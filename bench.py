@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a path
     python bench.py --impl reference --steps K --warmup W    # the reference's own CPU renderer on the host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write the last timed frame to DIR/*.npy
 
 A step = one full frame of BASELINE.json's headline config (helmet.glb, 1920x1080, 1024 spp, 8 bounces, synthetic
 environment) rendered by N GPUs, one process per GPU: every rank renders the share of the frame the library's policy
@@ -26,6 +27,7 @@ import ctypes as C
 import json
 import os
 import sys
+import tempfile
 import threading
 import time
 
@@ -55,6 +57,7 @@ FLOP_NODE, FLOP_LEAF, FLOP_ACCEPT, FLOP_SHADE, FLOP_ENV, FLOP_RAYGEN = 200.0, 45
 # cache-level bytes per unit of work (same section): 192 B per node, 288 B per leaf, 112 B per
 # accepted record, 4 taps x 4 textures x 4 B + 80 B material per shade
 BYTES_NODE, BYTES_LEAF, BYTES_ACCEPT, BYTES_SHADE = 192.0, 288.0, 112.0, 144.0
+DUMP_BYTES = 64 * 10 ** 6          # --dump-outputs writes at most this much
 
 
 def algorithmic_flops(c: dict) -> float:
@@ -142,8 +145,8 @@ def load_workload(args, **procs):
 
 class CpuRenderer:
     """The CPU arm: the reference's OWN raytracer.c / driver.c (oracle/_ref/libref.so — its sources compiled
-    unmodified where they lie, over the stand-in for its un-vendored stdlib; built by oracle/Makefile where
-    /root/reference exists and shipped with the repo snapshot) when that file is present, `kind: "reference"`;
+    unmodified where they lie, over the stand-in for its un-vendored stdlib; built by oracle/Makefile from
+    the reference checkout RT_REFERENCE_DIR names) when that file is present, `kind: "reference"`;
     otherwise the oracle port, `kind: "port"`.  Either way N host threads enter render_thread_proc with one
     context and pull 32x32 chunks from its atomic counter, exactly as the reference's driver starts them
     (driver.c:793-803)."""
@@ -304,6 +307,24 @@ def film_kernel_rates(gpu, gpu_check, torch, W, H, SPP, sptr, peak_gbs):
         out[name] = {"ms": round(ms, 4), "algorithmic_bytes": nbytes, "GB/s": round(gbs, 1),
                      "frac_of_hbm_peak": round(gbs / peak_gbs, 4), "note": "back-to-back launches: the 25 MB working set stays in the 126 MB L2"}
     return out
+
+
+def dump_outputs(out_dir: str, frames: dict, seed: int = 2026) -> None:
+    """Writes every (H, W, 3) array of `frames` as out_dir/<name>.npy in float32: whole when they fit in DUMP_BYTES
+    together, else the same seeded sample of pixels from each, (n, 3), with their row-major indices in
+    pixel_index.npy (float64, exact).  Two builds given the same arguments can then be compared file by file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in frames.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        h, w = next(iter(arrays.values())).shape[:2]
+        n = (DUMP_BYTES - 4096) // (total // (h * w) + 8)
+        idx = np.sort(np.random.default_rng(seed).choice(h * w, size=n, replace=False))
+        arrays = {k: a.reshape(h * w, -1)[idx] for k, a in arrays.items()}
+        arrays["pixel_index"] = idx.astype(np.float64)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def measured_peaks() -> dict:
@@ -517,6 +538,9 @@ def run_gpu(args) -> None:
     # the combined accumulator and image of the last timed step, for the parity check below
     accum_host = total.cpu().numpy() if rank == 0 else None
     pixels_host = pixels.cpu().numpy() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        # what the caller of the timed path receives: the summed radiance (accum / spp = mean) and the u8 sRGB film
+        dump_outputs(args.dump_outputs, {"accum": accum_host.reshape(H, W, 3), "pixels": pixels_host.reshape(H, W, 3)})
 
     # ---- e2e: through render_thread_proc with HOST buffers (N=1), or its device-level pieces + the cross-GPU film (N>1);
     # every step re-uploads the scene (H2D) and reads the image back (D2H)
@@ -579,9 +603,10 @@ def run_gpu(args) -> None:
         cpu, cpu_spp, cpu_dt = (None, None, None)
         if world == 1 and not args.no_cpu:
             cpu, cpu_spp, cpu_dt = cpu_reference_rate(args)
-        t0 = time.perf_counter()
-        driver.save_image("/tmp/bench_helmet.png", host_pixels if world == 1 else pinned.numpy().reshape(H, W, 3))
-        t_save = time.perf_counter() - t0
+        with tempfile.TemporaryDirectory() as tmp:
+            t0 = time.perf_counter()
+            driver.save_image(os.path.join(tmp, "frame.png"), host_pixels if world == 1 else pinned.numpy().reshape(H, W, 3))
+            t_save = time.perf_counter() - t0
         mode_name = {SPLIT_SAMPLES: "sample-range", SPLIT_CHUNKS: "32x32-chunk round-robin"}[mode_used.value]
         film = {"p2p": "rank 0's fused reduce+resolve kernel reads the peers' accumulators over NVLink (CUDA IPC), two 4-byte NCCL all-reduces as fences",
                 "nccl": "NCCL reduce(sum) of the f32 accumulators to rank 0, then the resolve kernel"}.get(reduce_how, reduce_how)
@@ -633,7 +658,14 @@ def main() -> None:
     ap.add_argument("--fast", action="store_true",
                     help="opt-in fast mode (RT_GPU_Options.fast_math): FMA-contracted bounce stages with hardware transcendentals; "
                          "NOT the headline — the default is the bit-exact path")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="GPU path (--impl ours) only: write the accumulator and the u8 film of the last timed step to "
+                         "DIR/accum.npy, DIR/pixels.npy (float32; a seeded pixel sample when they exceed 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's frame: not available with --impl reference")
     for key in ("width", "height", "spp"):
         if getattr(args, key) is None:
             setattr(args, key, WORKLOADS[args.workload][key])

@@ -3,7 +3,7 @@
  * raytracer.c:3-7, scene.c:1-6, driver.c:1-8) but which is not vendored.
  *
  * Purpose: let the UNMODIFIED reference sources compile, from where they lie
- * under /root/reference, into oracle/_ref/libref.so (recipe: oracle/Makefile,
+ * in a reference checkout (RT_REFERENCE_DIR), into oracle/_ref/libref.so (recipe: oracle/Makefile,
  * target `ref`), so the oracle's restatement can be checked against the
  * reference's own code.  Only what those sources use is provided; every other
  * codin/X.h in this directory just includes this file.

@@ -8,7 +8,7 @@
  * (SURVEY.md §4) and cannot be built as shipped (its stdlib "Codin" is not
  * vendored).  This oracle is pinned against the reference's own raytracer.c /
  * scene.c / denoiser.c / driver.c compiled unmodified, from where they lie
- * under /root/reference, over a Codin shim (oracle/codin_shim, recipe
+ * in a reference checkout (RT_REFERENCE_DIR), over a Codin shim (oracle/codin_shim, recipe
  * oracle/Makefile target `ref`, output oracle/_ref/libref.so) — see
  * tests/test_oracle_vs_ref.py and the committed fixtures under tests/golden/.
  * The shim itself carries the UNPINNED Codin choices listed in DESIGN.md.

@@ -4,6 +4,7 @@
 #include "oracle.h"
 #include "oracle_vec.h"
 #include "rt_seed.h"
+#include <immintrin.h>
 
 f32 oracle_powf(f32 x, f32 y)    { return rt_powf(x, y); }
 f32 oracle_sinf(f32 x)           { return rt_sinf(x); }
@@ -21,6 +22,17 @@ void oracle_sincos_array(f32 const *x, f32 *s, f32 *c, isize n) { for (isize i =
 void oracle_sincos_fused_array(f32 const *x, f32 *s, f32 *c, isize n) { for (isize i = 0; i < n; i++) rt_sincosf(x[i], &s[i], &c[i]); }
 void oracle_atan2_array(f32 const *y, f32 const *x, f32 *out, isize n) { for (isize i = 0; i < n; i++) out[i] = rt_atan2f(y[i], x[i]); }
 void oracle_asin_array(f32 const *x, f32 *out, isize n) { for (isize i = 0; i < n; i++) out[i] = rt_asinf(x[i]); }
+
+/* _mm256_rsqrt_ps, which raytracer.c:663 uses for primary rays: its bits are the CPU's choice, not IEEE's, so a
+ * reference-seed-mode image recorded on one CPU holds on another only where this array comes out the same. */
+void oracle_rsqrt_ps_array(f32 const *x, f32 *out, isize n) {
+  for (isize i = 0; i < n; i += 8) {
+    f32 in[8] = {1, 1, 1, 1, 1, 1, 1, 1}, res[8];
+    for (isize k = 0; k < 8 && i + k < n; k++) in[k] = x[i + k];
+    _mm256_storeu_ps(res, _mm256_rsqrt_ps(_mm256_loadu_ps(in)));
+    for (isize k = 0; k < 8 && i + k < n; k++) out[i + k] = res[k];
+  }
+}
 
 /* Primary ray of sample s at pixel (x, y): raytracer.c:644-677 with the exact
  * 1/sqrt (the form the parity mode uses on both sides). */

@@ -123,6 +123,14 @@ def denoise(src: np.ndarray, n_threads: int = 1) -> np.ndarray:
     return dst
 
 
+def rsqrt_ps(x: np.ndarray) -> np.ndarray:
+    """_mm256_rsqrt_ps of every element on this CPU (the approximation of reference seed mode's primary rays)."""
+    x = np.ascontiguousarray(x, dtype=np.float32)
+    out = np.empty_like(x)
+    lib().oracle_rsqrt_ps_array(x.ctypes.data, out.ctypes.data, C.c_ssize_t(x.size))
+    return out
+
+
 def resolve(accum: np.ndarray, samples: int) -> np.ndarray:
     accum = np.ascontiguousarray(accum, dtype=np.float32)
     out = np.zeros(accum.shape, dtype=np.uint8)

@@ -1,8 +1,8 @@
 """ctypes bindings of oracle/_ref/libref.so — the reference's OWN raytracer.c / scene.c / denoiser.c /
 driver.c compiled unmodified over the Codin stand-in (oracle/codin_shim).  TEST INFRASTRUCTURE ONLY.
 
-The library can only be (re)built where /root/reference exists; the built file travels with the
-repo snapshot.  available() says whether the tests that need it can run.
+The library can only be (re)built from a checkout of the reference named by RT_REFERENCE_DIR.
+available() says whether the tests that need it can run.
 """
 from __future__ import annotations
 
@@ -26,7 +26,7 @@ class RefHit(C.Structure):
 def available() -> bool:
     if os.path.exists(REF_LIB):
         return True
-    if os.path.isdir("/root/reference"):
+    if os.path.isdir(os.environ.get("RT_REFERENCE_DIR", "")):
         return subprocess.run(["make", "-C", ORACLE_DIR, "ref"], capture_output=True).returncode == 0
     return False
 
@@ -37,7 +37,7 @@ _lib = None
 def lib() -> C.CDLL:
     global _lib
     if _lib is None:
-        assert available(), "oracle/_ref/libref.so is missing and /root/reference is not mounted"
+        assert available(), "oracle/_ref/libref.so is missing and RT_REFERENCE_DIR names no reference checkout"
         r = C.CDLL(REF_LIB)
         r.ref_scene_init.argtypes = [C.POINTER(Scene), TriangleSlice]
         r.render_thread_proc.argtypes = [C.POINTER(RenderingContext)]

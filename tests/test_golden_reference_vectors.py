@@ -2,7 +2,7 @@
 
 tests/golden/reference_vectors.npz was generated (tools/make_golden.py) by oracle/_ref/libref.so —
 raytracer.c, scene.c, denoiser.c and driver.c compiled unmodified over the Codin stand-in.  These
-tests need neither /root/reference nor a GPU; they are what pins the oracle on every machine.
+tests need neither the reference checkout nor a GPU; they are what pins the oracle on every machine.
 """
 import ctypes as C
 

@@ -1,6 +1,6 @@
 """Generate tests/golden/reference_vectors.npz from the reference's OWN code.
 
-Runs only in the build container (needs /root/reference): builds oracle/_ref/libref.so — the
+Needs a reference checkout named by RT_REFERENCE_DIR: builds oracle/_ref/libref.so — the
 reference's raytracer.c / scene.c / denoiser.c / driver.c compiled unmodified over the Codin
 stand-in — and records small input/output vectors of the hot path:
 
@@ -14,6 +14,10 @@ stand-in — and records small input/output vectors of the hot path:
   background_dir / _out       sample_background (driver.c:95)
   lightmap/<case>             lightmap_bake (raytracer.c:722), u8 image, both generator copies started from the
                               recorded states (the sequential "reference" seed mode)
+  reference_mode/<case>       render_thread_proc as shipped (one thread, one RNG stream from 0, _mm256_rsqrt_ps primary
+                              rays), u8 image; rsqrt_in / rsqrt_out fingerprint the recording CPU's _mm256_rsqrt_ps
+  per_sample/<case>           cast_ray per (pixel, sample) with a non-zero user seed; denoise_frame_in / _out:
+                              denoise_image on the oracle's u8 frame of the same render
 
 quad.obj and fov_test.obj are absent from bvh_sha256: the reference's builder has undefined
 behaviour on them (SURVEY.md §2.3 Q1/Q2).
@@ -32,6 +36,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import oracle_ffi  # noqa: E402
 import ref_ffi  # noqa: E402
+from helpers import CAMERAS  # noqa: E402
 from raytracing_c_b200 import driver  # noqa: E402
 from raytracing_c_b200._ffi import Vec2, Vec3  # noqa: E402
 
@@ -53,6 +58,20 @@ LIGHTMAP_CASES = {
     "tower_64x48x3": ("tower.obj", 64, 48, 3, (30.0, 20.0, 10.0), 123, 7),
     "spheres_48x48x2": ("spheres.glb", 48, 48, 2, (30.0, 20.0, 10.0), 99, 5),
 }
+
+
+# tests/test_oracle_vs_ref.py reads these under the same keys: (model, width, height, spp, material override)
+REFERENCE_MODE_CASES = [("spheres.glb", 96, 64, 4, {}), ("helmet.glb", 64, 48, 3, {}),
+                        ("sheen.glb", 48, 48, 4, {"sheen": 1.0, "sheen_tint": 1.0}), ("tower.obj", 48, 32, 2, {})]
+SEEDED_CASE = ("spheres.glb", 20, 12, 3, 99)         # model, width, height, spp, user seed
+
+
+def reference_mode_key(model, w, h, spp):
+    return f"reference_mode/{model}_{w}x{h}x{spp}"
+
+
+def seeded_key(model, w, h, spp, seed):
+    return f"per_sample/{model}_{w}x{h}x{spp}_seed{seed}"
 
 
 def scene_digest(scene) -> str:
@@ -119,8 +138,25 @@ def main():
     arrays["background_out"] = np.array([(c.x, c.y, c.z) for c in (r.ref_sample_background(C.byref(loaded.background), Vec3(*p)) for p in d)], dtype=np.float32)
     loaded.close()
 
+    for model, w, h, spp, override in REFERENCE_MODE_CASES:
+        loaded = load_ref(model, override, CAMERAS.get(model))
+        arrays[reference_mode_key(model, w, h, spp)] = ref_ffi.render_reference_mode(loaded, w, h, spp)
+        loaded.close()
+    rng = np.random.default_rng(663)
+    x = np.concatenate([np.geomspace(1e-4, 1e4, 2048), rng.uniform(0.0, 8.0, 2048)]).astype(np.float32)
+    arrays["rsqrt_in"], arrays["rsqrt_out"] = x, oracle_ffi.rsqrt_ps(x)
+    model, w, h, spp, seed = SEEDED_CASE
+    loaded = load_ref(model)
+    arrays[seeded_key(*SEEDED_CASE)] = ref_ffi.cast_rays_per_sample(loaded, w, h, spp, user_seed=seed)
+    loaded.close()
+    loaded = driver.load_scene(os.path.join(MODELS, model), shader_proc=oracle_ffi.shader_proc(),
+                               background_proc=oracle_ffi.background_proc())
+    frame = oracle_ffi.render(loaded, w, h, spp, 8, n_threads=2, user_seed=seed)["pixels"]
+    loaded.close()
+    arrays["denoise_frame_in"], arrays["denoise_frame_out"] = frame, ref_ffi.denoise(frame)
+
     np.savez_compressed(os.path.join(OUT, "reference_vectors.npz"), **arrays)
-    meta = {"generator": "tools/make_golden.py", "source": "oracle/_ref/libref.so = /root/reference/{raytracer,scene,denoiser,driver}.c unmodified + oracle/codin_shim",
+    meta = {"generator": "tools/make_golden.py", "source": "oracle/_ref/libref.so = $RT_REFERENCE_DIR/{raytracer,scene,denoiser,driver}.c unmodified + oracle/codin_shim",
             "bvh": digests, "radiance_cases": {k: dict(model=v[0], width=v[1], height=v[2], spp=v[3], bounces=v[4], override=v[5], camera=v[6]) for k, v in RADIANCE_CASES.items()},
             "lightmap_cases": {k: dict(model=v[0], width=v[1], height=v[2], samples=v[3], emission=list(v[4]), dir_state=v[5], shader_state=v[6])
                                for k, v in LIGHTMAP_CASES.items()}}
