@@ -167,6 +167,42 @@ int rt_gpu_resolve_device(f32 const *d_accum, isize width, isize height, isize s
 int rt_gpu_denoise_device(u8 const *d_src, u8 *d_dst, isize width, isize height,
                           isize src_stride, isize dst_stride, i32 components, void *stream);
 
+/* ---- ray queries on a resident scene (csrc/rt_query.cu) ----
+ * A query is the reference's ray_scene_hit (raytracer.c:443-503) with hit.distance set to t_max before the walk:
+ *   - a ray is the reference's Ray (24 B, f32 alignment).  Directions are not normalised; t is in units of
+ *     |direction|, as in the reference;
+ *   - a triangle counts when it passes the Moller-Trumbore test of raytracer.c:115-159 with EPSILON <= t < t_max
+ *     (strict).  t_max is per ray; a NULL t_max array means +inf for every ray.  A t_max that is NaN, negative or
+ *     <= EPSILON gives a miss: that is what the reference's compares give, with no special case;
+ *   - the walk visits nodes in the reference's order with its compares and tie rules, so the closest hit (ties
+ *     included) is the reference's triangle slot.
+ * Closest hit: t, the barycentrics u, v of the hit and the padded triangle slot (the numbering of rt_gpu_read_hit_ids:
+ * scene->triangles.aos[slot] is the triangle).  A miss is t = +inf, u = v = 0, slot = -1.  The optional surface
+ * record is raytracer.c:164-182 in the f32 expressions the renderer uses: point = o + d * t, the interpolated
+ * shading normal (not normalised, as in the reference), the geometric normal and the interpolated texture
+ * coordinates; all zero for a miss.
+ * Occlusion: one byte per ray, 1 = some triangle counts.  It is the same ordered walk, stopped at the first leaf
+ * that accepts a triangle.  Until that acceptance hit.distance is still t_max, so the occlusion walk is a prefix of
+ * the closest-hit walk with the same t_max: occluded[i] == (closest hit of ray i has slot >= 0) exactly, and its
+ * node, leaf and accept counts never exceed those of the closest-hit query.
+ * Queries are always exact: RT_GPU_Options.fast_math does not apply to them.
+ * They run on the first device, do not wait for the scene's textures (only for its geometry), and do not serialise
+ * against renders; two queries on one device are serialised by the library (they share a work counter). */
+typedef struct { f32 t, u, v; i32 slot; } RT_GPU_Hit;                                   /* 16 B */
+typedef struct { Vec3 point, normal, normal_geo; Vec2 tex_coords; } RT_GPU_Surface;     /* 44 B */
+/* device pointers, stream-ordered (stream: cudaStream_t as void*, NULL = the legacy default stream).  d_hits must be
+ * 16-byte aligned; d_t_max, d_surface and d_counters are optional.  d_counters: four u64, atomically added, as
+ * RT_GPU_CTR_RAYS / NODES / LEAVES / ACCEPTS.  n_rays in [0, INT32_MAX]; 0 is a no-op. */
+int rt_gpu_closest_hit_device(Scene const *scene, Ray const *d_rays, f32 const *d_t_max, isize n_rays,
+                              RT_GPU_Hit *d_hits, RT_GPU_Surface *d_surface, u64 *d_counters, void *stream);
+int rt_gpu_occluded_device(Scene const *scene, Ray const *d_rays, f32 const *d_t_max, isize n_rays,
+                           u8 *d_occluded, u64 *d_counters, void *stream);
+/* host memory: staged through library-owned device buffers, queried, copied back; returns when the results are in
+ * place.  t_max and surface are optional. */
+int rt_gpu_closest_hit(Scene const *scene, Ray const *rays, f32 const *t_max, isize n_rays,
+                       RT_GPU_Hit *hits, RT_GPU_Surface *surface);
+int rt_gpu_occluded(Scene const *scene, Ray const *rays, f32 const *t_max, isize n_rays, u8 *occluded);
+
 #ifdef __cplusplus
 }
 #endif

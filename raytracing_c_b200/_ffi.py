@@ -97,6 +97,18 @@ class GPUOptions(C.Structure):
                 ("pixel_world", C.c_int32), ("fast_math", C.c_int32)]
 
 
+class Ray(C.Structure):
+    _fields_ = [("position", Vec3), ("direction", Vec3)]
+
+
+class GPUHit(C.Structure):
+    _fields_ = [("t", C.c_float), ("u", C.c_float), ("v", C.c_float), ("slot", C.c_int32)]
+
+
+class GPUSurface(C.Structure):
+    _fields_ = [("point", Vec3), ("normal", Vec3), ("normal_geo", Vec3), ("tex_coords", Vec2)]
+
+
 SPLIT_AUTO, SPLIT_SAMPLES, SPLIT_CHUNKS = 0, 1, 2
 REDUCE_P2P, REDUCE_NCCL = 0, 1
 
@@ -122,6 +134,7 @@ GPU_EXPORTS = [
     "rt_gpu_read_counters_ex", "rt_gpu_last_launches",
     "rt_gpu_last_kernel_ms", "rt_gpu_stage_profile_enable", "rt_gpu_stage_profile_read", "rt_gpu_stage_profile_read_bounces",
     "rt_gpu_render_accum_device", "rt_gpu_resolve_device", "rt_gpu_denoise_device",
+    "rt_gpu_closest_hit_device", "rt_gpu_occluded_device", "rt_gpu_closest_hit", "rt_gpu_occluded",
 ]
 
 HOST_EXPORTS = [
@@ -243,6 +256,12 @@ def gpu_lib() -> C.CDLL:
                                                    C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.rt_gpu_resolve_device.argtypes = [C.c_void_p, isize, isize, isize, C.c_void_p, isize, C.c_int32, C.c_void_p]
         lib.rt_gpu_denoise_device.argtypes = [C.c_void_p, C.c_void_p, isize, isize, isize, isize, C.c_int32, C.c_void_p]
+        lib.rt_gpu_closest_hit_device.argtypes = [C.POINTER(Scene), C.c_void_p, C.c_void_p, isize, C.c_void_p, C.c_void_p,
+                                                  C.c_void_p, C.c_void_p]
+        lib.rt_gpu_occluded_device.argtypes = [C.POINTER(Scene), C.c_void_p, C.c_void_p, isize, C.c_void_p, C.c_void_p,
+                                               C.c_void_p]
+        lib.rt_gpu_closest_hit.argtypes = [C.POINTER(Scene), C.c_void_p, C.c_void_p, isize, C.c_void_p, C.c_void_p]
+        lib.rt_gpu_occluded.argtypes = [C.POINTER(Scene), C.c_void_p, C.c_void_p, isize, C.c_void_p]
         lib.render_thread_proc.argtypes = [C.POINTER(RenderingContext)]
         lib.render_thread_proc.restype = None
         lib.rendering_context_is_finished.argtypes = [C.POINTER(RenderingContext)]

@@ -433,6 +433,126 @@ int rt_gpu_denoise_device(u8 const *d_src, u8 *d_dst, isize width, isize height,
   return 0;
 }
 
+// ------------------------------------------------------------------ ray queries
+}  // extern "C"
+
+namespace {
+
+int query_validate(const char *what, const Scene *scene, const void *rays, isize n_rays, const void *out, const void *hits) {
+  if (n_rays < 0 || n_rays > INT32_MAX) return fail("%s: n_rays = %lld, must be in [0, INT32_MAX]", what, (long long)n_rays);
+  if (n_rays == 0) return 0;
+  if (!scene) return fail("%s: null scene", what);
+  if (!rays) return fail("%s: null rays", what);
+  if (!out) return fail("%s: null output", what);
+  if (reinterpret_cast<uintptr_t>(hits) & 15) return fail("%s: hits must be 16-byte aligned", what);
+  return 0;
+}
+
+// One query launch on the first device, ordered on `stream`.  It reads the scene's geometry only, so it waits for
+// geom_ready and not for the texels; it touches neither the render workspace nor the camera-relative copies, so it
+// does not wait for renders.  Queries of one device share its work counter: each waits for the previous one.
+int query_on_device(const Scene *scene, const Ray *rays, const f32 *t_max, isize n_rays, bool any, RT_GPU_Hit *hits,
+                    RT_GPU_Surface *surface, u8 *occluded, u64 *counters, cudaStream_t stream) {
+  Device &d = g.devs[0];
+  CUDA_TRY(cudaSetDevice(d.id));
+  const DeviceScene &ds = d.scenes.find(scene)->second;
+  if (!d.d_query_fetch) CUDA_TRY(cudaMalloc(reinterpret_cast<void **>(&d.d_query_fetch), sizeof(unsigned)));
+  if (!d.query_busy) CUDA_TRY(cudaEventCreateWithFlags(&d.query_busy, cudaEventDisableTiming));
+  CUDA_TRY(cudaStreamWaitEvent(stream, ds.geom_ready, 0));
+  if (d.query_busy_valid) CUDA_TRY(cudaStreamWaitEvent(stream, d.query_busy, 0));
+  CUDA_TRY(cudaMemsetAsync(d.d_query_fetch, 0, sizeof(unsigned), stream));
+  QueryParams p{};
+  p.scene = ds.dev;
+  p.rays = reinterpret_cast<const float *>(rays);
+  p.t_max = t_max;
+  p.n_rays = (unsigned)n_rays;
+  p.hits = reinterpret_cast<float4 *>(hits);
+  p.surface = reinterpret_cast<float *>(surface);
+  p.occluded = occluded;
+  p.fetch = d.d_query_fetch;
+  p.counters = reinterpret_cast<unsigned long long *>(counters);
+  int e = rt_launch_query(p, any, d.sm_count, stream);
+  if (e) return fail("query kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
+  g.last_launches++;
+  CUDA_TRY(cudaEventRecord(d.query_busy, stream));
+  d.query_busy_valid = true;
+  return 0;
+}
+
+int query_device_call(const char *what, const Scene *scene, const Ray *d_rays, const f32 *d_t_max, isize n_rays, bool any,
+                      RT_GPU_Hit *d_hits, RT_GPU_Surface *d_surface, u8 *d_occluded, u64 *d_counters, void *stream) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  if (query_validate(what, scene, d_rays, n_rays, any ? static_cast<const void *>(d_occluded) : d_hits, d_hits)) return 1;
+  if (n_rays == 0) return 0;
+  if (ensure_init()) return 1;
+  if (scene_on_devices(scene)) return 1;
+  return query_on_device(scene, d_rays, d_t_max, n_rays, any, d_hits, d_surface, d_occluded, d_counters,
+                         static_cast<cudaStream_t>(stream));
+}
+
+// Host memory: rays (and t_max) up through the first device's staging block, query, results back, synchronise.
+int query_host_call(const char *what, const Scene *scene, const Ray *rays, const f32 *t_max, isize n_rays, bool any,
+                    RT_GPU_Hit *hits, RT_GPU_Surface *surface, u8 *occluded) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  g.last_launches = 0;
+  // host arrays need no alignment: the device copy of hits is the staging block's first part
+  if (query_validate(what, scene, rays, n_rays, any ? static_cast<const void *>(occluded) : hits, nullptr)) return 1;
+  if (n_rays == 0) return 0;
+  if (ensure_init()) return 1;
+  if (scene_on_devices(scene)) return 1;
+  Device &d = g.devs[0];
+  CUDA_TRY(cudaSetDevice(d.id));
+  // staging layout, every part 16-byte aligned: hits | surface | rays | t_max | occluded
+  const size_t n = (size_t)n_rays;
+  auto up16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
+  const size_t o_surface = up16(any ? 0 : n * sizeof(RT_GPU_Hit));
+  const size_t o_rays = o_surface + up16(surface && !any ? n * sizeof(RT_GPU_Surface) : 0);
+  const size_t o_t_max = o_rays + up16(n * sizeof(Ray));
+  const size_t o_occluded = o_t_max + up16(t_max ? n * sizeof(f32) : 0);
+  const size_t total = o_occluded + up16(any ? n : 0);
+  if (grow(&d.d_query_stage, &d.query_stage_bytes, total)) return 1;
+  char *base = static_cast<char *>(d.d_query_stage);
+  RT_GPU_Hit *d_hits = any ? nullptr : reinterpret_cast<RT_GPU_Hit *>(base);
+  RT_GPU_Surface *d_surface = surface && !any ? reinterpret_cast<RT_GPU_Surface *>(base + o_surface) : nullptr;
+  Ray *d_rays = reinterpret_cast<Ray *>(base + o_rays);
+  f32 *d_t_max = t_max ? reinterpret_cast<f32 *>(base + o_t_max) : nullptr;
+  u8 *d_occluded = any ? reinterpret_cast<u8 *>(base + o_occluded) : nullptr;
+  CUDA_TRY(cudaMemcpyAsync(d_rays, rays, n * sizeof(Ray), cudaMemcpyHostToDevice, d.stream));
+  if (t_max) CUDA_TRY(cudaMemcpyAsync(d_t_max, t_max, n * sizeof(f32), cudaMemcpyHostToDevice, d.stream));
+  if (query_on_device(scene, d_rays, d_t_max, n_rays, any, d_hits, d_surface, d_occluded, nullptr, d.stream)) return 1;
+  if (any) {
+    CUDA_TRY(cudaMemcpyAsync(occluded, d_occluded, n, cudaMemcpyDeviceToHost, d.stream));
+  } else {
+    CUDA_TRY(cudaMemcpyAsync(hits, d_hits, n * sizeof(RT_GPU_Hit), cudaMemcpyDeviceToHost, d.stream));
+    if (surface) CUDA_TRY(cudaMemcpyAsync(surface, d_surface, n * sizeof(RT_GPU_Surface), cudaMemcpyDeviceToHost, d.stream));
+  }
+  CUDA_TRY(cudaStreamSynchronize(d.stream));
+  return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int rt_gpu_closest_hit_device(Scene const *scene, Ray const *d_rays, f32 const *d_t_max, isize n_rays, RT_GPU_Hit *d_hits,
+                              RT_GPU_Surface *d_surface, u64 *d_counters, void *stream) {
+  return query_device_call("closest_hit", scene, d_rays, d_t_max, n_rays, false, d_hits, d_surface, nullptr, d_counters, stream);
+}
+
+int rt_gpu_occluded_device(Scene const *scene, Ray const *d_rays, f32 const *d_t_max, isize n_rays, u8 *d_occluded,
+                           u64 *d_counters, void *stream) {
+  return query_device_call("occluded", scene, d_rays, d_t_max, n_rays, true, nullptr, nullptr, d_occluded, d_counters, stream);
+}
+
+int rt_gpu_closest_hit(Scene const *scene, Ray const *rays, f32 const *t_max, isize n_rays, RT_GPU_Hit *hits,
+                       RT_GPU_Surface *surface) {
+  return query_host_call("closest_hit", scene, rays, t_max, n_rays, false, hits, surface, nullptr);
+}
+
+int rt_gpu_occluded(Scene const *scene, Ray const *rays, f32 const *t_max, isize n_rays, u8 *occluded) {
+  return query_host_call("occluded", scene, rays, t_max, n_rays, true, nullptr, nullptr, occluded);
+}
+
 // ----------------------------------------------------------------- parity hooks
 int rt_gpu_read_accum(f32 *out, isize n_floats) {
   std::lock_guard<std::mutex> lock(g_mutex);

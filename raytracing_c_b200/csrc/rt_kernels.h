@@ -34,6 +34,20 @@ int rt_launch_texel_expand(const uchar4 *src, size_t n, float4 *dst, cudaStream_
 // tri_pos / tri_rec from the host's vertex arrays, Triangle_AOS records and per-slot material indices (rt_denoise.cu)
 int rt_launch_scene_pack(const float *soa, const float4 *aos, const int *mat_index, int n_slots, float4 *tri_pos, float4 *tri_rec,
                          cudaStream_t stream);
+// ray queries (rt_query.cu): closest hit (any = false: hits, optional surface) or occlusion (any = true: occluded)
+// of n_rays rays at their own index; `fetch` is a zeroed work counter no other launch uses at the same time
+struct QueryParams {
+  SceneDev  scene;
+  const float *rays;                     // [n_rays][6]: the reference's Ray (position, direction)
+  const float *t_max;                    // optional [n_rays], NULL = +inf
+  unsigned  n_rays;
+  float4   *hits;                        // [n_rays] (t, u, v, slot bits)
+  float    *surface;                     // optional [n_rays][11]: point, normal, normal_geo, tex_coords
+  unsigned char *occluded;               // [n_rays]
+  unsigned *fetch;
+  unsigned long long *counters;          // optional 4: rays, nodes, leaves, accepts
+};
+int rt_launch_query(const QueryParams &p, bool any, int sm_count, cudaStream_t stream);
 // per-stage CUDA-event timing of rt_launch_render's kernels (off by default)
 // slot = stage * RT_STAGE_BOUNCES + min(bounce, RT_STAGE_BOUNCES - 1)
 enum { RT_STAGE_TRACE = 0, RT_STAGE_MISS, RT_STAGE_SHADE, RT_STAGE_ACCUMULATE, RT_N_STAGES, RT_STAGE_BOUNCES = 16 };

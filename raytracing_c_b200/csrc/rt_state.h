@@ -75,6 +75,12 @@ struct Device {
   size_t workspace_denied = 0;                    // a request at least this large failed before: do not retry it
   unsigned char *d_image = nullptr, *d_image2 = nullptr; size_t image_bytes = 0, image2_bytes = 0;
   unsigned char *h_pinned = nullptr; size_t pinned_bytes = 0;
+  // ray queries (rt_gpu_closest_hit* / rt_gpu_occluded*): the kernel's work counter, the event that serialises queries
+  // on this device (they share the counter), staging for the host-memory calls
+  unsigned *d_query_fetch = nullptr;
+  cudaEvent_t query_busy = nullptr;
+  bool  query_busy_valid = false;
+  void *d_query_stage = nullptr; size_t query_stage_bytes = 0;
   bool l2_window_set = false;
   size_t l2_persist_max = 0, l2_window_max = 0;    // device limits (persistingL2CacheMaxSize, accessPolicyMaxWindowSize)
   cudaStream_t l2_stream = nullptr; const void *l2_base = nullptr;   // where the window was last set

@@ -217,6 +217,47 @@ def lightmap_bake(loaded: LoadedScene, width: int, height: int, samples: int, ou
     return dict(pixels=pixels, values=values, owner=owner)
 
 
+def _query_rays(origins, directions, t_max):
+    """(n, 6) float32 rays (the C Ray: position, direction) and the optional (n,) float32 t_max, both contiguous."""
+    o = np.asarray(origins, dtype=np.float32).reshape(-1, 3)
+    d = np.asarray(directions, dtype=np.float32).reshape(-1, 3)
+    if o.shape != d.shape:
+        raise ValueError(f"origins {o.shape} and directions {d.shape} differ")
+    rays = np.ascontiguousarray(np.concatenate([o, d], axis=1))
+    if t_max is not None:
+        t_max = np.ascontiguousarray(np.broadcast_to(np.asarray(t_max, dtype=np.float32), (len(rays),)))
+    return rays, t_max
+
+
+def closest_hit(loaded: LoadedScene, origins, directions, t_max=None, surface: bool = False) -> dict:
+    """Closest hit of each ray (rt_gpu_closest_hit; semantics in include/rt_gpu.h): the reference's ray_scene_hit with
+    hit.distance = t_max (None = +inf; a scalar applies to every ray).  Returns t, u, v (float32) and slot (int32,
+    -1 = miss); with surface, also point, normal (interpolated, not normalised), normal_geo (n, 3) and tex_coords (n, 2)."""
+    register_callbacks(loaded)
+    rays, t_max = _query_rays(origins, directions, t_max)
+    n = len(rays)
+    hits = np.zeros(n, dtype=[("t", np.float32), ("u", np.float32), ("v", np.float32), ("slot", np.int32)])
+    surf = np.zeros((n, 11), dtype=np.float32) if surface else None
+    gpu_check(gpu_lib().rt_gpu_closest_hit(C.byref(loaded.scene), rays.ctypes.data,
+                                           t_max.ctypes.data if t_max is not None else None, n, hits.ctypes.data,
+                                           surf.ctypes.data if surf is not None else None))
+    out = {k: np.ascontiguousarray(hits[k]) for k in ("t", "u", "v", "slot")}
+    if surf is not None:
+        out.update(point=surf[:, 0:3], normal=surf[:, 3:6], normal_geo=surf[:, 6:9], tex_coords=surf[:, 9:11])
+    return out
+
+
+def occluded(loaded: LoadedScene, origins, directions, t_max=None) -> np.ndarray:
+    """Whether any triangle lies along each ray before t_max (rt_gpu_occluded): exactly closest_hit(...)["slot"] >= 0
+    for the same rays and t_max, with a walk that stops at the first accepted triangle."""
+    register_callbacks(loaded)
+    rays, t_max = _query_rays(origins, directions, t_max)
+    out = np.zeros(len(rays), dtype=np.uint8)
+    gpu_check(gpu_lib().rt_gpu_occluded(C.byref(loaded.scene), rays.ctypes.data,
+                                        t_max.ctypes.data if t_max is not None else None, len(rays), out.ctypes.data))
+    return out.astype(bool)
+
+
 def read_accum(width: int, height: int) -> np.ndarray:
     out = np.empty((height, width, 3), dtype=np.float32)
     gpu_check(gpu_lib().rt_gpu_read_accum(out.ctypes.data, out.size))
