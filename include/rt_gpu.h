@@ -203,6 +203,41 @@ int rt_gpu_closest_hit(Scene const *scene, Ray const *rays, f32 const *t_max, is
                        RT_GPU_Hit *hits, RT_GPU_Surface *surface);
 int rt_gpu_occluded(Scene const *scene, Ray const *rays, f32 const *t_max, isize n_rays, u8 *occluded);
 
+/* ---- radiance for caller rays on a resident scene (csrc/rt_render.cu) ----
+ * The reference's cast_ray (raytracer.c:505-558) for a batch of n_rays rays, each traced for `samples` samples with
+ * sample indices sample_begin + s, s in [0, samples):
+ *   - a ray is the reference's Ray (24 B, f32 alignment), as for the queries.  Directions are used as given: the
+ *     renderer normalises its camera rays, cast_ray itself does not;
+ *   - path (i, s) is cast_ray(scene, ray_i, max_bounces) with the shader generator seeded to
+ *     rt_path_seed(key_i, sample_begin + s, user_seed) just before the call (rt_seed.h, the renderer's rule).  key_i is
+ *     keys[i], or i when keys is NULL.  Results therefore depend neither on the order of the batch nor on how it is
+ *     split into calls; a host that passes the renderer's camera ray of (pixel p, sample s) with key p gets the
+ *     renderer's radiance of that sample bit for bit;
+ *   - radiance[i] (3 f32) is the sum over the samples in sample order, before any division (the meaning of
+ *     rt_gpu_read_accum).  With accumulate != 0 the sums continue from what the buffer holds, so samples [0, k) then
+ *     [k, n) equal [0, n) bit for bit.  With samples == 0 nothing is traced: radiance is zeroed unless accumulate
+ *     is set, in which case it is left as it is (as rt_gpu_render_accum_device does with an empty range);
+ *   - per_sample (optional, [n_rays][samples][3] f32) receives each path's radiance, as the renderer's per-sample output;
+ *   - d_counters (optional, 8 u64, atomically added) as RT_GPU_CTR_*; SAMPLES grows by n_rays * samples;
+ *   - NaN radiance is summed as the renderer sums it (there is no film here, so the film's NaN -> 0 does not apply);
+ *   - max_bounces = 0 gives zero radiance for every path, as cast_ray does.
+ * Always exact: RT_GPU_Options.fast_math does not apply.  First device only.  The call shades, so it waits for the
+ * scene's texels as well as its geometry; it uses the device's path-queue workspace, so it is serialised with renders
+ * and lightmap bakes on that device (not with ray queries).  A batch larger than one workspace chunk is split over rays
+ * and samples inside the call.
+ * Refused before any launch: n_rays outside [0, INT32_MAX], samples < 0, sample_begin < 0,
+ * sample_begin + samples > INT32_MAX, max_bounces < 0, NULL rays or radiance with n_rays > 0, a scene that is not
+ * resident (rt_gpu_scene_upload).  n_rays = 0 is a no-op. */
+int rt_gpu_cast_rays_device(Scene const *scene, Ray const *d_rays, u32 const *d_keys, isize n_rays, isize sample_begin,
+                            isize samples, isize max_bounces, u32 user_seed, i32 accumulate,
+                            f32 *d_radiance,          /* n_rays*3 */
+                            f32 *d_per_sample,        /* optional n_rays*samples*3 */
+                            u64 *d_counters,          /* optional 8 */
+                            void *stream);
+/* host memory: staged through library-owned device buffers; returns when the results are in place */
+int rt_gpu_cast_rays(Scene const *scene, Ray const *rays, u32 const *keys, isize n_rays, isize sample_begin, isize samples,
+                     isize max_bounces, u32 user_seed, i32 accumulate, f32 *radiance, f32 *per_sample);
+
 #ifdef __cplusplus
 }
 #endif

@@ -135,6 +135,7 @@ GPU_EXPORTS = [
     "rt_gpu_last_kernel_ms", "rt_gpu_stage_profile_enable", "rt_gpu_stage_profile_read", "rt_gpu_stage_profile_read_bounces",
     "rt_gpu_render_accum_device", "rt_gpu_resolve_device", "rt_gpu_denoise_device",
     "rt_gpu_closest_hit_device", "rt_gpu_occluded_device", "rt_gpu_closest_hit", "rt_gpu_occluded",
+    "rt_gpu_cast_rays_device", "rt_gpu_cast_rays",
 ]
 
 HOST_EXPORTS = [
@@ -262,6 +263,10 @@ def gpu_lib() -> C.CDLL:
                                                C.c_void_p]
         lib.rt_gpu_closest_hit.argtypes = [C.POINTER(Scene), C.c_void_p, C.c_void_p, isize, C.c_void_p, C.c_void_p]
         lib.rt_gpu_occluded.argtypes = [C.POINTER(Scene), C.c_void_p, C.c_void_p, isize, C.c_void_p]
+        lib.rt_gpu_cast_rays_device.argtypes = [C.POINTER(Scene), C.c_void_p, C.c_void_p, isize, isize, isize, isize,
+                                                C.c_uint32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.rt_gpu_cast_rays.argtypes = [C.POINTER(Scene), C.c_void_p, C.c_void_p, isize, isize, isize, isize, C.c_uint32,
+                                         C.c_int32, C.c_void_p, C.c_void_p]
         lib.render_thread_proc.argtypes = [C.POINTER(RenderingContext)]
         lib.render_thread_proc.restype = None
         lib.rendering_context_is_finished.argtypes = [C.POINTER(RenderingContext)]

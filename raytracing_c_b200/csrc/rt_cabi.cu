@@ -553,6 +553,107 @@ int rt_gpu_occluded(Scene const *scene, Ray const *rays, f32 const *t_max, isize
   return query_host_call("occluded", scene, rays, t_max, n_rays, true, nullptr, nullptr, occluded);
 }
 
+// ------------------------------------------------------------- radiance for caller rays
+}  // extern "C"
+
+namespace {
+
+// Everything that is refused before a launch; afterwards the scene is resident (and current) on the first device.
+int cast_rays_validate(const char *what, const Scene *scene, const void *rays, isize n_rays, isize sample_begin,
+                       isize samples, isize max_bounces, const void *radiance) {
+  if (n_rays < 0 || n_rays > INT32_MAX) return fail("%s: n_rays = %lld, must be in [0, INT32_MAX]", what, (long long)n_rays);
+  if (samples < 0 || sample_begin < 0 || sample_begin > INT32_MAX - samples)
+    return fail("%s: samples [%lld, %lld + %lld) must lie in [0, INT32_MAX]", what, (long long)sample_begin,
+                (long long)sample_begin, (long long)samples);
+  if (max_bounces < 0 || max_bounces > INT32_MAX) return fail("%s: max_bounces = %lld, must be >= 0", what, (long long)max_bounces);
+  if (n_rays == 0) return 0;
+  if (!rays) return fail("%s: null rays", what);
+  if (!radiance) return fail("%s: null radiance", what);
+  if (!scene) return fail("%s: null scene", what);
+  if (ensure_init()) return 1;
+  if (g.devs[0].scenes.find(scene) == g.devs[0].scenes.end())
+    return fail("%s: scene is not resident (rt_gpu_scene_upload it first)", what);
+  return scene_on_devices(scene);
+}
+
+// One cast_rays call on the first device, ordered on `stream`.  It uses the device's path-queue workspace, so like a
+// render it waits for the previous user of the workspace (busy) and records busy after its last kernel; it shades, so
+// it waits for the scene's texels as well as its geometry.
+int cast_rays_on_device(const Scene *scene, const Ray *rays, const u32 *keys, isize n_rays, isize sample_begin, isize samples,
+                        isize max_bounces, u32 user_seed, int accumulate, float *radiance, float *per_sample,
+                        unsigned long long *counters, cudaStream_t stream) {
+  Device &d = g.devs[0];
+  CUDA_TRY(cudaSetDevice(d.id));
+  const DeviceScene &ds = d.scenes.find(scene)->second;
+  const size_t n_paths = (size_t)n_rays * (size_t)samples;
+  if (n_paths > 0 && ensure_workspace(d, rt_cast_rays_workspace_bytes(n_paths, (int)max_bounces, false),
+                                      rt_cast_rays_workspace_bytes(n_paths, (int)max_bounces, true), stream))
+    return 1;
+  if (d.busy_valid) CUDA_TRY(cudaStreamWaitEvent(stream, d.busy, 0));
+  CUDA_TRY(cudaStreamWaitEvent(stream, ds.geom_ready, 0));
+  CUDA_TRY(cudaStreamWaitEvent(stream, ds.tex_ready, 0));
+  set_l2_window(d, ds, stream);
+  int e = rt_launch_cast_rays(ds.dev, reinterpret_cast<const float *>(rays), keys, (int)n_rays, (int)sample_begin,
+                              (int)samples, (int)max_bounces, user_seed, accumulate, radiance, per_sample, counters,
+                              d.sm_count, d.d_workspace, d.workspace_bytes, stream, &g.last_launches);
+  if (e) return fail("cast_rays kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
+  CUDA_TRY(cudaEventRecord(d.busy, stream));
+  d.busy_valid = true;
+  return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int rt_gpu_cast_rays_device(Scene const *scene, Ray const *d_rays, u32 const *d_keys, isize n_rays, isize sample_begin,
+                            isize samples, isize max_bounces, u32 user_seed, i32 accumulate, f32 *d_radiance,
+                            f32 *d_per_sample, u64 *d_counters, void *stream) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  if (cast_rays_validate("cast_rays", scene, d_rays, n_rays, sample_begin, samples, max_bounces, d_radiance)) return 1;
+  if (n_rays == 0) return 0;
+  return cast_rays_on_device(scene, d_rays, d_keys, n_rays, sample_begin, samples, max_bounces, user_seed, accumulate,
+                             d_radiance, d_per_sample, reinterpret_cast<unsigned long long *>(d_counters),
+                             static_cast<cudaStream_t>(stream));
+}
+
+// Host memory: rays, keys (and the sums to continue from) up through the first device's staging block, cast, results
+// back, synchronise.
+int rt_gpu_cast_rays(Scene const *scene, Ray const *rays, u32 const *keys, isize n_rays, isize sample_begin, isize samples,
+                     isize max_bounces, u32 user_seed, i32 accumulate, f32 *radiance, f32 *per_sample) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  g.last_launches = 0;
+  if (cast_rays_validate("cast_rays", scene, rays, n_rays, sample_begin, samples, max_bounces, radiance)) return 1;
+  if (n_rays == 0) return 0;
+  Device &d = g.devs[0];
+  CUDA_TRY(cudaSetDevice(d.id));
+  // staging layout, every part 16-byte aligned: radiance | per_sample | rays | keys
+  const size_t n = (size_t)n_rays;
+  auto up16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
+  const size_t sums_bytes = n * 3 * sizeof(float);
+  const size_t per_sample_bytes = per_sample ? n * (size_t)samples * 3 * sizeof(float) : 0;
+  const size_t o_per_sample = up16(sums_bytes);
+  const size_t o_rays = o_per_sample + up16(per_sample_bytes);
+  const size_t o_keys = o_rays + up16(n * sizeof(Ray));
+  const size_t total = o_keys + up16(keys ? n * sizeof(u32) : 0);
+  if (grow(&d.d_cast_stage, &d.cast_stage_bytes, total)) return 1;
+  char *base = static_cast<char *>(d.d_cast_stage);
+  float *d_radiance = reinterpret_cast<float *>(base);
+  float *d_per_sample = per_sample ? reinterpret_cast<float *>(base + o_per_sample) : nullptr;
+  Ray *d_rays = reinterpret_cast<Ray *>(base + o_rays);
+  u32 *d_keys = keys ? reinterpret_cast<u32 *>(base + o_keys) : nullptr;
+  CUDA_TRY(cudaMemcpyAsync(d_rays, rays, n * sizeof(Ray), cudaMemcpyHostToDevice, d.stream));
+  if (keys) CUDA_TRY(cudaMemcpyAsync(d_keys, keys, n * sizeof(u32), cudaMemcpyHostToDevice, d.stream));
+  if (accumulate) CUDA_TRY(cudaMemcpyAsync(d_radiance, radiance, sums_bytes, cudaMemcpyHostToDevice, d.stream));
+  if (cast_rays_on_device(scene, d_rays, d_keys, n_rays, sample_begin, samples, max_bounces, user_seed, accumulate, d_radiance,
+                          d_per_sample, nullptr, d.stream))
+    return 1;
+  CUDA_TRY(cudaMemcpyAsync(radiance, d_radiance, sums_bytes, cudaMemcpyDeviceToHost, d.stream));
+  if (per_sample_bytes) CUDA_TRY(cudaMemcpyAsync(per_sample, d_per_sample, per_sample_bytes, cudaMemcpyDeviceToHost, d.stream));
+  CUDA_TRY(cudaStreamSynchronize(d.stream));
+  return 0;
+}
+
 // ----------------------------------------------------------------- parity hooks
 int rt_gpu_read_accum(f32 *out, isize n_floats) {
   std::lock_guard<std::mutex> lock(g_mutex);

@@ -18,6 +18,14 @@ int rt_launch_lightmap(const SceneDev &scene, int width, int height, int samples
                        unsigned char *d_pixels, int stride, int components, float *d_values, int *d_owner_out,
                        void *scratch, int sm_count, void *workspace, size_t workspace_bytes, cudaStream_t stream,
                        int *n_launches, unsigned *n_jobs_out);
+// cast_ray (raytracer.c:505-558) for caller rays on the wavefront, samples [sample_begin, sample_begin + samples) of each
+// ray summed into radiance (see rt_render.cu); `workspace` holds the path queues: rt_cast_rays_workspace_bytes for
+// n_rays * samples paths at the preferred chunk size, or with `floor` the smallest one the launch accepts
+size_t rt_cast_rays_workspace_bytes(size_t n_paths, int max_bounces, bool floor);
+int rt_launch_cast_rays(const SceneDev &scene, const float *rays, const unsigned *keys, int n_rays, int sample_begin,
+                        int samples, int max_bounces, uint32_t user_seed, int accumulate, float *radiance, float *per_sample,
+                        unsigned long long *counters, int sm_count, void *workspace, size_t workspace_bytes,
+                        cudaStream_t stream, int *n_launches);
 int rt_launch_resolve(const float *accum, int width, int height, int samples, unsigned char *pixels,
                       int stride, int components, cudaStream_t stream);
 // sum of parts.n accumulators (own + peer-mapped) in rank order, optional copy of the sum, optional resolve to u8

@@ -172,6 +172,7 @@ rt_reduce_resolve_kernel(const ReduceParts parts, float *__restrict__ sum_out, i
 // ------------------------------------------------------------------- launchers
 #define RT_PATH_BYTES ((2 + 3 + 1 + 2) * sizeof(float4))       // ray + hit + miss records and the tint / emission(=rad) state of one path
 #define RT_CHUNK_PATHS_MAX (512u << 20)
+#define RT_CAST_RAYS_MIN_CHUNK (1u << 16)                      // paths of the smallest workspace a cast_rays call accepts
 
 static size_t counts_bytes(int max_bounces) {
   size_t b = (size_t)(max_bounces + 1) * Q_STRIDE * sizeof(unsigned);
@@ -632,6 +633,152 @@ int rt_launch_lightmap(const SceneDev &scene, int width, int height, int samples
   }
   rt_lightmap_store_kernel<<<flat_grid, 256, 0, stream>>>(L, n_jobs, d_pixels, stride, components, d_values);
   launches++;
+  if (n_launches) *n_launches += launches;
+  return (int)cudaGetLastError();
+}
+
+// ===================================================================== cast_rays
+// Reference raytracer.c:505-558 for caller-supplied rays: path (ray i, sample s) is cast_ray(scene, ray_i, max_bounces)
+// with the shader generator seeded to rt_path_seed(key_i, s, user_seed) (rt_seed.h) just before the call.  The first ray
+// of a path is the caller's, as given (not normalised); the bounces run on the renderer's unchanged stage kernels, and
+// the per-ray sum is taken in sample order.  A chunk holds R rays x S samples, path id = ray_in_chunk * S + s: a warp is
+// consecutive samples of one ray, as in the renderer's layout.
+struct CastRaysParams {
+  const float    *rays;          // [n_rays][6]: the reference's Ray (position, direction)
+  const unsigned *keys;          // optional [n_rays]: seed key of each ray, NULL = its index
+  unsigned  ray0, n_rays;        // this chunk: rays [ray0, ray0 + n_rays)
+  float    *radiance;            // [n_rays total][3] running sums
+  float    *per_sample;          // optional [n_rays total][per_sample_stride][3], this chunk at +per_sample_offset
+  int       per_sample_stride, per_sample_offset;
+};
+
+// first ray of path (ray, sample): the caller's ray and the path's seed, appended to the RAY queue of bounce 0.  Without
+// bounces (max_bounces = 0) cast_ray returns its zero emission: the path ends here with radiance 0 and counts as a sample
+// (otherwise the miss or shade kernel that ends it counts it).
+__global__ void __launch_bounds__(256)
+rt_cast_rays_raygen_kernel(const __grid_constant__ StageParams P, const CastRaysParams C) {
+  const unsigned lane = threadIdx.x & 31u;
+  const unsigned S = (unsigned)P.n_samples, n = P.n_paths, n_round = (n + 31u) & ~31u;
+  unsigned c_samples = 0;
+  for (unsigned path = blockIdx.x * blockDim.x + threadIdx.x; path < n_round; path += gridDim.x * blockDim.x) {
+    bool shoot = false;
+    float4 a = make_float4(0, 0, 0, 0), b = make_float4(0, 0, 0, 0);
+    if (path < n) {
+      const unsigned r = path / S, ray = C.ray0 + r;
+      const int s = P.sample0 + (int)(path - r * S);
+      const float *src = C.rays + (size_t)ray * 6;
+      const uint32_t key = C.keys ? C.keys[ray] : ray;
+      const uint32_t rng = rt_path_seed(key, (uint32_t)s, P.user_seed);
+      shoot = P.max_bounces > 0;
+      a = make_float4(src[0], src[1], src[2], src[3]);
+      b = make_float4(src[4], src[5], __uint_as_float(path), __uint_as_float(rng));
+      if (!shoot) { P.q.rad[path] = make_float4(0, 0, 0, 0); c_samples++; }
+    }
+    const unsigned pos = warp_append(&P.q.counts[Q_RAYS], shoot, lane);
+    if (shoot) { P.q.ray_a[pos] = a; P.q.ray_b[pos] = b; }
+  }
+  if (P.counters) add_counter(P.counters, 7, c_samples);
+}
+
+// raytracer.c:696-700 per ray: radiance += cast_ray(...) in sample order, from zero on the first chunk of a call without
+// `accumulate`, else from the buffer
+__global__ void __launch_bounds__(256)
+rt_cast_rays_accumulate_kernel(const __grid_constant__ StageParams P, const CastRaysParams C) {
+  for (unsigned r = blockIdx.x * blockDim.x + threadIdx.x; r < C.n_rays; r += gridDim.x * blockDim.x) {
+    const size_t ray = (size_t)C.ray0 + r;
+    float *dst = C.radiance + 3 * ray;
+    V3 sum = P.accumulate ? mk3(dst[0], dst[1], dst[2]) : mk3(0, 0, 0);
+    const float4 *rad = P.q.rad + (size_t)r * (size_t)P.n_samples;
+    for (int s = 0; s < P.n_samples; s++) {
+      const float4 v = rad[s];
+      sum = add3(sum, mk3(v.x, v.y, v.z));
+      if (C.per_sample) {
+        float *ps = C.per_sample + (ray * (size_t)C.per_sample_stride + (size_t)(C.per_sample_offset + s)) * 3;
+        ps[0] = v.x; ps[1] = v.y; ps[2] = v.z;
+      }
+    }
+    dst[0] = sum.x; dst[1] = sum.y; dst[2] = sum.z;
+  }
+}
+
+size_t rt_cast_rays_workspace_bytes(size_t n_paths, int max_bounces, bool floor) {
+  size_t paths = floor ? (size_t)RT_CAST_RAYS_MIN_CHUNK : chunk_paths_max();
+  if (paths > n_paths) paths = n_paths;
+  if (paths < 1) paths = 1;
+  return counts_bytes(max_bounces > 0 ? max_bounces : 1) + paths * RT_PATH_BYTES;
+}
+
+int rt_launch_cast_rays(const SceneDev &scene, const float *rays, const unsigned *keys, int n_rays, int sample_begin,
+                        int samples, int max_bounces, uint32_t user_seed, int accumulate, float *radiance, float *per_sample,
+                        unsigned long long *counters, int sm_count, void *workspace, size_t workspace_bytes,
+                        cudaStream_t stream, int *n_launches) {
+  if (n_rays <= 0) return (int)cudaGetLastError();
+  if (samples <= 0) {
+    // no samples: the sums gain nothing (as rt_launch_render)
+    if (!accumulate) cudaMemsetAsync(radiance, 0, (size_t)n_rays * 3 * sizeof(float), stream);
+    return (int)cudaGetLastError();
+  }
+  size_t level_bytes = 0;
+  int dev = 0;
+  if (int e = trace_launch_setup(scene, &dev, &level_bytes)) return e;
+
+  StageParams P{};
+  P.scene = scene;
+  P.width = 1; P.height = 1;                 // no camera: the bounce trace does not use them
+  P.max_bounces = max_bounces;
+  P.user_seed = user_seed;
+  P.counters = counters;
+  CastRaysParams C{};
+  C.rays = rays; C.keys = keys; C.radiance = radiance; C.per_sample = per_sample;
+  C.per_sample_stride = samples;
+
+  // chunking: R rays x S samples per chunk, at most `cap` paths.  Every sample of every ray when they fit; otherwise
+  // samples of a ray stay together up to a warp's worth (or all of them, if the rays are few) and the rays are split
+  const size_t cb = counts_bytes(max_bounces > 0 ? max_bounces : 1);
+  if (workspace_bytes < cb + RT_PATH_BYTES) return (int)cudaErrorMemoryAllocation;
+  size_t cap = (workspace_bytes - cb) / RT_PATH_BYTES;
+  if (cap > chunk_paths_max()) cap = chunk_paths_max();
+  size_t S = (size_t)samples, R = (size_t)n_rays;
+  if (R * S > cap) {
+    const size_t warp = cap < 32 ? cap : 32;
+    S = cap / R > warp ? cap / R : warp;
+    if (S > (size_t)samples) S = (size_t)samples;
+    R = cap / S;
+    if (R > (size_t)n_rays) R = (size_t)n_rays;
+  }
+  bind_queues(P.q, static_cast<char *>(workspace), cb, R * S);
+
+  const unsigned trace_grid = (unsigned)(sm_count * g_trace_blocks_per_sm[dev]);
+  const unsigned wide_grid = (unsigned)(sm_count * g_wide_blocks_per_sm[dev]);
+  const unsigned flat_grid = (unsigned)(sm_count * 8);
+  // the renderer's per-bounce launch shapes (rt_launch_render); bounce 0 is a generic trace of a long queue
+  auto miss_grid  = [&](int b) { return (unsigned)sm_count * (b == 0 ? 64u : b == 1 ? 32u : 8u); };
+  auto shade_grid = [&](int b) { return (unsigned)sm_count * (b == 0 ? 64u : 8u); };
+  int launches = 0;
+  for (size_t r0 = 0; r0 < (size_t)n_rays; r0 += R) {
+    C.ray0 = (unsigned)r0;
+    C.n_rays = (unsigned)((size_t)n_rays - r0 < R ? (size_t)n_rays - r0 : R);
+    for (int s0 = sample_begin; s0 < sample_begin + samples; s0 += (int)S) {
+      const int n_s = sample_begin + samples - s0 < (int)S ? sample_begin + samples - s0 : (int)S;
+      P.sample0 = s0; P.n_samples = n_s;
+      P.n_paths = C.n_rays * (unsigned)n_s;
+      P.accumulate = (accumulate || s0 > sample_begin) ? 1 : 0;
+      C.per_sample_offset = s0 - sample_begin;
+      cudaMemsetAsync(P.q.counts, 0, cb, stream);
+      rt_cast_rays_raygen_kernel<<<flat_grid, 256, 0, stream>>>(P, C);
+      launches++;
+      for (int b = 0; b < max_bounces; b++) {
+        P.bounce = b;
+        if (b <= RT_TRACE_WIDE_BOUNCES) rt_trace_kernel<false, RT_TRACE_MIN_BLOCKS_WIDE><<<wide_grid, RT_BLOCK, level_bytes, stream>>>(P);
+        else                            rt_trace_kernel<false><<<trace_grid, RT_BLOCK, level_bytes, stream>>>(P);
+        rt_miss_kernel<<<miss_grid(b), 256, 0, stream>>>(P);
+        rt_shade_kernel<<<shade_grid(b), 256, 0, stream>>>(P);
+        launches += 3;
+      }
+      rt_cast_rays_accumulate_kernel<<<flat_grid * 4, 256, 0, stream>>>(P, C);
+      launches++;
+    }
+  }
   if (n_launches) *n_launches += launches;
   return (int)cudaGetLastError();
 }

@@ -258,6 +258,31 @@ def occluded(loaded: LoadedScene, origins, directions, t_max=None) -> np.ndarray
     return out.astype(bool)
 
 
+def cast_rays(loaded: LoadedScene, origins, directions, samples: int, max_bounces: int = 8, sample_begin: int = 0,
+              user_seed: int = 0, keys=None, per_sample: bool = False):
+    """Path-traced radiance along each ray (rt_gpu_cast_rays; semantics in include/rt_gpu.h): the reference's cast_ray
+    for samples [sample_begin, sample_begin + samples), the shader generator of path (i, s) seeded to
+    rt_path_seed(keys[i] (default i), s, user_seed).  Directions are used as given.  Uploads the scene if it is not
+    resident.  Returns the (n, 3) float32 sums over the samples (not divided); with per_sample, also the
+    (n, samples, 3) radiance of every path, as (radiance, per_sample)."""
+    gpu = gpu_lib()
+    register_callbacks(loaded)
+    rays, _ = _query_rays(origins, directions, None)
+    n = len(rays)
+    if keys is not None:
+        keys = np.ascontiguousarray(np.asarray(keys, dtype=np.uint32).reshape(-1))
+        if len(keys) != n:
+            raise ValueError(f"{len(keys)} keys for {n} rays")
+    if gpu.rt_gpu_scene_device_bytes(C.byref(loaded.scene)) == 0:
+        gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+    radiance = np.zeros((n, 3), dtype=np.float32)
+    per = np.zeros((n, samples, 3), dtype=np.float32) if per_sample else None
+    gpu_check(gpu.rt_gpu_cast_rays(C.byref(loaded.scene), rays.ctypes.data, keys.ctypes.data if keys is not None else None,
+                                   n, sample_begin, samples, max_bounces, user_seed, 0, radiance.ctypes.data,
+                                   per.ctypes.data if per is not None else None))
+    return (radiance, per) if per_sample else radiance
+
+
 def read_accum(width: int, height: int) -> np.ndarray:
     out = np.empty((height, width, 3), dtype=np.float32)
     gpu_check(gpu_lib().rt_gpu_read_accum(out.ctypes.data, out.size))
