@@ -238,6 +238,57 @@ int rt_gpu_cast_rays_device(Scene const *scene, Ray const *d_rays, u32 const *d_
 int rt_gpu_cast_rays(Scene const *scene, Ray const *rays, u32 const *keys, isize n_rays, isize sample_begin, isize samples,
                      isize max_bounces, u32 user_seed, i32 accumulate, f32 *radiance, f32 *per_sample);
 
+/* ---- first-surface AOVs of the renderer's camera samples on a resident scene (csrc/rt_render.cu) ----
+ * Per-pixel buffers aligned with the beauty image: what surface each sample of the renderer's path (pixel p, sample s)
+ * shades first, for s in [sample_begin, sample_end), with max_bounces:
+ *   1. the camera ray of (p, s) is the one the renderer traces, from the scene's current camera as a render reads it;
+ *   2. while the hit is a back face (dot(ng, d) > 0 || dot(normal, d) > 0, raytracer.c:516-522) and fewer than
+ *      max_bounces walks have been made, the walk continues from point + d * EPSILON, as the renderer's path does;
+ *   3. the first front-face hit within max_bounces walks is the sample's surface: where the path runs its first shader.
+ *      A sample that escapes, or uses up its walks on back faces, has no surface.
+ * Values at the surface are the renderer's f32 expressions:
+ *   albedo    the base colour the BSDF receives: base_color times the sRGB-decoded albedo texel where there is one;
+ *   normal    the shading normal handed to the BSDF: the normalised interpolated normal, normal-mapped where the
+ *             material has a normal map;
+ *   position  o + d * t of the last walk (the shaded point);
+ *   depth     sqrt((position - eye) . (position - eye)), eye the camera origin: three products summed left to right,
+ *             one IEEE square root;
+ *   emission  the emission the shader returns (emission times the decoded emissive texel);
+ *   roughness, metalness  after their texture, the clamp and min(., 0.9) / 0.9;
+ *   coverage  1.
+ * A sample with no surface adds nothing to any field.  Nothing random happens before a path's first shade (the jitter
+ * is a hash of pixel and sample, the back-face step is deterministic, the material fetch draws no random numbers), so
+ * every record is exact per (pixel, sample), with no seed; NaN values (a degenerate interpolated normal) are summed as
+ * they come.
+ * aov[y * width + x] holds the SUMS over the samples in sample order, before any division (the meaning of
+ * rt_gpu_read_accum): divide by coverage for the mean over covered samples, or by the sample count.  With
+ * accumulate != 0 the sums continue from what the buffer holds, so [0, k) then [k, n) equals [0, n) bit for bit.  With
+ * an empty range or max_bounces = 0 nothing is traced: the records are zeroed unless accumulate is set, in which case
+ * they are left as they are, and the counters are not touched.
+ * d_counters (optional, 8 u64, atomically added) as RT_GPU_CTR_*: RAYS, NODES, LEAVES, ACCEPTS of every walk; SHADES =
+ * samples with a surface; MISSES = walks that escaped; PASSTHROUGH = back-face hits; SAMPLES = W * H * (end - begin).
+ * Always exact: RT_GPU_Options.fast_math does not apply, and pixel_rank / pixel_world do not either (the call covers the
+ * whole image).  First device only.  The call reads texels, so it waits for the scene's texels as well as its geometry;
+ * it uses the device's path-queue workspace and rewrites the camera-relative scene copies, so it is serialised with
+ * renders, lightmap bakes and cast_rays on that device.
+ * Refused before any launch: width or height < 1, or an image whose one sample per pixel exceeds 2^31 path ids;
+ * sample_begin < 0, sample_end < sample_begin, sample_end > INT32_MAX; max_bounces < 0; a NULL record buffer, or
+ * (device form) one that is not 16-byte aligned; a scene that is not resident (rt_gpu_scene_upload). */
+typedef struct {
+  Vec3 albedo;   f32 coverage;
+  Vec3 normal;   f32 depth;
+  Vec3 position; f32 roughness;
+  Vec3 emission; f32 metalness;
+} RT_GPU_AOV;                                   /* 64 B: four 16-byte vectors per pixel */
+int rt_gpu_render_aov_device(Scene const *scene, isize width, isize height, isize sample_begin, isize sample_end,
+                             isize max_bounces, i32 accumulate,
+                             RT_GPU_AOV *d_aov,       /* W*H, 16-byte aligned */
+                             u64 *d_counters,         /* optional 8 */
+                             void *stream);
+/* host memory: staged through a library-owned device buffer, from zero; returns when the records are in place */
+int rt_gpu_render_aov(Scene const *scene, isize width, isize height, isize sample_begin, isize sample_end,
+                      isize max_bounces, RT_GPU_AOV *aov);
+
 #ifdef __cplusplus
 }
 #endif

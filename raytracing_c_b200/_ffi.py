@@ -109,6 +109,12 @@ class GPUSurface(C.Structure):
     _fields_ = [("point", Vec3), ("normal", Vec3), ("normal_geo", Vec3), ("tex_coords", Vec2)]
 
 
+class GPUAOV(C.Structure):
+    """RT_GPU_AOV: per-pixel sums of the first-surface AOVs (64 B)."""
+    _fields_ = [("albedo", Vec3), ("coverage", C.c_float), ("normal", Vec3), ("depth", C.c_float),
+                ("position", Vec3), ("roughness", C.c_float), ("emission", Vec3), ("metalness", C.c_float)]
+
+
 SPLIT_AUTO, SPLIT_SAMPLES, SPLIT_CHUNKS = 0, 1, 2
 REDUCE_P2P, REDUCE_NCCL = 0, 1
 
@@ -136,6 +142,7 @@ GPU_EXPORTS = [
     "rt_gpu_render_accum_device", "rt_gpu_resolve_device", "rt_gpu_denoise_device",
     "rt_gpu_closest_hit_device", "rt_gpu_occluded_device", "rt_gpu_closest_hit", "rt_gpu_occluded",
     "rt_gpu_cast_rays_device", "rt_gpu_cast_rays",
+    "rt_gpu_render_aov_device", "rt_gpu_render_aov",
 ]
 
 HOST_EXPORTS = [
@@ -267,6 +274,9 @@ def gpu_lib() -> C.CDLL:
                                                 C.c_uint32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.rt_gpu_cast_rays.argtypes = [C.POINTER(Scene), C.c_void_p, C.c_void_p, isize, isize, isize, isize, C.c_uint32,
                                          C.c_int32, C.c_void_p, C.c_void_p]
+        lib.rt_gpu_render_aov_device.argtypes = [C.POINTER(Scene), isize, isize, isize, isize, isize, C.c_int32, C.c_void_p,
+                                                 C.c_void_p, C.c_void_p]
+        lib.rt_gpu_render_aov.argtypes = [C.POINTER(Scene), isize, isize, isize, isize, isize, C.c_void_p]
         lib.render_thread_proc.argtypes = [C.POINTER(RenderingContext)]
         lib.render_thread_proc.restype = None
         lib.rendering_context_is_finished.argtypes = [C.POINTER(RenderingContext)]

@@ -654,6 +654,88 @@ int rt_gpu_cast_rays(Scene const *scene, Ray const *rays, u32 const *keys, isize
   return 0;
 }
 
+// ------------------------------------------------------------- first-surface AOVs
+}  // extern "C"
+
+namespace {
+
+// Everything that is refused before a launch; afterwards the scene is resident on the first device with the camera the
+// Scene holds now (scene_on_devices refreshes it, as for a render).
+int aov_validate(const char *what, const Scene *scene, isize width, isize height, isize sample_begin, isize sample_end,
+                 isize max_bounces, const void *aov) {
+  if (width < 1 || height < 1) return fail("%s: image %lld x %lld is empty", what, (long long)width, (long long)height);
+  // one sample of every pixel must fit one chunk of 32-bit path ids
+  if (width > INT32_MAX || height > INT32_MAX ||
+      (size_t)((width + 7) / 8) * (size_t)((height + 3) / 4) * 32 > ((size_t)1 << 31))
+    return fail("%s: image %lld x %lld is too large", what, (long long)width, (long long)height);
+  if (sample_begin < 0 || sample_end < sample_begin || sample_end > INT32_MAX)
+    return fail("%s: samples [%lld, %lld) must be a range inside [0, INT32_MAX]", what, (long long)sample_begin,
+                (long long)sample_end);
+  if (max_bounces < 0 || max_bounces > INT32_MAX) return fail("%s: max_bounces = %lld, must be >= 0", what, (long long)max_bounces);
+  if (!aov) return fail("%s: null aov", what);
+  if (!scene) return fail("%s: null scene", what);
+  if (ensure_init()) return 1;
+  if (g.devs[0].scenes.find(scene) == g.devs[0].scenes.end())
+    return fail("%s: scene is not resident (rt_gpu_scene_upload it first)", what);
+  return scene_on_devices(scene);
+}
+
+// One AOV call on the first device, ordered on `stream`.  Like a render it uses the device's path-queue workspace and
+// rewrites the camera-relative copies, so it waits for the previous user of both (busy) and records busy after its last
+// kernel; it reads texels, so it waits for the scene's texels as well as its geometry.
+int aov_on_device(const Scene *scene, isize width, isize height, isize sample_begin, isize sample_end, isize max_bounces,
+                  int accumulate, float *aov, unsigned long long *counters, cudaStream_t stream) {
+  Device &d = g.devs[0];
+  CUDA_TRY(cudaSetDevice(d.id));
+  const DeviceScene &ds = d.scenes.find(scene)->second;
+  const int n_samples = (int)(sample_end - sample_begin);
+  if (n_samples > 0 && max_bounces > 0 &&
+      ensure_workspace(d, rt_render_workspace_bytes((int)width, (int)height, n_samples, (int)max_bounces, 0, 1),
+                       rt_render_workspace_bytes((int)width, (int)height, 1, (int)max_bounces, 1, 1), stream))
+    return 1;
+  if (d.busy_valid) CUDA_TRY(cudaStreamWaitEvent(stream, d.busy, 0));
+  CUDA_TRY(cudaStreamWaitEvent(stream, ds.geom_ready, 0));
+  CUDA_TRY(cudaStreamWaitEvent(stream, ds.tex_ready, 0));
+  set_l2_window(d, ds, stream);
+  int e = rt_launch_aov(ds.dev, (int)width, (int)height, (int)sample_begin, (int)sample_end, (int)max_bounces, accumulate,
+                        aov, counters, d.sm_count, d.d_workspace, d.workspace_bytes, stream, &g.last_launches);
+  if (e) return fail("aov kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
+  CUDA_TRY(cudaEventRecord(d.busy, stream));
+  d.busy_valid = true;
+  return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int rt_gpu_render_aov_device(Scene const *scene, isize width, isize height, isize sample_begin, isize sample_end,
+                             isize max_bounces, i32 accumulate, RT_GPU_AOV *d_aov, u64 *d_counters, void *stream) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  if (aov_validate("render_aov", scene, width, height, sample_begin, sample_end, max_bounces, d_aov)) return 1;
+  if (reinterpret_cast<uintptr_t>(d_aov) & 15) return fail("render_aov: d_aov is not 16-byte aligned");
+  return aov_on_device(scene, width, height, sample_begin, sample_end, max_bounces, accumulate,
+                       reinterpret_cast<float *>(d_aov), reinterpret_cast<unsigned long long *>(d_counters),
+                       static_cast<cudaStream_t>(stream));
+}
+
+// Host memory: the records go through the first device's AOV staging block and come back; synchronises.
+int rt_gpu_render_aov(Scene const *scene, isize width, isize height, isize sample_begin, isize sample_end,
+                      isize max_bounces, RT_GPU_AOV *aov) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  g.last_launches = 0;
+  if (aov_validate("render_aov", scene, width, height, sample_begin, sample_end, max_bounces, aov)) return 1;
+  Device &d = g.devs[0];
+  CUDA_TRY(cudaSetDevice(d.id));
+  const size_t bytes = (size_t)width * (size_t)height * sizeof(RT_GPU_AOV);
+  if (grow(&d.d_aov_stage, &d.aov_stage_bytes, bytes)) return 1;
+  float *d_aov = static_cast<float *>(d.d_aov_stage);
+  if (aov_on_device(scene, width, height, sample_begin, sample_end, max_bounces, 0, d_aov, nullptr, d.stream)) return 1;
+  CUDA_TRY(cudaMemcpyAsync(aov, d_aov, bytes, cudaMemcpyDeviceToHost, d.stream));
+  CUDA_TRY(cudaStreamSynchronize(d.stream));
+  return 0;
+}
+
 // ----------------------------------------------------------------- parity hooks
 int rt_gpu_read_accum(f32 *out, isize n_floats) {
   std::lock_guard<std::mutex> lock(g_mutex);

@@ -26,6 +26,12 @@ int rt_launch_cast_rays(const SceneDev &scene, const float *rays, const unsigned
                         int samples, int max_bounces, uint32_t user_seed, int accumulate, float *radiance, float *per_sample,
                         unsigned long long *counters, int sm_count, void *workspace, size_t workspace_bytes,
                         cudaStream_t stream, int *n_launches);
+// first-surface AOVs of the renderer's camera samples [sample_begin, sample_end), whole image, summed per pixel into aov
+// (W*H records of 16 floats, 16-byte aligned; see rt_render.cu).  The workspace is the renderer's
+// (rt_render_workspace_bytes with split_world 1)
+int rt_launch_aov(const SceneDev &scene, int width, int height, int sample_begin, int sample_end, int max_bounces,
+                  int accumulate, float *aov, unsigned long long *counters, int sm_count, void *workspace,
+                  size_t workspace_bytes, cudaStream_t stream, int *n_launches);
 int rt_launch_resolve(const float *accum, int width, int height, int samples, unsigned char *pixels,
                       int stride, int components, cudaStream_t stream);
 // sum of parts.n accumulators (own + peer-mapped) in rank order, optional copy of the sum, optional resolve to u8

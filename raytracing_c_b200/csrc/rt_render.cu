@@ -783,6 +783,193 @@ int rt_launch_cast_rays(const SceneDev &scene, const float *rays, const unsigned
   return (int)cudaGetLastError();
 }
 
+// ===================================================================== first-surface AOVs
+// What surface the renderer's path (pixel, sample) shades first: its camera ray (the unchanged primary trace), walked
+// through back faces as shade_hit steps through them (raytracer.c:516-522), to the first front face within max_bounces
+// walks.  Nothing random happens before that shade, so the record is exact per (pixel, sample).  The surface kernel
+// keeps, per path id, (point.xyz, slot) in `tint` and (u, v) in `emis` (path state the trace kernel never touches;
+// slot -1 = no surface); the accumulate kernel evaluates the material there (pbr_surface, as shade_pbr does) and sums
+// per pixel in sample order.
+
+// the HIT queue of bounce b: a back face goes on to the RAY queue of b + 1 while walks remain; a front face is the path's
+// surface.  Misses have no kernel (their record stays "no surface"): their count comes from the queue length.
+__global__ void __launch_bounds__(256)
+rt_aov_surface_kernel(const __grid_constant__ StageParams P) {
+  const SceneDev &sc = P.scene;
+  const unsigned lane = threadIdx.x & 31u;
+  const unsigned n = P.q.counts[P.bounce * Q_STRIDE + Q_HITS];
+  unsigned *next_rays = &P.q.counts[(P.bounce + 1) * Q_STRIDE + Q_RAYS];
+  const unsigned n_round = (n + 31u) & ~31u;          // whole warps stay in the loop for the collective append
+  unsigned c_shades = 0, c_pass = 0;
+  for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n_round; i += gridDim.x * blockDim.x) {
+    bool cont = false;
+    float4 ra = make_float4(0, 0, 0, 0), rb = make_float4(0, 0, 0, 0);
+    if (i < n) {
+      const float4 a = P.q.hit_a[i], b = P.q.hit_b[i], h = P.q.hit_h[i];
+      const V3 o = mk3(a.x, a.y, a.z), d = mk3(a.w, b.x, b.y);
+      const unsigned path = __float_as_uint(b.z);
+      const int slot = __float_as_int(h.w);
+      // shade_hit's point, interpolated normal and back-face test (rt_stages.cuh)
+      const float4 *rec = sc.tri_rec + (size_t)slot * 7;
+      const float4 r0 = __ldg(rec + 0), r1 = __ldg(rec + 1), r2 = __ldg(rec + 2);
+      const V3 ng = mk3(r0.x, r0.y, r0.z);
+      const V3 na = mk3(r0.w, r1.x, r1.y), nb = mk3(r1.z, r1.w, r2.x), nc = mk3(r2.y, r2.z, r2.w);
+      const float w1 = h.y, w2 = h.z, w0 = 1 - w1 - w2;
+      const V3 point = add3(o, scale3(d, h.x));
+      const V3 normal = mk3(na.x * w0 + nb.x * w1 + nc.x * w2,
+                            na.y * w0 + nb.y * w1 + nc.y * w2,
+                            na.z * w0 + nb.z * w1 + nc.z * w2);
+      if (dot3(ng, d) > 0 || dot3(normal, d) > 0) {
+        c_pass++;
+        cont = P.bounce + 1 < P.max_bounces;
+        const V3 next = add3(point, scale3(d, RT_EPS));
+        ra = make_float4(next.x, next.y, next.z, d.x);
+        rb = make_float4(d.y, d.z, b.z, b.w);
+      } else {
+        c_shades++;
+        P.q.tint[path] = make_float4(point.x, point.y, point.z, h.w);
+        P.q.emis[path] = make_float4(w1, w2, 0, 0);
+      }
+    }
+    const unsigned pos = warp_append(next_rays, cont, lane);
+    if (cont) { P.q.ray_a[pos] = ra; P.q.ray_b[pos] = rb; }
+  }
+  if (P.counters) {
+    add_counter(P.counters, 4, c_shades);
+    add_counter(P.counters, 6, c_pass);
+    if (blockIdx.x == 0 && threadIdx.x == 0)
+      atomicAdd(&P.counters[5], (unsigned long long)P.q.counts[P.bounce * Q_STRIDE + Q_MISSES]);
+  }
+}
+
+// per pixel: the records of its samples in sample order, each sample's material evaluated at its surface, summed into
+// aov[pixel] = (albedo, coverage) (normal, depth) (position, roughness) (emission, metalness) — from zero on the first
+// chunk of a call without `accumulate`, else from the buffer
+__global__ void __launch_bounds__(256)
+rt_aov_accumulate_kernel(const __grid_constant__ StageParams P, float4 *__restrict__ aov) {
+  const SceneDev &sc = P.scene;
+  const float ex = sc.view[0][3], ey = sc.view[1][3], ez = sc.view[2][3];          // the camera origin (raytracer.c:612)
+  const unsigned n = P.n_tiles * 32u;
+  unsigned c_samples = 0;
+  for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const unsigned tile = i >> 5, in_tile = i & 31u;
+    int x0, y0;
+    tile_origin(P, tile, x0, y0);
+    const int px = x0 + (int)(in_tile & 7u), py = y0 + (int)(in_tile >> 3);
+    if (px >= P.width || py >= P.height) continue;
+    float4 *dst = aov + 4 * ((size_t)py * (size_t)P.width + (size_t)px);
+    float4 s0 = make_float4(0, 0, 0, 0), s1 = s0, s2 = s0, s3 = s0;
+    if (P.accumulate) { s0 = dst[0]; s1 = dst[1]; s2 = dst[2]; s3 = dst[3]; }
+    const size_t first = (size_t)i * (size_t)P.n_samples;            // RT_PATH_LAYOUT 1: path id = pixel * S + s
+    for (int s = 0; s < P.n_samples; s++) {
+      const float4 surf = P.q.tint[first + s];
+      const int slot = __float_as_int(surf.w);
+      if (slot < 0) continue;
+      const float4 bary = P.q.emis[first + s];
+      // shade_hit's shading input (rt_stages.cuh) at the recorded surface
+      const float4 *rec = sc.tri_rec + (size_t)slot * 7;
+      const float4 r0 = __ldg(rec + 0), r1 = __ldg(rec + 1), r2 = __ldg(rec + 2), r3 = __ldg(rec + 3);
+      const float4 r4 = __ldg(rec + 4), r5 = __ldg(rec + 5), r6 = __ldg(rec + 6);
+      const V3 na = mk3(r0.w, r1.x, r1.y), nb = mk3(r1.z, r1.w, r2.x), nc = mk3(r2.y, r2.z, r2.w);
+      const float w1 = bary.x, w2 = bary.y, w0 = 1 - w1 - w2;
+      const V3 normal = mk3(na.x * w0 + nb.x * w1 + nc.x * w2,
+                            na.y * w0 + nb.y * w1 + nc.y * w2,
+                            na.z * w0 + nb.z * w1 + nc.z * w2);
+      ShadeIn in;
+      in.dir = mk3(0, 0, 0);                                         // the material fetch does not read it
+      in.normal = normalize3(normal);
+      in.normal_geo = mk3(r0.x, r0.y, r0.z);
+      in.tangent   = mk3(r3.x, r3.y, r3.z);
+      in.bitangent = mk3(r3.w, r4.x, r4.y);
+      in.u = r4.z * w0 + r5.x * w1 + r5.z * w2;
+      in.v = r4.w * w0 + r5.y * w1 + r5.w * w2;
+      V3 nrm, base, glow;
+      float roughness, metalness;
+      pbr_surface(sc, sc.materials[__float_as_int(r6.x)], in, nrm, base, roughness, metalness, glow);
+      const float dx = surf.x - ex, dy = surf.y - ey, dz = surf.z - ez;
+      const float depth = __fsqrt_rn(dx * dx + dy * dy + dz * dz);
+      s0.x += base.x; s0.y += base.y; s0.z += base.z; s0.w += 1.0f;
+      s1.x += nrm.x;  s1.y += nrm.y;  s1.z += nrm.z;  s1.w += depth;
+      s2.x += surf.x; s2.y += surf.y; s2.z += surf.z; s2.w += roughness;
+      s3.x += glow.x; s3.y += glow.y; s3.z += glow.z; s3.w += metalness;
+    }
+    dst[0] = s0; dst[1] = s1; dst[2] = s2; dst[3] = s3;
+    c_samples += (unsigned)P.n_samples;
+  }
+  if (P.counters) add_counter(P.counters, 7, c_samples);
+}
+
+int rt_launch_aov(const SceneDev &scene, int width, int height, int sample_begin, int sample_end, int max_bounces,
+                  int accumulate, float *aov, unsigned long long *counters, int sm_count, void *workspace,
+                  size_t workspace_bytes, cudaStream_t stream, int *n_launches) {
+  const int n_total = sample_end - sample_begin;
+  if (n_total <= 0 || max_bounces < 1) {
+    // no samples, or no walk: no sample has a surface (as rt_launch_render)
+    if (!accumulate) cudaMemsetAsync(aov, 0, (size_t)width * (size_t)height * 16 * sizeof(float), stream);
+    return (int)cudaGetLastError();
+  }
+  size_t level_bytes = 0;
+  int dev = 0;
+  if (int e = trace_launch_setup(scene, &dev, &level_bytes)) return e;
+
+  // the renderer's frame set-up (rt_launch_render, whole image)
+  StageParams P{};
+  P.scene = scene;
+  P.width = width; P.height = height;
+  P.tiles_x = (width + 7) / 8; P.tiles_y = (height + 3) / 4;
+  P.split_rank = 0; P.split_world = 1;
+  P.chunks_x = (width + 31) / 32;
+  P.n_tiles = rt_render_tiles(width, height, 0, 1);
+  P.div_tiles_x = rt_fastdiv_make((uint32_t)P.tiles_x, 0xffffffffu >> 5);
+  P.div_chunks_x = rt_fastdiv_make((uint32_t)P.chunks_x, 0xffffffffu);
+  P.max_bounces = max_bounces;
+  P.counters = counters;
+
+  const size_t per_sample = (size_t)P.n_tiles * 32;
+  const size_t cb = counts_bytes(max_bounces);
+  if (workspace_bytes < cb + per_sample * RT_PATH_BYTES) return (int)cudaErrorMemoryAllocation;
+  size_t cap = (workspace_bytes - cb) / RT_PATH_BYTES;
+  size_t fit = chunk_samples(per_sample, n_total, 0);
+  if (fit > cap / per_sample) fit = cap / per_sample;
+  const int chunk = (int)fit;
+  cap = (size_t)chunk * per_sample;
+  bind_queues(P.q, static_cast<char *>(workspace), cb, cap);
+
+  rt_camera_relative_kernel<<<(unsigned)sm_count, 256, 0, stream>>>(scene);
+  const unsigned trace_grid = (unsigned)(sm_count * g_trace_blocks_per_sm[dev]);
+  const unsigned wide_grid = (unsigned)(sm_count * g_wide_blocks_per_sm[dev]);
+  const unsigned primary_grid = (unsigned)(sm_count * g_primary_blocks_per_sm[dev]);
+  const unsigned flat_grid = (unsigned)(sm_count * 8);
+  auto surface_grid = [&](int b) { return (unsigned)sm_count * (b == 0 ? 64u : 8u); };    // the renderer's shade_grid
+  int launches = 1;
+  for (int s0 = sample_begin; s0 < sample_end; s0 += chunk) {
+    const int S = (sample_end - s0 < chunk) ? sample_end - s0 : chunk;
+    P.sample0 = s0; P.n_samples = S;
+    P.n_paths = (unsigned)(per_sample * (size_t)S);
+    P.div_samples = rt_fastdiv_make((uint32_t)S, P.n_paths);
+    P.accumulate = (accumulate || s0 > sample_begin) ? 1 : 0;
+    cudaMemsetAsync(P.q.counts, 0, cb, stream);
+    cudaMemsetAsync(P.q.tint, 0xff, (size_t)P.n_paths * sizeof(float4), stream);    // slot -1: no surface yet
+    P.bounce = 0;
+    rt_trace_kernel<true><<<primary_grid, RT_BLOCK, level_bytes, stream>>>(P);
+    launches++;
+    for (int b = 0; b < max_bounces; b++) {
+      P.bounce = b;
+      if (b > 0) {
+        if (b <= RT_TRACE_WIDE_BOUNCES) rt_trace_kernel<false, RT_TRACE_MIN_BLOCKS_WIDE><<<wide_grid, RT_BLOCK, level_bytes, stream>>>(P);
+        else                            rt_trace_kernel<false><<<trace_grid, RT_BLOCK, level_bytes, stream>>>(P);
+        launches++;
+      }
+      rt_aov_surface_kernel<<<surface_grid(b), 256, 0, stream>>>(P);
+      launches++;
+    }
+    rt_aov_accumulate_kernel<<<flat_grid * 4, 256, 0, stream>>>(P, reinterpret_cast<float4 *>(aov));
+    launches++;
+  }
+  if (n_launches) *n_launches += launches;
+  return (int)cudaGetLastError();
+}
+
 int rt_launch_resolve(const float *accum, int width, int height, int samples, unsigned char *pixels,
                       int stride, int components, cudaStream_t stream) {
   int n = width * height;

@@ -178,12 +178,14 @@ __device__ __forceinline__ V3 sheen_term(float sheen, V3 base, float sheen_tint,
   return scale3(lerp3(mk3(1, 1, 1), tint, sheen_tint), sheen * w);
 }
 
-// driver.c:350-409 with :287-348 inlined
-__device__ __forceinline__ void shade_pbr(const SceneDev &sc, int material, const ShadeIn &in, uint32_t &rng, ShadeOut &out) {
-  const MaterialDev &mat = sc.materials[material];
-
+// driver.c:129-153,350-367: the material fetch — what the BSDF receives at a surface: the shading normal (normal-mapped
+// where the material has a map), the base colour after the albedo texture, roughness and metalness after their texture,
+// clamp and rescale, and the emission.  No random numbers are drawn.  shade_pbr and the first-surface AOVs
+// (rt_render.cu) both evaluate it here, so the AOVs are what the shader saw.
+__device__ __forceinline__ void pbr_surface(const SceneDev &sc, const MaterialDev &mat, const ShadeIn &in, V3 &n, V3 &base,
+                                            float &roughness, float &metalness, V3 &glow) {
   // driver.c:129-153
-  V3 n = in.normal;
+  n = in.normal;
   if (mat.tex_normal >= 0) {
     V3 s = sample_bilinear(sc.textures[mat.tex_normal], in.u, in.v);
     s = add3(scale3(s, 2.0f), mk3(-1, -1, -1));
@@ -195,10 +197,10 @@ __device__ __forceinline__ void shade_pbr(const SceneDev &sc, int material, cons
                        k * (s.x * t.z + s.y * b.z + s.z * n.z) + n.z * (1 - k)));
   }
 
-  V3 base = mk3(mat.base[0], mat.base[1], mat.base[2]);
+  base = mk3(mat.base[0], mat.base[1], mat.base[2]);
   if (mat.tex_albedo >= 0) base = mul3(base, decode_srgb(sample_bilinear(sc.textures[mat.tex_albedo], in.u, in.v)));
 
-  float roughness = mat.roughness, metalness = mat.metalness;
+  roughness = mat.roughness; metalness = mat.metalness;
   if (mat.tex_mr >= 0) {
     V3 mr = sample_bilinear(sc.textures[mat.tex_mr], in.u, in.v);
     roughness *= mr.y;
@@ -208,7 +210,7 @@ __device__ __forceinline__ void shade_pbr(const SceneDev &sc, int material, cons
   if (metalness > 0.9f) metalness = 0.9f;
   metalness /= 0.9f;
 
-  V3 glow = mk3(mat.emission[0], mat.emission[1], mat.emission[2]);
+  glow = mk3(mat.emission[0], mat.emission[1], mat.emission[2]);
   if (mat.tex_emission >= 0) {
     // emissive maps are mostly black, and a black bilinear tap decodes to one constant (common.h:82-88 has no linear toe:
     // pow(0.055 / 1.055, 2.4)) — sc.srgb_of_zero holds it, evaluated once by the same rt_math.h code, so a warp whose
@@ -218,6 +220,14 @@ __device__ __forceinline__ void shade_pbr(const SceneDev &sc, int material, cons
     const V3 lin = black ? mk3(sc.srgb_of_zero, sc.srgb_of_zero, sc.srgb_of_zero) : decode_srgb(e);
     glow = mul3(glow, lin);
   }
+}
+
+// driver.c:350-409 with :287-348 inlined
+__device__ __forceinline__ void shade_pbr(const SceneDev &sc, int material, const ShadeIn &in, uint32_t &rng, ShadeOut &out) {
+  const MaterialDev &mat = sc.materials[material];
+  V3 n, base, glow;
+  float roughness, metalness;
+  pbr_surface(sc, mat, in, n, base, roughness, metalness, glow);
   out.emission = glow;
   out.terminate = false;
   out.tint = mk3(0, 0, 0);

@@ -83,6 +83,8 @@ struct Device {
   void *d_query_stage = nullptr; size_t query_stage_bytes = 0;
   // staging of the host-memory rt_gpu_cast_rays: rays, keys, sums, per-sample radiance
   void *d_cast_stage = nullptr; size_t cast_stage_bytes = 0;
+  // staging of the host-memory rt_gpu_render_aov: the W*H records
+  void *d_aov_stage = nullptr; size_t aov_stage_bytes = 0;
   bool l2_window_set = false;
   size_t l2_persist_max = 0, l2_window_max = 0;    // device limits (persistingL2CacheMaxSize, accessPolicyMaxWindowSize)
   cudaStream_t l2_stream = nullptr; const void *l2_base = nullptr;   // where the window was last set

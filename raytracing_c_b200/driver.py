@@ -283,6 +283,28 @@ def cast_rays(loaded: LoadedScene, origins, directions, samples: int, max_bounce
     return (radiance, per) if per_sample else radiance
 
 
+def render_aov(loaded: LoadedScene, width: int, height: int, samples: int, max_bounces: int = 8,
+               sample_begin: int = 0) -> dict:
+    """First-surface AOVs of the renderer's camera samples [sample_begin, sample_begin + samples) (rt_gpu_render_aov;
+    semantics in include/rt_gpu.h): per pixel, the sums over the samples of albedo, shading normal, position and
+    emission ((H, W, 3) float32) and of coverage, depth, roughness and metalness ((H, W) float32), at the first front
+    face each sample's path shades.  The sums are not divided: divide by coverage for the mean over the covered samples.
+    Uploads the scene if it is not resident."""
+    gpu = gpu_lib()
+    register_callbacks(loaded)
+    if gpu.rt_gpu_scene_device_bytes(C.byref(loaded.scene)) == 0:
+        gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+    floats = C.sizeof(_ffi.GPUAOV) // 4
+    records = np.zeros((height, width, floats), dtype=np.float32)
+    gpu_check(gpu.rt_gpu_render_aov(C.byref(loaded.scene), width, height, sample_begin, sample_begin + samples,
+                                    max_bounces, records.ctypes.data))
+    out = {}
+    for name, ctype in _ffi.GPUAOV._fields_:
+        first = getattr(_ffi.GPUAOV, name).offset // 4
+        out[name] = records[:, :, first:first + 3].copy() if ctype is Vec3 else records[:, :, first].copy()
+    return out
+
+
 def read_accum(width: int, height: int) -> np.ndarray:
     out = np.empty((height, width, 3), dtype=np.float32)
     gpu_check(gpu_lib().rt_gpu_read_accum(out.ctypes.data, out.size))
