@@ -121,10 +121,20 @@ int ensure_init() {
   return init_devices_locked(1, &zero);
 }
 
+// bytes of path-queue workspace a call asks for: the preferred size and the least it accepts (want 0: none)
+struct WorkspaceRequest { size_t want = 0, floor = 0; };
+
+// the camera path's request (render, AOV) for n_samples samples of every pixel: one chunk of them, or one sample
+WorkspaceRequest camera_workspace(isize width, isize height, isize n_samples, isize max_bounces, int split_world) {
+  return {rt_render_workspace_bytes((int)width, (int)height, (int)n_samples, (int)max_bounces, split_world),
+          rt_render_workspace_bytes((int)width, (int)height, 1, (int)max_bounces, split_world)};
+}
+
 // Path-queue workspace of one device.  The preferred size (up to 26.6 GB) is a throughput choice, not a requirement:
-// on a device that cannot spare it the request is halved down to one sample of every pixel per chunk, and the size
-// that was refused is remembered so later calls do not walk the same ladder again.
-int ensure_workspace(Device &d, size_t want, size_t floor_bytes, cudaStream_t stream) {
+// on a device that cannot spare it the request is halved down to the floor (one sample of every pixel per chunk for
+// a render), and the size that was refused is remembered so later calls do not walk the same ladder again.
+int ensure_workspace(Device &d, const WorkspaceRequest &r, cudaStream_t stream) {
+  const size_t want = r.want, floor_bytes = r.floor;
   if (d.workspace_bytes >= want) return 0;
   if (d.workspace_denied && want >= d.workspace_denied && d.workspace_bytes >= floor_bytes) return 0;
   CUDA_TRY(cudaStreamSynchronize(stream));      // an earlier launch may still read the old queues
@@ -142,33 +152,49 @@ int ensure_workspace(Device &d, size_t want, size_t floor_bytes, cudaStream_t st
   return 0;
 }
 
+// Every user of a device's path-queue workspace (render, lightmap bake, cast_rays, AOV) is serialised on the device
+// whatever stream it comes from: it waits for the event the previous user recorded (busy) and records busy after its
+// last kernel.  Renders and AOV calls also rewrite the scene's camera-relative copies, which the same event covers.
+// A user waits for the scene's geometry, and for its texels unless its launch defers that wait (the renderer's
+// shading_ready).
+int workspace_begin(Device &d, const DeviceScene &ds, const WorkspaceRequest &r, bool wait_texels, cudaStream_t stream) {
+  if (ensure_workspace(d, r, stream)) return 1;
+  if (d.busy_valid) CUDA_TRY(cudaStreamWaitEvent(stream, d.busy, 0));
+  CUDA_TRY(cudaStreamWaitEvent(stream, ds.geom_ready, 0));
+  if (wait_texels) CUDA_TRY(cudaStreamWaitEvent(stream, ds.tex_ready, 0));
+  set_l2_window(d, ds, stream);
+  return 0;
+}
+
+int workspace_end(Device &d, const char *what, int launch_error, cudaStream_t stream) {
+  if (launch_error) return fail("%s kernel launch failed: %s", what, cudaGetErrorString((cudaError_t)launch_error));
+  CUDA_TRY(cudaEventRecord(d.busy, stream));
+  d.busy_valid = true;
+  return 0;
+}
+
 struct Share {            // what one device (or process) renders of a frame
   isize s_begin, s_end;
   int   split_rank, split_world;
 };
 
-// One render of `share` on device d, enqueued on `stream`.  Every render of a device uses the device's one workspace
-// and rewrites the scene's camera-relative copies, so renders are serialised on the device whatever stream they come
-// from: each waits for the event the previous one recorded.
+// One render of `share` on device d, enqueued on `stream`: a workspace user.
 int render_on_device(Device &d, const Scene *scene, isize width, isize height, const Share &share, isize max_bounces,
                      u32 seed, int accumulate, float *d_accum, float *d_per_sample, int *d_hit_ids,
-                     unsigned long long *d_counters, cudaStream_t stream, int slice_cap = 0) {
+                     unsigned long long *d_counters, cudaStream_t stream) {
   if (width < 1 || height < 1) return fail("render: empty image");
   CUDA_TRY(cudaSetDevice(d.id));
   auto it = d.scenes.find(scene);
   if (it == d.scenes.end()) return fail("render: scene is not resident on device %d", d.id);
   const DeviceScene &ds = it->second;
+  const isize n_samples = share.s_end - share.s_begin;
+  if (workspace_begin(d, ds, n_samples > 0 ? camera_workspace(width, height, n_samples, max_bounces, share.split_world)
+                                           : WorkspaceRequest{}, false, stream))
+    return 1;
   RenderParams p{};
   p.scene = ds.dev;
-  const int n_samples = (int)(share.s_end - share.s_begin);
-  const size_t want = rt_render_workspace_bytes((int)width, (int)height, n_samples, (int)max_bounces, slice_cap, share.split_world);
-  const size_t floor_bytes = rt_render_workspace_bytes((int)width, (int)height, 1, (int)max_bounces, 1, share.split_world);
-  if (n_samples > 0 && ensure_workspace(d, want, floor_bytes, stream)) return 1;
-  if (d.busy_valid) CUDA_TRY(cudaStreamWaitEvent(stream, d.busy, 0));
-  CUDA_TRY(cudaStreamWaitEvent(stream, ds.geom_ready, 0));
   p.shading_ready = ds.tex_ready;
   p.fast = g.options.fast_math != 0;
-  set_l2_window(d, ds, stream);
   p.width = (int)width; p.height = (int)height;
   p.split_rank = share.split_rank; p.split_world = share.split_world;
   p.sample_begin = (int)share.s_begin; p.sample_end = (int)share.s_end; p.max_bounces = (int)max_bounces;
@@ -177,11 +203,8 @@ int render_on_device(Device &d, const Scene *scene, isize width, isize height, c
   p.accum = d_accum; p.per_sample = d_per_sample; p.hit_ids = d_hit_ids;
   p.counters = d_counters;
   p.counters_ex = (d_counters && d_counters == d.d_counters) ? d_counters + 8 : nullptr;   // the library's own buffer has 16 slots
-  int e = rt_launch_render(p, d.sm_count, d.d_workspace, d.workspace_bytes, stream, &g.last_launches);
-  if (e) return fail("render kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
-  CUDA_TRY(cudaEventRecord(d.busy, stream));
-  d.busy_valid = true;
-  return 0;
+  return workspace_end(d, "render", rt_launch_render(p, d.sm_count, d.d_workspace, d.workspace_bytes, stream, &g.last_launches),
+                       stream);
 }
 
 int ensure_frame_buffers(Device &d, size_t n_pixels, bool hit_ids) {
@@ -335,9 +358,7 @@ int rt_gpu_prepare_frame(isize width, isize height, isize samples, isize max_bou
   if (slice > share) slice = share;
   for (Device &d : g.devs) {
     if (ensure_frame_buffers(d, (size_t)width * (size_t)height, g.options.keep_hit_ids != 0)) return 1;
-    const size_t want = rt_render_workspace_bytes((int)width, (int)height, (int)slice, (int)max_bounces, 0, world);
-    const size_t floor_bytes = rt_render_workspace_bytes((int)width, (int)height, 1, (int)max_bounces, 1, world);
-    if (ensure_workspace(d, want, floor_bytes, d.stream)) return 1;
+    if (ensure_workspace(d, camera_workspace(width, height, slice, max_bounces, world), d.stream)) return 1;
   }
   if (n_dev > 1 && g.options.reduce_mode == RT_GPU_REDUCE_NCCL && nccl_prepare()) return 1;
   CUDA_TRY(cudaSetDevice(g.devs[0].id));
@@ -438,6 +459,27 @@ int rt_gpu_denoise_device(u8 const *d_src, u8 *d_dst, isize width, isize height,
 
 namespace {
 
+// Staging of a host-memory call (queries, cast_rays, AOV) in the first device's staging block: part i gets bytes[i]
+// (0: none, NULL), every part 16-byte aligned.  The calls share the block: each runs on d.stream under g_mutex and
+// synchronises before it returns, and grow() frees the old block through cudaFree, which waits for the device.
+template <int N>
+int stage(Device &d, const size_t (&bytes)[N], void *(&parts)[N]) {
+  size_t offset[N], total = 0;
+  for (int i = 0; i < N; i++) { offset[i] = total; total += (bytes[i] + 15) & ~(size_t)15; }
+  if (grow(&d.d_stage, &d.stage_bytes, total)) return 1;
+  for (int i = 0; i < N; i++) parts[i] = bytes[i] ? static_cast<char *>(d.d_stage) + offset[i] : nullptr;
+  return 0;
+}
+
+// the tail of the cast_rays and AOV validations: afterwards the scene is resident (and current) on every device
+int scene_resident(const char *what, const Scene *scene) {
+  if (!scene) return fail("%s: null scene", what);
+  if (ensure_init()) return 1;
+  if (g.devs[0].scenes.find(scene) == g.devs[0].scenes.end())
+    return fail("%s: scene is not resident (rt_gpu_scene_upload it first)", what);
+  return scene_on_devices(scene);
+}
+
 int query_validate(const char *what, const Scene *scene, const void *rays, isize n_rays, const void *out, const void *hits) {
   if (n_rays < 0 || n_rays > INT32_MAX) return fail("%s: n_rays = %lld, must be in [0, INT32_MAX]", what, (long long)n_rays);
   if (n_rays == 0) return 0;
@@ -502,21 +544,16 @@ int query_host_call(const char *what, const Scene *scene, const Ray *rays, const
   if (scene_on_devices(scene)) return 1;
   Device &d = g.devs[0];
   CUDA_TRY(cudaSetDevice(d.id));
-  // staging layout, every part 16-byte aligned: hits | surface | rays | t_max | occluded
   const size_t n = (size_t)n_rays;
-  auto up16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
-  const size_t o_surface = up16(any ? 0 : n * sizeof(RT_GPU_Hit));
-  const size_t o_rays = o_surface + up16(surface && !any ? n * sizeof(RT_GPU_Surface) : 0);
-  const size_t o_t_max = o_rays + up16(n * sizeof(Ray));
-  const size_t o_occluded = o_t_max + up16(t_max ? n * sizeof(f32) : 0);
-  const size_t total = o_occluded + up16(any ? n : 0);
-  if (grow(&d.d_query_stage, &d.query_stage_bytes, total)) return 1;
-  char *base = static_cast<char *>(d.d_query_stage);
-  RT_GPU_Hit *d_hits = any ? nullptr : reinterpret_cast<RT_GPU_Hit *>(base);
-  RT_GPU_Surface *d_surface = surface && !any ? reinterpret_cast<RT_GPU_Surface *>(base + o_surface) : nullptr;
-  Ray *d_rays = reinterpret_cast<Ray *>(base + o_rays);
-  f32 *d_t_max = t_max ? reinterpret_cast<f32 *>(base + o_t_max) : nullptr;
-  u8 *d_occluded = any ? reinterpret_cast<u8 *>(base + o_occluded) : nullptr;
+  void *part[5];
+  if (stage(d, {any ? 0 : n * sizeof(RT_GPU_Hit), surface && !any ? n * sizeof(RT_GPU_Surface) : 0, n * sizeof(Ray),
+                t_max ? n * sizeof(f32) : 0, any ? n : 0}, part))
+    return 1;
+  RT_GPU_Hit *d_hits = static_cast<RT_GPU_Hit *>(part[0]);
+  RT_GPU_Surface *d_surface = static_cast<RT_GPU_Surface *>(part[1]);
+  Ray *d_rays = static_cast<Ray *>(part[2]);
+  f32 *d_t_max = static_cast<f32 *>(part[3]);
+  u8 *d_occluded = static_cast<u8 *>(part[4]);
   CUDA_TRY(cudaMemcpyAsync(d_rays, rays, n * sizeof(Ray), cudaMemcpyHostToDevice, d.stream));
   if (t_max) CUDA_TRY(cudaMemcpyAsync(d_t_max, t_max, n * sizeof(f32), cudaMemcpyHostToDevice, d.stream));
   if (query_on_device(scene, d_rays, d_t_max, n_rays, any, d_hits, d_surface, d_occluded, nullptr, d.stream)) return 1;
@@ -569,16 +606,11 @@ int cast_rays_validate(const char *what, const Scene *scene, const void *rays, i
   if (n_rays == 0) return 0;
   if (!rays) return fail("%s: null rays", what);
   if (!radiance) return fail("%s: null radiance", what);
-  if (!scene) return fail("%s: null scene", what);
-  if (ensure_init()) return 1;
-  if (g.devs[0].scenes.find(scene) == g.devs[0].scenes.end())
-    return fail("%s: scene is not resident (rt_gpu_scene_upload it first)", what);
-  return scene_on_devices(scene);
+  return scene_resident(what, scene);
 }
 
-// One cast_rays call on the first device, ordered on `stream`.  It uses the device's path-queue workspace, so like a
-// render it waits for the previous user of the workspace (busy) and records busy after its last kernel; it shades, so
-// it waits for the scene's texels as well as its geometry.
+// One cast_rays call on the first device, ordered on `stream`: a workspace user that shades, so it waits for the
+// scene's texels as well as its geometry.
 int cast_rays_on_device(const Scene *scene, const Ray *rays, const u32 *keys, isize n_rays, isize sample_begin, isize samples,
                         isize max_bounces, u32 user_seed, int accumulate, float *radiance, float *per_sample,
                         unsigned long long *counters, cudaStream_t stream) {
@@ -586,20 +618,14 @@ int cast_rays_on_device(const Scene *scene, const Ray *rays, const u32 *keys, is
   CUDA_TRY(cudaSetDevice(d.id));
   const DeviceScene &ds = d.scenes.find(scene)->second;
   const size_t n_paths = (size_t)n_rays * (size_t)samples;
-  if (n_paths > 0 && ensure_workspace(d, rt_cast_rays_workspace_bytes(n_paths, (int)max_bounces, false),
-                                      rt_cast_rays_workspace_bytes(n_paths, (int)max_bounces, true), stream))
-    return 1;
-  if (d.busy_valid) CUDA_TRY(cudaStreamWaitEvent(stream, d.busy, 0));
-  CUDA_TRY(cudaStreamWaitEvent(stream, ds.geom_ready, 0));
-  CUDA_TRY(cudaStreamWaitEvent(stream, ds.tex_ready, 0));
-  set_l2_window(d, ds, stream);
+  WorkspaceRequest r;
+  if (n_paths > 0)
+    r = {rt_cast_rays_workspace_bytes(n_paths, (int)max_bounces, false), rt_cast_rays_workspace_bytes(n_paths, (int)max_bounces, true)};
+  if (workspace_begin(d, ds, r, true, stream)) return 1;
   int e = rt_launch_cast_rays(ds.dev, reinterpret_cast<const float *>(rays), keys, (int)n_rays, (int)sample_begin,
                               (int)samples, (int)max_bounces, user_seed, accumulate, radiance, per_sample, counters,
                               d.sm_count, d.d_workspace, d.workspace_bytes, stream, &g.last_launches);
-  if (e) return fail("cast_rays kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
-  CUDA_TRY(cudaEventRecord(d.busy, stream));
-  d.busy_valid = true;
-  return 0;
+  return workspace_end(d, "cast_rays", e, stream);
 }
 
 }  // namespace
@@ -627,21 +653,15 @@ int rt_gpu_cast_rays(Scene const *scene, Ray const *rays, u32 const *keys, isize
   if (n_rays == 0) return 0;
   Device &d = g.devs[0];
   CUDA_TRY(cudaSetDevice(d.id));
-  // staging layout, every part 16-byte aligned: radiance | per_sample | rays | keys
   const size_t n = (size_t)n_rays;
-  auto up16 = [](size_t b) { return (b + 15) & ~(size_t)15; };
   const size_t sums_bytes = n * 3 * sizeof(float);
   const size_t per_sample_bytes = per_sample ? n * (size_t)samples * 3 * sizeof(float) : 0;
-  const size_t o_per_sample = up16(sums_bytes);
-  const size_t o_rays = o_per_sample + up16(per_sample_bytes);
-  const size_t o_keys = o_rays + up16(n * sizeof(Ray));
-  const size_t total = o_keys + up16(keys ? n * sizeof(u32) : 0);
-  if (grow(&d.d_cast_stage, &d.cast_stage_bytes, total)) return 1;
-  char *base = static_cast<char *>(d.d_cast_stage);
-  float *d_radiance = reinterpret_cast<float *>(base);
-  float *d_per_sample = per_sample ? reinterpret_cast<float *>(base + o_per_sample) : nullptr;
-  Ray *d_rays = reinterpret_cast<Ray *>(base + o_rays);
-  u32 *d_keys = keys ? reinterpret_cast<u32 *>(base + o_keys) : nullptr;
+  void *part[4];
+  if (stage(d, {sums_bytes, per_sample_bytes, n * sizeof(Ray), keys ? n * sizeof(u32) : 0}, part)) return 1;
+  float *d_radiance = static_cast<float *>(part[0]);
+  float *d_per_sample = static_cast<float *>(part[1]);
+  Ray *d_rays = static_cast<Ray *>(part[2]);
+  u32 *d_keys = static_cast<u32 *>(part[3]);
   CUDA_TRY(cudaMemcpyAsync(d_rays, rays, n * sizeof(Ray), cudaMemcpyHostToDevice, d.stream));
   if (keys) CUDA_TRY(cudaMemcpyAsync(d_keys, keys, n * sizeof(u32), cudaMemcpyHostToDevice, d.stream));
   if (accumulate) CUDA_TRY(cudaMemcpyAsync(d_radiance, radiance, sums_bytes, cudaMemcpyHostToDevice, d.stream));
@@ -673,36 +693,23 @@ int aov_validate(const char *what, const Scene *scene, isize width, isize height
                 (long long)sample_end);
   if (max_bounces < 0 || max_bounces > INT32_MAX) return fail("%s: max_bounces = %lld, must be >= 0", what, (long long)max_bounces);
   if (!aov) return fail("%s: null aov", what);
-  if (!scene) return fail("%s: null scene", what);
-  if (ensure_init()) return 1;
-  if (g.devs[0].scenes.find(scene) == g.devs[0].scenes.end())
-    return fail("%s: scene is not resident (rt_gpu_scene_upload it first)", what);
-  return scene_on_devices(scene);
+  return scene_resident(what, scene);
 }
 
-// One AOV call on the first device, ordered on `stream`.  Like a render it uses the device's path-queue workspace and
-// rewrites the camera-relative copies, so it waits for the previous user of both (busy) and records busy after its last
-// kernel; it reads texels, so it waits for the scene's texels as well as its geometry.
+// One AOV call on the first device, ordered on `stream`: a workspace user that rewrites the camera-relative copies as
+// a render does, and reads texels, so it waits for the scene's texels as well as its geometry.
 int aov_on_device(const Scene *scene, isize width, isize height, isize sample_begin, isize sample_end, isize max_bounces,
                   int accumulate, float *aov, unsigned long long *counters, cudaStream_t stream) {
   Device &d = g.devs[0];
   CUDA_TRY(cudaSetDevice(d.id));
   const DeviceScene &ds = d.scenes.find(scene)->second;
-  const int n_samples = (int)(sample_end - sample_begin);
-  if (n_samples > 0 && max_bounces > 0 &&
-      ensure_workspace(d, rt_render_workspace_bytes((int)width, (int)height, n_samples, (int)max_bounces, 0, 1),
-                       rt_render_workspace_bytes((int)width, (int)height, 1, (int)max_bounces, 1, 1), stream))
+  const isize n_samples = sample_end - sample_begin;
+  if (workspace_begin(d, ds, n_samples > 0 && max_bounces > 0 ? camera_workspace(width, height, n_samples, max_bounces, 1)
+                                                              : WorkspaceRequest{}, true, stream))
     return 1;
-  if (d.busy_valid) CUDA_TRY(cudaStreamWaitEvent(stream, d.busy, 0));
-  CUDA_TRY(cudaStreamWaitEvent(stream, ds.geom_ready, 0));
-  CUDA_TRY(cudaStreamWaitEvent(stream, ds.tex_ready, 0));
-  set_l2_window(d, ds, stream);
   int e = rt_launch_aov(ds.dev, (int)width, (int)height, (int)sample_begin, (int)sample_end, (int)max_bounces, accumulate,
                         aov, counters, d.sm_count, d.d_workspace, d.workspace_bytes, stream, &g.last_launches);
-  if (e) return fail("aov kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
-  CUDA_TRY(cudaEventRecord(d.busy, stream));
-  d.busy_valid = true;
-  return 0;
+  return workspace_end(d, "aov", e, stream);
 }
 
 }  // namespace
@@ -719,7 +726,7 @@ int rt_gpu_render_aov_device(Scene const *scene, isize width, isize height, isiz
                        static_cast<cudaStream_t>(stream));
 }
 
-// Host memory: the records go through the first device's AOV staging block and come back; synchronises.
+// Host memory: the records go through the first device's staging block and come back; synchronises.
 int rt_gpu_render_aov(Scene const *scene, isize width, isize height, isize sample_begin, isize sample_end,
                       isize max_bounces, RT_GPU_AOV *aov) {
   std::lock_guard<std::mutex> lock(g_mutex);
@@ -728,8 +735,9 @@ int rt_gpu_render_aov(Scene const *scene, isize width, isize height, isize sampl
   Device &d = g.devs[0];
   CUDA_TRY(cudaSetDevice(d.id));
   const size_t bytes = (size_t)width * (size_t)height * sizeof(RT_GPU_AOV);
-  if (grow(&d.d_aov_stage, &d.aov_stage_bytes, bytes)) return 1;
-  float *d_aov = static_cast<float *>(d.d_aov_stage);
+  void *part[1];
+  if (stage(d, {bytes}, part)) return 1;
+  float *d_aov = static_cast<float *>(part[0]);
   if (aov_on_device(scene, width, height, sample_begin, sample_end, max_bounces, 0, d_aov, nullptr, d.stream)) return 1;
   CUDA_TRY(cudaMemcpyAsync(aov, d_aov, bytes, cudaMemcpyDeviceToHost, d.stream));
   CUDA_TRY(cudaStreamSynchronize(d.stream));
@@ -954,9 +962,7 @@ static int render_owner(Rendering_Context *ctx, isize n_chunks) {
     const isize n = sh.s_end - sh.s_begin < slice ? sh.s_end - sh.s_begin : slice;
     if (n <= 0) continue;
     CUDA_TRY(cudaSetDevice(d.id));
-    const size_t want = rt_render_workspace_bytes((int)im.width, (int)im.height, (int)n, (int)ctx->max_bounces, 0, sh.split_world);
-    const size_t floor_bytes = rt_render_workspace_bytes((int)im.width, (int)im.height, 1, (int)ctx->max_bounces, 1, sh.split_world);
-    if (ensure_workspace(d, want, floor_bytes, d.stream)) return 1;
+    if (ensure_workspace(d, camera_workspace(im.width, im.height, n, ctx->max_bounces, sh.split_world), d.stream)) return 1;
   }
   // slices round-robin over the devices, so the host's progress bar (driver.c:810-818) follows all of them
   for (size_t k = 0; k < n_dev; k++) {
@@ -1111,17 +1117,9 @@ int rt_gpu_lightmap_bake(Image const *lightmap, Scene const *scene, isize sample
   char *scratch = static_cast<char *>(d.d_texel_stage);
   float *d_values = values_out ? reinterpret_cast<float *>(scratch + rt_lightmap_workspace_bytes(W, H)) : nullptr;
   int *d_owner = owner_out ? reinterpret_cast<int *>(scratch + rt_lightmap_workspace_bytes(W, H) + (values_out ? n_texels * 3 * sizeof(float) : 0)) : nullptr;
-  // path queues: at most one chunk's worth, at least one sample of every texel
-  const size_t per_path = rt_render_workspace_bytes(8, 4, 1, max_bounces, 1, 1) / 32 + sizeof(float) + 16;
-  size_t paths = n_texels * (size_t)samples;
-  const size_t chunk_paths = (size_t)rt_render_chunk_samples(8, 4, 1) * 32;
-  if (paths > chunk_paths) paths = chunk_paths;
-  if (paths < n_texels) paths = n_texels;
-  if (ensure_workspace(d, paths * per_path + 4096, n_texels * per_path + 4096, d.stream)) return 1;
-
-  if (d.busy_valid) CUDA_TRY(cudaStreamWaitEvent(d.stream, d.busy, 0));
-  CUDA_TRY(cudaStreamWaitEvent(d.stream, ds.geom_ready, 0));
-  CUDA_TRY(cudaStreamWaitEvent(d.stream, ds.tex_ready, 0));
+  const WorkspaceRequest r{rt_lightmap_paths_workspace_bytes(n_texels, (int)samples, max_bounces, false),
+                           rt_lightmap_paths_workspace_bytes(n_texels, (int)samples, max_bounces, true)};
+  if (workspace_begin(d, ds, r, true, d.stream)) return 1;
   memcpy(d.h_pinned, lightmap->pixels.data, image_bytes);            // untouched texels keep their bytes
   CUDA_TRY(cudaMemcpyAsync(d.d_image, d.h_pinned, image_bytes, cudaMemcpyHostToDevice, d.stream));
   if (d_values) CUDA_TRY(cudaMemsetAsync(d_values, 0, n_texels * 3 * sizeof(float), d.stream));
@@ -1129,9 +1127,7 @@ int rt_gpu_lightmap_bake(Image const *lightmap, Scene const *scene, isize sample
   int e = rt_launch_lightmap(ds.dev, W, H, (int)samples, max_bounces, g.options.user_seed, d.d_image, (int)lightmap->stride,
                              lightmap->components, d_values, d_owner, scratch, d.sm_count, d.d_workspace, d.workspace_bytes,
                              d.stream, &g.last_launches, &n_jobs);
-  if (e) return fail("lightmap kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
-  CUDA_TRY(cudaEventRecord(d.busy, d.stream));
-  d.busy_valid = true;
+  if (workspace_end(d, "lightmap", e, d.stream)) return 1;
   CUDA_TRY(cudaMemcpyAsync(d.h_pinned, d.d_image, image_bytes, cudaMemcpyDeviceToHost, d.stream));
   CUDA_TRY(cudaStreamSynchronize(d.stream));
   memcpy(lightmap->pixels.data, d.h_pinned, image_bytes);

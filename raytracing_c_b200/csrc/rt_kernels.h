@@ -7,13 +7,16 @@
 
 // wavefront render of samples [p.sample_begin, p.sample_end) into p.accum; `workspace` holds the path queues
 // (rt_render_workspace_bytes; a smaller one only means more, smaller chunks).  *n_launches += kernels launched.
-size_t rt_render_workspace_bytes(int width, int height, int n_samples, int max_bounces, int slice_samples, int split_world);
+size_t rt_render_workspace_bytes(int width, int height, int n_samples, int max_bounces, int split_world);
 int rt_render_chunk_samples(int width, int height, int split_world);
 unsigned rt_render_tiles(int width, int height, int split_rank, int split_world);
 int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_t workspace_bytes,
                      cudaStream_t stream, int *n_launches);
-// lightmap_bake (raytracer.c:722-784) on the wavefront: see rt_render.cu
+// lightmap_bake (raytracer.c:722-784) on the wavefront: see rt_render.cu.  `scratch` holds rt_lightmap_workspace_bytes,
+// `workspace` the path queues: rt_lightmap_paths_workspace_bytes for n_texels * samples paths at the preferred chunk
+// size, or with `floor` the smallest one the bake asks for (one sample of every texel)
 size_t rt_lightmap_workspace_bytes(int width, int height);
+size_t rt_lightmap_paths_workspace_bytes(size_t n_texels, int samples, int max_bounces, bool floor);
 int rt_launch_lightmap(const SceneDev &scene, int width, int height, int samples, int max_bounces, uint32_t user_seed,
                        unsigned char *d_pixels, int stride, int components, float *d_values, int *d_owner_out,
                        void *scratch, int sm_count, void *workspace, size_t workspace_bytes, cudaStream_t stream,

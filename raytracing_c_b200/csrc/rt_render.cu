@@ -174,8 +174,9 @@ rt_reduce_resolve_kernel(const ReduceParts parts, float *__restrict__ sum_out, i
 #define RT_CHUNK_PATHS_MAX (512u << 20)
 #define RT_CAST_RAYS_MIN_CHUNK (1u << 16)                      // paths of the smallest workspace a cast_rays call accepts
 
+// queue lengths of bounces 0 .. max_bounces (at least one bounce's worth)
 static size_t counts_bytes(int max_bounces) {
-  size_t b = (size_t)(max_bounces + 1) * Q_STRIDE * sizeof(unsigned);
+  size_t b = (size_t)((max_bounces > 0 ? max_bounces : 1) + 1) * Q_STRIDE * sizeof(unsigned);
   return (b + 255) & ~(size_t)255;
 }
 
@@ -194,13 +195,18 @@ static size_t chunk_paths_max() {
   return RT_CHUNK_PATHS_MAX;
 }
 
-// samples of every pixel per chunk
-static size_t chunk_samples(size_t per_sample, int n_samples, int slice_samples) {
+// samples of every pixel per chunk (n_samples > 0: at most that many)
+static size_t chunk_samples(size_t per_sample, int n_samples) {
   size_t s = chunk_paths_max() / per_sample;
   if (s < 1) s = 1;
-  if (slice_samples > 0 && s > (size_t)slice_samples) s = (size_t)slice_samples;
   if (n_samples > 0 && s > (size_t)n_samples) s = (size_t)n_samples;
   return s;
+}
+
+// paths a workspace holds past its queue lengths, at per_path bytes each
+static size_t path_capacity(size_t workspace_bytes, int max_bounces, size_t per_path) {
+  const size_t cb = counts_bytes(max_bounces);
+  return workspace_bytes < cb ? 0 : (workspace_bytes - cb) / per_path;
 }
 
 // job tiles (8x4 pixels) one render covers: the whole image, or the 32x32 chunks congruent to split_rank
@@ -215,19 +221,22 @@ unsigned rt_render_tiles(int width, int height, int split_rank, int split_world)
 int rt_render_chunk_samples(int width, int height, int split_world) {
   size_t per_sample = (size_t)rt_render_tiles(width, height, 0, split_world) * 32;
   if (per_sample < 32) per_sample = 32;
-  return (int)chunk_samples(per_sample, 0, 0);
+  return (int)chunk_samples(per_sample, 0);
 }
 
-size_t rt_render_workspace_bytes(int width, int height, int n_samples, int max_bounces, int slice_samples, int split_world) {
+size_t rt_render_workspace_bytes(int width, int height, int n_samples, int max_bounces, int split_world) {
   size_t per_sample = (size_t)rt_render_tiles(width, height, 0, split_world) * 32;
   if (per_sample < 32) per_sample = 32;
-  return counts_bytes(max_bounces > 0 ? max_bounces : 1) +
-         chunk_samples(per_sample, n_samples, slice_samples) * per_sample * RT_PATH_BYTES;
+  return counts_bytes(max_bounces) + chunk_samples(per_sample, n_samples) * per_sample * RT_PATH_BYTES;
 }
 
-// occupancy of the trace kernel and its dynamic-shared-memory opt-in, per device (cudaFuncSetAttribute is per device)
-static int g_trace_blocks_per_sm[RT_MAX_DEVICES], g_wide_blocks_per_sm[RT_MAX_DEVICES], g_primary_blocks_per_sm[RT_MAX_DEVICES], g_fast_blocks_per_sm[RT_MAX_DEVICES], g_fast_wide_blocks_per_sm[RT_MAX_DEVICES];
-static size_t g_level_bytes[RT_MAX_DEVICES];
+// trace kernels' blocks per SM at the level-store size they were measured for, per device (cudaFuncSetAttribute is per device)
+struct TraceOccupancy { size_t level_bytes; int primary, generic, wide, fast, fast_wide; };
+static TraceOccupancy g_occupancy[RT_MAX_DEVICES];
+
+// what a launcher needs of trace_launch_setup: the device, the level store, and the trace kernels' persistent grids
+// (one wave: blocks per SM x SMs)
+struct TraceLaunch { int dev; size_t level_bytes; unsigned primary, generic, wide, fast, fast_wide; };
 
 // ---- optional per-stage timing (bench.py's roofline leg): CUDA events around every launch, on the
 // launching stream; read back and summed by rt_stage_profile_read
@@ -274,15 +283,33 @@ int rt_stage_profile_read(double ms[RT_N_STAGES * RT_STAGE_BOUNCES], long long l
   return 0;
 }
 
-static void bind_queues(PathQueues &q, char *w, size_t cb, size_t cap) {
-  q.counts = reinterpret_cast<unsigned *>(w); w += cb;
+// the queue lengths, then eight arrays of `paths` records; returns the end of the last array
+static char *bind_queues(PathQueues &q, void *workspace, int max_bounces, size_t paths) {
+  char *w = static_cast<char *>(workspace);
+  q.counts = reinterpret_cast<unsigned *>(w); w += counts_bytes(max_bounces);
   float4 **arrays[] = { &q.ray_a, &q.ray_b, &q.hit_a, &q.hit_b, &q.hit_h, &q.miss_a, &q.tint, &q.emis };
-  for (float4 **a : arrays) { *a = reinterpret_cast<float4 *>(w); w += cap * sizeof(float4); }
+  for (float4 **a : arrays) { *a = reinterpret_cast<float4 *>(w); w += paths * sizeof(float4); }
   q.rad = q.emis;
+  return w;
+}
+
+// Chunk fitting of a call that runs paths_per_sample paths per sample and n_samples samples: as many samples per chunk
+// as the preferred chunk size and the workspace allow, each path taking RT_PATH_BYTES + extra_bytes.  Binds the queues
+// for one chunk, points *extra (if given) at the chunk's extra bytes, and returns the samples per chunk, or 0 when one
+// sample does not fit.
+static int fit_chunk(StageParams &P, size_t paths_per_sample, int n_samples, size_t extra_bytes, void *workspace,
+                     size_t workspace_bytes, char **extra) {
+  const size_t cap = path_capacity(workspace_bytes, P.max_bounces, RT_PATH_BYTES + extra_bytes);
+  if (cap < paths_per_sample) return 0;
+  size_t fit = chunk_samples(paths_per_sample, n_samples);
+  if (fit > cap / paths_per_sample) fit = cap / paths_per_sample;
+  char *end = bind_queues(P.q, workspace, P.max_bounces, fit * paths_per_sample);
+  if (extra) *extra = end;
+  return (int)fit;
 }
 
 // Dynamic shared memory opt-in and occupancy of the trace kernels on the current device (once per device and depth).
-static int trace_launch_setup(const SceneDev &scene, int *dev_out, size_t *level_bytes_out) {
+static int trace_launch_setup(const SceneDev &scene, int sm_count, TraceLaunch &t) {
   // level store: [depth - 1][2][RT_BLOCK] float4 of dynamic shared memory (see rt_trace.cuh)
   // (levels 2 .. depth only: 24 KB per block for the depth-4 trees of the shipped models; the driver's default carve-out is the
   // smallest that holds the resident blocks — forcing a larger one costs up to 6 %, L1 beyond 96 KB gains nothing: measured)
@@ -290,23 +317,66 @@ static int trace_launch_setup(const SceneDev &scene, int *dev_out, size_t *level
   int dev = 0;
   cudaGetDevice(&dev);
   if (dev < 0 || dev >= RT_MAX_DEVICES) return (int)cudaErrorInvalidDevice;
-  if (g_trace_blocks_per_sm[dev] == 0 || level_bytes != g_level_bytes[dev]) {
-    int n = 0;
-    cudaFuncSetAttribute(rt_trace_kernel<true>,  cudaFuncAttributeMaxDynamicSharedMemorySize, RT_MAX_DEPTH * 2 * RT_BLOCK * 16);
-    cudaFuncSetAttribute(rt_trace_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_MAX_DEPTH * 2 * RT_BLOCK * 16);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, rt_trace_kernel<false>, RT_BLOCK, level_bytes) != cudaSuccess || n < 1) n = 1;
-    g_trace_blocks_per_sm[dev] = n;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, rt_trace_kernel<true>, RT_BLOCK, level_bytes) != cudaSuccess || n < 1) n = 1;
-    g_primary_blocks_per_sm[dev] = n;
-    cudaFuncSetAttribute(rt_trace_kernel<false, RT_TRACE_MIN_BLOCKS_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_MAX_DEPTH * 2 * RT_BLOCK * 16);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, rt_trace_kernel<false, RT_TRACE_MIN_BLOCKS_WIDE>, RT_BLOCK, level_bytes) != cudaSuccess || n < 1) n = 1;
-    g_wide_blocks_per_sm[dev] = n;
-    g_fast_blocks_per_sm[dev] = rt_fast_trace_setup(level_bytes, &g_fast_wide_blocks_per_sm[dev]);
-    g_level_bytes[dev] = level_bytes;
+  TraceOccupancy &o = g_occupancy[dev];
+  if (o.generic == 0 || level_bytes != o.level_bytes) {
+    auto blocks_per_sm = [&](const void *kernel) {
+      int n = 0;
+      cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_MAX_DEPTH * 2 * RT_BLOCK * 16);
+      return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel, RT_BLOCK, level_bytes) == cudaSuccess && n >= 1 ? n : 1;
+    };
+    o.primary = blocks_per_sm((const void *)rt_trace_kernel<true>);
+    o.generic = blocks_per_sm((const void *)rt_trace_kernel<false>);
+    o.wide = blocks_per_sm((const void *)rt_trace_kernel<false, RT_TRACE_MIN_BLOCKS_WIDE>);
+    o.fast = rt_fast_trace_setup(level_bytes, &o.fast_wide);
+    o.level_bytes = level_bytes;
   }
-  *dev_out = dev;
-  *level_bytes_out = level_bytes;
+  t = TraceLaunch{dev, level_bytes, (unsigned)(sm_count * o.primary), (unsigned)(sm_count * o.generic),
+                  (unsigned)(sm_count * o.wide), (unsigned)(sm_count * o.fast), (unsigned)(sm_count * o.fast_wide)};
   return 0;
+}
+
+// grid-stride kernels (miss, shade, accumulate): blocks per SM by queue length.  The items of a queue cost unevenly
+// (texture taps, lobe picks), so the long queues of the first bounces want many short-lived blocks to even out the
+// last wave (bounce-0 miss 2073 / 1950 / 1889 / 1864 / 1856 us at 8 / 16 / 32 / 64 / 128 blocks per SM), the short late
+// queues want few (every block builds its texel table first: bounce-7 shade 23 / 31 / 41 us at 8 / 64 / 128).
+static unsigned flat_grid(int sm_count) { return (unsigned)(sm_count * 8); }
+static unsigned miss_grid(int sm_count, int b) { return (unsigned)sm_count * (b == 0 ? 64u : b == 1 ? 32u : 8u); }
+static unsigned shade_grid(int sm_count, int b) { return (unsigned)sm_count * (b == 0 ? 64u : 8u); }
+
+// the trace of bounce P.bounce's RAY queue, exact or fast: the wide build for the long queues of the first bounces, the
+// generic one after.  The lightmap bake launches its own (the generic build at every bounce).
+static void launch_bounce_trace(const StageParams &P, const TraceLaunch &t, bool fast, cudaStream_t stream) {
+  const bool wide = P.bounce <= RT_TRACE_WIDE_BOUNCES;
+  if (fast)      rt_fast_launch_trace(P, wide ? t.fast_wide : t.fast, t.level_bytes, stream, wide);
+  else if (wide) rt_trace_kernel<false, RT_TRACE_MIN_BLOCKS_WIDE><<<t.wide, RT_BLOCK, t.level_bytes, stream>>>(P);
+  else           rt_trace_kernel<false><<<t.generic, RT_BLOCK, t.level_bytes, stream>>>(P);
+}
+
+// The camera frame of a render or AOV call: job tiles, the split's share of them, fastdiv magic.
+static StageParams camera_frame(const SceneDev &scene, int width, int height, int split_rank, int split_world, int max_bounces) {
+  StageParams P{};
+  P.scene = scene;
+  P.width = width; P.height = height;
+  P.tiles_x = (width + 7) / 8; P.tiles_y = (height + 3) / 4;
+  P.split_rank = split_rank; P.split_world = split_world > 1 ? split_world : 1;
+  P.chunks_x = (width + 31) / 32;
+  P.n_tiles = rt_render_tiles(width, height, P.split_rank, P.split_world);
+  // a path id is at most n_paths (32-bit), so a tile id is below 2^27 and a chunk id below tiles/32 * world + world
+  P.div_tiles_x = rt_fastdiv_make((uint32_t)P.tiles_x, 0xffffffffu >> 5);
+  P.div_chunks_x = rt_fastdiv_make((uint32_t)P.chunks_x, 0xffffffffu);
+  P.max_bounces = max_bounces;
+  return P;
+}
+
+// The header of a camera-path chunk: samples [s0, s0 + chunk) clipped to sample_end of every pixel, the accumulator
+// continued or not, empty queues.
+static void camera_chunk(StageParams &P, int s0, int sample_end, int chunk, bool continues, cudaStream_t stream) {
+  const int S = (sample_end - s0 < chunk) ? sample_end - s0 : chunk;
+  P.sample0 = s0; P.n_samples = S;
+  P.n_paths = (unsigned)((size_t)P.n_tiles * 32 * (size_t)S);
+  P.div_samples = rt_fastdiv_make((uint32_t)S, P.n_paths);
+  P.accumulate = continues ? 1 : 0;
+  cudaMemsetAsync(P.q.counts, 0, counts_bytes(P.max_bounces), stream);
 }
 
 int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_t workspace_bytes,
@@ -317,21 +387,10 @@ int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_
     if (!p.accumulate) cudaMemsetAsync(p.accum, 0, (size_t)p.width * p.height * 3 * sizeof(float), stream);
     return (int)cudaGetLastError();
   }
-  size_t level_bytes = 0;
-  int dev = 0;
-  if (int e = trace_launch_setup(p.scene, &dev, &level_bytes)) return e;
+  TraceLaunch t;
+  if (int e = trace_launch_setup(p.scene, sm_count, t)) return e;
 
-  StageParams P{};
-  P.scene = p.scene;
-  P.width = p.width; P.height = p.height;
-  P.tiles_x = (p.width + 7) / 8; P.tiles_y = (p.height + 3) / 4;
-  P.split_rank = p.split_rank; P.split_world = p.split_world > 1 ? p.split_world : 1;
-  P.chunks_x = (p.width + 31) / 32;
-  P.n_tiles = rt_render_tiles(p.width, p.height, P.split_rank, P.split_world);
-  // a path id is at most n_paths (32-bit), so a tile id is below 2^27 and a chunk id below tiles/32 * world + world
-  P.div_tiles_x = rt_fastdiv_make((uint32_t)P.tiles_x, 0xffffffffu >> 5);
-  P.div_chunks_x = rt_fastdiv_make((uint32_t)P.chunks_x, 0xffffffffu);
-  P.max_bounces = p.max_bounces;
+  StageParams P = camera_frame(p.scene, p.width, p.height, p.split_rank, p.split_world, p.max_bounces);
   P.user_seed = p.user_seed;
   P.accum = p.accum;
   P.per_sample = p.per_sample;
@@ -341,43 +400,20 @@ int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_
 
   // chunking: as many samples of every pixel per chunk as the workspace holds paths
   const size_t per_sample = (size_t)P.n_tiles * 32;
-  const size_t cb = counts_bytes(p.max_bounces);
   if (P.split_world > 1 && !p.accumulate)      // the pixels of other ranks stay zero (the cross-rank sum adds them)
     cudaMemsetAsync(p.accum, 0, (size_t)p.width * p.height * 3 * sizeof(float), stream);
   if (per_sample == 0) return (int)cudaGetLastError();
-  if (workspace_bytes < cb + per_sample * RT_PATH_BYTES) return (int)cudaErrorMemoryAllocation;
-  size_t cap = (workspace_bytes - cb) / RT_PATH_BYTES;
-  size_t fit = chunk_samples(per_sample, n_total, 0);
-  if (fit > cap / per_sample) fit = cap / per_sample;
-  const int chunk = (int)fit;
-  cap = (size_t)chunk * per_sample;
-  bind_queues(P.q, static_cast<char *>(workspace), cb, cap);
+  const int chunk = fit_chunk(P, per_sample, n_total, 0, workspace, workspace_bytes, nullptr);
+  if (chunk == 0) return (int)cudaErrorMemoryAllocation;
 
   rt_camera_relative_kernel<<<(unsigned)sm_count, 256, 0, stream>>>(p.scene);
-  const unsigned trace_grid = (unsigned)(sm_count * g_trace_blocks_per_sm[dev]);     // persistent: one wave
-  const unsigned wide_grid = (unsigned)(sm_count * g_wide_blocks_per_sm[dev]);
-  const unsigned primary_grid = (unsigned)(sm_count * g_primary_blocks_per_sm[dev]);
-  const unsigned fast_grid = (unsigned)(sm_count * g_fast_blocks_per_sm[dev]);
-  const unsigned fast_wide_grid = (unsigned)(sm_count * g_fast_wide_blocks_per_sm[dev]);
-  // grid-stride kernels (miss, shade, accumulate): blocks per SM by queue length.  The items of a queue cost unevenly
-  // (texture taps, lobe picks), so the long queues of the first bounces want many short-lived blocks to even out the
-  // last wave (bounce-0 miss 2073 / 1950 / 1889 / 1864 / 1856 us at 8 / 16 / 32 / 64 / 128 blocks per SM), the short late
-  // queues want few (every block builds its texel table first: bounce-7 shade 23 / 31 / 41 us at 8 / 64 / 128).
-  const unsigned flat_grid  = (unsigned)(sm_count * 8);
-  auto miss_grid  = [&](int b) { return (unsigned)sm_count * (b == 0 ? 64u : b == 1 ? 32u : 8u); };
-  auto shade_grid = [&](int b) { return (unsigned)sm_count * (b == 0 ? 64u : 8u); };
   int launches = 1;
   for (int s0 = p.sample_begin; s0 < p.sample_end; s0 += chunk) {
-    const int S = (p.sample_end - s0 < chunk) ? p.sample_end - s0 : chunk;
-    P.sample0 = s0; P.n_samples = S;
-    P.n_paths = (unsigned)(per_sample * (size_t)S);
-    P.div_samples = rt_fastdiv_make((uint32_t)S, P.n_paths);
-    P.accumulate = (p.accumulate || s0 > p.sample_begin || P.split_world > 1) ? 1 : 0;
     P.per_sample_offset = s0 - p.sample_begin;
     P.hit_ids = (s0 == p.sample_begin) ? p.hit_ids : nullptr;
-    cudaMemsetAsync(P.q.counts, 0, cb, stream);
+    camera_chunk(P, s0, p.sample_end, chunk, p.accumulate || s0 > p.sample_begin || P.split_world > 1, stream);
     P.bounce = 0;
-    { StageTimer t(RT_STAGE_TRACE * RT_STAGE_BOUNCES, stream, dev); rt_trace_kernel<true><<<primary_grid, RT_BLOCK, level_bytes, stream>>>(P); }
+    { StageTimer st(RT_STAGE_TRACE * RT_STAGE_BOUNCES, stream, t.dev); rt_trace_kernel<true><<<t.primary, RT_BLOCK, t.level_bytes, stream>>>(P); }
     launches++;
     // textures and the environment may still be in flight on the upload's copy stream: the primary trace reads
     // nodes and triangles only, everything after it waits here (rt_scene.cu)
@@ -386,25 +422,23 @@ int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_
       P.bounce = b;
       const int bslot = b < RT_STAGE_BOUNCES ? b : RT_STAGE_BOUNCES - 1;
       if (b > 0) {
-        StageTimer t(RT_STAGE_TRACE * RT_STAGE_BOUNCES + bslot, stream, dev);
-        if (p.fast) rt_fast_launch_trace(P, b <= RT_TRACE_WIDE_BOUNCES ? fast_wide_grid : fast_grid, level_bytes, stream, b <= RT_TRACE_WIDE_BOUNCES);
-        else if (b <= RT_TRACE_WIDE_BOUNCES) rt_trace_kernel<false, RT_TRACE_MIN_BLOCKS_WIDE><<<wide_grid, RT_BLOCK, level_bytes, stream>>>(P);
-        else        rt_trace_kernel<false><<<trace_grid, RT_BLOCK, level_bytes, stream>>>(P);
+        StageTimer st(RT_STAGE_TRACE * RT_STAGE_BOUNCES + bslot, stream, t.dev);
+        launch_bounce_trace(P, t, p.fast, stream);
         launches++;
       }
       {
-        StageTimer t(RT_STAGE_MISS * RT_STAGE_BOUNCES + bslot, stream, dev);
-        if (p.fast) rt_fast_launch_miss(P, miss_grid(b), stream);
-        else        rt_miss_kernel<<<miss_grid(b), 256, 0, stream>>>(P);
+        StageTimer st(RT_STAGE_MISS * RT_STAGE_BOUNCES + bslot, stream, t.dev);
+        if (p.fast) rt_fast_launch_miss(P, miss_grid(sm_count, b), stream);
+        else        rt_miss_kernel<<<miss_grid(sm_count, b), 256, 0, stream>>>(P);
       }
       {
-        StageTimer t(RT_STAGE_SHADE * RT_STAGE_BOUNCES + bslot, stream, dev);
-        if (p.fast) rt_fast_launch_shade(P, shade_grid(b), stream);
-        else        rt_shade_kernel<<<shade_grid(b), 256, 0, stream>>>(P);
+        StageTimer st(RT_STAGE_SHADE * RT_STAGE_BOUNCES + bslot, stream, t.dev);
+        if (p.fast) rt_fast_launch_shade(P, shade_grid(sm_count, b), stream);
+        else        rt_shade_kernel<<<shade_grid(sm_count, b), 256, 0, stream>>>(P);
       }
       launches += 2;
     }
-    { StageTimer t(RT_STAGE_ACCUMULATE * RT_STAGE_BOUNCES, stream, dev); rt_accumulate_kernel<<<flat_grid * 4, 256, 0, stream>>>(P); }
+    { StageTimer st(RT_STAGE_ACCUMULATE * RT_STAGE_BOUNCES, stream, t.dev); rt_accumulate_kernel<<<flat_grid(sm_count) * 4, 256, 0, stream>>>(P); }
     launches++;
   }
   if (n_launches) *n_launches += launches;
@@ -574,9 +608,8 @@ int rt_launch_lightmap(const SceneDev &scene, int width, int height, int samples
                        unsigned char *d_pixels, int stride, int components, float *d_values, int *d_owner_out,
                        void *scratch, int sm_count, void *workspace, size_t workspace_bytes, cudaStream_t stream,
                        int *n_launches, unsigned *n_jobs_out) {
-  size_t level_bytes = 0;
-  int dev = 0;
-  if (int e = trace_launch_setup(scene, &dev, &level_bytes)) return e;
+  TraceLaunch t;
+  if (int e = trace_launch_setup(scene, sm_count, t)) return e;
   const size_t n_texels = (size_t)width * (size_t)height;
   LightmapParams L{};
   L.width = width; L.height = height; L.samples = samples;
@@ -587,9 +620,9 @@ int rt_launch_lightmap(const SceneDev &scene, int width, int height, int samples
   L.sums = reinterpret_cast<float *>(sp);
   cudaMemsetAsync(L.n_jobs, 0, 256, stream);
   cudaMemsetAsync(L.owner, 0xff, n_texels * sizeof(int), stream);
-  const unsigned flat_grid = (unsigned)(sm_count * 8);
+  const unsigned flat = flat_grid(sm_count);
   rt_lightmap_owner_kernel<<<(unsigned)scene.n_slots, 128, 0, stream>>>(scene, L);
-  rt_lightmap_jobs_kernel<<<flat_grid, 256, 0, stream>>>(L);
+  rt_lightmap_jobs_kernel<<<flat, 256, 0, stream>>>(L);
   int launches = 2;
   unsigned n_jobs = 0;
   cudaMemcpyAsync(&n_jobs, L.n_jobs, sizeof n_jobs, cudaMemcpyDeviceToHost, stream);
@@ -603,35 +636,29 @@ int rt_launch_lightmap(const SceneDev &scene, int width, int height, int samples
   P.width = width; P.height = height;
   P.max_bounces = max_bounces;
   P.user_seed = user_seed;
-  const size_t cb = counts_bytes(max_bounces);
-  const size_t per_path = RT_PATH_BYTES + sizeof(float);
-  if (workspace_bytes < cb + (size_t)n_jobs * per_path) return (int)cudaErrorMemoryAllocation;
-  size_t cap = (workspace_bytes - cb) / per_path;
-  size_t fit = chunk_samples(n_jobs, samples, 0);
-  if (fit > cap / n_jobs) fit = cap / n_jobs;
-  const int chunk = (int)fit;
-  cap = (size_t)chunk * n_jobs;
-  bind_queues(P.q, static_cast<char *>(workspace), cb, cap);
-  L.cosw = reinterpret_cast<float *>(static_cast<char *>(workspace) + cb + cap * RT_PATH_BYTES);
-  const unsigned trace_grid = (unsigned)(sm_count * g_trace_blocks_per_sm[dev]);
+  char *cosw = nullptr;
+  const int chunk = fit_chunk(P, n_jobs, samples, sizeof(float), workspace, workspace_bytes, &cosw);
+  if (chunk == 0) return (int)cudaErrorMemoryAllocation;
+  L.cosw = reinterpret_cast<float *>(cosw);
   for (int s0 = 0; s0 < samples; s0 += chunk) {
     const int S = samples - s0 < chunk ? samples - s0 : chunk;
     P.sample0 = s0; P.n_samples = S;
     P.n_paths = n_jobs * (unsigned)S;
-    cudaMemsetAsync(P.q.counts, 0, cb, stream);
-    rt_lightmap_raygen_kernel<<<flat_grid, 256, 0, stream>>>(P, L, n_jobs);
+    cudaMemsetAsync(P.q.counts, 0, counts_bytes(max_bounces), stream);
+    rt_lightmap_raygen_kernel<<<flat, 256, 0, stream>>>(P, L, n_jobs);
     launches++;
+    // the generic trace and flat grids at every bounce, not the camera path's per-bounce shapes
     for (int b = 0; b < max_bounces; b++) {
       P.bounce = b;
-      rt_trace_kernel<false><<<trace_grid, RT_BLOCK, level_bytes, stream>>>(P);
-      rt_miss_kernel<<<flat_grid, 256, 0, stream>>>(P);
-      rt_shade_kernel<<<flat_grid, 256, 0, stream>>>(P);
+      rt_trace_kernel<false><<<t.generic, RT_BLOCK, t.level_bytes, stream>>>(P);
+      rt_miss_kernel<<<flat, 256, 0, stream>>>(P);
+      rt_shade_kernel<<<flat, 256, 0, stream>>>(P);
       launches += 3;
     }
-    rt_lightmap_accumulate_kernel<<<flat_grid, 256, 0, stream>>>(P, L, n_jobs, s0 == 0);
+    rt_lightmap_accumulate_kernel<<<flat, 256, 0, stream>>>(P, L, n_jobs, s0 == 0);
     launches++;
   }
-  rt_lightmap_store_kernel<<<flat_grid, 256, 0, stream>>>(L, n_jobs, d_pixels, stride, components, d_values);
+  rt_lightmap_store_kernel<<<flat, 256, 0, stream>>>(L, n_jobs, d_pixels, stride, components, d_values);
   launches++;
   if (n_launches) *n_launches += launches;
   return (int)cudaGetLastError();
@@ -705,7 +732,17 @@ size_t rt_cast_rays_workspace_bytes(size_t n_paths, int max_bounces, bool floor)
   size_t paths = floor ? (size_t)RT_CAST_RAYS_MIN_CHUNK : chunk_paths_max();
   if (paths > n_paths) paths = n_paths;
   if (paths < 1) paths = 1;
-  return counts_bytes(max_bounces > 0 ? max_bounces : 1) + paths * RT_PATH_BYTES;
+  return counts_bytes(max_bounces) + paths * RT_PATH_BYTES;
+}
+
+size_t rt_lightmap_paths_workspace_bytes(size_t n_texels, int samples, int max_bounces, bool floor) {
+  // a path's records and its cosine, plus slack: the queue lengths' share of a 32-path tile and 16 B (156 B at 8 bounces)
+  const size_t per_path = RT_PATH_BYTES + sizeof(float) + counts_bytes(max_bounces) / 32 + 16;
+  const size_t chunk = chunk_samples(32, 0) * 32;
+  size_t paths = floor ? n_texels : n_texels * (size_t)samples;
+  if (paths > chunk) paths = chunk;
+  if (paths < n_texels) paths = n_texels;
+  return paths * per_path + 4096;
 }
 
 int rt_launch_cast_rays(const SceneDev &scene, const float *rays, const unsigned *keys, int n_rays, int sample_begin,
@@ -718,9 +755,8 @@ int rt_launch_cast_rays(const SceneDev &scene, const float *rays, const unsigned
     if (!accumulate) cudaMemsetAsync(radiance, 0, (size_t)n_rays * 3 * sizeof(float), stream);
     return (int)cudaGetLastError();
   }
-  size_t level_bytes = 0;
-  int dev = 0;
-  if (int e = trace_launch_setup(scene, &dev, &level_bytes)) return e;
+  TraceLaunch t;
+  if (int e = trace_launch_setup(scene, sm_count, t)) return e;
 
   StageParams P{};
   P.scene = scene;
@@ -734,9 +770,8 @@ int rt_launch_cast_rays(const SceneDev &scene, const float *rays, const unsigned
 
   // chunking: R rays x S samples per chunk, at most `cap` paths.  Every sample of every ray when they fit; otherwise
   // samples of a ray stay together up to a warp's worth (or all of them, if the rays are few) and the rays are split
-  const size_t cb = counts_bytes(max_bounces > 0 ? max_bounces : 1);
-  if (workspace_bytes < cb + RT_PATH_BYTES) return (int)cudaErrorMemoryAllocation;
-  size_t cap = (workspace_bytes - cb) / RT_PATH_BYTES;
+  size_t cap = path_capacity(workspace_bytes, max_bounces, RT_PATH_BYTES);
+  if (cap < 1) return (int)cudaErrorMemoryAllocation;
   if (cap > chunk_paths_max()) cap = chunk_paths_max();
   size_t S = (size_t)samples, R = (size_t)n_rays;
   if (R * S > cap) {
@@ -746,14 +781,9 @@ int rt_launch_cast_rays(const SceneDev &scene, const float *rays, const unsigned
     R = cap / S;
     if (R > (size_t)n_rays) R = (size_t)n_rays;
   }
-  bind_queues(P.q, static_cast<char *>(workspace), cb, R * S);
+  bind_queues(P.q, workspace, max_bounces, R * S);
 
-  const unsigned trace_grid = (unsigned)(sm_count * g_trace_blocks_per_sm[dev]);
-  const unsigned wide_grid = (unsigned)(sm_count * g_wide_blocks_per_sm[dev]);
-  const unsigned flat_grid = (unsigned)(sm_count * 8);
   // the renderer's per-bounce launch shapes (rt_launch_render); bounce 0 is a generic trace of a long queue
-  auto miss_grid  = [&](int b) { return (unsigned)sm_count * (b == 0 ? 64u : b == 1 ? 32u : 8u); };
-  auto shade_grid = [&](int b) { return (unsigned)sm_count * (b == 0 ? 64u : 8u); };
   int launches = 0;
   for (size_t r0 = 0; r0 < (size_t)n_rays; r0 += R) {
     C.ray0 = (unsigned)r0;
@@ -764,18 +794,17 @@ int rt_launch_cast_rays(const SceneDev &scene, const float *rays, const unsigned
       P.n_paths = C.n_rays * (unsigned)n_s;
       P.accumulate = (accumulate || s0 > sample_begin) ? 1 : 0;
       C.per_sample_offset = s0 - sample_begin;
-      cudaMemsetAsync(P.q.counts, 0, cb, stream);
-      rt_cast_rays_raygen_kernel<<<flat_grid, 256, 0, stream>>>(P, C);
+      cudaMemsetAsync(P.q.counts, 0, counts_bytes(max_bounces), stream);
+      rt_cast_rays_raygen_kernel<<<flat_grid(sm_count), 256, 0, stream>>>(P, C);
       launches++;
       for (int b = 0; b < max_bounces; b++) {
         P.bounce = b;
-        if (b <= RT_TRACE_WIDE_BOUNCES) rt_trace_kernel<false, RT_TRACE_MIN_BLOCKS_WIDE><<<wide_grid, RT_BLOCK, level_bytes, stream>>>(P);
-        else                            rt_trace_kernel<false><<<trace_grid, RT_BLOCK, level_bytes, stream>>>(P);
-        rt_miss_kernel<<<miss_grid(b), 256, 0, stream>>>(P);
-        rt_shade_kernel<<<shade_grid(b), 256, 0, stream>>>(P);
+        launch_bounce_trace(P, t, false, stream);
+        rt_miss_kernel<<<miss_grid(sm_count, b), 256, 0, stream>>>(P);
+        rt_shade_kernel<<<shade_grid(sm_count, b), 256, 0, stream>>>(P);
         launches += 3;
       }
-      rt_cast_rays_accumulate_kernel<<<flat_grid * 4, 256, 0, stream>>>(P, C);
+      rt_cast_rays_accumulate_kernel<<<flat_grid(sm_count) * 4, 256, 0, stream>>>(P, C);
       launches++;
     }
   }
@@ -908,62 +937,33 @@ int rt_launch_aov(const SceneDev &scene, int width, int height, int sample_begin
     if (!accumulate) cudaMemsetAsync(aov, 0, (size_t)width * (size_t)height * 16 * sizeof(float), stream);
     return (int)cudaGetLastError();
   }
-  size_t level_bytes = 0;
-  int dev = 0;
-  if (int e = trace_launch_setup(scene, &dev, &level_bytes)) return e;
+  TraceLaunch t;
+  if (int e = trace_launch_setup(scene, sm_count, t)) return e;
 
-  // the renderer's frame set-up (rt_launch_render, whole image)
-  StageParams P{};
-  P.scene = scene;
-  P.width = width; P.height = height;
-  P.tiles_x = (width + 7) / 8; P.tiles_y = (height + 3) / 4;
-  P.split_rank = 0; P.split_world = 1;
-  P.chunks_x = (width + 31) / 32;
-  P.n_tiles = rt_render_tiles(width, height, 0, 1);
-  P.div_tiles_x = rt_fastdiv_make((uint32_t)P.tiles_x, 0xffffffffu >> 5);
-  P.div_chunks_x = rt_fastdiv_make((uint32_t)P.chunks_x, 0xffffffffu);
-  P.max_bounces = max_bounces;
+  // the renderer's frame and chunking (rt_launch_render, whole image)
+  StageParams P = camera_frame(scene, width, height, 0, 1, max_bounces);
   P.counters = counters;
-
-  const size_t per_sample = (size_t)P.n_tiles * 32;
-  const size_t cb = counts_bytes(max_bounces);
-  if (workspace_bytes < cb + per_sample * RT_PATH_BYTES) return (int)cudaErrorMemoryAllocation;
-  size_t cap = (workspace_bytes - cb) / RT_PATH_BYTES;
-  size_t fit = chunk_samples(per_sample, n_total, 0);
-  if (fit > cap / per_sample) fit = cap / per_sample;
-  const int chunk = (int)fit;
-  cap = (size_t)chunk * per_sample;
-  bind_queues(P.q, static_cast<char *>(workspace), cb, cap);
+  const int chunk = fit_chunk(P, (size_t)P.n_tiles * 32, n_total, 0, workspace, workspace_bytes, nullptr);
+  if (chunk == 0) return (int)cudaErrorMemoryAllocation;
 
   rt_camera_relative_kernel<<<(unsigned)sm_count, 256, 0, stream>>>(scene);
-  const unsigned trace_grid = (unsigned)(sm_count * g_trace_blocks_per_sm[dev]);
-  const unsigned wide_grid = (unsigned)(sm_count * g_wide_blocks_per_sm[dev]);
-  const unsigned primary_grid = (unsigned)(sm_count * g_primary_blocks_per_sm[dev]);
-  const unsigned flat_grid = (unsigned)(sm_count * 8);
-  auto surface_grid = [&](int b) { return (unsigned)sm_count * (b == 0 ? 64u : 8u); };    // the renderer's shade_grid
   int launches = 1;
   for (int s0 = sample_begin; s0 < sample_end; s0 += chunk) {
-    const int S = (sample_end - s0 < chunk) ? sample_end - s0 : chunk;
-    P.sample0 = s0; P.n_samples = S;
-    P.n_paths = (unsigned)(per_sample * (size_t)S);
-    P.div_samples = rt_fastdiv_make((uint32_t)S, P.n_paths);
-    P.accumulate = (accumulate || s0 > sample_begin) ? 1 : 0;
-    cudaMemsetAsync(P.q.counts, 0, cb, stream);
+    camera_chunk(P, s0, sample_end, chunk, accumulate || s0 > sample_begin, stream);
     cudaMemsetAsync(P.q.tint, 0xff, (size_t)P.n_paths * sizeof(float4), stream);    // slot -1: no surface yet
     P.bounce = 0;
-    rt_trace_kernel<true><<<primary_grid, RT_BLOCK, level_bytes, stream>>>(P);
+    rt_trace_kernel<true><<<t.primary, RT_BLOCK, t.level_bytes, stream>>>(P);
     launches++;
     for (int b = 0; b < max_bounces; b++) {
       P.bounce = b;
       if (b > 0) {
-        if (b <= RT_TRACE_WIDE_BOUNCES) rt_trace_kernel<false, RT_TRACE_MIN_BLOCKS_WIDE><<<wide_grid, RT_BLOCK, level_bytes, stream>>>(P);
-        else                            rt_trace_kernel<false><<<trace_grid, RT_BLOCK, level_bytes, stream>>>(P);
+        launch_bounce_trace(P, t, false, stream);
         launches++;
       }
-      rt_aov_surface_kernel<<<surface_grid(b), 256, 0, stream>>>(P);
+      rt_aov_surface_kernel<<<shade_grid(sm_count, b), 256, 0, stream>>>(P);     // in place of miss and shade
       launches++;
     }
-    rt_aov_accumulate_kernel<<<flat_grid * 4, 256, 0, stream>>>(P, reinterpret_cast<float4 *>(aov));
+    rt_aov_accumulate_kernel<<<flat_grid(sm_count) * 4, 256, 0, stream>>>(P, reinterpret_cast<float4 *>(aov));
     launches++;
   }
   if (n_launches) *n_launches += launches;
@@ -989,5 +989,5 @@ int rt_launch_reduce_resolve(const ReduceParts &parts, float *sum_out, int width
 int rt_render_blocks_per_sm(void) {
   int dev = 0;
   cudaGetDevice(&dev);
-  return dev >= 0 && dev < RT_MAX_DEVICES ? g_trace_blocks_per_sm[dev] : 0;
+  return dev >= 0 && dev < RT_MAX_DEVICES ? g_occupancy[dev].generic : 0;
 }

@@ -78,8 +78,7 @@ void release_device(Device &d) {
   for (auto &kv : d.block_pool) cudaFree(kv.second);
   d.block_pool.clear();
   cudaFree(d.d_accum); cudaFree(d.d_hit_ids); cudaFree(d.d_counters); cudaFree(d.d_workspace); cudaFree(d.d_texel_stage);
-  cudaFree(d.d_image); cudaFree(d.d_image2); cudaFree(d.d_query_fetch); cudaFree(d.d_query_stage);
-  cudaFree(d.d_cast_stage); cudaFree(d.d_aov_stage);
+  cudaFree(d.d_image); cudaFree(d.d_image2); cudaFree(d.d_query_fetch); cudaFree(d.d_stage);
   if (d.h_pinned) cudaFreeHost(d.h_pinned);
   if (d.ring.base) cudaFreeHost(d.ring.base);
   for (cudaEvent_t e : d.ring.drained) if (e) cudaEventDestroy(e);

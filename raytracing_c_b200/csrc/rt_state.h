@@ -76,15 +76,12 @@ struct Device {
   unsigned char *d_image = nullptr, *d_image2 = nullptr; size_t image_bytes = 0, image2_bytes = 0;
   unsigned char *h_pinned = nullptr; size_t pinned_bytes = 0;
   // ray queries (rt_gpu_closest_hit* / rt_gpu_occluded*): the kernel's work counter, the event that serialises queries
-  // on this device (they share the counter), staging for the host-memory calls
+  // on this device (they share the counter)
   unsigned *d_query_fetch = nullptr;
   cudaEvent_t query_busy = nullptr;
   bool  query_busy_valid = false;
-  void *d_query_stage = nullptr; size_t query_stage_bytes = 0;
-  // staging of the host-memory rt_gpu_cast_rays: rays, keys, sums, per-sample radiance
-  void *d_cast_stage = nullptr; size_t cast_stage_bytes = 0;
-  // staging of the host-memory rt_gpu_render_aov: the W*H records
-  void *d_aov_stage = nullptr; size_t aov_stage_bytes = 0;
+  // staging of the host-memory queries, rt_gpu_cast_rays and rt_gpu_render_aov (rt_cabi.cu: stage)
+  void *d_stage = nullptr; size_t stage_bytes = 0;
   bool l2_window_set = false;
   size_t l2_persist_max = 0, l2_window_max = 0;    // device limits (persistingL2CacheMaxSize, accessPolicyMaxWindowSize)
   cudaStream_t l2_stream = nullptr; const void *l2_base = nullptr;   // where the window was last set

@@ -52,7 +52,8 @@ def test_lightmap_through_the_reference_entry_point_and_in_chunks(monkeypatch):
         n_jobs = int((ref["owner"] >= 0).sum())
         monkeypatch.setenv("RT_GPU_CHUNK_PATHS", str(n_jobs * 2))        # 2 samples per chunk
         assert np.array_equal(driver.lightmap_bake(loaded, w, h, samples), whole)
-        assert gpu_lib().rt_gpu_last_launches() >= 3 * (2 + 8 * 3)
+        # owner and jobs, 3 chunks x (raygen, 8 x trace / miss / shade, accumulate), store
+        assert gpu_lib().rt_gpu_last_launches() == 2 + 3 * (1 + 8 * 3 + 1) + 1
     finally:
         loaded.close()
 
