@@ -289,6 +289,48 @@ int rt_gpu_render_aov_device(Scene const *scene, isize width, isize height, isiz
 int rt_gpu_render_aov(Scene const *scene, isize width, isize height, isize sample_begin, isize sample_end,
                       isize max_bounces, RT_GPU_AOV *aov);
 
+/* ---- adaptive sampling: masked sample passes and a film for per-pixel sample counts (csrc/rt_render.cu) ----
+ * rt_gpu_render_masked_device renders samples [sample_begin, sample_end) of the pixels d_mask selects, by the
+ * renderer's own camera paths.  The library supplies the mechanism; the host keeps the policy (which pixels have
+ * converged, how many samples a pass takes, when to stop).
+ *   - mask: W*H bytes, row-major; non-zero = render the pixel.  NULL = every pixel.
+ *   - radiance: for a selected pixel p and sample s the path is the renderer's path (p, s): the same camera ray, the
+ *     seed rt_path_seed(p, s, user_seed) and the same per-sample radiance as rt_gpu_render_accum_device.  d_accum[p]
+ *     (3 f32) is the sum in sample order, before any division.
+ *   - second moment (d_accum_sq, optional, W*H*3 f32): the per-channel sum of v * v in sample order; the product is
+ *     rounded, then the add (IEEE f32 without contraction: numpy float32 reproduces it).
+ *   - accumulate = 0: every pixel of d_accum, and of d_accum_sq if given, is written: selected pixels get their sums
+ *     from zero, the others 0 (as the shard call is zero outside its share).  accumulate != 0: selected pixels continue
+ *     from the buffers, the others are not touched.
+ *   - an empty range or max_bounces = 0 is handled as the renderer handles it: nothing is traced or counted, and the
+ *     buffers are zeroed unless accumulate is set, in which case they are left as they are.
+ *   - d_counters (optional, 8 u64, atomically added) as RT_GPU_CTR_*, over the selected paths only: SAMPLES grows by
+ *     (selected pixels) * (end - begin).
+ *   - RT_GPU_Options.fast_math applies exactly as it does to rt_gpu_render_accum_device: the call is the renderer with
+ *     a mask.  pixel_rank / pixel_world do not apply (the call covers the whole image).  First device only.
+ * Key property: because every path is seeded per (pixel, sample) and the sums continue in sample order, after passes
+ * that cover samples [0, n_p) of pixel p, chained with accumulate, d_accum[p] and d_accum_sq[p] equal a uniform render
+ * of [0, n_p) at that pixel bit for bit, whatever the passes in between selected elsewhere.
+ * Ordering: the call uses the device's path-queue workspace and rewrites the camera-relative scene copies, so it is
+ * serialised with renders, lightmap bakes, cast_rays and AOV calls on that device; like a render it waits for the
+ * scene's geometry before its primary trace and for its texels after it.
+ * Refused before any launch: width or height < 1, or an image whose one sample per pixel exceeds 2^31 path ids;
+ * sample_begin < 0, sample_end < sample_begin, sample_end > INT32_MAX; max_bounces < 0; a NULL d_accum; a scene that
+ * is not resident (rt_gpu_scene_upload). */
+int rt_gpu_render_masked_device(Scene const *scene, isize width, isize height,
+                                u8 const *d_mask,        /* optional W*H, row-major: non-zero = render; NULL = every pixel */
+                                isize sample_begin, isize sample_end, isize max_bounces, u32 user_seed, i32 accumulate,
+                                f32 *d_accum,            /* W*H*3 */
+                                f32 *d_accum_sq,         /* optional W*H*3 */
+                                u64 *d_counters,         /* optional 8 */
+                                void *stream);
+/* The film with a sample count per pixel: reference raytracer.c:700-716 with samples = d_samples[pixel].  Each channel
+ * is sum * (1.0f / (f32)n), clamped, sRGB-encoded and truncated to u8, as rt_gpu_resolve_device does; a count <= 0
+ * gives 0 bytes and a NaN sum gives 0.  With every count equal to n the bytes equal rt_gpu_resolve_device(..., n, ...).
+ * Refused: a NULL d_samples, components < 3. */
+int rt_gpu_resolve_counts_device(f32 const *d_accum, i32 const *d_samples, isize width, isize height,
+                                 u8 *d_pixels, isize stride, i32 components, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -143,6 +143,7 @@ GPU_EXPORTS = [
     "rt_gpu_closest_hit_device", "rt_gpu_occluded_device", "rt_gpu_closest_hit", "rt_gpu_occluded",
     "rt_gpu_cast_rays_device", "rt_gpu_cast_rays",
     "rt_gpu_render_aov_device", "rt_gpu_render_aov",
+    "rt_gpu_render_masked_device", "rt_gpu_resolve_counts_device",
 ]
 
 HOST_EXPORTS = [
@@ -277,6 +278,10 @@ def gpu_lib() -> C.CDLL:
         lib.rt_gpu_render_aov_device.argtypes = [C.POINTER(Scene), isize, isize, isize, isize, isize, C.c_int32, C.c_void_p,
                                                  C.c_void_p, C.c_void_p]
         lib.rt_gpu_render_aov.argtypes = [C.POINTER(Scene), isize, isize, isize, isize, isize, C.c_void_p]
+        lib.rt_gpu_render_masked_device.argtypes = [C.POINTER(Scene), isize, isize, C.c_void_p, isize, isize, isize,
+                                                    C.c_uint32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.rt_gpu_resolve_counts_device.argtypes = [C.c_void_p, C.c_void_p, isize, isize, C.c_void_p, isize, C.c_int32,
+                                                     C.c_void_p]
         lib.render_thread_proc.argtypes = [C.POINTER(RenderingContext)]
         lib.render_thread_proc.restype = None
         lib.rendering_context_is_finished.argtypes = [C.POINTER(RenderingContext)]

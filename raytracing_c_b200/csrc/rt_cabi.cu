@@ -178,10 +178,12 @@ struct Share {            // what one device (or process) renders of a frame
   int   split_rank, split_world;
 };
 
-// One render of `share` on device d, enqueued on `stream`: a workspace user.
+// One render of `share` on device d, enqueued on `stream`: a workspace user.  d_mask / d_accum_sq (optional) make it a
+// masked pass (rt_gpu_render_masked_device).
 int render_on_device(Device &d, const Scene *scene, isize width, isize height, const Share &share, isize max_bounces,
                      u32 seed, int accumulate, float *d_accum, float *d_per_sample, int *d_hit_ids,
-                     unsigned long long *d_counters, cudaStream_t stream) {
+                     unsigned long long *d_counters, cudaStream_t stream, const u8 *d_mask = nullptr,
+                     float *d_accum_sq = nullptr) {
   if (width < 1 || height < 1) return fail("render: empty image");
   CUDA_TRY(cudaSetDevice(d.id));
   auto it = d.scenes.find(scene);
@@ -203,6 +205,7 @@ int render_on_device(Device &d, const Scene *scene, isize width, isize height, c
   p.accum = d_accum; p.per_sample = d_per_sample; p.hit_ids = d_hit_ids;
   p.counters = d_counters;
   p.counters_ex = (d_counters && d_counters == d.d_counters) ? d_counters + 8 : nullptr;   // the library's own buffer has 16 slots
+  p.pixel_mask = d_mask; p.accum_sq = d_accum_sq;
   return workspace_end(d, "render", rt_launch_render(p, d.sm_count, d.d_workspace, d.workspace_bytes, stream, &g.last_launches),
                        stream);
 }
@@ -430,6 +433,16 @@ int rt_gpu_reduce_resolve_device(f32 const *const *d_parts, i32 n_parts, f32 *d_
   int e = rt_launch_reduce_resolve(parts, d_sum_out, (int)width, (int)height, (int)samples, d_pixels, (int)stride, components,
                                    static_cast<cudaStream_t>(stream));
   if (e) return fail("reduce+resolve kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
+  g.last_launches++;
+  return 0;
+}
+
+int rt_gpu_resolve_counts_device(f32 const *d_accum, i32 const *d_samples, isize width, isize height, u8 *d_pixels,
+                                 isize stride, i32 components, void *stream) {
+  if (!d_samples || components < 3) return fail("resolve_counts: d_samples and components >= 3 required");
+  int e = rt_launch_resolve_counts(d_accum, d_samples, (int)width, (int)height, d_pixels, (int)stride, components,
+                                   static_cast<cudaStream_t>(stream));
+  if (e) return fail("resolve kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
   g.last_launches++;
   return 0;
 }
@@ -679,10 +692,11 @@ int rt_gpu_cast_rays(Scene const *scene, Ray const *rays, u32 const *keys, isize
 
 namespace {
 
-// Everything that is refused before a launch; afterwards the scene is resident on the first device with the camera the
-// Scene holds now (scene_on_devices refreshes it, as for a render).
-int aov_validate(const char *what, const Scene *scene, isize width, isize height, isize sample_begin, isize sample_end,
-                 isize max_bounces, const void *aov) {
+// Everything that is refused before a launch of a whole-image camera call (AOV, masked render) writing into `out`;
+// afterwards the scene is resident on the first device with the camera the Scene holds now (scene_on_devices
+// refreshes it, as for a render).
+int camera_validate(const char *what, const Scene *scene, isize width, isize height, isize sample_begin, isize sample_end,
+                    isize max_bounces, const void *out, const char *out_name) {
   if (width < 1 || height < 1) return fail("%s: image %lld x %lld is empty", what, (long long)width, (long long)height);
   // one sample of every pixel must fit one chunk of 32-bit path ids
   if (width > INT32_MAX || height > INT32_MAX ||
@@ -692,7 +706,7 @@ int aov_validate(const char *what, const Scene *scene, isize width, isize height
     return fail("%s: samples [%lld, %lld) must be a range inside [0, INT32_MAX]", what, (long long)sample_begin,
                 (long long)sample_end);
   if (max_bounces < 0 || max_bounces > INT32_MAX) return fail("%s: max_bounces = %lld, must be >= 0", what, (long long)max_bounces);
-  if (!aov) return fail("%s: null aov", what);
+  if (!out) return fail("%s: null %s", what, out_name);
   return scene_resident(what, scene);
 }
 
@@ -719,7 +733,7 @@ extern "C" {
 int rt_gpu_render_aov_device(Scene const *scene, isize width, isize height, isize sample_begin, isize sample_end,
                              isize max_bounces, i32 accumulate, RT_GPU_AOV *d_aov, u64 *d_counters, void *stream) {
   std::lock_guard<std::mutex> lock(g_mutex);
-  if (aov_validate("render_aov", scene, width, height, sample_begin, sample_end, max_bounces, d_aov)) return 1;
+  if (camera_validate("render_aov", scene, width, height, sample_begin, sample_end, max_bounces, d_aov, "aov")) return 1;
   if (reinterpret_cast<uintptr_t>(d_aov) & 15) return fail("render_aov: d_aov is not 16-byte aligned");
   return aov_on_device(scene, width, height, sample_begin, sample_end, max_bounces, accumulate,
                        reinterpret_cast<float *>(d_aov), reinterpret_cast<unsigned long long *>(d_counters),
@@ -731,7 +745,7 @@ int rt_gpu_render_aov(Scene const *scene, isize width, isize height, isize sampl
                       isize max_bounces, RT_GPU_AOV *aov) {
   std::lock_guard<std::mutex> lock(g_mutex);
   g.last_launches = 0;
-  if (aov_validate("render_aov", scene, width, height, sample_begin, sample_end, max_bounces, aov)) return 1;
+  if (camera_validate("render_aov", scene, width, height, sample_begin, sample_end, max_bounces, aov, "aov")) return 1;
   Device &d = g.devs[0];
   CUDA_TRY(cudaSetDevice(d.id));
   const size_t bytes = (size_t)width * (size_t)height * sizeof(RT_GPU_AOV);
@@ -742,6 +756,21 @@ int rt_gpu_render_aov(Scene const *scene, isize width, isize height, isize sampl
   CUDA_TRY(cudaMemcpyAsync(aov, d_aov, bytes, cudaMemcpyDeviceToHost, d.stream));
   CUDA_TRY(cudaStreamSynchronize(d.stream));
   return 0;
+}
+
+// ------------------------------------------------------------- masked sample passes
+// The renderer itself (render_on_device, whole image, first device) with its primary trace and accumulate swapped for
+// their masked builds: the launch sequence, chunking, fast_math and the deferred texel wait are a render's.
+int rt_gpu_render_masked_device(Scene const *scene, isize width, isize height, u8 const *d_mask, isize sample_begin,
+                                isize sample_end, isize max_bounces, u32 user_seed, i32 accumulate, f32 *d_accum,
+                                f32 *d_accum_sq, u64 *d_counters, void *stream) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  if (camera_validate("render_masked", scene, width, height, sample_begin, sample_end, max_bounces, d_accum, "accum"))
+    return 1;
+  const Share share{sample_begin, sample_end, 0, 1};
+  return render_on_device(g.devs[0], scene, width, height, share, max_bounces, user_seed, accumulate, d_accum, nullptr,
+                          nullptr, reinterpret_cast<unsigned long long *>(d_counters), static_cast<cudaStream_t>(stream),
+                          d_mask, d_accum_sq);
 }
 
 // ----------------------------------------------------------------- parity hooks

@@ -82,6 +82,8 @@ struct RenderParams {
   int      *hit_ids;
   unsigned long long *counters;
   unsigned long long *counters_ex;
+  const unsigned char *pixel_mask;       // optional W*H: only pixels with a non-zero byte are rendered (masked passes)
+  float    *accum_sq;                    // optional W*H*3: per-channel sum of squared radiance in sample order
 };
 
 __device__ __forceinline__ V3 mk3(float x, float y, float z) { V3 v; v.x = x; v.y = y; v.z = z; return v; }

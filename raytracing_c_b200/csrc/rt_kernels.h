@@ -7,6 +7,8 @@
 
 // wavefront render of samples [p.sample_begin, p.sample_end) into p.accum; `workspace` holds the path queues
 // (rt_render_workspace_bytes; a smaller one only means more, smaller chunks).  *n_launches += kernels launched.
+// With p.pixel_mask and/or p.accum_sq the primary trace and the accumulate run their masked builds: only the selected
+// pixels are rendered (the others are zeroed without p.accumulate, untouched with it) and the second moments are summed.
 size_t rt_render_workspace_bytes(int width, int height, int n_samples, int max_bounces, int split_world);
 int rt_render_chunk_samples(int width, int height, int split_world);
 unsigned rt_render_tiles(int width, int height, int split_rank, int split_world);
@@ -37,6 +39,9 @@ int rt_launch_aov(const SceneDev &scene, int width, int height, int sample_begin
                   size_t workspace_bytes, cudaStream_t stream, int *n_launches);
 int rt_launch_resolve(const float *accum, int width, int height, int samples, unsigned char *pixels,
                       int stride, int components, cudaStream_t stream);
+// the film with a sample count per pixel (samples[W*H]; a count <= 0 gives 0 bytes)
+int rt_launch_resolve_counts(const float *accum, const int *samples, int width, int height, unsigned char *pixels,
+                             int stride, int components, cudaStream_t stream);
 // sum of parts.n accumulators (own + peer-mapped) in rank order, optional copy of the sum, optional resolve to u8
 int rt_launch_reduce_resolve(const ReduceParts &parts, float *sum_out, int width, int height, int samples,
                              unsigned char *pixels, int stride, int components, cudaStream_t stream);

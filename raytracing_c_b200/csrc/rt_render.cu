@@ -67,9 +67,11 @@ __global__ void rt_camera_relative_kernel(const SceneDev sc) {
 }
 
 // ----------------------------------------------------------------- accumulate
-// raytracer.c:696-700: color += cast_ray(...) in sample order, one thread per pixel.
-__global__ void __launch_bounds__(256)
-rt_accumulate_kernel(const __grid_constant__ StageParams P) {
+// raytracer.c:696-700: color += cast_ray(...) in sample order, one thread per pixel.  MASKED (a masked pass, or one with
+// second moments): a pixel P.pixel_mask does not select is written 0 when the call does not accumulate and is left as
+// it is otherwise; P.accum_sq (optional) gains v * v per sample alongside the sum (product rounded, then the add).
+template <bool MASKED>
+__device__ __forceinline__ void accumulate_pixels(const StageParams &P) {
   const unsigned n = P.n_tiles * 32u;
   for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const unsigned tile = i >> 5, in_tile = i & 31u;
@@ -78,7 +80,16 @@ rt_accumulate_kernel(const __grid_constant__ StageParams P) {
     const int px = x0 + (int)(in_tile & 7u), py = y0 + (int)(in_tile >> 3);
     if (px >= P.width || py >= P.height) continue;
     const int pixel = py * P.width + px;
+    if (MASKED && P.pixel_mask && !P.pixel_mask[pixel]) {
+      if (!P.accumulate) {
+        P.accum[3 * pixel + 0] = 0; P.accum[3 * pixel + 1] = 0; P.accum[3 * pixel + 2] = 0;
+        if (P.accum_sq) { P.accum_sq[3 * pixel + 0] = 0; P.accum_sq[3 * pixel + 1] = 0; P.accum_sq[3 * pixel + 2] = 0; }
+      }
+      continue;
+    }
     V3 sum = P.accumulate ? mk3(P.accum[3 * pixel], P.accum[3 * pixel + 1], P.accum[3 * pixel + 2]) : mk3(0, 0, 0);
+    V3 sq = mk3(0, 0, 0);
+    if (MASKED && P.accum_sq && P.accumulate) sq = mk3(P.accum_sq[3 * pixel], P.accum_sq[3 * pixel + 1], P.accum_sq[3 * pixel + 2]);
 #if RT_PATH_LAYOUT == 1
     const float4 *r = P.q.rad + (size_t)i * (size_t)P.n_samples;
     const size_t r_step = 1;
@@ -89,6 +100,7 @@ rt_accumulate_kernel(const __grid_constant__ StageParams P) {
     for (int s = 0; s < P.n_samples; s++) {
       const float4 v = r[(size_t)s * r_step];
       sum = add3(sum, mk3(v.x, v.y, v.z));
+      if (MASKED && P.accum_sq) sq = add3(sq, mul3(mk3(v.x, v.y, v.z), mk3(v.x, v.y, v.z)));
       if (P.per_sample) {
         float *dst = P.per_sample + ((size_t)pixel * (size_t)P.per_sample_stride + (size_t)(P.per_sample_offset + s)) * 3;
         dst[0] = v.x; dst[1] = v.y; dst[2] = v.z;
@@ -97,8 +109,15 @@ rt_accumulate_kernel(const __grid_constant__ StageParams P) {
     P.accum[3 * pixel + 0] = sum.x;
     P.accum[3 * pixel + 1] = sum.y;
     P.accum[3 * pixel + 2] = sum.z;
+    if (MASKED && P.accum_sq) { P.accum_sq[3 * pixel + 0] = sq.x; P.accum_sq[3 * pixel + 1] = sq.y; P.accum_sq[3 * pixel + 2] = sq.z; }
   }
 }
+
+__global__ void __launch_bounds__(256)
+rt_accumulate_kernel(const __grid_constant__ StageParams P) { accumulate_pixels<false>(P); }
+
+__global__ void __launch_bounds__(256)
+rt_accumulate_masked_kernel(const __grid_constant__ StageParams P) { accumulate_pixels<true>(P); }
 
 // ----------------------------------------------------------------------- film
 // raytracer.c:700-716 + common.h:90-92: /spp, clamp, sRGB OETF, *255.999, truncate.
@@ -119,6 +138,19 @@ __global__ void rt_resolve_kernel(const float *__restrict__ accum, int width, in
   unsigned char *dst = pixels + (size_t)components * (size_t)(x + y * stride);
   #pragma unroll
   for (int c = 0; c < 3; c++) dst[c] = film_u8(accum[3 * i + c], inv_samples);
+}
+
+// the film of a pixel with its own sample count: 1 / samples[i] taken per pixel, a count <= 0 gives 0 bytes
+__global__ void rt_resolve_counts_kernel(const float *__restrict__ accum, const int *__restrict__ samples, int width,
+                                         int height, unsigned char *__restrict__ pixels, int stride, int components) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= width * height) return;
+  int x = i % width, y = i / width;
+  const int n = samples[i];
+  const float inv_samples = 1.0f / (float)n;
+  unsigned char *dst = pixels + (size_t)components * (size_t)(x + y * stride);
+  #pragma unroll
+  for (int c = 0; c < 3; c++) dst[c] = n > 0 ? film_u8(accum[3 * i + c], inv_samples) : 0;
 }
 
 // Multi-GPU film: the per-device accumulators are combined and resolved by ONE kernel on the device that owns
@@ -231,12 +263,12 @@ size_t rt_render_workspace_bytes(int width, int height, int n_samples, int max_b
 }
 
 // trace kernels' blocks per SM at the level-store size they were measured for, per device (cudaFuncSetAttribute is per device)
-struct TraceOccupancy { size_t level_bytes; int primary, generic, wide, fast, fast_wide; };
+struct TraceOccupancy { size_t level_bytes; int primary, generic, wide, fast, fast_wide, masked; };
 static TraceOccupancy g_occupancy[RT_MAX_DEVICES];
 
 // what a launcher needs of trace_launch_setup: the device, the level store, and the trace kernels' persistent grids
 // (one wave: blocks per SM x SMs)
-struct TraceLaunch { int dev; size_t level_bytes; unsigned primary, generic, wide, fast, fast_wide; };
+struct TraceLaunch { int dev; size_t level_bytes; unsigned primary, generic, wide, fast, fast_wide, masked; };
 
 // ---- optional per-stage timing (bench.py's roofline leg): CUDA events around every launch, on the
 // launching stream; read back and summed by rt_stage_profile_read
@@ -328,10 +360,12 @@ static int trace_launch_setup(const SceneDev &scene, int sm_count, TraceLaunch &
     o.generic = blocks_per_sm((const void *)rt_trace_kernel<false>);
     o.wide = blocks_per_sm((const void *)rt_trace_kernel<false, RT_TRACE_MIN_BLOCKS_WIDE>);
     o.fast = rt_fast_trace_setup(level_bytes, &o.fast_wide);
+    o.masked = blocks_per_sm((const void *)rt_trace_kernel<true, RT_TRACE_MIN_BLOCKS_PRIMARY, true>);
     o.level_bytes = level_bytes;
   }
   t = TraceLaunch{dev, level_bytes, (unsigned)(sm_count * o.primary), (unsigned)(sm_count * o.generic),
-                  (unsigned)(sm_count * o.wide), (unsigned)(sm_count * o.fast), (unsigned)(sm_count * o.fast_wide)};
+                  (unsigned)(sm_count * o.wide), (unsigned)(sm_count * o.fast), (unsigned)(sm_count * o.fast_wide),
+                  (unsigned)(sm_count * o.masked)};
   return 0;
 }
 
@@ -384,7 +418,10 @@ int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_
   const int n_total = p.sample_end - p.sample_begin;
   if (n_total <= 0 || p.max_bounces < 1) {
     // no samples, or cast_ray's loop body never runs (raytracer.c:512,557): the sum gains nothing
-    if (!p.accumulate) cudaMemsetAsync(p.accum, 0, (size_t)p.width * p.height * 3 * sizeof(float), stream);
+    if (!p.accumulate) {
+      cudaMemsetAsync(p.accum, 0, (size_t)p.width * p.height * 3 * sizeof(float), stream);
+      if (p.accum_sq) cudaMemsetAsync(p.accum_sq, 0, (size_t)p.width * p.height * 3 * sizeof(float), stream);
+    }
     return (int)cudaGetLastError();
   }
   TraceLaunch t;
@@ -397,6 +434,9 @@ int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_
   P.per_sample_stride = n_total;
   P.counters = p.counters;
   P.counters_ex = p.counters_ex;
+  P.pixel_mask = p.pixel_mask;
+  P.accum_sq = p.accum_sq;
+  const bool masked_sum = p.pixel_mask || p.accum_sq;      // the MASKED accumulate: mask, second moments or both
 
   // chunking: as many samples of every pixel per chunk as the workspace holds paths
   const size_t per_sample = (size_t)P.n_tiles * 32;
@@ -413,7 +453,11 @@ int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_
     P.hit_ids = (s0 == p.sample_begin) ? p.hit_ids : nullptr;
     camera_chunk(P, s0, p.sample_end, chunk, p.accumulate || s0 > p.sample_begin || P.split_world > 1, stream);
     P.bounce = 0;
-    { StageTimer st(RT_STAGE_TRACE * RT_STAGE_BOUNCES, stream, t.dev); rt_trace_kernel<true><<<t.primary, RT_BLOCK, t.level_bytes, stream>>>(P); }
+    {
+      StageTimer st(RT_STAGE_TRACE * RT_STAGE_BOUNCES, stream, t.dev);
+      if (p.pixel_mask) rt_trace_kernel<true, RT_TRACE_MIN_BLOCKS_PRIMARY, true><<<t.masked, RT_BLOCK, t.level_bytes, stream>>>(P);
+      else              rt_trace_kernel<true><<<t.primary, RT_BLOCK, t.level_bytes, stream>>>(P);
+    }
     launches++;
     // textures and the environment may still be in flight on the upload's copy stream: the primary trace reads
     // nodes and triangles only, everything after it waits here (rt_scene.cu)
@@ -438,7 +482,11 @@ int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_
       }
       launches += 2;
     }
-    { StageTimer st(RT_STAGE_ACCUMULATE * RT_STAGE_BOUNCES, stream, t.dev); rt_accumulate_kernel<<<flat_grid(sm_count) * 4, 256, 0, stream>>>(P); }
+    {
+      StageTimer st(RT_STAGE_ACCUMULATE * RT_STAGE_BOUNCES, stream, t.dev);
+      if (masked_sum) rt_accumulate_masked_kernel<<<flat_grid(sm_count) * 4, 256, 0, stream>>>(P);
+      else            rt_accumulate_kernel<<<flat_grid(sm_count) * 4, 256, 0, stream>>>(P);
+    }
     launches++;
   }
   if (n_launches) *n_launches += launches;
@@ -975,6 +1023,13 @@ int rt_launch_resolve(const float *accum, int width, int height, int samples, un
   int n = width * height;
   float inv_samples = 1.0f / (float)samples;
   rt_resolve_kernel<<<(n + 255) / 256, 256, 0, stream>>>(accum, width, height, inv_samples, pixels, stride, components);
+  return (int)cudaGetLastError();
+}
+
+int rt_launch_resolve_counts(const float *accum, const int *samples, int width, int height, unsigned char *pixels,
+                             int stride, int components, cudaStream_t stream) {
+  int n = width * height;
+  rt_resolve_counts_kernel<<<(n + 255) / 256, 256, 0, stream>>>(accum, samples, width, height, pixels, stride, components);
   return (int)cudaGetLastError();
 }
 

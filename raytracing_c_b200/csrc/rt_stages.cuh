@@ -83,6 +83,9 @@ struct StageParams {
   int       *hit_ids;                 // optional, written by the primary trace for sample `sample0`
   unsigned long long *counters;
   unsigned long long *counters_ex;    // optional 8 more: [0] rays whose walk was the root-union test alone, [1] primary rays
+  // masked passes (rt_gpu_render_masked_device), last so that the fields above keep their offsets
+  const unsigned char *pixel_mask;    // optional [pixel]: non-zero = render; read by the MASKED trace and accumulate only
+  float     *accum_sq;                // optional [pixel][3]: sum of v * v in sample order
 };
 
 // raytracer.c:582-594, one lane of hash12x8
@@ -175,7 +178,8 @@ __device__ __forceinline__ unsigned warp_append(unsigned *count, bool want, unsi
 // (64 registers; -2.8 % on their kernel).  Bounce rays: the long queues of the first bounces gain too (-2.7 % at
 // bounce 1: more warps to cover the divergent loads), the short late queues lose 5-10 % to it (their time is the
 // slowest ray's latency, which spills lengthen) — the host picks per bounce (rt_render.cu, RT_TRACE_WIDE_BOUNCES).
-template <bool PRIMARY, int MIN_BLOCKS = (PRIMARY ? RT_TRACE_MIN_BLOCKS_PRIMARY : RT_TRACE_MIN_BLOCKS)>
+// MASKED (primary only): a path id whose pixel P.pixel_mask does not select takes no ray, as one outside the image.
+template <bool PRIMARY, int MIN_BLOCKS = (PRIMARY ? RT_TRACE_MIN_BLOCKS_PRIMARY : RT_TRACE_MIN_BLOCKS), bool MASKED = false>
 __global__ void __launch_bounds__(RT_BLOCK, MIN_BLOCKS)
 RT_KN(rt_trace_kernel)(const __grid_constant__ StageParams P) {
   extern __shared__ float4 level_store[];          // [depth - 1][2][RT_BLOCK] entry distances of pending levels (2 .. depth)
@@ -283,6 +287,7 @@ RT_KN(rt_trace_kernel)(const __grid_constant__ StageParams P) {
             int px = 0, py = 0, ls = 0;
             path_pixel(P, q, px, py, ls);
             ok = px < P.width && py < P.height;
+            if (MASKED && ok) ok = P.pixel_mask[py * P.width + px] != 0;
             if (ok) {
               // raytracer.c:644-677; rand_a == rand_b; exact 1/sqrt instead of rsqrt_ps
               const int s = P.sample0 + ls;
@@ -317,7 +322,7 @@ RT_KN(rt_trace_kernel)(const __grid_constant__ StageParams P) {
       if (walking == 0) {
         // nobody walks: rays that finished at their root visit go out on the next turn; with none of those either
         // the queue is drained — or (chunk split) the 32 ids just taken were a job tile that lies outside the
-        // image, and the warp's reserved range goes on
+        // image, or (MASKED) pixels the mask does not select, and the warp's reserved range goes on
         if (exhausted && __ballot_sync(RT_FULL, w.flags & WALK_RAY) == 0) break;
         continue;
       }

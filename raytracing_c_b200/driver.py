@@ -305,6 +305,56 @@ def render_aov(loaded: LoadedScene, width: int, height: int, samples: int, max_b
     return out
 
 
+def render_masked(loaded: LoadedScene, accum, sample_begin: int, sample_end: int, mask=None, accum_sq=None,
+                  max_bounces: int = 8, user_seed: int = 0, accumulate: bool = False, counters=None, stream=None) -> None:
+    """Samples [sample_begin, sample_end) of the pixels `mask` selects (rt_gpu_render_masked_device; semantics in
+    include/rt_gpu.h), enqueued on `stream` (default: torch's current stream).  `accum` and `accum_sq` (optional) are
+    contiguous (H, W, 3) float32 CUDA tensors: the sums and the per-channel sums of squares in sample order, continued
+    with `accumulate`.  `mask` is an (H, W) bool or uint8 CUDA tensor (None = every pixel); `counters` an optional
+    8-element int64 CUDA tensor the work counters are added to.  Uploads the scene if it is not resident."""
+    import torch
+    gpu = gpu_lib()
+    height, width = accum.shape[0], accum.shape[1]
+
+    def check(t, shape, dtypes, what):
+        if t.device.type != "cuda" or t.dtype not in dtypes or tuple(t.shape) != shape or not t.is_contiguous():
+            raise ValueError(f"{what}: a contiguous CUDA tensor of shape {shape} and dtype {dtypes[0]} is required")
+    check(accum, (height, width, 3), (torch.float32,), "accum")
+    if accum_sq is not None:
+        check(accum_sq, (height, width, 3), (torch.float32,), "accum_sq")
+    if mask is not None:
+        check(mask, (height, width), (torch.uint8, torch.bool), "mask")
+    if counters is not None:
+        check(counters, (8,), (torch.int64,), "counters")
+    register_callbacks(loaded)
+    if gpu.rt_gpu_scene_device_bytes(C.byref(loaded.scene)) == 0:
+        gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+    st = stream or torch.cuda.current_stream()
+    gpu_check(gpu.rt_gpu_render_masked_device(
+        C.byref(loaded.scene), width, height, mask.data_ptr() if mask is not None else None, sample_begin, sample_end,
+        max_bounces, user_seed, int(accumulate), accum.data_ptr(), accum_sq.data_ptr() if accum_sq is not None else None,
+        counters.data_ptr() if counters is not None else None, st.cuda_stream))
+
+
+def resolve_counts(accum, samples, stream=None):
+    """The film with a sample count per pixel (rt_gpu_resolve_counts_device): `accum` an (H, W, 3) float32 and `samples`
+    an (H, W) int32 CUDA tensor; returns the (H, W, 3) uint8 CUDA image, enqueued on `stream` (default: torch's current
+    stream).  A count <= 0 gives black."""
+    import torch
+    height, width = accum.shape[0], accum.shape[1]
+    if accum.dtype != torch.float32 or tuple(accum.shape) != (height, width, 3) or not accum.is_contiguous() \
+            or accum.device.type != "cuda":
+        raise ValueError("accum: a contiguous (H, W, 3) float32 CUDA tensor is required")
+    if samples.dtype != torch.int32 or tuple(samples.shape) != (height, width) or not samples.is_contiguous() \
+            or samples.device != accum.device:
+        raise ValueError("samples: a contiguous (H, W) int32 tensor on the device of accum is required")
+    pixels = torch.empty((height, width, 3), dtype=torch.uint8, device=accum.device)
+    st = stream or torch.cuda.current_stream()
+    gpu_check(gpu_lib().rt_gpu_resolve_counts_device(accum.data_ptr(), samples.data_ptr(), width, height,
+                                                     pixels.data_ptr(), width, 3, st.cuda_stream))
+    return pixels
+
+
 def read_accum(width: int, height: int) -> np.ndarray:
     out = np.empty((height, width, 3), dtype=np.float32)
     gpu_check(gpu_lib().rt_gpu_read_accum(out.ctypes.data, out.size))
