@@ -27,6 +27,7 @@
 #include <cuda_runtime.h>
 #include <math_constants.h>
 
+#include <cmath>
 #include <cstdlib>
 #include <vector>
 
@@ -37,6 +38,7 @@
 void rt_fast_launch_trace(const StageParams &P, unsigned grid, size_t smem, cudaStream_t stream, bool wide);
 void rt_fast_launch_miss(const StageParams &P, unsigned grid, cudaStream_t stream);
 void rt_fast_launch_shade(const StageParams &P, unsigned grid, cudaStream_t stream);
+void rt_fast_launch_sky(const StageParams &P, unsigned grid, cudaStream_t stream);
 int  rt_fast_trace_setup(size_t level_bytes, int *wide_blocks_per_sm);
 
 // ------------------------------------------------------------ camera-relative scene
@@ -70,13 +72,14 @@ __global__ void rt_camera_relative_kernel(const SceneDev sc) {
 // raytracer.c:696-700: color += cast_ray(...) in sample order, one thread per pixel.  MASKED (a masked pass, or one with
 // second moments): a pixel P.pixel_mask does not select is written 0 when the call does not accumulate and is left as
 // it is otherwise; P.accum_sq (optional) gains v * v per sample alongside the sum (product rounded, then the add).
+// With P.tiles: the traced tiles only (the sky kernel sums the others).
 template <bool MASKED>
 __device__ __forceinline__ void accumulate_pixels(const StageParams &P) {
-  const unsigned n = P.n_tiles * 32u;
+  const unsigned n = (P.tiles ? P.tiles[0] : P.n_tiles) * 32u;
   for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const unsigned tile = i >> 5, in_tile = i & 31u;
     int x0, y0;
-    tile_origin(P, tile, x0, y0);
+    tile_origin(P, P.tiles ? P.tiles[2 + tile] : tile, x0, y0);
     const int px = x0 + (int)(in_tile & 7u), py = y0 + (int)(in_tile >> 3);
     if (px >= P.width || py >= P.height) continue;
     const int pixel = py * P.width + px;
@@ -256,10 +259,14 @@ int rt_render_chunk_samples(int width, int height, int split_world) {
   return (int)chunk_samples(per_sample, 0);
 }
 
+// the tile lists of a render (StageParams.tiles): two counts and one id per job tile
+static size_t tile_list_bytes(unsigned n_tiles) { return ((2 + (size_t)n_tiles) * sizeof(unsigned) + 255) & ~(size_t)255; }
+
 size_t rt_render_workspace_bytes(int width, int height, int n_samples, int max_bounces, int split_world) {
-  size_t per_sample = (size_t)rt_render_tiles(width, height, 0, split_world) * 32;
+  const unsigned tiles = rt_render_tiles(width, height, 0, split_world);
+  size_t per_sample = (size_t)tiles * 32;
   if (per_sample < 32) per_sample = 32;
-  return counts_bytes(max_bounces) + chunk_samples(per_sample, n_samples) * per_sample * RT_PATH_BYTES;
+  return tile_list_bytes(tiles) + counts_bytes(max_bounces) + chunk_samples(per_sample, n_samples) * per_sample * RT_PATH_BYTES;
 }
 
 // trace kernels' blocks per SM at the level-store size they were measured for, per device (cudaFuncSetAttribute is per device)
@@ -413,6 +420,110 @@ static void camera_chunk(StageParams &P, int s0, int sample_end, int chunk, bool
   cudaMemsetAsync(P.q.counts, 0, counts_bytes(P.max_bounces), stream);
 }
 
+// ------------------------------------------------------------------ sky tiles
+// A job tile is sky when no jittered camera ray of its pixels can reach the root-union box: every such ray would end
+// its walk at walk_misses_root and its path at the bounce-0 miss kernel, and rt_sky_kernel renders it without the path
+// queues.  The argument is made in f64 on an inflated box and an enlarged footprint (DESIGN.md, "Sky tiles"), so a
+// tile is classified sky only when the f32 ray generation and slab test cannot disagree.
+#define RT_SKY_MARGIN 1e-3          // box inflation and zero-direction guard, relative
+#define RT_SKY_PIXELS 2.0           // footprint enlargement, pixels
+
+// Continuous pixel coordinates (u, v): pixel (px, py) casts its rays through u in [px - 0.5, px + 0.5] and v in
+// [py - 0.5, py + 0.5] (jitter in [0, 1], raytracer.c:644-677).  `rect` bounds the projection of the inflated box;
+// rot, aspect and focal give the camera-space direction of (u, v), whose components must keep one sign per tile.
+struct SkyFrame { double rect[4]; double rot[3][3]; double aspect, focal, width, height; };
+
+// The frame of a render, or false when no tile may be sky: a box corner at or behind the camera plane (this also
+// covers a camera inside the box), an empty or non-finite box, or a camera matrix without a finite inverse.
+static bool sky_frame(const SceneDev &sc, int width, int height, SkyFrame &f) {
+  double r[3][3], o[3], lo[3], hi[3], scale = 0, diag = 0;
+  for (int a = 0; a < 3; a++) {
+    for (int b = 0; b < 3; b++) r[a][b] = sc.view[a][b];
+    o[a] = sc.view[a][3]; lo[a] = sc.root_lo[a]; hi[a] = sc.root_hi[a];
+    if (!(lo[a] <= hi[a]) || !std::isfinite(lo[a]) || !std::isfinite(hi[a]) || !std::isfinite(o[a])) return false;
+    scale = std::fmax(scale, std::fmax(std::fabs(o[a]), std::fmax(std::fabs(lo[a]), std::fabs(hi[a]))));
+    diag += (hi[a] - lo[a]) * (hi[a] - lo[a]);
+  }
+  const double m = RT_SKY_MARGIN * (scale + std::sqrt(diag));
+  // inverse of the camera's 3x3 (camera space -> world is r, so world -> camera is its inverse)
+  const double det = r[0][0] * (r[1][1] * r[2][2] - r[1][2] * r[2][1]) - r[0][1] * (r[1][0] * r[2][2] - r[1][2] * r[2][0]) +
+                     r[0][2] * (r[1][0] * r[2][1] - r[1][1] * r[2][0]);
+  double inv[3][3];
+  for (int a = 0; a < 3; a++)
+    for (int b = 0; b < 3; b++) {
+      const int a1 = (b + 1) % 3, a2 = (b + 2) % 3, b1 = (a + 1) % 3, b2 = (a + 2) % 3;
+      inv[a][b] = (r[a1][b1] * r[a2][b2] - r[a1][b2] * r[a2][b1]) / det;
+      if (!std::isfinite(inv[a][b])) return false;
+    }
+  const double aspect = (double)((float)width / (float)height), focal = sc.focal_length;
+  if (!(focal > 0) || !std::isfinite(focal)) return false;
+  double u0 = INFINITY, u1 = -INFINITY, v0 = INFINITY, v1 = -INFINITY;
+  for (int c = 0; c < 8; c++) {
+    double w[3], p[3];
+    for (int a = 0; a < 3; a++) w[a] = ((c >> a) & 1 ? hi[a] + m : lo[a] - m) - o[a];
+    for (int a = 0; a < 3; a++) p[a] = inv[a][0] * w[0] + inv[a][1] * w[1] + inv[a][2] * w[2];
+    if (!(p[2] < 0)) return false;                          // camera looks down -z: the corner is not in front
+    // the camera-space direction (cx, cy, -focal) through the corner; cx = (2u / W - 1) * aspect, cy = 1 - 2v / H
+    const double cx = p[0] * (-focal / p[2]), cy = p[1] * (-focal / p[2]);
+    const double u = (cx / aspect + 1) * 0.5 * width, v = (1 - cy) * 0.5 * height;
+    if (!std::isfinite(u) || !std::isfinite(v)) return false;
+    u0 = std::fmin(u0, u); u1 = std::fmax(u1, u); v0 = std::fmin(v0, v); v1 = std::fmax(v1, v);
+  }
+  f = SkyFrame{{u0, u1, v0, v1}, {{r[0][0], r[0][1], r[0][2]}, {r[1][0], r[1][1], r[1][2]}, {r[2][0], r[2][1], r[2][2]}},
+               aspect, focal, (double)width, (double)height};
+  return true;
+}
+
+// tile sky? Its footprint, enlarged by RT_SKY_PIXELS, lies outside f.rect, and no direction component changes sign on it
+// or comes within RT_SKY_MARGIN of zero relative to its terms: a zero component makes the ray non-regular (WALK_REG),
+// whose walk does not take the root-union shortcut.  Tiles without pixels are sky (nothing renders them).
+__device__ bool sky_tile(const StageParams &P, const SkyFrame &f, unsigned tile) {
+  int x0, y0;
+  tile_origin(P, tile, x0, y0);
+  if (x0 >= P.width || y0 >= P.height) return true;
+  const double ua = x0 - 0.5 - RT_SKY_PIXELS, ub = x0 + 7.5 + RT_SKY_PIXELS;
+  const double va = y0 - 0.5 - RT_SKY_PIXELS, vb = y0 + 3.5 + RT_SKY_PIXELS;
+  if (!(ub < f.rect[0] || ua > f.rect[1] || vb < f.rect[2] || va > f.rect[3])) return false;
+  for (int a = 0; a < 3; a++) {
+    double g_min = INFINITY, g_max = -INFINITY, terms = 0;
+    for (int c = 0; c < 4; c++) {
+      const double cx = ((c & 1 ? ub : ua) * 2 / f.width - 1) * f.aspect, cy = 1 - (c & 2 ? vb : va) * 2 / f.height;
+      const double g = f.rot[a][0] * cx + f.rot[a][1] * cy - f.rot[a][2] * f.focal;
+      g_min = fmin(g_min, g); g_max = fmax(g_max, g);
+      terms = fmax(terms, fabs(f.rot[a][0] * cx) + fabs(f.rot[a][1] * cy) + fabs(f.rot[a][2] * f.focal));
+    }
+    if (!(g_min > RT_SKY_MARGIN * terms || g_max < -RT_SKY_MARGIN * terms)) return false;
+  }
+  return true;
+}
+
+// One block: the traced tiles to P.tiles[2 ..] ascending, the sky tiles from the end, the two counts to [0] and [1].
+__global__ void __launch_bounds__(1024)
+rt_sky_tiles_kernel(const __grid_constant__ StageParams P, const SkyFrame f, unsigned *tiles) {
+  __shared__ unsigned warp_sky[32];
+  __shared__ unsigned base_sky;
+  const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5, lt = (1u << lane) - 1u;
+  if (threadIdx.x == 0) base_sky = 0;
+  for (unsigned t0 = 0; t0 < P.n_tiles; t0 += blockDim.x) {
+    const unsigned tile = t0 + threadIdx.x;
+    const bool sky = tile < P.n_tiles && sky_tile(P, f, tile);
+    const unsigned m = __ballot_sync(RT_FULL, sky);
+    if (lane == 0) warp_sky[warp] = __popc(m);
+    __syncthreads();
+    unsigned before = base_sky;
+    for (unsigned w = 0; w < warp; w++) before += warp_sky[w];
+    const unsigned sky_rank = before + __popc(m & lt);
+    if (tile < P.n_tiles) {
+      if (sky) tiles[2 + P.n_tiles - 1 - sky_rank] = tile;
+      else     tiles[2 + tile - sky_rank] = tile;                 // tiles before it that are traced
+    }
+    __syncthreads();
+    if (threadIdx.x == blockDim.x - 1) base_sky = sky_rank + (sky ? 1u : 0u);
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) { tiles[0] = P.n_tiles - base_sky; tiles[1] = base_sky; }
+}
+
 int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_t workspace_bytes,
                      cudaStream_t stream, int *n_launches) {
   const int n_total = p.sample_end - p.sample_begin;
@@ -443,11 +554,22 @@ int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_
   if (P.split_world > 1 && !p.accumulate)      // the pixels of other ranks stay zero (the cross-rank sum adds them)
     cudaMemsetAsync(p.accum, 0, (size_t)p.width * p.height * 3 * sizeof(float), stream);
   if (per_sample == 0) return (int)cudaGetLastError();
-  const int chunk = fit_chunk(P, per_sample, n_total, 0, workspace, workspace_bytes, nullptr);
+  // the tile lists first, then the path queues
+  const size_t list_bytes = tile_list_bytes(P.n_tiles);
+  if (workspace_bytes < list_bytes) return (int)cudaErrorMemoryAllocation;
+  unsigned *tiles = static_cast<unsigned *>(workspace);
+  const int chunk = fit_chunk(P, per_sample, n_total, 0, static_cast<char *>(workspace) + list_bytes,
+                              workspace_bytes - list_bytes, nullptr);
   if (chunk == 0) return (int)cudaErrorMemoryAllocation;
 
   rt_camera_relative_kernel<<<(unsigned)sm_count, 256, 0, stream>>>(p.scene);
   int launches = 1;
+  SkyFrame sky;
+  if (sky_frame(p.scene, p.width, p.height, sky)) {
+    rt_sky_tiles_kernel<<<1, 1024, 0, stream>>>(P, sky, tiles);
+    P.tiles = tiles;
+    launches++;
+  }
   for (int s0 = p.sample_begin; s0 < p.sample_end; s0 += chunk) {
     P.per_sample_offset = s0 - p.sample_begin;
     P.hit_ids = (s0 == p.sample_begin) ? p.hit_ids : nullptr;
@@ -462,6 +584,17 @@ int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_
     // textures and the environment may still be in flight on the upload's copy stream: the primary trace reads
     // nodes and triangles only, everything after it waits here (rt_scene.cu)
     if (s0 == p.sample_begin && p.shading_ready) cudaStreamWaitEvent(stream, p.shading_ready, 0);
+    if (s0 == p.sample_begin && P.tiles) {
+      // every sample of the call's sky tiles in one launch, timed as a bounce-0 miss stage
+      StageParams S = P;
+      S.sample0 = p.sample_begin; S.n_samples = n_total;
+      S.per_sample_offset = 0;
+      S.hit_ids = p.hit_ids;
+      StageTimer st(RT_STAGE_MISS * RT_STAGE_BOUNCES, stream, t.dev);
+      if (p.fast) rt_fast_launch_sky(S, flat_grid(sm_count) * 4, stream);
+      else        rt_sky_kernel<<<flat_grid(sm_count) * 4, 256, 0, stream>>>(S);
+      launches++;
+    }
     for (int b = 0; b < p.max_bounces; b++) {
       P.bounce = b;
       const int bslot = b < RT_STAGE_BOUNCES ? b : RT_STAGE_BOUNCES - 1;

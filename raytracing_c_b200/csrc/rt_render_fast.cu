@@ -24,6 +24,10 @@ void rt_fast_launch_shade(const StageParams &P, unsigned grid, cudaStream_t stre
   rt_shade_kernel_fast<<<grid, 256, 0, stream>>>(P);
 }
 
+void rt_fast_launch_sky(const StageParams &P, unsigned grid, cudaStream_t stream) {
+  rt_sky_kernel_fast<<<grid, 256, 0, stream>>>(P);
+}
+
 int rt_fast_trace_setup(size_t level_bytes, int *wide_blocks_per_sm) {
   int n = 0, w = 0;
   cudaFuncSetAttribute(rt_trace_kernel_fast<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_MAX_DEPTH * 2 * RT_BLOCK * 16);

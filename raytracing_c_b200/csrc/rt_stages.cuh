@@ -63,7 +63,7 @@ struct PathQueues {
   unsigned *counts;                                 // [max_bounces + 1][Q_STRIDE]
 };
 
-struct StageParams {
+struct __align__(16) StageParams {
   SceneDev   scene;
   PathQueues q;
   int        width, height, tiles_x, tiles_y;
@@ -86,17 +86,37 @@ struct StageParams {
   // masked passes (rt_gpu_render_masked_device), last so that the fields above keep their offsets
   const unsigned char *pixel_mask;    // optional [pixel]: non-zero = render; read by the MASKED trace and accumulate only
   float     *accum_sq;                // optional [pixel][3]: sum of v * v in sample order
+  // optional job-tile lists of a render with sky tiles (rt_render.cu): [0] traced tiles, [1] sky tiles, then the traced
+  // tile ids ascending from [2] and the sky tile ids from [2 + n_tiles - 1] down.  The primary trace and the accumulate
+  // cover the traced tiles only (path ids are built on the list), rt_sky_kernel the sky tiles.  NULL = every tile traced.
+  const unsigned *tiles;
 };
 
-// raytracer.c:582-594, one lane of hash12x8
-__device__ __forceinline__ float fract1(float v) { return v - floorf(v); }
+// raytracer.c:582-594, one lane of hash12x8.  Ray generation is spelled with round-to-nearest intrinsics, which are
+// never fused: the exact build compiles them to what it compiles the plain operators to, and the fast build
+// (rt_render_fast.cu, FMA contraction on) generates the same rays as the exact one.
+__device__ __forceinline__ float fract1(float v) { return __fsub_rn(v, floorf(v)); }
 __device__ __forceinline__ float hash12(float px, float py) {
-  float a = fract1(px * 0.1031f);
-  float b = fract1(py * 0.1031f);
-  float c = fract1(px * 0.1031f);
+  float a = fract1(__fmul_rn(px, 0.1031f));
+  float b = fract1(__fmul_rn(py, 0.1031f));
+  float c = fract1(__fmul_rn(px, 0.1031f));
   float k = 33.33f;
-  float d = a * (b + k) + b * (c + k) + c * (a + k);
-  return fract1((a + b + d * 2.0f) * (c + d));
+  float d = __fadd_rn(__fadd_rn(__fmul_rn(a, __fadd_rn(b, k)), __fmul_rn(b, __fadd_rn(c, k))), __fmul_rn(c, __fadd_rn(a, k)));
+  return fract1(__fmul_rn(__fadd_rn(__fadd_rn(a, b), __fmul_rn(d, 2.0f)), __fadd_rn(c, d)));
+}
+
+// raytracer.c:644-677: the direction of camera sample s of pixel (px, py); rand_a == rand_b, exact 1/sqrt instead of
+// rsqrt_ps.  inv_w = 1 / width, inv_h = 1 / height, aspect = width / height.  The origin is the camera's (view column 3).
+__device__ __forceinline__ void camera_dir(const SceneDev &sc, int px, int py, int s, float inv_w, float inv_h, float aspect,
+                                           float &dx, float &dy, float &dz) {
+  const float jit = hash12(__fadd_rn(__fmul_rn((float)px, 50.0f), (float)s), (float)py);
+  const float ux = __fsub_rn(__fmul_rn(__fmul_rn(__fsub_rn(__fadd_rn((float)px, jit), 0.5f), 2.0f), inv_w), 1.0f);
+  const float uy = __fsub_rn(__fmul_rn(__fmul_rn(__fsub_rn(__fadd_rn((float)py, jit), 0.5f), 2.0f), inv_h), 1.0f);
+  const float cx = __fmul_rn(ux, aspect), cy = -uy, cz = -sc.focal_length;
+  const float inv_len = 1.0f / __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(cx, cx), __fmul_rn(cy, cy)), __fmul_rn(cz, cz)));
+  dx = __fmul_rn(__fadd_rn(__fadd_rn(__fmul_rn(sc.view[0][0], cx), __fmul_rn(sc.view[0][1], cy)), __fmul_rn(sc.view[0][2], cz)), inv_len);
+  dy = __fmul_rn(__fadd_rn(__fadd_rn(__fmul_rn(sc.view[1][0], cx), __fmul_rn(sc.view[1][1], cy)), __fmul_rn(sc.view[1][2], cz)), inv_len);
+  dz = __fmul_rn(__fadd_rn(__fadd_rn(__fmul_rn(sc.view[2][0], cx), __fmul_rn(sc.view[2][1], cy)), __fmul_rn(sc.view[2][2], cz)), inv_len);
 }
 
 // top-left pixel of job tile `tile` (8x4 pixels): row-major over the image, or — pixel-space split — the
@@ -124,11 +144,12 @@ __device__ __forceinline__ void path_pixel(const StageParams &P, unsigned path, 
 #if RT_PATH_LAYOUT == 1
   const unsigned pix = rt_fastdiv(path, P.div_samples, (unsigned)P.n_samples);
   ls = (int)(path - pix * (unsigned)P.n_samples);
-  const unsigned in_tile = pix & 31u, tile = pix >> 5;
+  const unsigned in_tile = pix & 31u, tile = P.tiles ? P.tiles[2 + (pix >> 5)] : pix >> 5;
 #else
   unsigned in_tile = path & 31u, rest = path >> 5;
   unsigned tile = rest / (unsigned)P.n_samples;
   ls = (int)(rest - tile * (unsigned)P.n_samples);
+  if (P.tiles) tile = P.tiles[2 + tile];
 #endif
   int x0, y0;
   tile_origin(P, tile, x0, y0);
@@ -188,7 +209,7 @@ RT_KN(rt_trace_kernel)(const __grid_constant__ StageParams P) {
   const unsigned lt_mask = (1u << lane) - 1u;
   float4 *levels = level_store + threadIdx.x;
   unsigned *counts = P.q.counts + P.bounce * Q_STRIDE;
-  const unsigned n_in = PRIMARY ? P.n_paths : counts[Q_RAYS];
+  const unsigned n_in = PRIMARY ? (P.tiles ? P.tiles[0] * 32u * (unsigned)P.n_samples : P.n_paths) : counts[Q_RAYS];
   unsigned c_rays = 0, c_nodes = 0, c_leaves = 0, c_accepts = 0, c_root_miss = 0;
 
   const float inv_w = 1.0f / (float)P.width, inv_h = 1.0f / (float)P.height;
@@ -289,16 +310,8 @@ RT_KN(rt_trace_kernel)(const __grid_constant__ StageParams P) {
             ok = px < P.width && py < P.height;
             if (MASKED && ok) ok = P.pixel_mask[py * P.width + px] != 0;
             if (ok) {
-              // raytracer.c:644-677; rand_a == rand_b; exact 1/sqrt instead of rsqrt_ps
               const int s = P.sample0 + ls;
-              float jit = hash12((float)px * 50.0f + (float)s, (float)py);
-              float ux = ((float)px + jit - 0.5f) * 2.0f * inv_w - 1.0f;
-              float uy = ((float)py + jit - 0.5f) * 2.0f * inv_h - 1.0f;
-              float cx = ux * aspect, cy = -uy, cz = -sc.focal_length;
-              float inv_len = 1.0f / __fsqrt_rn(cx * cx + cy * cy + cz * cz);
-              dx = (sc.view[0][0] * cx + sc.view[0][1] * cy + sc.view[0][2] * cz) * inv_len;
-              dy = (sc.view[1][0] * cx + sc.view[1][1] * cy + sc.view[1][2] * cz) * inv_len;
-              dz = (sc.view[2][0] * cx + sc.view[2][1] * cy + sc.view[2][2] * cz) * inv_len;
+              camera_dir(sc, px, py, s, inv_w, inv_h, aspect, dx, dy, dz);
               ox = sc.view[0][3]; oy = sc.view[1][3]; oz = sc.view[2][3];       // raytracer.c:612
               seed0 = rt_path_seed((uint32_t)(py * P.width + px), (uint32_t)s, P.user_seed);
             }
@@ -388,6 +401,72 @@ RT_KN(rt_miss_kernel)(const __grid_constant__ StageParams P) {
   if (P.counters) {
     add_counter(P.counters, 5, done);
     add_counter(P.counters, 7, done);
+  }
+}
+
+// ------------------------------------------------------------------------ sky
+// The camera samples of the sky tiles: job tiles no jittered camera ray of which can reach the root-union box
+// (rt_render.cu), so every such ray is one the primary trace would end at walk_misses_root and the bounce-0 miss kernel
+// would give the environment.  Here that is done without the path queues: one thread per pixel (a warp is one sky tile,
+// so its lanes look up neighbouring directions together), looping over the call's samples [sample0, sample0 + n_samples)
+// and summing each one as it comes — the sum (and v * v) in sample order exactly as accumulate_pixels forms it.  The
+// counters gain what the trace and the miss kernel add for such rays.
+// P.accumulate: the sum starts from P.accum (else +0); P.hit_ids gets -1 (no primary hit) for the call's first sample.
+// 60 registers, 4 blocks per SM: 4.36 ms for the 286 M sky samples of a 256-spp helmet frame.  Capped at 48 / 40 registers
+// (5 / 6 blocks) the environment lookup spills: the bounce-0 miss stage (miss + sky) takes 7.09 / 7.12 / 7.22 ms at 4 / 5 / 6
+#ifndef RT_SKY_MIN_BLOCKS
+#define RT_SKY_MIN_BLOCKS 4
+#endif
+__global__ void __launch_bounds__(256, RT_SKY_MIN_BLOCKS)
+RT_KN(rt_sky_kernel)(const __grid_constant__ StageParams P) {
+  const SceneDev &sc = P.scene;
+  const float inv_w = 1.0f / (float)P.width, inv_h = 1.0f / (float)P.height;
+  const float aspect = (float)P.width / (float)P.height;
+  const unsigned n_pixels = P.tiles[1] * 32u;
+  const unsigned *sky = P.tiles + 2 + P.n_tiles - 1;          // sky tile j at sky[-j]
+  unsigned c_samples = 0;
+  for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n_pixels; i += gridDim.x * blockDim.x) {
+    int x0, y0;
+    tile_origin(P, sky[-(int)(i >> 5)], x0, y0);
+    const int px = x0 + (int)(i & 7u), py = y0 + (int)((i >> 3) & 3u);
+    if (px >= P.width || py >= P.height) continue;
+    const int pixel = py * P.width + px;
+    if (P.pixel_mask && !P.pixel_mask[pixel]) {              // as the masked accumulate: zeroed or left alone
+      if (!P.accumulate) {
+        P.accum[3 * pixel + 0] = 0; P.accum[3 * pixel + 1] = 0; P.accum[3 * pixel + 2] = 0;
+        if (P.accum_sq) { P.accum_sq[3 * pixel + 0] = 0; P.accum_sq[3 * pixel + 1] = 0; P.accum_sq[3 * pixel + 2] = 0; }
+      }
+      continue;
+    }
+    V3 sum = P.accumulate ? mk3(P.accum[3 * pixel], P.accum[3 * pixel + 1], P.accum[3 * pixel + 2]) : mk3(0, 0, 0);
+    V3 sq = mk3(0, 0, 0);
+    if (P.accum_sq && P.accumulate) sq = mk3(P.accum_sq[3 * pixel], P.accum_sq[3 * pixel + 1], P.accum_sq[3 * pixel + 2]);
+    for (int s = 0; s < P.n_samples; s++) {
+      float dx, dy, dz;
+      camera_dir(sc, px, py, P.sample0 + s, inv_w, inv_h, aspect, dx, dy, dz);
+      const V3 v = environment(sc, mk3(dx, dy, dz));          // bounce 0: tint 1, emission 0 (rt_miss_kernel)
+      sum = add3(sum, v);
+      if (P.accum_sq) sq = add3(sq, mul3(v, v));
+      if (P.per_sample) {
+        float *dst = P.per_sample + ((size_t)pixel * (size_t)P.per_sample_stride + (size_t)(P.per_sample_offset + s)) * 3;
+        dst[0] = v.x; dst[1] = v.y; dst[2] = v.z;
+      }
+    }
+    P.accum[3 * pixel + 0] = sum.x; P.accum[3 * pixel + 1] = sum.y; P.accum[3 * pixel + 2] = sum.z;
+    if (P.accum_sq) { P.accum_sq[3 * pixel + 0] = sq.x; P.accum_sq[3 * pixel + 1] = sq.y; P.accum_sq[3 * pixel + 2] = sq.z; }
+    if (P.hit_ids) P.hit_ids[pixel] = -1;
+    c_samples += (unsigned)P.n_samples;
+  }
+  // per ray: the trace's ray, root visit and root-union miss (and primary ray), the miss kernel's miss and sample
+  if (P.counters) {
+    add_counter(P.counters, 0, c_samples);
+    add_counter(P.counters, 1, c_samples);
+    add_counter(P.counters, 5, c_samples);
+    add_counter(P.counters, 7, c_samples);
+  }
+  if (P.counters_ex) {
+    add_counter(P.counters_ex, 0, c_samples);
+    add_counter(P.counters_ex, 1, c_samples);
   }
 }
 

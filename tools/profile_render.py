@@ -23,12 +23,15 @@ ap.add_argument("--spp", type=int, default=64)
 ap.add_argument("--reps", type=int, default=3)
 ap.add_argument("--denoise", action="store_true")
 ap.add_argument("--stages", action="store_true", help="print CUDA-event time per stage and bounce of the last rep")
+ap.add_argument("--eye", type=float, nargs=3, default=None, help="camera position (with --target; default: the model's camera)")
+ap.add_argument("--target", type=float, nargs=3, default=(0.0, 0.0, 0.0))
 args = ap.parse_args()
 
 gpu = gpu_lib()
 gpu_check(gpu.rt_gpu_init(0))
 torch.cuda.set_device(0)
-loaded = driver.load_scene(os.path.join(ROOT, "assets", "models", args.model))
+camera = driver.look_at(args.eye, args.target) if args.eye else None
+loaded = driver.load_scene(os.path.join(ROOT, "assets", "models", args.model), camera=camera)
 driver.register_callbacks(loaded)
 scene = C.byref(loaded.scene)
 gpu_check(gpu.rt_gpu_scene_upload(scene))
