@@ -14,6 +14,7 @@
 //                                  vertex normals, tangent, bitangent, three UVs,
 //                                  material index (Triangle_AOS with the Shader
 //                                  function pointer replaced by a table index).
+//                                  Read through the rec_* accessors below.
 //   materials, textures            PBR_Shader_Data with Image* -> texture slot;
 //                                  texels repacked RGB8 -> RGBA8 (one 32-bit load per tap).
 // Everything is read-only during a render and small enough (<= ~75 MB with the
@@ -105,3 +106,23 @@ __device__ __forceinline__ V3 lerp3(V3 a, V3 b, float t) { return mk3(lerp1(a.x,
 __device__ __forceinline__ float sel_min(float a, float b) { return a < b ? a : b; }   // MINPS: b when unordered
 __device__ __forceinline__ float sel_max(float a, float b) { return a > b ? a : b; }   // MAXPS: b when unordered
 __device__ __forceinline__ float clamp1(float x, float lo, float hi) { return x < lo ? lo : (x > hi ? hi : x); }
+
+// ---- the shading record of a hit (tri_rec above, rows r0..r6 as float4): raytracer.c:164-182 in the f32 expressions
+// every reader uses.  Barycentric weights of hit (u, v): w1 = u, w2 = v, w0 = 1 - w1 - w2 (raytracer.c:164-166).
+__device__ __forceinline__ V3 rec_normal_geo(float4 r0) { return mk3(r0.x, r0.y, r0.z); }
+// the vertex normals (r0.w, r1.xy) (r1.zw, r2.x) (r2.yzw), interpolated (raytracer.c:167-172; not normalised)
+__device__ __forceinline__ V3 rec_normal(float4 r0, float4 r1, float4 r2, float w0, float w1, float w2) {
+  return mk3(r0.w * w0 + r1.z * w1 + r2.y * w2,
+             r1.x * w0 + r1.w * w1 + r2.z * w2,
+             r1.y * w0 + r2.x * w1 + r2.w * w2);
+}
+// the three UVs (r4.zw) (r5.xy) (r5.zw), interpolated (raytracer.c:175-176)
+__device__ __forceinline__ float rec_tex_u(float4 r4, float4 r5, float w0, float w1, float w2) { return r4.z * w0 + r5.x * w1 + r5.z * w2; }
+__device__ __forceinline__ float rec_tex_v(float4 r4, float4 r5, float w0, float w1, float w2) { return r4.w * w0 + r5.y * w1 + r5.w * w2; }
+__device__ __forceinline__ V3 rec_tangent(float4 r3) { return mk3(r3.x, r3.y, r3.z); }
+__device__ __forceinline__ V3 rec_bitangent(float4 r3, float4 r4) { return mk3(r3.w, r4.x, r4.y); }
+__device__ __forceinline__ int rec_material(float4 r6) { return __float_as_int(r6.x); }
+// the hit point o + d * t (raytracer.c:173)
+__device__ __forceinline__ V3 hit_point(V3 o, V3 d, float t) { return add3(o, scale3(d, t)); }
+// raytracer.c:516: the ray leaves through the back of the geometric or of the interpolated normal
+__device__ __forceinline__ bool hit_back_face(V3 ng, V3 normal, V3 d) { return dot3(ng, d) > 0 || dot3(normal, d) > 0; }

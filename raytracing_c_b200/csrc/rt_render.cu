@@ -349,25 +349,17 @@ static int fit_chunk(StageParams &P, size_t paths_per_sample, int n_samples, siz
 
 // Dynamic shared memory opt-in and occupancy of the trace kernels on the current device (once per device and depth).
 static int trace_launch_setup(const SceneDev &scene, int sm_count, TraceLaunch &t) {
-  // level store: [depth - 1][2][RT_BLOCK] float4 of dynamic shared memory (see rt_trace.cuh)
-  // (levels 2 .. depth only: 24 KB per block for the depth-4 trees of the shipped models; the driver's default carve-out is the
-  // smallest that holds the resident blocks — forcing a larger one costs up to 6 %, L1 beyond 96 KB gains nothing: measured)
-  const size_t level_bytes = (size_t)(scene.depth > 1 ? scene.depth - 1 : 1) * 2 * RT_BLOCK * sizeof(float4);
+  const size_t level_bytes = level_store_bytes(scene.depth);
   int dev = 0;
   cudaGetDevice(&dev);
   if (dev < 0 || dev >= RT_MAX_DEVICES) return (int)cudaErrorInvalidDevice;
   TraceOccupancy &o = g_occupancy[dev];
   if (o.generic == 0 || level_bytes != o.level_bytes) {
-    auto blocks_per_sm = [&](const void *kernel) {
-      int n = 0;
-      cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_MAX_DEPTH * 2 * RT_BLOCK * 16);
-      return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel, RT_BLOCK, level_bytes) == cudaSuccess && n >= 1 ? n : 1;
-    };
-    o.primary = blocks_per_sm((const void *)rt_trace_kernel<true>);
-    o.generic = blocks_per_sm((const void *)rt_trace_kernel<false>);
-    o.wide = blocks_per_sm((const void *)rt_trace_kernel<false, RT_TRACE_MIN_BLOCKS_WIDE>);
+    o.primary = level_store_blocks_per_sm((const void *)rt_trace_kernel<true>, level_bytes);
+    o.generic = level_store_blocks_per_sm((const void *)rt_trace_kernel<false>, level_bytes);
+    o.wide = level_store_blocks_per_sm((const void *)rt_trace_kernel<false, RT_TRACE_MIN_BLOCKS_WIDE>, level_bytes);
     o.fast = rt_fast_trace_setup(level_bytes, &o.fast_wide);
-    o.masked = blocks_per_sm((const void *)rt_trace_kernel<true, RT_TRACE_MIN_BLOCKS_PRIMARY, true>);
+    o.masked = level_store_blocks_per_sm((const void *)rt_trace_kernel<true, RT_TRACE_MIN_BLOCKS_PRIMARY, true>, level_bytes);
     o.level_bytes = level_bytes;
   }
   t = TraceLaunch{dev, level_bytes, (unsigned)(sm_count * o.primary), (unsigned)(sm_count * o.generic),
@@ -725,6 +717,8 @@ rt_lightmap_raygen_kernel(const __grid_constant__ StageParams P, const LightmapP
                               soa[6 * N] * w0 + soa[7 * N] * w1 + soa[8 * N] * w2);
       const float4 *rec = sc.tri_rec + (size_t)slot * 7;
       const float4 r0 = __ldg(rec), r1 = __ldg(rec + 1), r2 = __ldg(rec + 2);
+      // rec_normal's expressions (rt_device.cuh), written out: through the call one instruction of this kernel is
+      // scheduled one slot later
       const V3 normal = mk3(r0.w * w0 + r1.z * w1 + r2.y * w2, r1.x * w0 + r1.w * w1 + r2.z * w2, r1.y * w0 + r2.x * w1 + r2.w * w2);
       o = add3(position, scale3(normal, RT_EPS));
       uint32_t dir_state = rt_path_seed(texel, (uint32_t)s, P.user_seed ^ RT_LIGHTMAP_DIR_SALT);
@@ -1022,14 +1016,11 @@ rt_aov_surface_kernel(const __grid_constant__ StageParams P) {
       // shade_hit's point, interpolated normal and back-face test (rt_stages.cuh)
       const float4 *rec = sc.tri_rec + (size_t)slot * 7;
       const float4 r0 = __ldg(rec + 0), r1 = __ldg(rec + 1), r2 = __ldg(rec + 2);
-      const V3 ng = mk3(r0.x, r0.y, r0.z);
-      const V3 na = mk3(r0.w, r1.x, r1.y), nb = mk3(r1.z, r1.w, r2.x), nc = mk3(r2.y, r2.z, r2.w);
+      const V3 ng = rec_normal_geo(r0);
       const float w1 = h.y, w2 = h.z, w0 = 1 - w1 - w2;
-      const V3 point = add3(o, scale3(d, h.x));
-      const V3 normal = mk3(na.x * w0 + nb.x * w1 + nc.x * w2,
-                            na.y * w0 + nb.y * w1 + nc.y * w2,
-                            na.z * w0 + nb.z * w1 + nc.z * w2);
-      if (dot3(ng, d) > 0 || dot3(normal, d) > 0) {
+      const V3 point = hit_point(o, d, h.x);
+      const V3 normal = rec_normal(r0, r1, r2, w0, w1, w2);
+      if (hit_back_face(ng, normal, d)) {
         c_pass++;
         cont = P.bounce + 1 < P.max_bounces;
         const V3 next = add3(point, scale3(d, RT_EPS));
@@ -1080,22 +1071,13 @@ rt_aov_accumulate_kernel(const __grid_constant__ StageParams P, float4 *__restri
       const float4 *rec = sc.tri_rec + (size_t)slot * 7;
       const float4 r0 = __ldg(rec + 0), r1 = __ldg(rec + 1), r2 = __ldg(rec + 2), r3 = __ldg(rec + 3);
       const float4 r4 = __ldg(rec + 4), r5 = __ldg(rec + 5), r6 = __ldg(rec + 6);
-      const V3 na = mk3(r0.w, r1.x, r1.y), nb = mk3(r1.z, r1.w, r2.x), nc = mk3(r2.y, r2.z, r2.w);
       const float w1 = bary.x, w2 = bary.y, w0 = 1 - w1 - w2;
-      const V3 normal = mk3(na.x * w0 + nb.x * w1 + nc.x * w2,
-                            na.y * w0 + nb.y * w1 + nc.y * w2,
-                            na.z * w0 + nb.z * w1 + nc.z * w2);
-      ShadeIn in;
-      in.dir = mk3(0, 0, 0);                                         // the material fetch does not read it
-      in.normal = normalize3(normal);
-      in.normal_geo = mk3(r0.x, r0.y, r0.z);
-      in.tangent   = mk3(r3.x, r3.y, r3.z);
-      in.bitangent = mk3(r3.w, r4.x, r4.y);
-      in.u = r4.z * w0 + r5.x * w1 + r5.z * w2;
-      in.v = r4.w * w0 + r5.y * w1 + r5.w * w2;
+      const V3 normal = rec_normal(r0, r1, r2, w0, w1, w2);
+      // the material fetch does not read the direction
+      const ShadeIn in = shade_input(mk3(0, 0, 0), normal, rec_normal_geo(r0), r3, r4, r5, w0, w1, w2);
       V3 nrm, base, glow;
       float roughness, metalness;
-      pbr_surface(sc, sc.materials[__float_as_int(r6.x)], in, nrm, base, roughness, metalness, glow);
+      pbr_surface(sc, sc.materials[rec_material(r6)], in, nrm, base, roughness, metalness, glow);
       const float dx = surf.x - ex, dy = surf.y - ey, dz = surf.z - ez;
       const float depth = __fsqrt_rn(dx * dx + dy * dy + dz * dz);
       s0.x += base.x; s0.y += base.y; s0.z += base.z; s0.w += 1.0f;

@@ -29,11 +29,6 @@ void rt_fast_launch_sky(const StageParams &P, unsigned grid, cudaStream_t stream
 }
 
 int rt_fast_trace_setup(size_t level_bytes, int *wide_blocks_per_sm) {
-  int n = 0, w = 0;
-  cudaFuncSetAttribute(rt_trace_kernel_fast<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_MAX_DEPTH * 2 * RT_BLOCK * 16);
-  cudaFuncSetAttribute(rt_trace_kernel_fast<false, RT_TRACE_MIN_BLOCKS_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_MAX_DEPTH * 2 * RT_BLOCK * 16);
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, rt_trace_kernel_fast<false>, RT_BLOCK, level_bytes) != cudaSuccess || n < 1) n = 1;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&w, rt_trace_kernel_fast<false, RT_TRACE_MIN_BLOCKS_WIDE>, RT_BLOCK, level_bytes) != cudaSuccess || w < 1) w = 1;
-  *wide_blocks_per_sm = w;
-  return n;
+  *wide_blocks_per_sm = level_store_blocks_per_sm((const void *)rt_trace_kernel_fast<false, RT_TRACE_MIN_BLOCKS_WIDE>, level_bytes);
+  return level_store_blocks_per_sm((const void *)rt_trace_kernel_fast<false>, level_bytes);
 }

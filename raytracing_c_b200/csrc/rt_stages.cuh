@@ -32,18 +32,8 @@
 #ifndef RT_TRACE_WIDE_BOUNCES
 #define RT_TRACE_WIDE_BOUNCES 2
 #endif
-#define RT_FULL 0xffffffffu
-// rays a warp reserves per atomic on a long queue: 5823 / 5500 / 5372 / 5411 / 5831 us for the primary trace of a 64-spp helmet
-// chunk at 64 / 128 / 256 / 512 / 1024 (consecutive ids are neighbouring pixels: short shares scatter a warp over the image
-// and lose L1 reuse, long ones unbalance the last wave)
 #ifndef RT_EMIT_ONE_ATOMIC
 #define RT_EMIT_ONE_ATOMIC 1
-#endif
-#ifndef RT_BATCH_MAX
-#define RT_BATCH_MAX 256u
-#endif
-#ifndef RT_ROOT_STEP_AT_REFILL
-#define RT_ROOT_STEP_AT_REFILL 1
 #endif
 
 // counts[bounce][...]: queue lengths written by one stage and read by the next
@@ -157,44 +147,10 @@ __device__ __forceinline__ void path_pixel(const StageParams &P, unsigned path, 
   py = y0 + (int)(in_tile >> 3);
 }
 
-__device__ __forceinline__ void add_counter(unsigned long long *counters, int k, unsigned v) {
-  v += __shfl_xor_sync(RT_FULL, v, 16);
-  v += __shfl_xor_sync(RT_FULL, v, 8);
-  v += __shfl_xor_sync(RT_FULL, v, 4);
-  v += __shfl_xor_sync(RT_FULL, v, 2);
-  v += __shfl_xor_sync(RT_FULL, v, 1);
-  if ((threadIdx.x & 31) == 0 && v) atomicAdd(&counters[k], (unsigned long long)v);
-}
-
-// warp-aggregated append: returns this lane's slot in the queue whose length is *count
-__device__ __forceinline__ unsigned warp_append(unsigned *count, bool want, unsigned lane) {
-  const unsigned mask = __ballot_sync(RT_FULL, want);
-  unsigned base = 0;
-  if (lane == 0 && mask) base = atomicAdd(count, (unsigned)__popc(mask));
-  base = __shfl_sync(RT_FULL, base, 0);
-  return base + (unsigned)__popc(mask & ((1u << lane) - 1u));
-}
-
 // ---------------------------------------------------------------------- trace
-// Persistent warps pull rays from the input queue (the GPU form of the reference's atomic
-// 32x32 chunk queue, raytracer.c:619-627) and keep their lanes full: whenever RT_REFILL_MIN_*
-// lanes have finished, those lanes append their results to the HIT / MISS queues and take the
-// next rays, while the others keep their walk state.  PRIMARY: the ray is generated from the
-// path id — 32 consecutive ids are 32 samples of one pixel (RT_PATH_LAYOUT 1), so a warp's rays are coherent.
-#ifndef RT_MIN_BATCH
-#define RT_MIN_BATCH 4u
-#endif
-// Lanes that must have finished before the warp stops to emit results and take new rays.  The stop
-// itself costs ~300 instructions at partial width, waiting costs idle lanes: measured optimum is "all
-// 32" for primary rays (most finish in the same turn anyway; 9.17 / 8.60 / 8.20 / 8.08 ms per 64-spp
-// chunk at 8 / 16 / 24 / 32) and 20 for bounce rays (7.36 / 7.15 / 7.13 / 7.27 / 8.90 ms at 12 / 16 / 20 / 24 / 32).
-#ifndef RT_REFILL_MIN_PRIMARY
-#define RT_REFILL_MIN_PRIMARY 32
-#endif
-#ifndef RT_REFILL_MIN_BOUNCE
-#define RT_REFILL_MIN_BOUNCE 20
-#endif
-
+// Persistent warps walk the input queue's rays, scheduled as rt_trace.cuh describes: whenever RT_REFILL_MIN_* lanes have
+// finished, those lanes append their results to the HIT / MISS queues and take the next rays.  PRIMARY: the ray is generated from the path id — 32 consecutive ids are 32 samples of one pixel
+// (RT_PATH_LAYOUT 1), so a warp's rays are coherent.
 // MIN_BLOCKS: resident blocks per SM the kernel is compiled for.  Coherent primary rays gain from a fourth block
 // (64 registers; -2.8 % on their kernel).  Bounce rays: the long queues of the first bounces gain too (-2.7 % at
 // bounce 1: more warps to cover the divergent loads), the short late queues lose 5-10 % to it (their time is the
@@ -220,17 +176,8 @@ RT_KN(rt_trace_kernel)(const __grid_constant__ StageParams P) {
   bool     exhausted = false;
   unsigned q = 0, range_next = 0, range_end = 0;
   uint32_t seed0 = 0;                      // primary: the path's RNG seed, fixed when the ray is generated
-  // rays reserved per atomic: large queues amortise the round trip, small ones (late bounces)
-  // spread over all warps of the grid
   const unsigned total_warps = gridDim.x * (RT_BLOCK / 32);
-  unsigned batch = (n_in / (total_warps * 4u)) & ~31u;
-  if (batch > RT_BATCH_MAX) batch = RT_BATCH_MAX;
-  if (batch < 32u) {
-    // a short queue: one share per warp, so the kernel lasts as long as a few rays, not as 32 in lock step
-    batch = (n_in + total_warps - 1u) / total_warps;
-    if (batch < RT_MIN_BATCH) batch = RT_MIN_BATCH;
-    if (batch > 32u) batch = 32u;
-  }
+  unsigned batch = ray_batch_first(n_in, total_warps);
 
   unsigned walking = 0;                    // lanes whose walk is not finished (WALK_LIVE), kept current across turns
   for (;;) {
@@ -285,18 +232,11 @@ RT_KN(rt_trace_kernel)(const __grid_constant__ StageParams P) {
       if (!exhausted) {
         const unsigned idle = ~walking;
         if (range_next >= range_end) {
-          unsigned base = 0;
-          if (lane == 0) base = atomicAdd(&counts[Q_FETCH], batch);
-          base = __shfl_sync(RT_FULL, base, 0);
+          const unsigned base = ray_fetch(&counts[Q_FETCH], batch, lane);
           exhausted = base >= n_in;
           range_next = base;
           range_end = exhausted ? base : min(base + batch, n_in);
-          // guided self-scheduling: shares shrink as the queue drains, so the kernel's last wave is
-          // short (a 256-ray share held by one warp while the others idle is ~8 steps of 32 rays)
-          if (batch > 32u) {
-            const unsigned share = ((n_in - range_end) / (total_warps * 2u)) & ~31u;
-            batch = share < 32u ? 32u : (share < batch ? share : batch);
-          }
+          batch = ray_batch_next(batch, n_in - range_end, total_warps);
         }
         const unsigned take = min((unsigned)__popc(idle), range_end - range_next);
         const unsigned rank = (unsigned)__popc(idle & lt_mask);
@@ -323,10 +263,8 @@ RT_KN(rt_trace_kernel)(const __grid_constant__ StageParams P) {
             walk_begin(w, sc, ox, oy, oz, dx, dy, dz);
             c_rays++;
             if (walk_misses_root<PRIMARY>(w, sc)) { w.flags = WALK_RAY; c_nodes++; c_root_miss++; }      // the root visit, nothing entered
-#if RT_ROOT_STEP_AT_REFILL
             // the root visit here, among the lanes that just took a ray (all at the same node), instead of in a voted turn
             else walk_node_step<PRIMARY, true>(w, sc, levels, c_nodes);
-#endif
           }
         }
         range_next += take;
@@ -349,14 +287,7 @@ RT_KN(rt_trace_kernel)(const __grid_constant__ StageParams P) {
       __syncwarp();
       if (w.flags & WALK_LEAF) walk_leaf<PRIMARY>(w, sc, c_leaves, c_accepts);
     } else {
-      // incoherent rays: one step for the majority — node steps and leaf tests are different code, so the
-      // warp runs whichever more lanes wait for and the others keep their state for a later turn
-      const unsigned want_leaf = __ballot_sync(RT_FULL, w.flags & WALK_LEAF);
-      if (2 * __popc(want_leaf) <= __popc(walking)) {        // node steps wanted by at least as many lanes
-        if ((w.flags & (WALK_LIVE | WALK_LEAF)) == WALK_LIVE) walk_node_step<PRIMARY>(w, sc, levels, c_nodes);
-      } else {
-        if (w.flags & WALK_LEAF) walk_leaf<PRIMARY>(w, sc, c_leaves, c_accepts);
-      }
+      walk_turn_voted<PRIMARY>(w, sc, levels, walking, c_nodes, c_leaves, c_accepts);
     }
     walking = __ballot_sync(RT_FULL, w.flags & WALK_LIVE);
   }
@@ -474,6 +405,21 @@ RT_KN(rt_sky_kernel)(const __grid_constant__ StageParams P) {
 // raytracer.c:514-552 for one hit: attribute interpolation (:164-182), back-face
 // pass-through, BSDF, emission/tint update, next origin.  Survivors go to the RAY
 // queue of bounce + 1; paths that terminate or exhaust max_bounces (:557) write rad.
+// raytracer.c:164-182: the shading input at a front-face hit of direction dir, from rows 3..5 of its record, its
+// interpolated normal and its geometric normal
+__device__ __forceinline__ ShadeIn shade_input(V3 dir, V3 normal, V3 ng, float4 r3, float4 r4, float4 r5,
+                                               float w0, float w1, float w2) {
+  ShadeIn in;
+  in.dir = dir;
+  in.normal = normalize3(normal);
+  in.normal_geo = ng;
+  in.tangent   = rec_tangent(r3);
+  in.bitangent = rec_bitangent(r3, r4);
+  in.u = rec_tex_u(r4, r5, w0, w1, w2);
+  in.v = rec_tex_v(r4, r5, w0, w1, w2);
+  return in;
+}
+
 // One surface interaction of cast_ray (raytracer.c:514-552) for the hit (t, u, v, slot) of the ray (o, d): returns
 // whether the path goes on; o, d, tint, emis and rng are updated in place (emis is the path's radiance if it ends).
 __device__ __forceinline__ bool shade_hit(const SceneDev &sc, V3 &o, V3 &d, V3 &tint, V3 &emis,
@@ -481,31 +427,21 @@ __device__ __forceinline__ bool shade_hit(const SceneDev &sc, V3 &o, V3 &d, V3 &
                                           unsigned &c_shades, unsigned &c_pass) {
   const float4 *rec = sc.tri_rec + (size_t)slot * 7;
   float4 r0 = __ldg(rec + 0), r1 = __ldg(rec + 1), r2 = __ldg(rec + 2);
-  V3 ng = mk3(r0.x, r0.y, r0.z);
-  V3 na = mk3(r0.w, r1.x, r1.y), nb = mk3(r1.z, r1.w, r2.x), nc = mk3(r2.y, r2.z, r2.w);
+  V3 ng = rec_normal_geo(r0);
   float w1 = hit_u, w2 = hit_v, w0 = 1 - w1 - w2;                       // raytracer.c:164-177
-  V3 point  = add3(o, scale3(d, hit_t));
-  V3 normal = mk3(na.x * w0 + nb.x * w1 + nc.x * w2,
-                  na.y * w0 + nb.y * w1 + nc.y * w2,
-                  na.z * w0 + nb.z * w1 + nc.z * w2);
-  if (dot3(ng, d) > 0 || dot3(normal, d) > 0) {
+  V3 point  = hit_point(o, d, hit_t);
+  V3 normal = rec_normal(r0, r1, r2, w0, w1, w2);
+  if (hit_back_face(ng, normal, d)) {
     // raytracer.c:516-522: back face — step through, the bounce is consumed
     c_pass++;
     o = add3(point, scale3(d, RT_EPS));
     return true;
   }
   float4 r3 = __ldg(rec + 3), r4 = __ldg(rec + 4), r5 = __ldg(rec + 5), r6 = __ldg(rec + 6);
-  ShadeIn in;
-  in.dir = d;
-  in.normal = normalize3(normal);
-  in.normal_geo = ng;
-  in.tangent   = mk3(r3.x, r3.y, r3.z);
-  in.bitangent = mk3(r3.w, r4.x, r4.y);
-  in.u = r4.z * w0 + r5.x * w1 + r5.z * w2;
-  in.v = r4.w * w0 + r5.y * w1 + r5.w * w2;
+  ShadeIn in = shade_input(d, normal, ng, r3, r4, r5, w0, w1, w2);
   ShadeOut out;
   c_shades++;
-  shade_pbr(sc, __float_as_int(r6.x), in, rng, out);
+  shade_pbr(sc, rec_material(r6), in, rng, out);
   emis = add3(emis, mul3(out.emission, tint));          // raytracer.c:537
   if (out.terminate) return false;
   d = out.dir;

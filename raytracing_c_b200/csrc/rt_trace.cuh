@@ -17,7 +17,7 @@
 #ifndef RT_BLOCK
 #define RT_BLOCK 256
 #endif
-
+#define RT_FULL 0xffffffffu
 
 // raytracer.c:190-230 for ONE child box, general form: the reference's nested MINPS/MAXPS with
 // their "second operand when unordered" rule, as operand-order selects.  Needed only when a
@@ -119,6 +119,19 @@ __device__ __forceinline__ float min8(const float (&e)[8]) {
 // per-thread slice of the level store: levels[(level - 1) * 2 + half][tid]
 // (levels 2 .. depth: a node of level 1 hands out leaves and never parks its entries — its slot is not allocated)
 #define RT_LEVELS(level, half) levels[(((level) - 2) * 2 + (half)) * RT_BLOCK]
+
+// The level store of a block: [depth - 1][2][RT_BLOCK] float4 of dynamic shared memory (levels 2 .. depth only: 24 KB
+// per block for the depth-4 trees of the shipped models; the driver's default carve-out is the smallest that holds the
+// resident blocks — forcing a larger one costs up to 6 %, L1 beyond 96 KB gains nothing: measured)
+static inline size_t level_store_bytes(int depth) { return (size_t)(depth > 1 ? depth - 1 : 1) * 2 * RT_BLOCK * sizeof(float4); }
+
+// Opts a walking kernel in to the level store of the deepest tree and returns its resident blocks per SM at level_bytes
+// on the current device (at least 1).  cudaFuncSetAttribute is per device: callers keep the result per device.
+static inline int level_store_blocks_per_sm(const void *kernel, size_t level_bytes) {
+  int n = 0;
+  cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, RT_MAX_DEPTH * 2 * RT_BLOCK * 16);
+  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel, RT_BLOCK, level_bytes) == cudaSuccess && n >= 1 ? n : 1;
+}
 
 // raytracer.c:443-503: closest hit of one ray, one thread per ray, as a resumable walk.
 // The reference recursion (8 entry distances per level on the C stack, up to 8 selection
@@ -299,4 +312,96 @@ __device__ __forceinline__ void walk_leaf(RayWalk &w, const SceneDev &sc, unsign
   }
   if (w.hit_t < t_before) c_accepts++;
   w.flags &= ~WALK_LEAF;
+}
+
+// incoherent rays: one step for the majority — node steps and leaf tests are different code, so the warp runs whichever
+// more lanes wait for and the others keep their state for a later turn (`walking`: the lanes with WALK_LIVE)
+template <bool REL>
+__device__ __forceinline__ void walk_turn_voted(RayWalk &w, const SceneDev &sc, float4 *levels, unsigned walking,
+                                                unsigned &c_nodes, unsigned &c_leaves, unsigned &c_accepts) {
+  const unsigned want_leaf = __ballot_sync(RT_FULL, w.flags & WALK_LEAF);
+  if (2 * __popc(want_leaf) <= __popc(walking)) {        // node steps wanted by at least as many lanes
+    if ((w.flags & (WALK_LIVE | WALK_LEAF)) == WALK_LIVE) walk_node_step<REL>(w, sc, levels, c_nodes);
+  } else {
+    if (w.flags & WALK_LEAF) walk_leaf<REL>(w, sc, c_leaves, c_accepts);
+  }
+}
+
+// ------------------------------------------------------------------ scheduling
+// The warp-level scheduling of every walk over an input of rays: the trace kernel (rt_stages.cuh) and the ray queries
+// (rt_query.cu) share its constants, the reservation of ray ranges and the voted turn.  Persistent warps pull rays from
+// the input (the GPU form of the reference's atomic 32x32 chunk queue, raytracer.c:619-627) and keep their lanes full:
+// whenever RT_REFILL_MIN_* lanes have finished, those lanes hand on their results and take the next rays of the warp's
+// reserved range, while the others keep their walk state.
+
+// rays a warp reserves per atomic on a long queue: 5823 / 5500 / 5372 / 5411 / 5831 us for the primary trace of a 64-spp helmet
+// chunk at 64 / 128 / 256 / 512 / 1024 (consecutive ids are neighbouring pixels: short shares scatter a warp over the image
+// and lose L1 reuse, long ones unbalance the last wave)
+#ifndef RT_BATCH_MAX
+#define RT_BATCH_MAX 256u
+#endif
+#ifndef RT_MIN_BATCH
+#define RT_MIN_BATCH 4u
+#endif
+// Lanes that must have finished before the warp stops to emit results and take new rays.  The stop
+// itself costs ~300 instructions at partial width, waiting costs idle lanes: measured optimum is "all
+// 32" for primary rays (most finish in the same turn anyway; 9.17 / 8.60 / 8.20 / 8.08 ms per 64-spp
+// chunk at 8 / 16 / 24 / 32) and 20 for bounce rays (7.36 / 7.15 / 7.13 / 7.27 / 8.90 ms at 12 / 16 / 20 / 24 / 32).
+#ifndef RT_REFILL_MIN_PRIMARY
+#define RT_REFILL_MIN_PRIMARY 32
+#endif
+#ifndef RT_REFILL_MIN_BOUNCE
+#define RT_REFILL_MIN_BOUNCE 20
+#endif
+
+__device__ __forceinline__ void add_counter(unsigned long long *counters, int k, unsigned v) {
+  v += __shfl_xor_sync(RT_FULL, v, 16);
+  v += __shfl_xor_sync(RT_FULL, v, 8);
+  v += __shfl_xor_sync(RT_FULL, v, 4);
+  v += __shfl_xor_sync(RT_FULL, v, 2);
+  v += __shfl_xor_sync(RT_FULL, v, 1);
+  if ((threadIdx.x & 31) == 0 && v) atomicAdd(&counters[k], (unsigned long long)v);
+}
+
+// warp-aggregated append: returns this lane's slot in the queue whose length is *count
+__device__ __forceinline__ unsigned warp_append(unsigned *count, bool want, unsigned lane) {
+  const unsigned mask = __ballot_sync(RT_FULL, want);
+  unsigned base = 0;
+  if (lane == 0 && mask) base = atomicAdd(count, (unsigned)__popc(mask));
+  base = __shfl_sync(RT_FULL, base, 0);
+  return base + (unsigned)__popc(mask & ((1u << lane) - 1u));
+}
+
+// The reservation of a warp's ray ranges: the caller keeps the range and the batch in its own variables, and the helpers
+// take and return plain values (helpers writing through references change the trace kernels' instruction schedule).
+
+// rays reserved per atomic: large queues amortise the round trip, small ones (late bounces)
+// spread over all warps of the grid
+__device__ __forceinline__ unsigned ray_batch_first(unsigned n_in, unsigned total_warps) {
+  unsigned batch = (n_in / (total_warps * 4u)) & ~31u;
+  if (batch > RT_BATCH_MAX) batch = RT_BATCH_MAX;
+  if (batch < 32u) {
+    // a short queue: one share per warp, so the kernel lasts as long as a few rays, not as 32 in lock step
+    batch = (n_in + total_warps - 1u) / total_warps;
+    if (batch < RT_MIN_BATCH) batch = RT_MIN_BATCH;
+    if (batch > 32u) batch = 32u;
+  }
+  return batch;
+}
+
+// the first index of the warp's next `batch` rays: one atomic on the input's fetch counter per range
+__device__ __forceinline__ unsigned ray_fetch(unsigned *fetch, unsigned batch, unsigned lane) {
+  unsigned base = 0;
+  if (lane == 0) base = atomicAdd(fetch, batch);
+  return __shfl_sync(RT_FULL, base, 0);
+}
+
+// guided self-scheduling: shares shrink as the queue drains (`left` rays after the range just reserved), so the kernel's
+// last wave is short (a 256-ray share held by one warp while the others idle is ~8 steps of 32 rays)
+__device__ __forceinline__ unsigned ray_batch_next(unsigned batch, unsigned left, unsigned total_warps) {
+  if (batch > 32u) {
+    const unsigned share = (left / (total_warps * 2u)) & ~31u;
+    batch = share < 32u ? 32u : (share < batch ? share : batch);
+  }
+  return batch;
 }
