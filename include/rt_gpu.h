@@ -331,6 +331,41 @@ int rt_gpu_render_masked_device(Scene const *scene, isize width, isize height,
 int rt_gpu_resolve_counts_device(f32 const *d_accum, i32 const *d_samples, isize width, isize height,
                                  u8 *d_pixels, isize stride, i32 components, void *stream);
 
+/* ---- moving geometry on a resident scene: refit the BVH and triangle records on the device (csrc/rt_refit.cu) ----
+ * A refit keeps the topology scene_init chose (which triangle sits in which slot, which child is which) and recomputes,
+ * from new vertex positions, everything that depends on them, with host/scene_build.c's f32 expressions:
+ *   - per occupied slot: the vertex arrays, the edges, the geometric normal, tangent and bitangent (pack_leaf), and the
+ *     vertex normals when given; UVs and materials are kept;
+ *   - per node child: the union of the subtree's triangle boxes inflated by EPSILON, exactly as scene_init computes it;
+ *     a child with no triangle keeps its all-zero box;
+ *   - the root-union box the renderer's sky tiles and root shortcut use.
+ * So refitting unchanged positions reproduces scene_init's bytes, and every render, query, AOV call and lightmap bake
+ * afterwards equals the same call on a host Scene built with the new positions under the same topology.  The boxes are
+ * exact, but under large motion they overlap more and tracing slows down: when to rebuild with scene_init is the host's
+ * choice.
+ * Occupancy is the upload's: a slot is a triangle when its Triangle_AOS had a shader at upload.  Inputs of padding
+ * slots are ignored; those slots stay zero.
+ * Ordering: the refit waits on the device for every earlier render, lightmap bake, cast_rays, AOV, masked pass and
+ * query of the scene, and every later one waits for the refit; no caller needs a synchronisation of its own.  With
+ * several devices the peers receive the result over NVLink.
+ * The call SYNCHRONISES with the host before it returns (it reads back a validation flag and the root node).
+ * Refused, with the resident scene unchanged: a scene that is not resident (rt_gpu_scene_upload), NULL positions, a
+ * non-finite coordinate in an occupied slot. */
+/* device pointers on the first device, ordered on `stream` (cudaStream_t as void*, NULL = the legacy default stream).
+ * d_positions: f32[9][n_slots], the Scene's own block order x0 x1 x2 y0 y1 y2 z0 z1 z2; d_normals (optional):
+ * f32[n_slots][3][3], normal_a, normal_b, normal_c of each slot (Triangle_AOS order), NULL = keep.  The host buffers are
+ * not touched: a later rt_gpu_scene_upload, or the re-upload of a Scene whose buffers changed, replaces a device-only
+ * refit with what the host buffers hold. */
+int rt_gpu_scene_refit_device(Scene const *scene, f32 const *d_positions, f32 const *d_normals, void *stream);
+/* host form: the host has rewritten scene->triangles.x/y/z (and, with refit_normals, aos[s].normal_a/b/c) in slot
+ * order.  They are staged as the upload stages them (pinned memory in place, pageable through the staging ring), refit
+ * on the device, and the refit node boxes and each occupied slot's normal, tangent and bitangent are written back into
+ * scene->bvh.nodes.data and scene->triangles.aos; padding slots' positions (and normals) are zeroed.  Afterwards the host
+ * Scene is exactly what the device holds, for a CPU reference, a scene-cache save or a later re-upload. */
+int rt_gpu_scene_refit(Scene *scene, i32 refit_normals);
+/* parity hook: the node bytes resident on the first device (n_internal * 192 B into out) */
+int rt_gpu_read_nodes(Scene const *scene, BVH_Node *out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -144,6 +144,7 @@ GPU_EXPORTS = [
     "rt_gpu_cast_rays_device", "rt_gpu_cast_rays",
     "rt_gpu_render_aov_device", "rt_gpu_render_aov",
     "rt_gpu_render_masked_device", "rt_gpu_resolve_counts_device",
+    "rt_gpu_scene_refit_device", "rt_gpu_scene_refit", "rt_gpu_read_nodes",
 ]
 
 HOST_EXPORTS = [
@@ -151,7 +152,7 @@ HOST_EXPORTS = [
     "rt_image_decode", "rt_load_texture", "rt_image_free", "rt_image_alloc", "rt_generate_background",
     "rt_save_image", "rt_save_png", "rt_save_qoi", "rt_save_ppm", "rt_host_last_error",
     "rt_host_set_buffer_allocator", "rt_host_buffer_alloc", "rt_host_buffer_free", "rt_host_defer_jpeg_decode",
-    "scene_save_file", "scene_load_file",
+    "scene_save_file", "scene_load_file", "rt_scene_init_slots",
 ]
 
 
@@ -179,6 +180,8 @@ def host_lib() -> C.CDLL:
         lib.rt_load_model_file.argtypes = [C.c_char_p, C.c_void_p, C.POINTER(Model), C.POINTER(Camera)]
         lib.rt_model_free.argtypes = [C.POINTER(Model)]
         lib.scene_init.argtypes = [C.POINTER(Scene), TriangleSlice]
+        lib.rt_scene_init_slots.argtypes = [C.POINTER(Scene), TriangleSlice, C.c_void_p]
+        lib.rt_scene_init_slots.restype = None
         lib.scene_destroy.argtypes = [C.POINTER(Scene)]
         lib.rt_camera_default.argtypes = [C.POINTER(Camera)]
         lib.rt_camera_look_at.argtypes = [C.POINTER(Camera), Vec3, Vec3, Vec3, C.c_float]
@@ -282,6 +285,9 @@ def gpu_lib() -> C.CDLL:
                                                     C.c_uint32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.rt_gpu_resolve_counts_device.argtypes = [C.c_void_p, C.c_void_p, isize, isize, C.c_void_p, isize, C.c_int32,
                                                      C.c_void_p]
+        lib.rt_gpu_scene_refit_device.argtypes = [C.POINTER(Scene), C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.rt_gpu_scene_refit.argtypes = [C.POINTER(Scene), C.c_int32]
+        lib.rt_gpu_read_nodes.argtypes = [C.POINTER(Scene), C.c_void_p]
         lib.render_thread_proc.argtypes = [C.POINTER(RenderingContext)]
         lib.render_thread_proc.restype = None
         lib.rendering_context_is_finished.argtypes = [C.POINTER(RenderingContext)]

@@ -773,6 +773,28 @@ int rt_gpu_render_masked_device(Scene const *scene, isize width, isize height, u
                           d_mask, d_accum_sq);
 }
 
+// ------------------------------------------------------------------ moving geometry (rt_scene.cu: scene_refit)
+int rt_gpu_scene_refit_device(Scene const *scene, f32 const *d_positions, f32 const *d_normals, void *stream) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  if (scene_resident("scene_refit", scene)) return 1;
+  if (!d_positions) return fail("scene_refit: null positions");
+  return scene_refit(scene, d_positions, d_normals, 9, static_cast<cudaStream_t>(stream));
+}
+
+int rt_gpu_scene_refit(Scene *scene, i32 refit_normals) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  if (scene_resident("scene_refit", scene)) return 1;
+  if (!scene->triangles.x[0] || !scene->triangles.aos) return fail("scene_refit: null positions");
+  return scene_refit_host(scene, refit_normals != 0);
+}
+
+int rt_gpu_read_nodes(Scene const *scene, BVH_Node *out) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  if (scene_resident("read_nodes", scene)) return 1;
+  if (!out) return fail("read_nodes: null output");
+  return scene_read_nodes(scene, out);
+}
+
 // ----------------------------------------------------------------- parity hooks
 int rt_gpu_read_accum(f32 *out, isize n_floats) {
   std::lock_guard<std::mutex> lock(g_mutex);

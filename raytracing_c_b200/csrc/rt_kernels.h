@@ -56,6 +56,21 @@ int rt_launch_texel_expand(const uchar4 *src, size_t n, float4 *dst, cudaStream_
 // tri_pos / tri_rec from the host's vertex arrays, Triangle_AOS records and per-slot material indices (rt_denoise.cu)
 int rt_launch_scene_pack(const float *soa, const float4 *aos, const int *mat_index, int n_slots, float4 *tri_pos, float4 *tri_rec,
                          cudaStream_t stream);
+// refit of a resident scene from new positions (rt_refit.cu): validation, then one pass over the slots and one per
+// internal level, bottom-up.  A non-finite coordinate in an occupied slot sets *flag (zeroed by the caller) and nothing
+// is written.  masks: n_internal + n_slots / 8 bytes, the child (node) and slot (leaf) occupancy bits.
+struct RefitParams {
+  const float *positions;                // f32[9][n_slots]: x0 x1 x2 y0 y1 y2 z0 z1 z2
+  const float *normals;                  // optional: normal_a, normal_b, normal_c (9 floats) of slot s at normal_stride * s
+  int normal_stride;
+  int depth, n_internal, n_slots;
+  const unsigned char *masks;
+  int   *flag;
+  float *nodes;
+  float4 *tri_pos, *tri_rec;
+  float *tri_soa;
+};
+int rt_launch_refit(const RefitParams &p, cudaStream_t stream);
 // ray queries (rt_query.cu): closest hit (any = false: hits, optional surface) or occlusion (any = true: occluded)
 // of n_rays rays at their own index; `fetch` is a zeroed work counter no other launch uses at the same time
 struct QueryParams {

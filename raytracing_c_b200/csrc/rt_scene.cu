@@ -118,9 +118,9 @@ static int ring_init(Device &d) {
 }
 
 // asynchronous on d.copy; returns when the last piece is staged (pageable source) or at once (pinned source)
-static int h2d(Device &d, DeviceScene &ds, void *dst, const void *src, size_t n) {
+static int h2d(Device &d, size_t &counted, void *dst, const void *src, size_t n) {
   if (!n) return 0;
-  ds.h2d_bytes += n;
+  counted += n;
   if (is_pinned(src)) {
     CUDA_TRY(cudaMemcpyAsync(dst, src, n, cudaMemcpyHostToDevice, d.copy));
     return 0;
@@ -154,6 +154,7 @@ struct HostScene {
   int   depth = 0, n_internal = 0, n_slots = 0;
   float root_lo[3], root_hi[3];
   int   root_upper_empty = 0;             // children 4..7 of the root are padding (lo == hi on every axis)
+  std::vector<unsigned char> refit_masks; // occupancy of every node child and slot (rt_refit.cu)
   Fingerprint fp;
 };
 
@@ -163,6 +164,42 @@ static Fingerprint fingerprint(const Scene *scene) {
   f.background = scene->background.data;
   f.n_nodes = (long)scene->bvh.nodes.len; f.n_slots = (long)scene->triangles.len; f.depth = (long)scene->bvh.depth;
   return f;
+}
+
+// scene_init lays the nine vertex arrays out as one block x0 x1 x2 y0 y1 y2 z0 z1 z2 (scene.h:62-63, scene.c:86-96);
+// a host that assembled them differently gets them gathered into `copy` in that order
+static int vertex_block(const Scene *scene, std::vector<float> &copy, const float **out) {
+  const size_t n_slots = (size_t)scene->triangles.len;
+  const float *arrays[9] = { scene->triangles.x[0], scene->triangles.x[1], scene->triangles.x[2],
+                             scene->triangles.y[0], scene->triangles.y[1], scene->triangles.y[2],
+                             scene->triangles.z[0], scene->triangles.z[1], scene->triangles.z[2] };
+  bool one_block = true;
+  for (int a = 0; a < 9; a++) one_block &= arrays[a] == arrays[0] + (size_t)a * n_slots;
+  if (one_block) { *out = arrays[0]; return 0; }
+  copy.resize(n_slots * 9);
+  for (int a = 0; a < 9; a++) {
+    if (!arrays[a]) return fail("scene: null vertex array");
+    memcpy(copy.data() + (size_t)a * n_slots, arrays[a], n_slots * sizeof(float));
+  }
+  *out = copy.data();
+  return 0;
+}
+
+// union of the root's child boxes (n0: the root node's 48 floats); all-zero padding children (lo == hi) can never be
+// entered (enter >= leave), so they are left out.  The upload and every refit decide the box here.
+static void root_union(const float *n0, float lo[3], float hi[3], int *upper_empty) {
+  for (int a = 0; a < 3; a++) { lo[a] = INFINITY; hi[a] = -INFINITY; }
+  *upper_empty = 1;
+  for (int j = 0; j < 8; j++) {
+    bool empty = true;
+    for (int a = 0; a < 3; a++) empty &= (n0[a * 8 + j] == n0[(3 + a) * 8 + j]);
+    if (empty) continue;
+    if (j >= 4) *upper_empty = 0;
+    for (int a = 0; a < 3; a++) {
+      lo[a] = fminf(lo[a], n0[a * 8 + j]);
+      hi[a] = fmaxf(hi[a], n0[(3 + a) * 8 + j]);
+    }
+  }
 }
 
 static int flatten(const Scene *scene, HostScene &hs) {
@@ -177,25 +214,7 @@ static int flatten(const Scene *scene, HostScene &hs) {
 
   hs.nodes = reinterpret_cast<const float *>(scene->bvh.nodes.data);
   hs.aos = scene->triangles.aos;
-  // scene_init lays the nine vertex arrays out as one block x0 x1 x2 y0 y1 y2 z0 z1 z2 (scene.h:62-63, scene.c:86-96);
-  // a host that assembled them differently gets them gathered into that order
-  {
-    const float *arrays[9] = { scene->triangles.x[0], scene->triangles.x[1], scene->triangles.x[2],
-                               scene->triangles.y[0], scene->triangles.y[1], scene->triangles.y[2],
-                               scene->triangles.z[0], scene->triangles.z[1], scene->triangles.z[2] };
-    bool one_block = true;
-    for (int a = 0; a < 9; a++) one_block &= arrays[a] == arrays[0] + (size_t)a * (size_t)n_slots;
-    if (one_block) {
-      hs.soa = arrays[0];
-    } else {
-      hs.soa_copy.resize((size_t)n_slots * 9);
-      for (int a = 0; a < 9; a++) {
-        if (!arrays[a]) return fail("scene: null vertex array");
-        memcpy(hs.soa_copy.data() + (size_t)a * (size_t)n_slots, arrays[a], (size_t)n_slots * sizeof(float));
-      }
-      hs.soa = hs.soa_copy.data();
-    }
-  }
+  if (vertex_block(scene, hs.soa_copy, &hs.soa)) return 1;
 
   // materials / textures, de-duplicated by host pointer
   std::map<const void *, int> material_index, texture_index;
@@ -210,12 +229,14 @@ static int flatten(const Scene *scene, HostScene &hs) {
   };
 
   hs.mat_index.assign((size_t)n_slots, 0);
+  hs.refit_masks.assign((size_t)(n_nodes + n_slots / RT_SIMD_WIDTH), 0);
   const void *last_data = nullptr;
   int last_mat = 0;
   Shader_Proc last_proc = nullptr;
   for (isize s = 0; s < n_slots; s++) {
     const Triangle_AOS &a = scene->triangles.aos[s];
     if (!a.shader.proc && !a.shader.data) continue;
+    hs.refit_masks[(size_t)(n_nodes + s / RT_SIMD_WIDTH)] |= (unsigned char)(1u << (s % RT_SIMD_WIDTH));
     if (a.shader.proc != last_proc) {
       bool known = false;
       for (Shader_Proc p : g.pbr_procs) known |= (p == a.shader.proc);
@@ -258,20 +279,11 @@ static int flatten(const Scene *scene, HostScene &hs) {
         (hs.images[i]->pixel_type != PT_u8 && hs.images[i]->pixel_type != PT_RT_JPEG_BYTES))
       return fail("scene: texture %zu needs >= 3 u8 components (or compressed JPEG bytes) and a non-empty pixel buffer", i);
 
-  // union of the root's child boxes; all-zero padding slots (lo == hi) can never be entered (enter >= leave)
-  for (int a = 0; a < 3; a++) { hs.root_lo[a] = INFINITY; hs.root_hi[a] = -INFINITY; }
-  hs.root_upper_empty = 1;
-  for (int j = 0; j < 8; j++) {
-    const float *n0 = hs.nodes;
-    bool empty = true;
-    for (int a = 0; a < 3; a++) empty &= (n0[a * 8 + j] == n0[(3 + a) * 8 + j]);
-    if (empty) continue;
-    if (j >= 4) hs.root_upper_empty = 0;
-    for (int a = 0; a < 3; a++) {
-      hs.root_lo[a] = fminf(hs.root_lo[a], n0[a * 8 + j]);
-      hs.root_hi[a] = fmaxf(hs.root_hi[a], n0[(3 + a) * 8 + j]);
-    }
-  }
+  root_union(hs.nodes, hs.root_lo, hs.root_hi, &hs.root_upper_empty);
+
+  // occupancy for a later refit: the slot bits were set above; child bits per internal node, bottom-up
+  for (isize k = (isize)hs.refit_masks.size() - 1; k >= 1; k--)
+    if (hs.refit_masks[(size_t)k]) hs.refit_masks[(size_t)((k - 1) / RT_SIMD_WIDTH)] |= (unsigned char)(1u << ((k - 1) % RT_SIMD_WIDTH));
   return 0;
 }
 
@@ -375,12 +387,12 @@ static int upload_primary(Device &d, const HostScene &hs, const ArenaLayout &L, 
     if (grow(&d.d_texel_stage, &d.texel_stage_bytes, raw_max)) return 1;
   }
   char *raw_block = static_cast<char *>(d.d_texel_stage);
-  if (h2d(d, ds, base + L.nodes, hs.nodes, (size_t)hs.n_internal * 48 * sizeof(float))) return 1;
-  if (h2d(d, ds, base + L.tri_soa, hs.soa, (size_t)hs.n_slots * 9 * sizeof(float))) return 1;
-  if (h2d(d, ds, raw_block, hs.aos, aos_bytes)) return 1;
-  if (h2d(d, ds, raw_block + align256(aos_bytes), hs.mat_index.data(), idx_bytes)) return 1;
-  if (h2d(d, ds, base + L.materials, hs.materials.data(), hs.materials.size() * sizeof(MaterialDev))) return 1;
-  if (h2d(d, ds, base + L.table, table.data(), table.size() * sizeof(TextureDev))) return 1;
+  if (h2d(d, ds.h2d_bytes, base + L.nodes, hs.nodes, (size_t)hs.n_internal * 48 * sizeof(float))) return 1;
+  if (h2d(d, ds.h2d_bytes, base + L.tri_soa, hs.soa, (size_t)hs.n_slots * 9 * sizeof(float))) return 1;
+  if (h2d(d, ds.h2d_bytes, raw_block, hs.aos, aos_bytes)) return 1;
+  if (h2d(d, ds.h2d_bytes, raw_block + align256(aos_bytes), hs.mat_index.data(), idx_bytes)) return 1;
+  if (h2d(d, ds.h2d_bytes, base + L.materials, hs.materials.data(), hs.materials.size() * sizeof(MaterialDev))) return 1;
+  if (h2d(d, ds.h2d_bytes, base + L.table, table.data(), table.size() * sizeof(TextureDev))) return 1;
   {
     int e = rt_launch_scene_pack(reinterpret_cast<const float *>(base + L.tri_soa), reinterpret_cast<const float4 *>(raw_block),
                                  reinterpret_cast<const int *>(raw_block + align256(aos_bytes)), hs.n_slots,
@@ -410,7 +422,7 @@ static int upload_primary(Device &d, const HostScene &hs, const ArenaLayout &L, 
                                  (int)im->width, 3, reinterpret_cast<uchar4 *>(base + L.texel_off[i]), d.copy);
     } else {
       const size_t raw = (size_t)im->stride * (size_t)im->height * (size_t)im->components;
-      if (h2d(d, ds, d.d_texel_stage, im->pixels.data, raw)) return 1;
+      if (h2d(d, ds.h2d_bytes, d.d_texel_stage, im->pixels.data, raw)) return 1;
       e = rt_launch_texel_repack(static_cast<const unsigned char *>(d.d_texel_stage), (int)im->width, (int)im->height,
                                  (int)im->stride, im->components, reinterpret_cast<uchar4 *>(base + L.texel_off[i]), d.copy);
     }
@@ -442,7 +454,7 @@ static int upload_peer(Device &d, const Device &src_dev, const DeviceScene &src,
   CUDA_TRY(cudaStreamWaitEvent(d.copy, src.geom_ready, 0));
   CUDA_TRY(cudaMemcpyPeerAsync(base + L.nodes, d.id, src_base + L.nodes, src_dev.id, L.hot_end - L.nodes, d.copy));
   ds.p2p_bytes += L.hot_end - L.nodes;
-  if (h2d(d, ds, base + L.table, table.data(), table.size() * sizeof(TextureDev))) return 1;      // pointers differ per device
+  if (h2d(d, ds.h2d_bytes, base + L.table, table.data(), table.size() * sizeof(TextureDev))) return 1;      // pointers differ per device
   CUDA_TRY(cudaEventRecord(ds.geom_ready, d.copy));
   CUDA_TRY(cudaStreamWaitEvent(d.copy, src.tex_ready, 0));
   if (env_bytes) {
@@ -505,6 +517,7 @@ int scene_upload_all(const Scene *scene) {
   Device &d0 = g.devs[0];
   DeviceScene first;
   if (upload_primary(d0, hs, L, first)) { release_scene(d0, first); return 1; }
+  first.refit_masks = std::move(hs.refit_masks);
   auto it0 = d0.scenes.emplace(scene, std::move(first)).first;
   for (size_t k = 1; k < g.devs.size(); k++) {
     Device &d = g.devs[k];
@@ -543,6 +556,125 @@ void scene_release_all(const Scene *scene) {
     d.scenes.erase(it);
   }
   if (!g.devs.empty()) cudaSetDevice(g.devs[0].id);
+}
+
+// ---------------------------------------------------------------- refit (rt_gpu.h: moving geometry)
+// Device 0 refits on `stream` after every user of the scene's geometry there (renders and the other workspace users:
+// busy; queries: query_busy) and after the upload's own geometry; the flag and the root node come back in one
+// synchronisation.  Then geom_ready is re-recorded, so every later user waits for the new geometry as it waited for the
+// upload's, and the peers copy [nodes, hot_end) over NVLink as upload_peer does.
+int scene_refit(const Scene *scene, const float *positions, const float *normals, int normal_stride, cudaStream_t stream) {
+  Device &d = g.devs[0];
+  DeviceScene &ds = d.scenes.find(scene)->second;
+  CUDA_TRY(cudaSetDevice(d.id));
+  if (!ds.d_refit) {
+    void *block = nullptr;
+    if (pool_alloc(d, ds, 16 + ds.refit_masks.size(), &block)) return 1;
+    ds.d_refit = static_cast<unsigned char *>(block);
+    CUDA_TRY(cudaMemcpy(ds.d_refit + 16, ds.refit_masks.data(), ds.refit_masks.size(), cudaMemcpyHostToDevice));
+  }
+  if (d.busy_valid) CUDA_TRY(cudaStreamWaitEvent(stream, d.busy, 0));
+  if (d.query_busy_valid) CUDA_TRY(cudaStreamWaitEvent(stream, d.query_busy, 0));
+  CUDA_TRY(cudaStreamWaitEvent(stream, ds.geom_ready, 0));
+  int *flag = reinterpret_cast<int *>(ds.d_refit);
+  CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(int), stream));
+  RefitParams p{};
+  p.positions = positions; p.normals = normals; p.normal_stride = normal_stride;
+  p.depth = ds.dev.depth; p.n_internal = ds.dev.n_internal; p.n_slots = ds.dev.n_slots;
+  p.masks = ds.d_refit + 16; p.flag = flag;
+  p.nodes = const_cast<float *>(ds.dev.nodes);
+  p.tri_pos = const_cast<float4 *>(ds.dev.tri_pos);
+  p.tri_rec = const_cast<float4 *>(ds.dev.tri_rec);
+  p.tri_soa = const_cast<float *>(ds.dev.tri_soa);
+  const int e = rt_launch_refit(p, stream);
+  if (e) return fail("refit kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
+  if (grow_pinned(d, 256)) return 1;
+  CUDA_TRY(cudaMemcpyAsync(d.h_pinned, flag, sizeof(int), cudaMemcpyDeviceToHost, stream));
+  CUDA_TRY(cudaMemcpyAsync(d.h_pinned + 64, ds.dev.nodes, sizeof(BVH_Node), cudaMemcpyDeviceToHost, stream));
+  CUDA_TRY(cudaStreamSynchronize(stream));
+  int bad = 0;
+  memcpy(&bad, d.h_pinned, sizeof bad);
+  if (bad) return fail("scene_refit: a non-finite vertex coordinate in an occupied slot (the resident scene is unchanged)");
+  float root[48], lo[3], hi[3];
+  int upper_empty = 0;
+  memcpy(root, d.h_pinned + 64, sizeof root);
+  root_union(root, lo, hi, &upper_empty);
+  CUDA_TRY(cudaEventRecord(ds.geom_ready, stream));
+
+  const size_t head = (size_t)(reinterpret_cast<const char *>(ds.dev.nodes) - static_cast<const char *>(ds.hot_base));
+  for (Device &pd : g.devs) {
+    DeviceScene &ps = pd.scenes.find(scene)->second;
+    for (int a = 0; a < 3; a++) { ps.dev.root_lo[a] = lo[a]; ps.dev.root_hi[a] = hi[a]; }
+    ps.dev.root_upper_empty = upper_empty;
+    if (&pd == &d) continue;
+    CUDA_TRY(cudaSetDevice(pd.id));
+    if (pd.busy_valid) CUDA_TRY(cudaStreamWaitEvent(pd.copy, pd.busy, 0));
+    if (pd.query_busy_valid) CUDA_TRY(cudaStreamWaitEvent(pd.copy, pd.query_busy, 0));
+    CUDA_TRY(cudaStreamWaitEvent(pd.copy, ds.geom_ready, 0));
+    CUDA_TRY(cudaMemcpyPeerAsync(static_cast<char *>(ps.hot_base) + head, pd.id, static_cast<const char *>(ds.hot_base) + head,
+                                 d.id, ds.hot_bytes - head, pd.copy));
+    CUDA_TRY(cudaEventRecord(ps.geom_ready, pd.copy));
+    CUDA_TRY(cudaStreamSynchronize(pd.copy));       // the next refit of device 0 may overwrite what this copy reads
+  }
+  CUDA_TRY(cudaSetDevice(d.id));
+  return 0;
+}
+
+// The host form: the nine arrays (and the Triangle_AOS records, for their vertex normals) go up as the upload sends
+// them, on the copy stream; afterwards the refit node boxes and each occupied slot's geometric normal, tangent and
+// bitangent are written back, and padding slots are zeroed as they are on the device, so the host Scene is what the
+// device holds.
+int scene_refit_host(Scene *scene, bool refit_normals) {
+  Device &d = g.devs[0];
+  DeviceScene &ds = d.scenes.find(scene)->second;
+  CUDA_TRY(cudaSetDevice(d.id));
+  const size_t n = (size_t)ds.dev.n_slots, pos_bytes = n * 9 * sizeof(float), aos_bytes = n * sizeof(Triangle_AOS);
+  std::vector<float> gathered;
+  const float *soa = nullptr;
+  if (vertex_block(scene, gathered, &soa)) return 1;
+  const size_t need = align256(pos_bytes) + (refit_normals ? aos_bytes : 0);
+  if (need > d.texel_stage_bytes) {
+    CUDA_TRY(cudaStreamSynchronize(d.copy));
+    if (grow(&d.d_texel_stage, &d.texel_stage_bytes, need)) return 1;
+  }
+  char *stage = static_cast<char *>(d.d_texel_stage);
+  size_t staged = 0;
+  if (h2d(d, staged, stage, soa, pos_bytes)) return 1;
+  if (refit_normals && h2d(d, staged, stage + align256(pos_bytes), scene->triangles.aos, aos_bytes)) return 1;
+  // normal_a starts 12 bytes into a Triangle_AOS of 28 floats (scene.h)
+  const float *normals = refit_normals ? reinterpret_cast<const float *>(stage + align256(pos_bytes)) + 3 : nullptr;
+  if (scene_refit(scene, reinterpret_cast<const float *>(stage), normals, (int)(sizeof(Triangle_AOS) / sizeof(float)), d.copy))
+    return 1;
+  std::vector<float4> rec(n * 7);
+  CUDA_TRY(cudaMemcpyAsync(scene->bvh.nodes.data, ds.dev.nodes, (size_t)ds.dev.n_internal * sizeof(BVH_Node),
+                           cudaMemcpyDeviceToHost, d.copy));
+  CUDA_TRY(cudaMemcpyAsync(rec.data(), ds.dev.tri_rec, aos_bytes, cudaMemcpyDeviceToHost, d.copy));
+  CUDA_TRY(cudaStreamSynchronize(d.copy));
+  const size_t n_internal = (size_t)ds.dev.n_internal;
+  Triangles &t = scene->triangles;
+  for (size_t s = 0; s < n; s++) {
+    Triangle_AOS &a = t.aos[s];
+    if ((ds.refit_masks[n_internal + s / 8] >> (s % 8)) & 1) {
+      const float4 r0 = rec[7 * s], r3 = rec[7 * s + 3], r4 = rec[7 * s + 4];
+      a.normal.x = r0.x; a.normal.y = r0.y; a.normal.z = r0.z;
+      a.tangent.x = r3.x; a.tangent.y = r3.y; a.tangent.z = r3.z;
+      a.bitangent.x = r3.w; a.bitangent.y = r4.x; a.bitangent.z = r4.y;
+    } else {
+      for (int v = 0; v < 3; v++) t.x[v][s] = t.y[v][s] = t.z[v][s] = 0.0f;
+      if (refit_normals) a.normal_a = a.normal_b = a.normal_c = Vec3{};
+    }
+  }
+  return 0;
+}
+
+int scene_read_nodes(const Scene *scene, BVH_Node *out) {
+  Device &d = g.devs[0];
+  const DeviceScene &ds = d.scenes.find(scene)->second;
+  CUDA_TRY(cudaSetDevice(d.id));
+  CUDA_TRY(cudaStreamWaitEvent(d.stream, ds.geom_ready, 0));
+  CUDA_TRY(cudaMemcpyAsync(out, ds.dev.nodes, (size_t)ds.dev.n_internal * sizeof(BVH_Node), cudaMemcpyDeviceToHost, d.stream));
+  CUDA_TRY(cudaStreamSynchronize(d.stream));
+  return 0;
 }
 
 }  // namespace rt

@@ -44,6 +44,10 @@ struct DeviceScene {
   size_t hot_bytes = 0;
   int    n_textures = 0;
   Fingerprint fp;
+  // refit (first device only): the upload's occupancy bits (rt_refit.cu), and on the device [flag (16 B) | masks],
+  // allocated at the first refit
+  std::vector<unsigned char> refit_masks;
+  unsigned char *d_refit = nullptr;
 };
 
 // pinned staging ring for pageable host sources: the host memcpy of piece k+1 overlaps the DMA of piece k
@@ -122,6 +126,12 @@ int scene_upload_all(const Scene *scene);                     // (re-)upload: de
 void scene_release_all(const Scene *scene);
 void release_device(Device &d);                               // everything the device owns (shutdown)
 void set_l2_window(Device &d, const DeviceScene &ds, cudaStream_t stream);
+// refit of a resident scene (rt_gpu.h, "moving geometry"): scene_refit takes device pointers on the first device —
+// positions f32[9][n_slots], optional normals (9 floats at normal_stride * slot) — ordered on `stream`; scene_refit_host
+// stages the Scene's own buffers and writes the result back into them.  Both synchronise before they return.
+int scene_refit(const Scene *scene, const float *d_positions, const float *d_normals, int normal_stride, cudaStream_t stream);
+int scene_refit_host(Scene *scene, bool refit_normals);
+int scene_read_nodes(const Scene *scene, BVH_Node *out);
 
 // ---- rt_jpeg_gpu.cu
 int jpeg_begin_batch(cudaStream_t stream);

@@ -39,6 +39,8 @@ class LoadedScene:
     path: str
     n_triangles: int
     foreign_builder: bool = False      # scene buffers came from a test's builder (plain aligned_alloc), not scene_init
+    slot_of: Optional[np.ndarray] = None   # int32 [n_triangles]: the slot scene_init gave each source triangle (None
+                                           # with a foreign builder)
     _closed: bool = field(default=False)
 
     def close(self) -> None:
@@ -123,7 +125,11 @@ def load_scene(path: str, shader_proc: Optional[int] = None, background_proc: Op
                          background_proc=background_proc, path=path, n_triangles=model.triangles.len,
                          foreign_builder=builder is not None)
     loaded.scene.background.data = C.addressof(loaded.background)
-    (builder or host.scene_init)(C.byref(loaded.scene), model.triangles)
+    if builder is not None:
+        builder(C.byref(loaded.scene), model.triangles)
+    else:
+        loaded.slot_of = np.zeros(model.triangles.len, dtype=np.int32)
+        host.rt_scene_init_slots(C.byref(loaded.scene), model.triangles, loaded.slot_of.ctypes.data)
     return loaded
 
 
@@ -334,6 +340,80 @@ def render_masked(loaded: LoadedScene, accum, sample_begin: int, sample_end: int
         C.byref(loaded.scene), width, height, mask.data_ptr() if mask is not None else None, sample_begin, sample_end,
         max_bounces, user_seed, int(accumulate), accum.data_ptr(), accum_sq.data_ptr() if accum_sq is not None else None,
         counters.data_ptr() if counters is not None else None, st.cuda_stream))
+
+
+def scene_positions(loaded: LoadedScene) -> np.ndarray:
+    """A copy of the Scene's vertex positions in slot order, as the refit takes them: (3, 3, n_slots) float32, indexed
+    [axis][vertex][slot] (the block order x0 x1 x2 y0 y1 y2 z0 z1 z2)."""
+    t = loaded.scene.triangles
+    out = np.empty((3, 3, t.len), dtype=np.float32)
+    for a, arrays in enumerate((t.x, t.y, t.z)):
+        for v in range(3):
+            out[a, v] = np.ctypeslib.as_array((C.c_float * t.len).from_address(arrays[v]))
+    return out
+
+
+def scene_normals(loaded: LoadedScene) -> np.ndarray:
+    """A copy of the Scene's vertex normals in slot order: (n_slots, 3, 3) float32, normal_a, normal_b, normal_c."""
+    t = loaded.scene.triangles
+    aos = np.ctypeslib.as_array((C.c_float * (t.len * 28)).from_address(t.aos)).reshape(t.len, 28)
+    return aos[:, 3:12].reshape(t.len, 3, 3).copy()
+
+
+def refit(loaded: LoadedScene, positions=None, normals=None) -> None:
+    """Moves the geometry of a resident scene (rt_gpu_scene_refit; semantics in include/rt_gpu.h): `positions`
+    ((3, 3, n_slots) float32, scene_positions' layout) and `normals` ((n_slots, 3, 3), optional) are written into the
+    Scene's own buffers in slot order, the device refits, and the refit boxes, normals, tangents and bitangents are
+    written back, so the host Scene equals what the device holds.  positions=None refits from what the buffers already
+    hold.  LoadedScene.slot_of maps source triangles to slots.  Uploads the scene if it is not resident."""
+    gpu = gpu_lib()
+    t = loaded.scene.triangles
+    register_callbacks(loaded)
+    if gpu.rt_gpu_scene_device_bytes(C.byref(loaded.scene)) == 0:
+        gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+    if positions is not None:
+        positions = np.asarray(positions, dtype=np.float32)
+        if positions.shape != (3, 3, t.len):
+            raise ValueError(f"positions: shape (3, 3, {t.len}) required, got {positions.shape}")
+        for a, arrays in enumerate((t.x, t.y, t.z)):
+            for v in range(3):
+                np.ctypeslib.as_array((C.c_float * t.len).from_address(arrays[v]))[:] = positions[a, v]
+    if normals is not None:
+        normals = np.asarray(normals, dtype=np.float32)
+        if normals.shape != (t.len, 3, 3):
+            raise ValueError(f"normals: shape ({t.len}, 3, 3) required, got {normals.shape}")
+        aos = np.ctypeslib.as_array((C.c_float * (t.len * 28)).from_address(t.aos)).reshape(t.len, 28)
+        aos[:, 3:12] = normals.reshape(t.len, 9)
+    gpu_check(gpu.rt_gpu_scene_refit(C.byref(loaded.scene), int(normals is not None)))
+
+
+def refit_device(loaded: LoadedScene, positions, normals=None, stream=None) -> None:
+    """The device form (rt_gpu_scene_refit_device), enqueued on `stream` (default: torch's current stream): `positions`
+    a contiguous (3, 3, n_slots) float32 CUDA tensor, `normals` an optional contiguous (n_slots, 3, 3) one.  The host
+    buffers are not touched.  Returns after the refit (the call synchronises)."""
+    import torch
+    gpu = gpu_lib()
+    n = loaded.scene.triangles.len
+
+    def check(t, shape, what):
+        if t.device.type != "cuda" or t.dtype != torch.float32 or tuple(t.shape) != shape or not t.is_contiguous():
+            raise ValueError(f"{what}: a contiguous CUDA tensor of shape {shape} and dtype torch.float32 is required")
+    check(positions, (3, 3, n), "positions")
+    if normals is not None:
+        check(normals, (n, 3, 3), "normals")
+    register_callbacks(loaded)
+    if gpu.rt_gpu_scene_device_bytes(C.byref(loaded.scene)) == 0:
+        gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+    st = stream or torch.cuda.current_stream()
+    gpu_check(gpu.rt_gpu_scene_refit_device(C.byref(loaded.scene), positions.data_ptr(),
+                                            normals.data_ptr() if normals is not None else None, st.cuda_stream))
+
+
+def read_nodes(loaded: LoadedScene) -> bytes:
+    """The BVH node bytes resident on the first device (rt_gpu_read_nodes)."""
+    out = C.create_string_buffer(loaded.scene.bvh.nodes.len * _ffi.BVH_NODE_BYTES)
+    gpu_check(gpu_lib().rt_gpu_read_nodes(C.byref(loaded.scene), out))
+    return out.raw
 
 
 def resolve_counts(accum, samples, stream=None):

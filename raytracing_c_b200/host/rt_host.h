@@ -65,6 +65,11 @@ void  rt_host_buffer_free(void *p);
 bool scene_save_file(char const *path, Scene const *scene, PBR_Shader_Data const *materials, isize n_materials);
 bool scene_load_file(char const *path, Scene *scene, PBR_Shader_Data *materials, isize n_materials, Shader_Proc proc);
 
+/* scene_init that also reports where each source triangle went: slot_of_triangle[i] = the slot of src[i] (NULL
+ * allowed; scene_init is this call with NULL).  A host that keeps its vertices in source order (skinning output, a
+ * simulation) scatters them through this map into the slot order rt_gpu_scene_refit* takes. */
+void rt_scene_init_slots(Scene *scene, Triangle_Slice src, i32 *slot_of_triangle);
+
 char const *rt_host_last_error(void);
 
 #ifdef __cplusplus

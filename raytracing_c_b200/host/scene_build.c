@@ -42,6 +42,7 @@ typedef struct {
   Scene          *scene;
   Triangle const *tris;
   Tri_Info       *info;
+  i32            *slot_of;   /* optional: slot_of[source index] = slot (rt_scene_init_slots) */
 } Builder;
 
 typedef struct { u32 id; } Item;
@@ -124,6 +125,7 @@ static void pack_leaf(Builder *b, Item const *it, isize n, isize first_slot) {
   for (isize i = 0; i < n; i++) {
     Triangle const *t = &b->tris[it[i].id];
     isize s = first_slot + i;
+    if (b->slot_of) b->slot_of[it[i].id] = (i32)s;
     Vec3 const *p = t->positions;
     for (int v = 0; v < 3; v++) { dst->x[v][s] = p[v].x; dst->y[v][s] = p[v].y; dst->z[v][s] = p[v].z; }
 
@@ -250,7 +252,7 @@ static isize depth_for(isize n_triangles) {
   return d < 1 ? 1 : d;
 }
 
-void scene_init(Scene *scene, Triangle_Slice src) {
+void rt_scene_init_slots(Scene *scene, Triangle_Slice src, i32 *slot_of) {
   isize depth = depth_for(src.len);
   isize n_internal = bvh_n_internal_nodes(depth);
   scene->bvh.depth = depth;
@@ -272,7 +274,7 @@ void scene_init(Scene *scene, Triangle_Slice src) {
   scene->triangles.aos = (Triangle_AOS *)(block + slots * 9);
 
   isize n = src.len;
-  Builder b = { scene, src.data, malloc(sizeof(Tri_Info) * (size_t)(n ? n : 1)) };
+  Builder b = { scene, src.data, malloc(sizeof(Tri_Info) * (size_t)(n ? n : 1)), slot_of };
   Item *items = malloc(sizeof(Item) * (size_t)(n ? n : 1));
   for (isize i = 0; i < n; i++) {
     Vec3 const *p = src.data[i].positions;
@@ -300,6 +302,8 @@ void scene_init(Scene *scene, Triangle_Slice src) {
   free(items);
   free(b.info);
 }
+
+void scene_init(Scene *scene, Triangle_Slice src) { rt_scene_init_slots(scene, src, NULL); }
 
 void scene_destroy(Scene *scene) {
   rt_host_buffer_free(scene->bvh.nodes.data);
