@@ -51,6 +51,11 @@ void clear_error() {
   g_error_shared[0] = 0;
 }
 
+int launch_failed(const char *what, int launch_error) {
+  if (launch_error) return fail("%s kernel launch failed: %s", what, cudaGetErrorString((cudaError_t)launch_error));
+  return 0;
+}
+
 }  // namespace rt
 
 using namespace rt;
@@ -167,9 +172,54 @@ int workspace_begin(Device &d, const DeviceScene &ds, const WorkspaceRequest &r,
 }
 
 int workspace_end(Device &d, const char *what, int launch_error, cudaStream_t stream) {
-  if (launch_error) return fail("%s kernel launch failed: %s", what, cudaGetErrorString((cudaError_t)launch_error));
+  if (launch_failed(what, launch_error)) return 1;
   CUDA_TRY(cudaEventRecord(d.busy, stream));
   d.busy_valid = true;
+  return 0;
+}
+
+// the result of a launcher that enqueues one kernel: an error fails the call, a success counts the launch
+int launched(const char *what, int launch_error) {
+  if (launch_failed(what, launch_error)) return 1;
+  g.last_launches++;
+  return 0;
+}
+
+// The reference's entry points return void: whether `call` failed is left for rt_gpu_last_status, and a failure is
+// also reported on stderr.
+template <class Call>
+void report_status(const char *entry, Call call) {
+  clear_error();
+  g_status.store(0);
+  if (call()) {
+    g_status.store(1);
+    fprintf(stderr, "%s: %s\n", entry, rt_gpu_last_error());
+  }
+}
+
+// An image's round trip through the pinned buffer: d.d_image and the pinned buffer sized for it, the caller's image
+// up into d.d_image, and an image on the device back, all on d.stream.
+int image_buffers(Device &d, size_t bytes) {
+  if (grow(reinterpret_cast<void **>(&d.d_image), &d.image_bytes, bytes)) return 1;
+  return grow_pinned(d, bytes);
+}
+
+int image_to_device(Device &d, const void *pixels, size_t bytes) {
+  memcpy(d.h_pinned, pixels, bytes);
+  CUDA_TRY(cudaMemcpyAsync(d.d_image, d.h_pinned, bytes, cudaMemcpyHostToDevice, d.stream));
+  return 0;
+}
+
+// into the pinned buffer, synchronised: the renderer times its own copy out, the denoiser keeps padded rows' bytes
+int image_to_pinned(Device &d, const unsigned char *d_pixels, size_t bytes) {
+  CUDA_TRY(cudaMemcpyAsync(d.h_pinned, d_pixels, bytes, cudaMemcpyDeviceToHost, d.stream));
+  CUDA_TRY(cudaStreamSynchronize(d.stream));
+  return 0;
+}
+
+int image_from_device(Device &d, const unsigned char *d_pixels, size_t bytes, void *pixels) {
+  if (image_to_pinned(d, d_pixels, bytes)) return 1;
+  memcpy(pixels, d.h_pinned, bytes);
   return 0;
 }
 
@@ -430,41 +480,29 @@ int rt_gpu_reduce_resolve_device(f32 const *const *d_parts, i32 n_parts, f32 *d_
   ReduceParts parts{};
   parts.n = n_parts;
   for (int k = 0; k < n_parts; k++) parts.part[k] = d_parts[k];
-  int e = rt_launch_reduce_resolve(parts, d_sum_out, (int)width, (int)height, (int)samples, d_pixels, (int)stride, components,
-                                   static_cast<cudaStream_t>(stream));
-  if (e) return fail("reduce+resolve kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
-  g.last_launches++;
-  return 0;
+  return launched("reduce+resolve", rt_launch_reduce_resolve(parts, d_sum_out, (int)width, (int)height, (int)samples, d_pixels,
+                                                             (int)stride, components, static_cast<cudaStream_t>(stream)));
 }
 
 int rt_gpu_resolve_counts_device(f32 const *d_accum, i32 const *d_samples, isize width, isize height, u8 *d_pixels,
                                  isize stride, i32 components, void *stream) {
   if (!d_samples || components < 3) return fail("resolve_counts: d_samples and components >= 3 required");
-  int e = rt_launch_resolve_counts(d_accum, d_samples, (int)width, (int)height, d_pixels, (int)stride, components,
-                                   static_cast<cudaStream_t>(stream));
-  if (e) return fail("resolve kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
-  g.last_launches++;
-  return 0;
+  return launched("resolve", rt_launch_resolve_counts(d_accum, d_samples, (int)width, (int)height, d_pixels, (int)stride,
+                                                      components, static_cast<cudaStream_t>(stream)));
 }
 
 int rt_gpu_resolve_device(f32 const *d_accum, isize width, isize height, isize samples, u8 *d_pixels, isize stride,
                           i32 components, void *stream) {
   if (samples < 1 || components < 3) return fail("resolve: samples >= 1 and components >= 3 required");
-  int e = rt_launch_resolve(d_accum, (int)width, (int)height, (int)samples, d_pixels, (int)stride, components,
-                            static_cast<cudaStream_t>(stream));
-  if (e) return fail("resolve kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
-  g.last_launches++;
-  return 0;
+  return launched("resolve", rt_launch_resolve(d_accum, (int)width, (int)height, (int)samples, d_pixels, (int)stride, components,
+                                               static_cast<cudaStream_t>(stream)));
 }
 
 int rt_gpu_denoise_device(u8 const *d_src, u8 *d_dst, isize width, isize height, isize src_stride, isize dst_stride,
                           i32 components, void *stream) {
   if (d_src == d_dst) return fail("denoise: src and dst must differ (reference denoiser.c:130)");
-  int e = rt_launch_denoise(d_src, d_dst, (int)width, (int)height, (int)src_stride, (int)dst_stride, components,
-                            static_cast<cudaStream_t>(stream));
-  if (e) return fail("denoise kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
-  g.last_launches++;
-  return 0;
+  return launched("denoise", rt_launch_denoise(d_src, d_dst, (int)width, (int)height, (int)src_stride, (int)dst_stride,
+                                               components, static_cast<cudaStream_t>(stream)));
 }
 
 // ------------------------------------------------------------------ ray queries
@@ -472,35 +510,71 @@ int rt_gpu_denoise_device(u8 const *d_src, u8 *d_dst, isize width, isize height,
 
 namespace {
 
-// Staging of a host-memory call (queries, cast_rays, AOV) in the first device's staging block: part i gets bytes[i]
-// (0: none, NULL), every part 16-byte aligned.  The calls share the block: each runs on d.stream under g_mutex and
-// synchronises before it returns, and grow() frees the old block through cudaFree, which waits for the device.
-template <int N>
-int stage(Device &d, const size_t (&bytes)[N], void *(&parts)[N]) {
-  size_t offset[N], total = 0;
-  for (int i = 0; i < N; i++) { offset[i] = total; total += (bytes[i] + 15) & ~(size_t)15; }
-  if (grow(&d.d_stage, &d.stage_bytes, total)) return 1;
-  for (int i = 0; i < N; i++) parts[i] = bytes[i] ? static_cast<char *>(d.d_stage) + offset[i] : nullptr;
+// ---- the checks the validations are made of, in each validation's order; every message starts with the call's name
+int check_rays(const char *what, isize n_rays) {
+  if (n_rays < 0 || n_rays > INT32_MAX) return fail("%s: n_rays = %lld, must be in [0, INT32_MAX]", what, (long long)n_rays);
   return 0;
 }
 
-// the tail of the cast_rays and AOV validations: afterwards the scene is resident (and current) on every device
+int check_bounces(const char *what, isize max_bounces) {
+  if (max_bounces < 0 || max_bounces > INT32_MAX) return fail("%s: max_bounces = %lld, must be >= 0", what, (long long)max_bounces);
+  return 0;
+}
+
+int check_given(const char *what, const void *p, const char *name) {
+  if (!p) return fail("%s: null %s", what, name);
+  return 0;
+}
+
+// the tail of the cast_rays, AOV and refit validations: afterwards the scene is resident (and current) on every device
 int scene_resident(const char *what, const Scene *scene) {
-  if (!scene) return fail("%s: null scene", what);
+  if (check_given(what, scene, "scene")) return 1;
   if (ensure_init()) return 1;
   if (g.devs[0].scenes.find(scene) == g.devs[0].scenes.end())
     return fail("%s: scene is not resident (rt_gpu_scene_upload it first)", what);
   return scene_on_devices(scene);
 }
 
-int query_validate(const char *what, const Scene *scene, const void *rays, isize n_rays, const void *out, const void *hits) {
-  if (n_rays < 0 || n_rays > INT32_MAX) return fail("%s: n_rays = %lld, must be in [0, INT32_MAX]", what, (long long)n_rays);
-  if (n_rays == 0) return 0;
-  if (!scene) return fail("%s: null scene", what);
-  if (!rays) return fail("%s: null rays", what);
-  if (!out) return fail("%s: null output", what);
-  if (reinterpret_cast<uintptr_t>(hits) & 15) return fail("%s: hits must be 16-byte aligned", what);
+// A part of a host-memory call's staging: `bytes` on the device (0: none, NULL), filled from the host's `in` before the
+// device step and copied to the host's `out` after it (either may be NULL).
+struct HostPart { size_t bytes; const void *in; void *out; };
+
+// The host-memory form of a call (queries, cast_rays, AOV), after its validation: the parts are staged in the first
+// device's staging block, each 16-byte aligned; the inputs go up on d.stream, `step` enqueues the device form there
+// with the parts' device pointers, the outputs come back in part order and the call synchronises.  The calls share the
+// block: each runs on d.stream under g_mutex and synchronises before it returns, and grow() frees the old block
+// through cudaFree, which waits for the device.
+template <int N, class Step>
+int host_call(const HostPart (&parts)[N], Step step) {
+  Device &d = g.devs[0];
+  CUDA_TRY(cudaSetDevice(d.id));
+  size_t offset[N], total = 0;
+  for (int i = 0; i < N; i++) { offset[i] = total; total += (parts[i].bytes + 15) & ~(size_t)15; }
+  if (grow(&d.d_stage, &d.stage_bytes, total)) return 1;
+  void *dev[N];
+  for (int i = 0; i < N; i++) dev[i] = parts[i].bytes ? static_cast<char *>(d.d_stage) + offset[i] : nullptr;
+  for (int i = 0; i < N; i++)
+    if (parts[i].bytes && parts[i].in)
+      CUDA_TRY(cudaMemcpyAsync(dev[i], parts[i].in, parts[i].bytes, cudaMemcpyHostToDevice, d.stream));
+  if (step(dev, d.stream)) return 1;
+  for (int i = 0; i < N; i++)
+    if (parts[i].bytes && parts[i].out)
+      CUDA_TRY(cudaMemcpyAsync(parts[i].out, dev[i], parts[i].bytes, cudaMemcpyDeviceToHost, d.stream));
+  CUDA_TRY(cudaStreamSynchronize(d.stream));
   return 0;
+}
+
+// Everything that is refused before a query; afterwards the scene is resident (and current) on every device: unlike
+// the other calls, a query uploads a scene that is not.
+int query_validate(const char *what, const Scene *scene, const void *rays, isize n_rays, const void *out, const void *hits) {
+  if (check_rays(what, n_rays)) return 1;
+  if (n_rays == 0) return 0;
+  if (check_given(what, scene, "scene")) return 1;
+  if (check_given(what, rays, "rays")) return 1;
+  if (check_given(what, out, "output")) return 1;
+  if (reinterpret_cast<uintptr_t>(hits) & 15) return fail("%s: hits must be 16-byte aligned", what);
+  if (ensure_init()) return 1;
+  return scene_on_devices(scene);
 }
 
 // One query launch on the first device, ordered on `stream`.  It reads the scene's geometry only, so it waits for
@@ -509,15 +583,15 @@ int query_validate(const char *what, const Scene *scene, const void *rays, isize
 int query_on_device(const Scene *scene, const Ray *rays, const f32 *t_max, isize n_rays, bool any, RT_GPU_Hit *hits,
                     RT_GPU_Surface *surface, u8 *occluded, u64 *counters, cudaStream_t stream) {
   Device &d = g.devs[0];
-  CUDA_TRY(cudaSetDevice(d.id));
-  const DeviceScene &ds = d.scenes.find(scene)->second;
+  DeviceScene *ds = first_device_scene(scene);
+  if (!ds) return 1;
   if (!d.d_query_fetch) CUDA_TRY(cudaMalloc(reinterpret_cast<void **>(&d.d_query_fetch), sizeof(unsigned)));
   if (!d.query_busy) CUDA_TRY(cudaEventCreateWithFlags(&d.query_busy, cudaEventDisableTiming));
-  CUDA_TRY(cudaStreamWaitEvent(stream, ds.geom_ready, 0));
+  CUDA_TRY(cudaStreamWaitEvent(stream, ds->geom_ready, 0));
   if (d.query_busy_valid) CUDA_TRY(cudaStreamWaitEvent(stream, d.query_busy, 0));
   CUDA_TRY(cudaMemsetAsync(d.d_query_fetch, 0, sizeof(unsigned), stream));
   QueryParams p{};
-  p.scene = ds.dev;
+  p.scene = ds->dev;
   p.rays = reinterpret_cast<const float *>(rays);
   p.t_max = t_max;
   p.n_rays = (unsigned)n_rays;
@@ -526,9 +600,7 @@ int query_on_device(const Scene *scene, const Ray *rays, const f32 *t_max, isize
   p.occluded = occluded;
   p.fetch = d.d_query_fetch;
   p.counters = reinterpret_cast<unsigned long long *>(counters);
-  int e = rt_launch_query(p, any, d.sm_count, stream);
-  if (e) return fail("query kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
-  g.last_launches++;
+  if (launched("query", rt_launch_query(p, any, d.sm_count, stream))) return 1;
   CUDA_TRY(cudaEventRecord(d.query_busy, stream));
   d.query_busy_valid = true;
   return 0;
@@ -539,45 +611,29 @@ int query_device_call(const char *what, const Scene *scene, const Ray *d_rays, c
   std::lock_guard<std::mutex> lock(g_mutex);
   if (query_validate(what, scene, d_rays, n_rays, any ? static_cast<const void *>(d_occluded) : d_hits, d_hits)) return 1;
   if (n_rays == 0) return 0;
-  if (ensure_init()) return 1;
-  if (scene_on_devices(scene)) return 1;
   return query_on_device(scene, d_rays, d_t_max, n_rays, any, d_hits, d_surface, d_occluded, d_counters,
                          static_cast<cudaStream_t>(stream));
 }
 
-// Host memory: rays (and t_max) up through the first device's staging block, query, results back, synchronise.
+// Host memory: rays (and t_max) up, query, results back.
 int query_host_call(const char *what, const Scene *scene, const Ray *rays, const f32 *t_max, isize n_rays, bool any,
                     RT_GPU_Hit *hits, RT_GPU_Surface *surface, u8 *occluded) {
   std::lock_guard<std::mutex> lock(g_mutex);
   g.last_launches = 0;
-  // host arrays need no alignment: the device copy of hits is the staging block's first part
+  // host arrays need no alignment: the device copy of hits is a staging part
   if (query_validate(what, scene, rays, n_rays, any ? static_cast<const void *>(occluded) : hits, nullptr)) return 1;
   if (n_rays == 0) return 0;
-  if (ensure_init()) return 1;
-  if (scene_on_devices(scene)) return 1;
-  Device &d = g.devs[0];
-  CUDA_TRY(cudaSetDevice(d.id));
   const size_t n = (size_t)n_rays;
-  void *part[5];
-  if (stage(d, {any ? 0 : n * sizeof(RT_GPU_Hit), surface && !any ? n * sizeof(RT_GPU_Surface) : 0, n * sizeof(Ray),
-                t_max ? n * sizeof(f32) : 0, any ? n : 0}, part))
-    return 1;
-  RT_GPU_Hit *d_hits = static_cast<RT_GPU_Hit *>(part[0]);
-  RT_GPU_Surface *d_surface = static_cast<RT_GPU_Surface *>(part[1]);
-  Ray *d_rays = static_cast<Ray *>(part[2]);
-  f32 *d_t_max = static_cast<f32 *>(part[3]);
-  u8 *d_occluded = static_cast<u8 *>(part[4]);
-  CUDA_TRY(cudaMemcpyAsync(d_rays, rays, n * sizeof(Ray), cudaMemcpyHostToDevice, d.stream));
-  if (t_max) CUDA_TRY(cudaMemcpyAsync(d_t_max, t_max, n * sizeof(f32), cudaMemcpyHostToDevice, d.stream));
-  if (query_on_device(scene, d_rays, d_t_max, n_rays, any, d_hits, d_surface, d_occluded, nullptr, d.stream)) return 1;
-  if (any) {
-    CUDA_TRY(cudaMemcpyAsync(occluded, d_occluded, n, cudaMemcpyDeviceToHost, d.stream));
-  } else {
-    CUDA_TRY(cudaMemcpyAsync(hits, d_hits, n * sizeof(RT_GPU_Hit), cudaMemcpyDeviceToHost, d.stream));
-    if (surface) CUDA_TRY(cudaMemcpyAsync(surface, d_surface, n * sizeof(RT_GPU_Surface), cudaMemcpyDeviceToHost, d.stream));
-  }
-  CUDA_TRY(cudaStreamSynchronize(d.stream));
-  return 0;
+  return host_call({HostPart{any ? 0 : n * sizeof(RT_GPU_Hit), nullptr, hits},
+                    {surface && !any ? n * sizeof(RT_GPU_Surface) : 0, nullptr, surface},
+                    {n * sizeof(Ray), rays, nullptr},
+                    {t_max ? n * sizeof(f32) : 0, t_max, nullptr},
+                    {any ? n : 0, nullptr, occluded}},
+                   [&](void **part, cudaStream_t stream) {
+                     return query_on_device(scene, static_cast<Ray *>(part[2]), static_cast<f32 *>(part[3]), n_rays, any,
+                                            static_cast<RT_GPU_Hit *>(part[0]), static_cast<RT_GPU_Surface *>(part[1]),
+                                            static_cast<u8 *>(part[4]), nullptr, stream);
+                   });
 }
 
 }  // namespace
@@ -611,14 +667,14 @@ namespace {
 // Everything that is refused before a launch; afterwards the scene is resident (and current) on the first device.
 int cast_rays_validate(const char *what, const Scene *scene, const void *rays, isize n_rays, isize sample_begin,
                        isize samples, isize max_bounces, const void *radiance) {
-  if (n_rays < 0 || n_rays > INT32_MAX) return fail("%s: n_rays = %lld, must be in [0, INT32_MAX]", what, (long long)n_rays);
+  if (check_rays(what, n_rays)) return 1;
   if (samples < 0 || sample_begin < 0 || sample_begin > INT32_MAX - samples)
     return fail("%s: samples [%lld, %lld + %lld) must lie in [0, INT32_MAX]", what, (long long)sample_begin,
                 (long long)sample_begin, (long long)samples);
-  if (max_bounces < 0 || max_bounces > INT32_MAX) return fail("%s: max_bounces = %lld, must be >= 0", what, (long long)max_bounces);
+  if (check_bounces(what, max_bounces)) return 1;
   if (n_rays == 0) return 0;
-  if (!rays) return fail("%s: null rays", what);
-  if (!radiance) return fail("%s: null radiance", what);
+  if (check_given(what, rays, "rays")) return 1;
+  if (check_given(what, radiance, "radiance")) return 1;
   return scene_resident(what, scene);
 }
 
@@ -628,14 +684,14 @@ int cast_rays_on_device(const Scene *scene, const Ray *rays, const u32 *keys, is
                         isize max_bounces, u32 user_seed, int accumulate, float *radiance, float *per_sample,
                         unsigned long long *counters, cudaStream_t stream) {
   Device &d = g.devs[0];
-  CUDA_TRY(cudaSetDevice(d.id));
-  const DeviceScene &ds = d.scenes.find(scene)->second;
+  DeviceScene *ds = first_device_scene(scene);
+  if (!ds) return 1;
   const size_t n_paths = (size_t)n_rays * (size_t)samples;
   WorkspaceRequest r;
   if (n_paths > 0)
     r = {rt_cast_rays_workspace_bytes(n_paths, (int)max_bounces, false), rt_cast_rays_workspace_bytes(n_paths, (int)max_bounces, true)};
-  if (workspace_begin(d, ds, r, true, stream)) return 1;
-  int e = rt_launch_cast_rays(ds.dev, reinterpret_cast<const float *>(rays), keys, (int)n_rays, (int)sample_begin,
+  if (workspace_begin(d, *ds, r, true, stream)) return 1;
+  int e = rt_launch_cast_rays(ds->dev, reinterpret_cast<const float *>(rays), keys, (int)n_rays, (int)sample_begin,
                               (int)samples, (int)max_bounces, user_seed, accumulate, radiance, per_sample, counters,
                               d.sm_count, d.d_workspace, d.workspace_bytes, stream, &g.last_launches);
   return workspace_end(d, "cast_rays", e, stream);
@@ -656,35 +712,23 @@ int rt_gpu_cast_rays_device(Scene const *scene, Ray const *d_rays, u32 const *d_
                              static_cast<cudaStream_t>(stream));
 }
 
-// Host memory: rays, keys (and the sums to continue from) up through the first device's staging block, cast, results
-// back, synchronise.
+// Host memory: rays, keys (and the sums to continue from) up, cast, results back.
 int rt_gpu_cast_rays(Scene const *scene, Ray const *rays, u32 const *keys, isize n_rays, isize sample_begin, isize samples,
                      isize max_bounces, u32 user_seed, i32 accumulate, f32 *radiance, f32 *per_sample) {
   std::lock_guard<std::mutex> lock(g_mutex);
   g.last_launches = 0;
   if (cast_rays_validate("cast_rays", scene, rays, n_rays, sample_begin, samples, max_bounces, radiance)) return 1;
   if (n_rays == 0) return 0;
-  Device &d = g.devs[0];
-  CUDA_TRY(cudaSetDevice(d.id));
   const size_t n = (size_t)n_rays;
-  const size_t sums_bytes = n * 3 * sizeof(float);
-  const size_t per_sample_bytes = per_sample ? n * (size_t)samples * 3 * sizeof(float) : 0;
-  void *part[4];
-  if (stage(d, {sums_bytes, per_sample_bytes, n * sizeof(Ray), keys ? n * sizeof(u32) : 0}, part)) return 1;
-  float *d_radiance = static_cast<float *>(part[0]);
-  float *d_per_sample = static_cast<float *>(part[1]);
-  Ray *d_rays = static_cast<Ray *>(part[2]);
-  u32 *d_keys = static_cast<u32 *>(part[3]);
-  CUDA_TRY(cudaMemcpyAsync(d_rays, rays, n * sizeof(Ray), cudaMemcpyHostToDevice, d.stream));
-  if (keys) CUDA_TRY(cudaMemcpyAsync(d_keys, keys, n * sizeof(u32), cudaMemcpyHostToDevice, d.stream));
-  if (accumulate) CUDA_TRY(cudaMemcpyAsync(d_radiance, radiance, sums_bytes, cudaMemcpyHostToDevice, d.stream));
-  if (cast_rays_on_device(scene, d_rays, d_keys, n_rays, sample_begin, samples, max_bounces, user_seed, accumulate, d_radiance,
-                          d_per_sample, nullptr, d.stream))
-    return 1;
-  CUDA_TRY(cudaMemcpyAsync(radiance, d_radiance, sums_bytes, cudaMemcpyDeviceToHost, d.stream));
-  if (per_sample_bytes) CUDA_TRY(cudaMemcpyAsync(per_sample, d_per_sample, per_sample_bytes, cudaMemcpyDeviceToHost, d.stream));
-  CUDA_TRY(cudaStreamSynchronize(d.stream));
-  return 0;
+  return host_call({HostPart{n * 3 * sizeof(float), accumulate ? radiance : nullptr, radiance},
+                    {per_sample ? n * (size_t)samples * 3 * sizeof(float) : 0, nullptr, per_sample},
+                    {n * sizeof(Ray), rays, nullptr},
+                    {keys ? n * sizeof(u32) : 0, keys, nullptr}},
+                   [&](void **part, cudaStream_t stream) {
+                     return cast_rays_on_device(scene, static_cast<Ray *>(part[2]), static_cast<u32 *>(part[3]), n_rays,
+                                                sample_begin, samples, max_bounces, user_seed, accumulate,
+                                                static_cast<float *>(part[0]), static_cast<float *>(part[1]), nullptr, stream);
+                   });
 }
 
 // ------------------------------------------------------------- first-surface AOVs
@@ -705,8 +749,8 @@ int camera_validate(const char *what, const Scene *scene, isize width, isize hei
   if (sample_begin < 0 || sample_end < sample_begin || sample_end > INT32_MAX)
     return fail("%s: samples [%lld, %lld) must be a range inside [0, INT32_MAX]", what, (long long)sample_begin,
                 (long long)sample_end);
-  if (max_bounces < 0 || max_bounces > INT32_MAX) return fail("%s: max_bounces = %lld, must be >= 0", what, (long long)max_bounces);
-  if (!out) return fail("%s: null %s", what, out_name);
+  if (check_bounces(what, max_bounces)) return 1;
+  if (check_given(what, out, out_name)) return 1;
   return scene_resident(what, scene);
 }
 
@@ -715,13 +759,13 @@ int camera_validate(const char *what, const Scene *scene, isize width, isize hei
 int aov_on_device(const Scene *scene, isize width, isize height, isize sample_begin, isize sample_end, isize max_bounces,
                   int accumulate, float *aov, unsigned long long *counters, cudaStream_t stream) {
   Device &d = g.devs[0];
-  CUDA_TRY(cudaSetDevice(d.id));
-  const DeviceScene &ds = d.scenes.find(scene)->second;
+  DeviceScene *ds = first_device_scene(scene);
+  if (!ds) return 1;
   const isize n_samples = sample_end - sample_begin;
-  if (workspace_begin(d, ds, n_samples > 0 && max_bounces > 0 ? camera_workspace(width, height, n_samples, max_bounces, 1)
-                                                              : WorkspaceRequest{}, true, stream))
+  if (workspace_begin(d, *ds, n_samples > 0 && max_bounces > 0 ? camera_workspace(width, height, n_samples, max_bounces, 1)
+                                                               : WorkspaceRequest{}, true, stream))
     return 1;
-  int e = rt_launch_aov(ds.dev, (int)width, (int)height, (int)sample_begin, (int)sample_end, (int)max_bounces, accumulate,
+  int e = rt_launch_aov(ds->dev, (int)width, (int)height, (int)sample_begin, (int)sample_end, (int)max_bounces, accumulate,
                         aov, counters, d.sm_count, d.d_workspace, d.workspace_bytes, stream, &g.last_launches);
   return workspace_end(d, "aov", e, stream);
 }
@@ -740,22 +784,17 @@ int rt_gpu_render_aov_device(Scene const *scene, isize width, isize height, isiz
                        static_cast<cudaStream_t>(stream));
 }
 
-// Host memory: the records go through the first device's staging block and come back; synchronises.
+// Host memory: the records are computed from zero in a staging part and come back.
 int rt_gpu_render_aov(Scene const *scene, isize width, isize height, isize sample_begin, isize sample_end,
                       isize max_bounces, RT_GPU_AOV *aov) {
   std::lock_guard<std::mutex> lock(g_mutex);
   g.last_launches = 0;
   if (camera_validate("render_aov", scene, width, height, sample_begin, sample_end, max_bounces, aov, "aov")) return 1;
-  Device &d = g.devs[0];
-  CUDA_TRY(cudaSetDevice(d.id));
-  const size_t bytes = (size_t)width * (size_t)height * sizeof(RT_GPU_AOV);
-  void *part[1];
-  if (stage(d, {bytes}, part)) return 1;
-  float *d_aov = static_cast<float *>(part[0]);
-  if (aov_on_device(scene, width, height, sample_begin, sample_end, max_bounces, 0, d_aov, nullptr, d.stream)) return 1;
-  CUDA_TRY(cudaMemcpyAsync(aov, d_aov, bytes, cudaMemcpyDeviceToHost, d.stream));
-  CUDA_TRY(cudaStreamSynchronize(d.stream));
-  return 0;
+  return host_call({HostPart{(size_t)width * (size_t)height * sizeof(RT_GPU_AOV), nullptr, aov}},
+                   [&](void **part, cudaStream_t stream) {
+                     return aov_on_device(scene, width, height, sample_begin, sample_end, max_bounces, 0,
+                                          static_cast<float *>(part[0]), nullptr, stream);
+                   });
 }
 
 // ------------------------------------------------------------- masked sample passes
@@ -777,7 +816,7 @@ int rt_gpu_render_masked_device(Scene const *scene, isize width, isize height, u
 int rt_gpu_scene_refit_device(Scene const *scene, f32 const *d_positions, f32 const *d_normals, void *stream) {
   std::lock_guard<std::mutex> lock(g_mutex);
   if (scene_resident("scene_refit", scene)) return 1;
-  if (!d_positions) return fail("scene_refit: null positions");
+  if (check_given("scene_refit", d_positions, "positions")) return 1;
   return scene_refit(scene, d_positions, d_normals, 9, static_cast<cudaStream_t>(stream));
 }
 
@@ -791,7 +830,7 @@ int rt_gpu_scene_refit(Scene *scene, i32 refit_normals) {
 int rt_gpu_read_nodes(Scene const *scene, BVH_Node *out) {
   std::lock_guard<std::mutex> lock(g_mutex);
   if (scene_resident("read_nodes", scene)) return 1;
-  if (!out) return fail("read_nodes: null output");
+  if (check_given("read_nodes", out, "output")) return 1;
   return scene_read_nodes(scene, out);
 }
 
@@ -845,20 +884,23 @@ int rt_gpu_read_texture(Scene const *scene, i32 slot, u8 *out, isize *width, isi
   return 0;
 }
 
-int rt_gpu_read_counters(u64 out[8]) {
+// the first n_slots slots of every device's counter block, summed
+static int read_counters(u64 *out, int n_slots) {
   std::lock_guard<std::mutex> lock(g_mutex);
   if (g.devs.empty() || !g.devs[0].d_counters) return fail("read_counters: no render has run");
-  for (int i = 0; i < 8; i++) out[i] = 0;
+  for (int i = 0; i < n_slots; i++) out[i] = 0;
   for (Device &d : g.devs) {
     if (!d.d_counters) continue;
-    u64 part[8];
+    u64 part[16];
     CUDA_TRY(cudaSetDevice(d.id));
-    CUDA_TRY(cudaMemcpy(part, d.d_counters, sizeof part, cudaMemcpyDeviceToHost));
-    for (int i = 0; i < 8; i++) out[i] += part[i];
+    CUDA_TRY(cudaMemcpy(part, d.d_counters, n_slots * sizeof(u64), cudaMemcpyDeviceToHost));
+    for (int i = 0; i < n_slots; i++) out[i] += part[i];
   }
   CUDA_TRY(cudaSetDevice(g.devs[0].id));
   return 0;
 }
+
+int rt_gpu_read_counters(u64 out[8]) { return read_counters(out, 8); }
 
 // The library's own 16-slot counter block on the first device: [0..8) as RT_GPU_CTR_*, [8] rays whose whole walk
 // was the root-union test (they count as one node visit in [1], as in the reference, but cost 18 instructions),
@@ -886,20 +928,7 @@ int rt_gpu_counters_reset(void) {
   return 0;
 }
 
-int rt_gpu_read_counters_ex(u64 out[16]) {
-  std::lock_guard<std::mutex> lock(g_mutex);
-  if (g.devs.empty() || !g.devs[0].d_counters) return fail("read_counters: no render has run");
-  for (int i = 0; i < 16; i++) out[i] = 0;
-  for (Device &d : g.devs) {
-    if (!d.d_counters) continue;
-    u64 part[16];
-    CUDA_TRY(cudaSetDevice(d.id));
-    CUDA_TRY(cudaMemcpy(part, d.d_counters, sizeof part, cudaMemcpyDeviceToHost));
-    for (int i = 0; i < 16; i++) out[i] += part[i];
-  }
-  CUDA_TRY(cudaSetDevice(g.devs[0].id));
-  return 0;
-}
+int rt_gpu_read_counters_ex(u64 out[16]) { return read_counters(out, 16); }
 
 int rt_gpu_last_launches(void) { return g.last_launches; }
 
@@ -960,8 +989,7 @@ static int render_owner(Rendering_Context *ctx, isize n_chunks) {
     if (ensure_frame_buffers(d, n_pixels, opt.keep_hit_ids != 0)) return 1;
   Device &d0 = g.devs[0];
   CUDA_TRY(cudaSetDevice(d0.id));
-  if (grow(reinterpret_cast<void **>(&d0.d_image), &d0.image_bytes, image_bytes)) return 1;
-  if (grow_pinned(d0, image_bytes)) return 1;
+  if (image_buffers(d0, image_bytes)) return 1;
 
   // the samples this call renders (a multi-process host narrows them per rank), then their split over the devices
   isize s_begin = opt.sample_begin, s_end = opt.sample_end;
@@ -982,10 +1010,7 @@ static int render_owner(Rendering_Context *ctx, isize n_chunks) {
   g.last_has_hit_ids = opt.keep_hit_ids != 0;
   g.last_split_mode = mode;
   // rows padded by stride keep whatever the caller had there
-  if (im.stride != im.width || im.components != 3) {
-    memcpy(d0.h_pinned, im.pixels.data, image_bytes);
-    CUDA_TRY(cudaMemcpyAsync(d0.d_image, d0.h_pinned, image_bytes, cudaMemcpyHostToDevice, d0.stream));
-  }
+  if ((im.stride != im.width || im.components != 3) && image_to_device(d0, im.pixels.data, image_bytes)) return 1;
 
   CUDA_TRY(cudaEventRecord(d0.ev0, d0.stream));
   std::vector<Share> shares(n_dev);
@@ -1070,22 +1095,21 @@ static int render_owner(Rendering_Context *ctx, isize n_chunks) {
   if (n_dev > 1 && opt.reduce_mode == RT_GPU_REDUCE_NCCL) {
     if (nccl_reduce_to_first(n_pixels * 3)) return 1;
     CUDA_TRY(cudaSetDevice(d0.id));
-    int e = rt_launch_resolve(d0.d_accum, (int)im.width, (int)im.height, (int)ctx->samples, d0.d_image, (int)im.stride,
-                              im.components, d0.stream);
-    if (e) return fail("resolve kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
+    if (launched("resolve", rt_launch_resolve(d0.d_accum, (int)im.width, (int)im.height, (int)ctx->samples, d0.d_image,
+                                              (int)im.stride, im.components, d0.stream)))
+      return 1;
   } else {
     ReduceParts parts{};
     parts.n = (int)n_dev;
     for (size_t k = 0; k < n_dev; k++) parts.part[k] = g.devs[k].d_accum;
     // one device: the same kernel with a single part (x + nothing) — one film code path for every N
-    int e = rt_launch_reduce_resolve(parts, n_dev > 1 ? d0.d_accum : nullptr, (int)im.width, (int)im.height, (int)ctx->samples,
-                                     d0.d_image, (int)im.stride, im.components, d0.stream);
-    if (e) return fail("reduce+resolve kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
+    if (launched("reduce+resolve", rt_launch_reduce_resolve(parts, n_dev > 1 ? d0.d_accum : nullptr, (int)im.width,
+                                                            (int)im.height, (int)ctx->samples, d0.d_image, (int)im.stride,
+                                                            im.components, d0.stream)))
+      return 1;
   }
-  g.last_launches++;
   if (r1) CUDA_TRY(cudaEventRecord(r1, d0.stream));
-  CUDA_TRY(cudaMemcpyAsync(d0.h_pinned, d0.d_image, image_bytes, cudaMemcpyDeviceToHost, d0.stream));
-  CUDA_TRY(cudaStreamSynchronize(d0.stream));
+  if (image_to_pinned(d0, d0.d_image, image_bytes)) return 1;
   t0 = now_ms();
   memcpy(im.pixels.data, d0.h_pinned, image_bytes);
   g.last_d2h_ms = now_ms() - t0;
@@ -1117,12 +1141,7 @@ void render_thread_proc(Rendering_Context *ctx) {
   // raytracer.c:620: claim a chunk; whoever gets chunk 0 launches the whole frame
   i32 c = __atomic_fetch_add(const_cast<i32 *>(&ctx->_current_chunk), 1, __ATOMIC_SEQ_CST);
   if (c == 0) {
-    clear_error();
-    g_status.store(0);
-    if (render_owner(ctx, n_chunks)) {
-      g_status.store(1);
-      fprintf(stderr, "render_thread_proc: %s\n", rt_gpu_last_error());
-    }
+    report_status("render_thread_proc", [&] { return render_owner(ctx, n_chunks); });
     __atomic_store_n(const_cast<i32 *>(&ctx->_current_chunk), (i32)n_chunks + 1, __ATOMIC_SEQ_CST);
   }
   // raytracer.c:622
@@ -1151,8 +1170,8 @@ int rt_gpu_lightmap_bake(Image const *lightmap, Scene const *scene, isize sample
   if (samples < 1) return fail("lightmap_bake: samples must be >= 1");
   if (scene_on_devices(scene)) return 1;
   Device &d = g.devs[0];
-  CUDA_TRY(cudaSetDevice(d.id));
-  const DeviceScene &ds = d.scenes.find(scene)->second;
+  DeviceScene *ds = first_device_scene(scene);
+  if (!ds) return 1;
   const int W = (int)lightmap->width, H = (int)lightmap->height;
   const size_t n_texels = (size_t)W * (size_t)H;
   const size_t image_bytes = (size_t)lightmap->stride * (size_t)H * (size_t)lightmap->components;
@@ -1160,8 +1179,7 @@ int rt_gpu_lightmap_bake(Image const *lightmap, Scene const *scene, isize sample
 
   CUDA_TRY(cudaStreamSynchronize(d.stream));
   CUDA_TRY(cudaStreamSynchronize(d.copy));
-  if (grow(reinterpret_cast<void **>(&d.d_image), &d.image_bytes, image_bytes)) return 1;
-  if (grow_pinned(d, image_bytes)) return 1;
+  if (image_buffers(d, image_bytes)) return 1;
   const size_t scratch_bytes = rt_lightmap_workspace_bytes(W, H) + (values_out ? n_texels * 3 * sizeof(float) : 0) +
                                (owner_out ? n_texels * sizeof(int) : 0);
   if (grow(&d.d_texel_stage, &d.texel_stage_bytes, scratch_bytes)) return 1;       // the upload's raw-texel block doubles as scratch
@@ -1170,35 +1188,27 @@ int rt_gpu_lightmap_bake(Image const *lightmap, Scene const *scene, isize sample
   int *d_owner = owner_out ? reinterpret_cast<int *>(scratch + rt_lightmap_workspace_bytes(W, H) + (values_out ? n_texels * 3 * sizeof(float) : 0)) : nullptr;
   const WorkspaceRequest r{rt_lightmap_paths_workspace_bytes(n_texels, (int)samples, max_bounces, false),
                            rt_lightmap_paths_workspace_bytes(n_texels, (int)samples, max_bounces, true)};
-  if (workspace_begin(d, ds, r, true, d.stream)) return 1;
-  memcpy(d.h_pinned, lightmap->pixels.data, image_bytes);            // untouched texels keep their bytes
-  CUDA_TRY(cudaMemcpyAsync(d.d_image, d.h_pinned, image_bytes, cudaMemcpyHostToDevice, d.stream));
+  if (workspace_begin(d, *ds, r, true, d.stream)) return 1;
+  if (image_to_device(d, lightmap->pixels.data, image_bytes)) return 1;      // untouched texels keep their bytes
   if (d_values) CUDA_TRY(cudaMemsetAsync(d_values, 0, n_texels * 3 * sizeof(float), d.stream));
   unsigned n_jobs = 0;
-  int e = rt_launch_lightmap(ds.dev, W, H, (int)samples, max_bounces, g.options.user_seed, d.d_image, (int)lightmap->stride,
+  int e = rt_launch_lightmap(ds->dev, W, H, (int)samples, max_bounces, g.options.user_seed, d.d_image, (int)lightmap->stride,
                              lightmap->components, d_values, d_owner, scratch, d.sm_count, d.d_workspace, d.workspace_bytes,
                              d.stream, &g.last_launches, &n_jobs);
   if (workspace_end(d, "lightmap", e, d.stream)) return 1;
-  CUDA_TRY(cudaMemcpyAsync(d.h_pinned, d.d_image, image_bytes, cudaMemcpyDeviceToHost, d.stream));
-  CUDA_TRY(cudaStreamSynchronize(d.stream));
-  memcpy(lightmap->pixels.data, d.h_pinned, image_bytes);
+  if (image_from_device(d, d.d_image, image_bytes, lightmap->pixels.data)) return 1;
   if (values_out) CUDA_TRY(cudaMemcpy(values_out, d_values, n_texels * 3 * sizeof(float), cudaMemcpyDeviceToHost));
   if (owner_out) CUDA_TRY(cudaMemcpy(owner_out, d_owner, n_texels * sizeof(int), cudaMemcpyDeviceToHost));
   return 0;
 }
 
 void lightmap_bake(Image const *lightmap, Scene const *scene, isize samples) {
-  clear_error();
-  g_status.store(0);
-  if (rt_gpu_lightmap_bake(lightmap, scene, samples, nullptr, nullptr)) {
-    g_status.store(1);
-    fprintf(stderr, "lightmap_bake: %s\n", rt_gpu_last_error());
-  }
+  report_status("lightmap_bake", [&] { return rt_gpu_lightmap_bake(lightmap, scene, samples, nullptr, nullptr); });
 }
 
 void denoise_image(Image const *src, Image const *dst, isize n_threads) {
   (void)n_threads;
-  auto run = [&]() -> int {
+  report_status("denoise_image", [&]() -> int {
     std::lock_guard<std::mutex> lock(g_mutex);
     g.last_launches = 0;
     if (ensure_init()) return 1;
@@ -1214,20 +1224,17 @@ void denoise_image(Image const *src, Image const *dst, isize n_threads) {
     if (grow(reinterpret_cast<void **>(&d.d_image), &d.image_bytes, src_bytes)) return 1;
     if (grow(reinterpret_cast<void **>(&d.d_image2), &d.image2_bytes, dst_bytes)) return 1;
     if (grow_pinned(d, src_bytes > dst_bytes ? src_bytes : dst_bytes)) return 1;
-    memcpy(d.h_pinned, src->pixels.data, src_bytes);
-    CUDA_TRY(cudaMemcpyAsync(d.d_image, d.h_pinned, src_bytes, cudaMemcpyHostToDevice, d.stream));
+    if (image_to_device(d, src->pixels.data, src_bytes)) return 1;
     if (dst->stride != dst->width) CUDA_TRY(cudaMemsetAsync(d.d_image2, 0, dst_bytes, d.stream));
     CUDA_TRY(cudaEventRecord(d.ev0, d.stream));
-    int e = rt_launch_denoise(d.d_image, d.d_image2, (int)src->width, (int)src->height, (int)src->stride, (int)dst->stride,
-                              src->components, d.stream);
-    if (e) return fail("denoise kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
-    g.last_launches++;
+    if (launched("denoise", rt_launch_denoise(d.d_image, d.d_image2, (int)src->width, (int)src->height, (int)src->stride,
+                                              (int)dst->stride, src->components, d.stream)))
+      return 1;
     CUDA_TRY(cudaEventRecord(d.ev1, d.stream));
-    CUDA_TRY(cudaMemcpyAsync(d.h_pinned, d.d_image2, dst_bytes, cudaMemcpyDeviceToHost, d.stream));
-    CUDA_TRY(cudaStreamSynchronize(d.stream));
     if (dst->stride == dst->width) {
-      memcpy(dst->pixels.data, d.h_pinned, dst_bytes);
+      if (image_from_device(d, d.d_image2, dst_bytes, dst->pixels.data)) return 1;
     } else {
+      if (image_to_pinned(d, d.d_image2, dst_bytes)) return 1;
       for (isize y = 0; y < dst->height; y++)
         memcpy(dst->pixels.data + (size_t)y * (size_t)dst->stride * (size_t)dst->components,
                d.h_pinned + (size_t)y * (size_t)dst->stride * (size_t)dst->components,
@@ -1237,13 +1244,7 @@ void denoise_image(Image const *src, Image const *dst, isize n_threads) {
     cudaEventElapsedTime(&ms, d.ev0, d.ev1);
     g.last_kernel_ms = ms;
     return 0;
-  };
-  clear_error();
-  g_status.store(0);
-  if (run()) {
-    g_status.store(1);
-    fprintf(stderr, "denoise_image: %s\n", rt_gpu_last_error());
-  }
+  });
 }
 
 }  // extern "C"

@@ -546,6 +546,15 @@ int scene_on_devices(const Scene *scene) {
   return 0;
 }
 
+DeviceScene *first_device_scene(const Scene *scene) {
+  Device &d = g.devs[0];
+  auto it = d.scenes.find(scene);
+  if (it == d.scenes.end()) { fail("scene is not resident on device %d", d.id); return nullptr; }
+  const cudaError_t e = cudaSetDevice(d.id);
+  if (e != cudaSuccess) { fail("cudaSetDevice(d.id) failed: %s", cudaGetErrorString(e)); return nullptr; }
+  return &it->second;
+}
+
 void scene_release_all(const Scene *scene) {
   for (Device &d : g.devs) {
     auto it = d.scenes.find(scene);
@@ -565,32 +574,31 @@ void scene_release_all(const Scene *scene) {
 // upload's, and the peers copy [nodes, hot_end) over NVLink as upload_peer does.
 int scene_refit(const Scene *scene, const float *positions, const float *normals, int normal_stride, cudaStream_t stream) {
   Device &d = g.devs[0];
-  DeviceScene &ds = d.scenes.find(scene)->second;
-  CUDA_TRY(cudaSetDevice(d.id));
-  if (!ds.d_refit) {
+  DeviceScene *ds = first_device_scene(scene);
+  if (!ds) return 1;
+  if (!ds->d_refit) {
     void *block = nullptr;
-    if (pool_alloc(d, ds, 16 + ds.refit_masks.size(), &block)) return 1;
-    ds.d_refit = static_cast<unsigned char *>(block);
-    CUDA_TRY(cudaMemcpy(ds.d_refit + 16, ds.refit_masks.data(), ds.refit_masks.size(), cudaMemcpyHostToDevice));
+    if (pool_alloc(d, *ds, 16 + ds->refit_masks.size(), &block)) return 1;
+    ds->d_refit = static_cast<unsigned char *>(block);
+    CUDA_TRY(cudaMemcpy(ds->d_refit + 16, ds->refit_masks.data(), ds->refit_masks.size(), cudaMemcpyHostToDevice));
   }
   if (d.busy_valid) CUDA_TRY(cudaStreamWaitEvent(stream, d.busy, 0));
   if (d.query_busy_valid) CUDA_TRY(cudaStreamWaitEvent(stream, d.query_busy, 0));
-  CUDA_TRY(cudaStreamWaitEvent(stream, ds.geom_ready, 0));
-  int *flag = reinterpret_cast<int *>(ds.d_refit);
+  CUDA_TRY(cudaStreamWaitEvent(stream, ds->geom_ready, 0));
+  int *flag = reinterpret_cast<int *>(ds->d_refit);
   CUDA_TRY(cudaMemsetAsync(flag, 0, sizeof(int), stream));
   RefitParams p{};
   p.positions = positions; p.normals = normals; p.normal_stride = normal_stride;
-  p.depth = ds.dev.depth; p.n_internal = ds.dev.n_internal; p.n_slots = ds.dev.n_slots;
-  p.masks = ds.d_refit + 16; p.flag = flag;
-  p.nodes = const_cast<float *>(ds.dev.nodes);
-  p.tri_pos = const_cast<float4 *>(ds.dev.tri_pos);
-  p.tri_rec = const_cast<float4 *>(ds.dev.tri_rec);
-  p.tri_soa = const_cast<float *>(ds.dev.tri_soa);
-  const int e = rt_launch_refit(p, stream);
-  if (e) return fail("refit kernel launch failed: %s", cudaGetErrorString((cudaError_t)e));
+  p.depth = ds->dev.depth; p.n_internal = ds->dev.n_internal; p.n_slots = ds->dev.n_slots;
+  p.masks = ds->d_refit + 16; p.flag = flag;
+  p.nodes = const_cast<float *>(ds->dev.nodes);
+  p.tri_pos = const_cast<float4 *>(ds->dev.tri_pos);
+  p.tri_rec = const_cast<float4 *>(ds->dev.tri_rec);
+  p.tri_soa = const_cast<float *>(ds->dev.tri_soa);
+  if (launch_failed("refit", rt_launch_refit(p, stream))) return 1;
   if (grow_pinned(d, 256)) return 1;
   CUDA_TRY(cudaMemcpyAsync(d.h_pinned, flag, sizeof(int), cudaMemcpyDeviceToHost, stream));
-  CUDA_TRY(cudaMemcpyAsync(d.h_pinned + 64, ds.dev.nodes, sizeof(BVH_Node), cudaMemcpyDeviceToHost, stream));
+  CUDA_TRY(cudaMemcpyAsync(d.h_pinned + 64, ds->dev.nodes, sizeof(BVH_Node), cudaMemcpyDeviceToHost, stream));
   CUDA_TRY(cudaStreamSynchronize(stream));
   int bad = 0;
   memcpy(&bad, d.h_pinned, sizeof bad);
@@ -599,9 +607,9 @@ int scene_refit(const Scene *scene, const float *positions, const float *normals
   int upper_empty = 0;
   memcpy(root, d.h_pinned + 64, sizeof root);
   root_union(root, lo, hi, &upper_empty);
-  CUDA_TRY(cudaEventRecord(ds.geom_ready, stream));
+  CUDA_TRY(cudaEventRecord(ds->geom_ready, stream));
 
-  const size_t head = (size_t)(reinterpret_cast<const char *>(ds.dev.nodes) - static_cast<const char *>(ds.hot_base));
+  const size_t head = (size_t)(reinterpret_cast<const char *>(ds->dev.nodes) - static_cast<const char *>(ds->hot_base));
   for (Device &pd : g.devs) {
     DeviceScene &ps = pd.scenes.find(scene)->second;
     for (int a = 0; a < 3; a++) { ps.dev.root_lo[a] = lo[a]; ps.dev.root_hi[a] = hi[a]; }
@@ -610,9 +618,9 @@ int scene_refit(const Scene *scene, const float *positions, const float *normals
     CUDA_TRY(cudaSetDevice(pd.id));
     if (pd.busy_valid) CUDA_TRY(cudaStreamWaitEvent(pd.copy, pd.busy, 0));
     if (pd.query_busy_valid) CUDA_TRY(cudaStreamWaitEvent(pd.copy, pd.query_busy, 0));
-    CUDA_TRY(cudaStreamWaitEvent(pd.copy, ds.geom_ready, 0));
-    CUDA_TRY(cudaMemcpyPeerAsync(static_cast<char *>(ps.hot_base) + head, pd.id, static_cast<const char *>(ds.hot_base) + head,
-                                 d.id, ds.hot_bytes - head, pd.copy));
+    CUDA_TRY(cudaStreamWaitEvent(pd.copy, ds->geom_ready, 0));
+    CUDA_TRY(cudaMemcpyPeerAsync(static_cast<char *>(ps.hot_base) + head, pd.id, static_cast<const char *>(ds->hot_base) + head,
+                                 d.id, ds->hot_bytes - head, pd.copy));
     CUDA_TRY(cudaEventRecord(ps.geom_ready, pd.copy));
     CUDA_TRY(cudaStreamSynchronize(pd.copy));       // the next refit of device 0 may overwrite what this copy reads
   }
@@ -626,9 +634,9 @@ int scene_refit(const Scene *scene, const float *positions, const float *normals
 // device holds.
 int scene_refit_host(Scene *scene, bool refit_normals) {
   Device &d = g.devs[0];
-  DeviceScene &ds = d.scenes.find(scene)->second;
-  CUDA_TRY(cudaSetDevice(d.id));
-  const size_t n = (size_t)ds.dev.n_slots, pos_bytes = n * 9 * sizeof(float), aos_bytes = n * sizeof(Triangle_AOS);
+  DeviceScene *ds = first_device_scene(scene);
+  if (!ds) return 1;
+  const size_t n = (size_t)ds->dev.n_slots, pos_bytes = n * 9 * sizeof(float), aos_bytes = n * sizeof(Triangle_AOS);
   std::vector<float> gathered;
   const float *soa = nullptr;
   if (vertex_block(scene, gathered, &soa)) return 1;
@@ -646,15 +654,15 @@ int scene_refit_host(Scene *scene, bool refit_normals) {
   if (scene_refit(scene, reinterpret_cast<const float *>(stage), normals, (int)(sizeof(Triangle_AOS) / sizeof(float)), d.copy))
     return 1;
   std::vector<float4> rec(n * 7);
-  CUDA_TRY(cudaMemcpyAsync(scene->bvh.nodes.data, ds.dev.nodes, (size_t)ds.dev.n_internal * sizeof(BVH_Node),
+  CUDA_TRY(cudaMemcpyAsync(scene->bvh.nodes.data, ds->dev.nodes, (size_t)ds->dev.n_internal * sizeof(BVH_Node),
                            cudaMemcpyDeviceToHost, d.copy));
-  CUDA_TRY(cudaMemcpyAsync(rec.data(), ds.dev.tri_rec, aos_bytes, cudaMemcpyDeviceToHost, d.copy));
+  CUDA_TRY(cudaMemcpyAsync(rec.data(), ds->dev.tri_rec, aos_bytes, cudaMemcpyDeviceToHost, d.copy));
   CUDA_TRY(cudaStreamSynchronize(d.copy));
-  const size_t n_internal = (size_t)ds.dev.n_internal;
+  const size_t n_internal = (size_t)ds->dev.n_internal;
   Triangles &t = scene->triangles;
   for (size_t s = 0; s < n; s++) {
     Triangle_AOS &a = t.aos[s];
-    if ((ds.refit_masks[n_internal + s / 8] >> (s % 8)) & 1) {
+    if ((ds->refit_masks[n_internal + s / 8] >> (s % 8)) & 1) {
       const float4 r0 = rec[7 * s], r3 = rec[7 * s + 3], r4 = rec[7 * s + 4];
       a.normal.x = r0.x; a.normal.y = r0.y; a.normal.z = r0.z;
       a.tangent.x = r3.x; a.tangent.y = r3.y; a.tangent.z = r3.z;
@@ -669,10 +677,10 @@ int scene_refit_host(Scene *scene, bool refit_normals) {
 
 int scene_read_nodes(const Scene *scene, BVH_Node *out) {
   Device &d = g.devs[0];
-  const DeviceScene &ds = d.scenes.find(scene)->second;
-  CUDA_TRY(cudaSetDevice(d.id));
-  CUDA_TRY(cudaStreamWaitEvent(d.stream, ds.geom_ready, 0));
-  CUDA_TRY(cudaMemcpyAsync(out, ds.dev.nodes, (size_t)ds.dev.n_internal * sizeof(BVH_Node), cudaMemcpyDeviceToHost, d.stream));
+  DeviceScene *ds = first_device_scene(scene);
+  if (!ds) return 1;
+  CUDA_TRY(cudaStreamWaitEvent(d.stream, ds->geom_ready, 0));
+  CUDA_TRY(cudaMemcpyAsync(out, ds->dev.nodes, (size_t)ds->dev.n_internal * sizeof(BVH_Node), cudaMemcpyDeviceToHost, d.stream));
   CUDA_TRY(cudaStreamSynchronize(d.stream));
   return 0;
 }

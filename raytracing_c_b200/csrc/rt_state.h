@@ -84,7 +84,7 @@ struct Device {
   unsigned *d_query_fetch = nullptr;
   cudaEvent_t query_busy = nullptr;
   bool  query_busy_valid = false;
-  // staging of the host-memory queries, rt_gpu_cast_rays and rt_gpu_render_aov (rt_cabi.cu: stage)
+  // staging of the host-memory queries, rt_gpu_cast_rays and rt_gpu_render_aov (rt_cabi.cu: host_call)
   void *d_stage = nullptr; size_t stage_bytes = 0;
   bool l2_window_set = false;
   size_t l2_persist_max = 0, l2_window_max = 0;    // device limits (persistingL2CacheMaxSize, accessPolicyMaxWindowSize)
@@ -111,6 +111,7 @@ extern std::mutex g_mutex;
 
 int fail(const char *fmt, ...);
 void clear_error();
+int launch_failed(const char *what, int launch_error);       // a launcher's error code as the call's failure (0: none)
 
 #define CUDA_TRY(expr)                                                                          \
   do {                                                                                          \
@@ -122,6 +123,9 @@ void clear_error();
 int grow(void **ptr, size_t *have, size_t want);
 int grow_pinned(Device &d, size_t want);
 int scene_on_devices(const Scene *scene);                     // resident (and current) on every device of g.devs
+// the copy of a resident scene on the first device (g.devs[0]), made the current device; NULL (with the error set) if
+// the scene is not resident there or the device cannot be made current
+DeviceScene *first_device_scene(const Scene *scene);
 int scene_upload_all(const Scene *scene);                     // (re-)upload: device 0 over PCIe, peers over NVLink
 void scene_release_all(const Scene *scene);
 void release_device(Device &d);                               // everything the device owns (shutdown)

@@ -139,6 +139,21 @@ def register_callbacks(loaded: LoadedScene) -> None:
     gpu.rt_gpu_register_background(loaded.background_proc)
 
 
+def _resident(loaded: LoadedScene) -> None:
+    """Registers the scene's callbacks, then uploads the scene unless it is resident: the library refuses cast_rays,
+    AOV, masked and refit calls on a scene that is not."""
+    register_callbacks(loaded)
+    gpu = gpu_lib()
+    if gpu.rt_gpu_scene_device_bytes(C.byref(loaded.scene)) == 0:
+        gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+
+
+def _check_tensor(t, shape, dtypes, what) -> None:
+    """Raises unless `t` is a contiguous CUDA tensor of `shape` with one of `dtypes` (the first is the one named)."""
+    if t.device.type != "cuda" or t.dtype not in dtypes or tuple(t.shape) != shape or not t.is_contiguous():
+        raise ValueError(f"{what}: a contiguous CUDA tensor of shape {shape} and dtype {dtypes[0]} is required")
+
+
 def image_view(pixels: np.ndarray) -> Image:
     """Image header over a contiguous (H, W, C) uint8 array (driver.c:747-754)."""
     assert pixels.dtype == np.uint8 and pixels.ndim == 3 and pixels.flags["C_CONTIGUOUS"]
@@ -272,15 +287,13 @@ def cast_rays(loaded: LoadedScene, origins, directions, samples: int, max_bounce
     resident.  Returns the (n, 3) float32 sums over the samples (not divided); with per_sample, also the
     (n, samples, 3) radiance of every path, as (radiance, per_sample)."""
     gpu = gpu_lib()
-    register_callbacks(loaded)
     rays, _ = _query_rays(origins, directions, None)
     n = len(rays)
     if keys is not None:
         keys = np.ascontiguousarray(np.asarray(keys, dtype=np.uint32).reshape(-1))
         if len(keys) != n:
             raise ValueError(f"{len(keys)} keys for {n} rays")
-    if gpu.rt_gpu_scene_device_bytes(C.byref(loaded.scene)) == 0:
-        gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+    _resident(loaded)
     radiance = np.zeros((n, 3), dtype=np.float32)
     per = np.zeros((n, samples, 3), dtype=np.float32) if per_sample else None
     gpu_check(gpu.rt_gpu_cast_rays(C.byref(loaded.scene), rays.ctypes.data, keys.ctypes.data if keys is not None else None,
@@ -297,9 +310,7 @@ def render_aov(loaded: LoadedScene, width: int, height: int, samples: int, max_b
     face each sample's path shades.  The sums are not divided: divide by coverage for the mean over the covered samples.
     Uploads the scene if it is not resident."""
     gpu = gpu_lib()
-    register_callbacks(loaded)
-    if gpu.rt_gpu_scene_device_bytes(C.byref(loaded.scene)) == 0:
-        gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+    _resident(loaded)
     floats = C.sizeof(_ffi.GPUAOV) // 4
     records = np.zeros((height, width, floats), dtype=np.float32)
     gpu_check(gpu.rt_gpu_render_aov(C.byref(loaded.scene), width, height, sample_begin, sample_begin + samples,
@@ -321,20 +332,14 @@ def render_masked(loaded: LoadedScene, accum, sample_begin: int, sample_end: int
     import torch
     gpu = gpu_lib()
     height, width = accum.shape[0], accum.shape[1]
-
-    def check(t, shape, dtypes, what):
-        if t.device.type != "cuda" or t.dtype not in dtypes or tuple(t.shape) != shape or not t.is_contiguous():
-            raise ValueError(f"{what}: a contiguous CUDA tensor of shape {shape} and dtype {dtypes[0]} is required")
-    check(accum, (height, width, 3), (torch.float32,), "accum")
+    _check_tensor(accum, (height, width, 3), (torch.float32,), "accum")
     if accum_sq is not None:
-        check(accum_sq, (height, width, 3), (torch.float32,), "accum_sq")
+        _check_tensor(accum_sq, (height, width, 3), (torch.float32,), "accum_sq")
     if mask is not None:
-        check(mask, (height, width), (torch.uint8, torch.bool), "mask")
+        _check_tensor(mask, (height, width), (torch.uint8, torch.bool), "mask")
     if counters is not None:
-        check(counters, (8,), (torch.int64,), "counters")
-    register_callbacks(loaded)
-    if gpu.rt_gpu_scene_device_bytes(C.byref(loaded.scene)) == 0:
-        gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+        _check_tensor(counters, (8,), (torch.int64,), "counters")
+    _resident(loaded)
     st = stream or torch.cuda.current_stream()
     gpu_check(gpu.rt_gpu_render_masked_device(
         C.byref(loaded.scene), width, height, mask.data_ptr() if mask is not None else None, sample_begin, sample_end,
@@ -368,9 +373,7 @@ def refit(loaded: LoadedScene, positions=None, normals=None) -> None:
     hold.  LoadedScene.slot_of maps source triangles to slots.  Uploads the scene if it is not resident."""
     gpu = gpu_lib()
     t = loaded.scene.triangles
-    register_callbacks(loaded)
-    if gpu.rt_gpu_scene_device_bytes(C.byref(loaded.scene)) == 0:
-        gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+    _resident(loaded)
     if positions is not None:
         positions = np.asarray(positions, dtype=np.float32)
         if positions.shape != (3, 3, t.len):
@@ -394,16 +397,10 @@ def refit_device(loaded: LoadedScene, positions, normals=None, stream=None) -> N
     import torch
     gpu = gpu_lib()
     n = loaded.scene.triangles.len
-
-    def check(t, shape, what):
-        if t.device.type != "cuda" or t.dtype != torch.float32 or tuple(t.shape) != shape or not t.is_contiguous():
-            raise ValueError(f"{what}: a contiguous CUDA tensor of shape {shape} and dtype torch.float32 is required")
-    check(positions, (3, 3, n), "positions")
+    _check_tensor(positions, (3, 3, n), (torch.float32,), "positions")
     if normals is not None:
-        check(normals, (n, 3, 3), "normals")
-    register_callbacks(loaded)
-    if gpu.rt_gpu_scene_device_bytes(C.byref(loaded.scene)) == 0:
-        gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+        _check_tensor(normals, (n, 3, 3), (torch.float32,), "normals")
+    _resident(loaded)
     st = stream or torch.cuda.current_stream()
     gpu_check(gpu.rt_gpu_scene_refit_device(C.byref(loaded.scene), positions.data_ptr(),
                                             normals.data_ptr() if normals is not None else None, st.cuda_stream))
