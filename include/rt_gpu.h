@@ -331,6 +331,50 @@ int rt_gpu_render_masked_device(Scene const *scene, isize width, isize height,
 int rt_gpu_resolve_counts_device(f32 const *d_accum, i32 const *d_samples, isize width, isize height,
                                  u8 *d_pixels, isize stride, i32 components, void *stream);
 
+/* ---- many views of a resident scene in one call (csrc/rt_render.cu) ----
+ * rt_gpu_render_views_device renders samples [sample_begin, sample_end) of n_views whole images of one scene, view v
+ * from cameras[v], into slice v of d_accum ([n_views][H][W][3] f32).  After its primary trace a path no longer depends
+ * on the camera it came from, so each view runs its own primary trace (with the camera-relative copies and sky tiles
+ * of its camera) and every bounce launch is shared by the views: the renderer's fixed cost per call (launches, the
+ * tails of the late bounces) is paid once per call rather than once per view.
+ * Key property: slice v of d_accum equals, bit for bit,
+ *   rt_gpu_render_accum_device(scene, width, height, sample_begin, sample_end, max_bounces,
+ *                              user_seeds ? user_seeds[v] : 0, accumulate, ...)
+ * called with scene->camera = cameras[v], whatever the other views are, their number and order, and however the call is
+ * split into chunks inside.  The counters gain the sum of those per-view calls' counters, the extended slots [8..16)
+ * included when the library's own block (rt_gpu_counters_buffer) is passed.
+ *   - cameras: a host array; only the fields the renderer reads are used, rows 0..2 of view_matrix and focal_length.
+ *     scene->camera is neither read nor written by the call: a render after it uses scene->camera as before.
+ *   - seeds: view v's path (p, s) is seeded rt_path_seed(p, s, user_seeds[v]), the renderer's rule; NULL user_seeds =
+ *     0 for every view.  Pass distinct seeds for views whose noise should not be correlated.
+ *   - accumulate behaves per view as for a render: the sums continue from each slice, so [0, k) then [k, n) equals
+ *     [0, n).  An empty range or max_bounces = 0 traces and counts nothing and zeroes every slice unless accumulate is
+ *     set.  n_views = 0 is a no-op.
+ *   - RT_GPU_Options.fast_math applies as it does to a render (each view equals the fast single render); pixel_rank /
+ *     pixel_world do not apply (each view is a whole image).  First device only.
+ * Ordering: like a render, the call uses the device's path-queue workspace and rewrites the camera-relative scene
+ * copies, so it is serialised with renders, lightmap bakes, cast_rays and AOV calls on that device; it waits for the
+ * scene's geometry before its first primary trace and for its texels after it.
+ * Refused before any launch: width or height < 1, or an image whose one sample per pixel exceeds 2^31 path ids;
+ * sample_begin < 0, sample_end < sample_begin, sample_end > INT32_MAX; max_bounces < 0; n_views < 0; NULL cameras with
+ * n_views > 0; a NULL d_accum (device form) or both outputs NULL (host form); a scene that is not resident
+ * (rt_gpu_scene_upload).  No camera a render accepts is refused. */
+/* device pointers on the first device, ordered on `stream` (cudaStream_t as void*, NULL = the legacy default stream) */
+int rt_gpu_render_views_device(Scene const *scene, i32 n_views,
+                               Camera const *cameras,   /* host array [n_views] */
+                               u32 const *user_seeds,   /* optional host array [n_views]; NULL = 0 for every view */
+                               isize width, isize height, isize sample_begin, isize sample_end, isize max_bounces,
+                               i32 accumulate,
+                               f32 *d_accum,            /* [n_views][H][W][3] */
+                               u64 *d_counters,         /* optional 8 (16 with the library's own block) */
+                               void *stream);
+/* host memory: staged through the device's staging block, from zero; accum ([n_views][H][W][3] f32) and pixels
+ * ([n_views][H][W][3] u8, the film of rt_gpu_resolve_device with samples = sample_end - sample_begin; black when the
+ * range is empty) are each optional, but not both NULL; returns when the results are in place */
+int rt_gpu_render_views(Scene const *scene, i32 n_views, Camera const *cameras, u32 const *user_seeds,
+                        isize width, isize height, isize sample_begin, isize sample_end, isize max_bounces,
+                        f32 *accum, u8 *pixels);
+
 /* ---- moving geometry on a resident scene: refit the BVH and triangle records on the device (csrc/rt_refit.cu) ----
  * A refit keeps the topology scene_init chose (which triangle sits in which slot, which child is which) and recomputes,
  * from new vertex positions, everything that depends on them, with host/scene_build.c's f32 expressions:

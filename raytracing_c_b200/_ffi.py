@@ -145,6 +145,7 @@ GPU_EXPORTS = [
     "rt_gpu_render_aov_device", "rt_gpu_render_aov",
     "rt_gpu_render_masked_device", "rt_gpu_resolve_counts_device",
     "rt_gpu_scene_refit_device", "rt_gpu_scene_refit", "rt_gpu_read_nodes",
+    "rt_gpu_render_views_device", "rt_gpu_render_views",
 ]
 
 HOST_EXPORTS = [
@@ -288,6 +289,10 @@ def gpu_lib() -> C.CDLL:
         lib.rt_gpu_scene_refit_device.argtypes = [C.POINTER(Scene), C.c_void_p, C.c_void_p, C.c_void_p]
         lib.rt_gpu_scene_refit.argtypes = [C.POINTER(Scene), C.c_int32]
         lib.rt_gpu_read_nodes.argtypes = [C.POINTER(Scene), C.c_void_p]
+        lib.rt_gpu_render_views_device.argtypes = [C.POINTER(Scene), C.c_int32, C.c_void_p, C.c_void_p, isize, isize, isize,
+                                                   isize, isize, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.rt_gpu_render_views.argtypes = [C.POINTER(Scene), C.c_int32, C.c_void_p, C.c_void_p, isize, isize, isize, isize,
+                                            isize, C.c_void_p, C.c_void_p]
         lib.render_thread_proc.argtypes = [C.POINTER(RenderingContext)]
         lib.render_thread_proc.restype = None
         lib.rendering_context_is_finished.argtypes = [C.POINTER(RenderingContext)]

@@ -228,21 +228,29 @@ struct Share {            // what one device (or process) renders of a frame
   int   split_rank, split_world;
 };
 
+// the views of a many-view call (rt_gpu_render_views_device): cameras and optional seeds, host arrays of n
+struct Views { int n; const ViewCamera *cameras; const u32 *seeds; };
+
 // One render of `share` on device d, enqueued on `stream`: a workspace user.  d_mask / d_accum_sq (optional) make it a
-// masked pass (rt_gpu_render_masked_device).
+// masked pass (rt_gpu_render_masked_device); `views` (optional) renders each of them into its slice of d_accum
+// (rt_gpu_render_views_device).
 int render_on_device(Device &d, const Scene *scene, isize width, isize height, const Share &share, isize max_bounces,
                      u32 seed, int accumulate, float *d_accum, float *d_per_sample, int *d_hit_ids,
                      unsigned long long *d_counters, cudaStream_t stream, const u8 *d_mask = nullptr,
-                     float *d_accum_sq = nullptr) {
+                     float *d_accum_sq = nullptr, const Views *views = nullptr) {
   if (width < 1 || height < 1) return fail("render: empty image");
   CUDA_TRY(cudaSetDevice(d.id));
   auto it = d.scenes.find(scene);
   if (it == d.scenes.end()) return fail("render: scene is not resident on device %d", d.id);
   const DeviceScene &ds = it->second;
   const isize n_samples = share.s_end - share.s_begin;
-  if (workspace_begin(d, ds, n_samples > 0 ? camera_workspace(width, height, n_samples, max_bounces, share.split_world)
-                                           : WorkspaceRequest{}, false, stream))
-    return 1;
+  WorkspaceRequest r;
+  if (n_samples > 0 && views)
+    r = {rt_render_views_workspace_bytes((int)width, (int)height, views->n, (int)n_samples, (int)max_bounces, false),
+         rt_render_views_workspace_bytes((int)width, (int)height, views->n, 1, (int)max_bounces, true)};
+  else if (n_samples > 0)
+    r = camera_workspace(width, height, n_samples, max_bounces, share.split_world);
+  if (workspace_begin(d, ds, r, false, stream)) return 1;
   RenderParams p{};
   p.scene = ds.dev;
   p.shading_ready = ds.tex_ready;
@@ -256,6 +264,10 @@ int render_on_device(Device &d, const Scene *scene, isize width, isize height, c
   p.counters = d_counters;
   p.counters_ex = (d_counters && d_counters == d.d_counters) ? d_counters + 8 : nullptr;   // the library's own buffer has 16 slots
   p.pixel_mask = d_mask; p.accum_sq = d_accum_sq;
+  if (views) {
+    p.n_views = views->n; p.cameras = views->cameras; p.user_seeds = views->seeds;
+    p.view_stride = (size_t)width * (size_t)height * 3;
+  }
   return workspace_end(d, "render", rt_launch_render(p, d.sm_count, d.d_workspace, d.workspace_bytes, stream, &g.last_launches),
                        stream);
 }
@@ -810,6 +822,86 @@ int rt_gpu_render_masked_device(Scene const *scene, isize width, isize height, u
   return render_on_device(g.devs[0], scene, width, height, share, max_bounces, user_seed, accumulate, d_accum, nullptr,
                           nullptr, reinterpret_cast<unsigned long long *>(d_counters), static_cast<cudaStream_t>(stream),
                           d_mask, d_accum_sq);
+}
+
+// ------------------------------------------------------------- many views of a resident scene
+}  // extern "C"
+
+namespace {
+
+// Everything that is refused before a launch of a many-view call writing into `out`: camera_validate's refusals, a
+// negative view count, NULL cameras for a non-empty call.  The cameras themselves are not checked: a render accepts any.
+int views_validate(const char *what, const Scene *scene, i32 n_views, const Camera *cameras, isize width, isize height,
+                   isize sample_begin, isize sample_end, isize max_bounces, const void *out, const char *out_name) {
+  if (n_views < 0) return fail("%s: n_views = %d, must be >= 0", what, (int)n_views);
+  if (camera_validate(what, scene, width, height, sample_begin, sample_end, max_bounces, out, out_name)) return 1;
+  if (n_views > 0) return check_given(what, cameras, "cameras");
+  return 0;
+}
+
+// One many-view call on the first device, ordered on `stream`: the renderer with a camera and a seed per view, each view
+// into its W*H*3 slice of d_accum.  The cameras go to the launcher as copies; the resident scene's camera is not touched.
+int views_on_device(const Scene *scene, i32 n_views, const Camera *cameras, const u32 *seeds, isize width, isize height,
+                    isize sample_begin, isize sample_end, isize max_bounces, int accumulate, float *d_accum,
+                    unsigned long long *d_counters, cudaStream_t stream) {
+  std::vector<ViewCamera> views((size_t)n_views);
+  for (int v = 0; v < n_views; v++) {
+    for (int r = 0; r < 3; r++)
+      for (int c = 0; c < 4; c++) views[(size_t)v].view[r][c] = cameras[v].view_matrix.rows[r][c];
+    views[(size_t)v].focal_length = cameras[v].focal_length;
+  }
+  const Views vs{(int)n_views, views.data(), seeds};
+  const Share share{sample_begin, sample_end, 0, 1};
+  return render_on_device(g.devs[0], scene, width, height, share, max_bounces, 0, accumulate, d_accum, nullptr, nullptr,
+                          d_counters, stream, nullptr, nullptr, &vs);
+}
+
+}  // namespace
+
+extern "C" {
+
+int rt_gpu_render_views_device(Scene const *scene, i32 n_views, Camera const *cameras, u32 const *user_seeds, isize width,
+                               isize height, isize sample_begin, isize sample_end, isize max_bounces, i32 accumulate,
+                               f32 *d_accum, u64 *d_counters, void *stream) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  if (views_validate("render_views", scene, n_views, cameras, width, height, sample_begin, sample_end, max_bounces,
+                     d_accum, "accum"))
+    return 1;
+  if (n_views == 0) return 0;
+  return views_on_device(scene, n_views, cameras, user_seeds, width, height, sample_begin, sample_end, max_bounces,
+                         accumulate, d_accum, reinterpret_cast<unsigned long long *>(d_counters),
+                         static_cast<cudaStream_t>(stream));
+}
+
+// Host memory: the sums are computed from zero in a staging part; each view's image is the film of its slice.
+int rt_gpu_render_views(Scene const *scene, i32 n_views, Camera const *cameras, u32 const *user_seeds, isize width,
+                        isize height, isize sample_begin, isize sample_end, isize max_bounces, f32 *accum, u8 *pixels) {
+  std::lock_guard<std::mutex> lock(g_mutex);
+  g.last_launches = 0;
+  if (views_validate("render_views", scene, n_views, cameras, width, height, sample_begin, sample_end, max_bounces,
+                     accum ? static_cast<const void *>(accum) : pixels, "accum and pixels"))
+    return 1;
+  if (n_views == 0) return 0;
+  const size_t image = (size_t)width * (size_t)height * 3, n = (size_t)n_views * image;
+  const isize samples = sample_end - sample_begin;
+  return host_call({HostPart{n * sizeof(float), nullptr, accum}, {pixels ? n : 0, nullptr, pixels}},
+                   [&](void **part, cudaStream_t stream) {
+                     float *d_accum = static_cast<float *>(part[0]);
+                     u8 *d_pixels = static_cast<u8 *>(part[1]);
+                     if (views_on_device(scene, n_views, cameras, user_seeds, width, height, sample_begin, sample_end,
+                                         max_bounces, 0, d_accum, nullptr, stream))
+                       return 1;
+                     if (!pixels) return 0;
+                     if (samples < 1) {            // no samples: black images
+                       CUDA_TRY(cudaMemsetAsync(d_pixels, 0, n, stream));
+                       return 0;
+                     }
+                     for (size_t v = 0; v < (size_t)n_views; v++)
+                       if (launched("resolve", rt_launch_resolve(d_accum + v * image, (int)width, (int)height, (int)samples,
+                                                                 d_pixels + v * image, (int)width, 3, stream)))
+                         return 1;
+                     return 0;
+                   });
 }
 
 // ------------------------------------------------------------------ moving geometry (rt_scene.cu: scene_refit)

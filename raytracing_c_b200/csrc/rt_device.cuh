@@ -69,6 +69,9 @@ struct SceneDev {
 
 struct ReduceParts { const float *part[RT_MAX_PARTS]; int n; };
 
+// the fields of a Camera the renderer reads: rows 0..2 of the camera-to-world matrix and the focal length
+struct ViewCamera { float view[3][4]; float focal_length; };
+
 struct RenderParams {
   SceneDev  scene;
   int       width, height;
@@ -85,6 +88,12 @@ struct RenderParams {
   unsigned long long *counters_ex;
   const unsigned char *pixel_mask;       // optional W*H: only pixels with a non-zero byte are rendered (masked passes)
   float    *accum_sq;                    // optional W*H*3: per-channel sum of squared radiance in sample order
+  // many views of the scene in one call (rt_gpu_render_views_device): with cameras, view v renders from cameras[v] with
+  // the seed user_seeds[v] (NULL: user_seed) into accum + v * view_stride.  NULL cameras = one view, the scene's camera.
+  int       n_views;
+  const ViewCamera *cameras;             // host array [n_views]
+  const uint32_t   *user_seeds;          // optional host array [n_views]
+  size_t    view_stride;                 // floats between the views' accumulators
 };
 
 __device__ __forceinline__ V3 mk3(float x, float y, float z) { V3 v; v.x = x; v.y = y; v.z = z; return v; }

@@ -11,6 +11,9 @@
 // pixels are rendered (the others are zeroed without p.accumulate, untouched with it) and the second moments are summed.
 size_t rt_render_workspace_bytes(int width, int height, int n_samples, int max_bounces, int split_world);
 int rt_render_chunk_samples(int width, int height, int split_world);
+// a many-view call (RenderParams.cameras) of n_views whole images: the views' tile lists and one chunk of a group of views
+// at the preferred size, or with `floor` the least the launch accepts (one sample of one view)
+size_t rt_render_views_workspace_bytes(int width, int height, int n_views, int n_samples, int max_bounces, bool floor);
 unsigned rt_render_tiles(int width, int height, int split_rank, int split_world);
 int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_t workspace_bytes,
                      cudaStream_t stream, int *n_launches);

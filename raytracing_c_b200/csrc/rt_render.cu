@@ -28,6 +28,7 @@
 #include <math_constants.h>
 
 #include <cmath>
+#include <cstdint>
 #include <cstdlib>
 #include <vector>
 
@@ -269,13 +270,33 @@ size_t rt_render_workspace_bytes(int width, int height, int n_samples, int max_b
   return tile_list_bytes(tiles) + counts_bytes(max_bounces) + chunk_samples(per_sample, n_samples) * per_sample * RT_PATH_BYTES;
 }
 
+// Views per chunk of a many-view call: as many as one sample of each fits the preferred chunk size and `paths` (what the
+// workspace holds), at least one.  per_view: the paths of one sample of one view.
+static size_t view_group(int n_views, size_t per_view, size_t paths) {
+  size_t g = chunk_paths_max() / per_view;
+  if (g > paths / per_view) g = paths / per_view;
+  if (g < 1) g = 1;
+  return g < (size_t)n_views ? g : (size_t)n_views;
+}
+
+// The workspace of a many-view call: the views' tile lists, then one chunk of n_samples samples of a group of views at the
+// preferred size, or with `floor` one sample of one view.  n_views = 1 is rt_render_workspace_bytes.
+size_t rt_render_views_workspace_bytes(int width, int height, int n_views, int n_samples, int max_bounces, bool floor) {
+  const unsigned tiles = rt_render_tiles(width, height, 0, 1);
+  size_t per_view = (size_t)tiles * 32;
+  if (per_view < 32) per_view = 32;
+  const size_t per_sample = floor ? per_view : view_group(n_views, per_view, SIZE_MAX) * per_view;
+  return tile_list_bytes(tiles) * (size_t)n_views + counts_bytes(max_bounces) +
+         chunk_samples(per_sample, floor ? 1 : n_samples) * per_sample * RT_PATH_BYTES;
+}
+
 // trace kernels' blocks per SM at the level-store size they were measured for, per device (cudaFuncSetAttribute is per device)
-struct TraceOccupancy { size_t level_bytes; int primary, generic, wide, fast, fast_wide, masked; };
+struct TraceOccupancy { size_t level_bytes; int primary, generic, wide, fast, fast_wide, masked, based; };
 static TraceOccupancy g_occupancy[RT_MAX_DEVICES];
 
 // what a launcher needs of trace_launch_setup: the device, the level store, and the trace kernels' persistent grids
 // (one wave: blocks per SM x SMs)
-struct TraceLaunch { int dev; size_t level_bytes; unsigned primary, generic, wide, fast, fast_wide, masked; };
+struct TraceLaunch { int dev; size_t level_bytes; unsigned primary, generic, wide, fast, fast_wide, masked, based; };
 
 // ---- optional per-stage timing (bench.py's roofline leg): CUDA events around every launch, on the
 // launching stream; read back and summed by rt_stage_profile_read
@@ -360,11 +381,12 @@ static int trace_launch_setup(const SceneDev &scene, int sm_count, TraceLaunch &
     o.wide = level_store_blocks_per_sm((const void *)rt_trace_kernel<false, RT_TRACE_MIN_BLOCKS_WIDE>, level_bytes);
     o.fast = rt_fast_trace_setup(level_bytes, &o.fast_wide);
     o.masked = level_store_blocks_per_sm((const void *)rt_trace_kernel<true, RT_TRACE_MIN_BLOCKS_PRIMARY, true>, level_bytes);
+    o.based = level_store_blocks_per_sm((const void *)rt_trace_kernel<true, RT_TRACE_MIN_BLOCKS_PRIMARY, false, true>, level_bytes);
     o.level_bytes = level_bytes;
   }
   t = TraceLaunch{dev, level_bytes, (unsigned)(sm_count * o.primary), (unsigned)(sm_count * o.generic),
                   (unsigned)(sm_count * o.wide), (unsigned)(sm_count * o.fast), (unsigned)(sm_count * o.fast_wide),
-                  (unsigned)(sm_count * o.masked)};
+                  (unsigned)(sm_count * o.masked), (unsigned)(sm_count * o.based)};
   return 0;
 }
 
@@ -516,14 +538,34 @@ rt_sky_tiles_kernel(const __grid_constant__ StageParams P, const SkyFrame f, uns
   if (threadIdx.x == 0) { tiles[0] = P.n_tiles - base_sky; tiles[1] = base_sky; }
 }
 
+// The scene as view v of a render sees it: the scene's own camera, or (many views) cameras[v] on a copy.
+static SceneDev view_scene(const RenderParams &p, int v) {
+  SceneDev sc = p.scene;
+  if (p.cameras) {
+    for (int r = 0; r < 3; r++)
+      for (int c = 0; c < 4; c++) sc.view[r][c] = p.cameras[v].view[r][c];
+    sc.focal_length = p.cameras[v].focal_length;
+  }
+  return sc;
+}
+
+// Many views (p.cameras): each view is exactly the render it replaces.  A chunk covers a group of views and a sample
+// range; view v of the group owns the path ids [base_v, base_v + n_tiles * 32 * S), base_v = (v - v0) * n_tiles * 32 * S
+// (sky tiles leave holes, so the host knows every base).  Per view: the camera-relative copies (one copy, rewritten when
+// the view changes: stream order makes that safe), the primary trace with the view's camera, seed and tile list, and on
+// its first chunk the sky kernel; the bounce launches are shared by the group; then one accumulate per view.  A render is
+// one view with the scene's camera and enqueues what it always has.
 int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_t workspace_bytes,
                      cudaStream_t stream, int *n_launches) {
+  const int n_views = p.cameras ? p.n_views : 1;
+  const size_t image_bytes = (size_t)p.width * p.height * 3 * sizeof(float);
+  if (n_views < 1) return (int)cudaGetLastError();
   const int n_total = p.sample_end - p.sample_begin;
   if (n_total <= 0 || p.max_bounces < 1) {
     // no samples, or cast_ray's loop body never runs (raytracer.c:512,557): the sum gains nothing
     if (!p.accumulate) {
-      cudaMemsetAsync(p.accum, 0, (size_t)p.width * p.height * 3 * sizeof(float), stream);
-      if (p.accum_sq) cudaMemsetAsync(p.accum_sq, 0, (size_t)p.width * p.height * 3 * sizeof(float), stream);
+      for (int v = 0; v < n_views; v++) cudaMemsetAsync(p.accum + (size_t)v * p.view_stride, 0, image_bytes, stream);
+      if (p.accum_sq) cudaMemsetAsync(p.accum_sq, 0, image_bytes, stream);
     }
     return (int)cudaGetLastError();
   }
@@ -541,78 +583,110 @@ int rt_launch_render(const RenderParams &p, int sm_count, void *workspace, size_
   P.accum_sq = p.accum_sq;
   const bool masked_sum = p.pixel_mask || p.accum_sq;      // the MASKED accumulate: mask, second moments or both
 
-  // chunking: as many samples of every pixel per chunk as the workspace holds paths
+  // chunking: as many samples of every pixel (of a group of views) per chunk as the workspace holds paths
   const size_t per_sample = (size_t)P.n_tiles * 32;
   if (P.split_world > 1 && !p.accumulate)      // the pixels of other ranks stay zero (the cross-rank sum adds them)
-    cudaMemsetAsync(p.accum, 0, (size_t)p.width * p.height * 3 * sizeof(float), stream);
+    cudaMemsetAsync(p.accum, 0, image_bytes, stream);
   if (per_sample == 0) return (int)cudaGetLastError();
-  // the tile lists first, then the path queues
-  const size_t list_bytes = tile_list_bytes(P.n_tiles);
-  if (workspace_bytes < list_bytes) return (int)cudaErrorMemoryAllocation;
-  unsigned *tiles = static_cast<unsigned *>(workspace);
-  const int chunk = fit_chunk(P, per_sample, n_total, 0, static_cast<char *>(workspace) + list_bytes,
-                              workspace_bytes - list_bytes, nullptr);
+  // the tile lists first (one per view), then the path queues
+  const size_t list_bytes = tile_list_bytes(P.n_tiles), lists_bytes = list_bytes * (size_t)n_views;
+  if (workspace_bytes < lists_bytes) return (int)cudaErrorMemoryAllocation;
+  const size_t queue_bytes = workspace_bytes - lists_bytes;
+  const int group = (int)view_group(n_views, per_sample, path_capacity(queue_bytes, P.max_bounces, RT_PATH_BYTES));
+  const int chunk = fit_chunk(P, (size_t)group * per_sample, n_total, 0, static_cast<char *>(workspace) + lists_bytes,
+                              queue_bytes, nullptr);
   if (chunk == 0) return (int)cudaErrorMemoryAllocation;
 
-  rt_camera_relative_kernel<<<(unsigned)sm_count, 256, 0, stream>>>(p.scene);
-  int launches = 1;
-  SkyFrame sky;
-  if (sky_frame(p.scene, p.width, p.height, sky)) {
-    rt_sky_tiles_kernel<<<1, 1024, 0, stream>>>(P, sky, tiles);
-    P.tiles = tiles;
-    launches++;
-  }
-  for (int s0 = p.sample_begin; s0 < p.sample_end; s0 += chunk) {
-    P.per_sample_offset = s0 - p.sample_begin;
-    P.hit_ids = (s0 == p.sample_begin) ? p.hit_ids : nullptr;
-    camera_chunk(P, s0, p.sample_end, chunk, p.accumulate || s0 > p.sample_begin || P.split_world > 1, stream);
-    P.bounce = 0;
-    {
-      StageTimer st(RT_STAGE_TRACE * RT_STAGE_BOUNCES, stream, t.dev);
-      if (p.pixel_mask) rt_trace_kernel<true, RT_TRACE_MIN_BLOCKS_PRIMARY, true><<<t.masked, RT_BLOCK, t.level_bytes, stream>>>(P);
-      else              rt_trace_kernel<true><<<t.primary, RT_BLOCK, t.level_bytes, stream>>>(P);
-    }
-    launches++;
-    // textures and the environment may still be in flight on the upload's copy stream: the primary trace reads
-    // nodes and triangles only, everything after it waits here (rt_scene.cu)
-    if (s0 == p.sample_begin && p.shading_ready) cudaStreamWaitEvent(stream, p.shading_ready, 0);
-    if (s0 == p.sample_begin && P.tiles) {
-      // every sample of the call's sky tiles in one launch, timed as a bounce-0 miss stage
-      StageParams S = P;
-      S.sample0 = p.sample_begin; S.n_samples = n_total;
-      S.per_sample_offset = 0;
-      S.hit_ids = p.hit_ids;
-      StageTimer st(RT_STAGE_MISS * RT_STAGE_BOUNCES, stream, t.dev);
-      if (p.fast) rt_fast_launch_sky(S, flat_grid(sm_count) * 4, stream);
-      else        rt_sky_kernel<<<flat_grid(sm_count) * 4, 256, 0, stream>>>(S);
+  rt_camera_relative_kernel<<<(unsigned)sm_count, 256, 0, stream>>>(view_scene(p, 0));
+  int launches = 1, relative_view = 0;          // the view the camera-relative copies hold
+  std::vector<const unsigned *> tiles((size_t)n_views, nullptr);
+  for (int v = 0; v < n_views; v++) {
+    SkyFrame sky;
+    unsigned *list = reinterpret_cast<unsigned *>(static_cast<char *>(workspace) + (size_t)v * list_bytes);
+    if (sky_frame(view_scene(p, v), p.width, p.height, sky)) {
+      rt_sky_tiles_kernel<<<1, 1024, 0, stream>>>(P, sky, list);
+      tiles[(size_t)v] = list;
       launches++;
     }
-    for (int b = 0; b < p.max_bounces; b++) {
-      P.bounce = b;
-      const int bslot = b < RT_STAGE_BOUNCES ? b : RT_STAGE_BOUNCES - 1;
-      if (b > 0) {
-        StageTimer st(RT_STAGE_TRACE * RT_STAGE_BOUNCES + bslot, stream, t.dev);
-        launch_bounce_trace(P, t, p.fast, stream);
+  }
+  P.tiles = tiles[0];
+  bool shading_waited = false;
+  for (int v0 = 0; v0 < n_views; v0 += group) {
+    const int v1 = v0 + group < n_views ? v0 + group : n_views;
+    for (int s0 = p.sample_begin; s0 < p.sample_end; s0 += chunk) {
+      P.per_sample_offset = s0 - p.sample_begin;
+      P.hit_ids = (s0 == p.sample_begin) ? p.hit_ids : nullptr;
+      camera_chunk(P, s0, p.sample_end, chunk, p.accumulate || s0 > p.sample_begin || P.split_world > 1, stream);
+      P.bounce = 0;
+      for (int v = v0; v < v1; v++) {
+        // view v's primary trace: its camera, seed and tile list, its paths from base_v; the HIT / MISS appends continue
+        StageParams Pv = P;
+        Pv.scene = view_scene(p, v);
+        Pv.user_seed = p.user_seeds ? p.user_seeds[v] : p.user_seed;
+        Pv.tiles = tiles[(size_t)v];
+        Pv.accum = p.accum + (size_t)v * p.view_stride;
+        Pv.path_base = (unsigned)(v - v0) * P.n_paths;
+        if (v != relative_view) {
+          rt_camera_relative_kernel<<<(unsigned)sm_count, 256, 0, stream>>>(Pv.scene);
+          relative_view = v;
+          launches++;
+        }
+        if (v > v0) cudaMemsetAsync(&P.q.counts[Q_FETCH], 0, sizeof(unsigned), stream);
+        {
+          StageTimer st(RT_STAGE_TRACE * RT_STAGE_BOUNCES, stream, t.dev);
+          if (p.pixel_mask)   rt_trace_kernel<true, RT_TRACE_MIN_BLOCKS_PRIMARY, true><<<t.masked, RT_BLOCK, t.level_bytes, stream>>>(Pv);
+          else if (p.cameras) rt_trace_kernel<true, RT_TRACE_MIN_BLOCKS_PRIMARY, false, true><<<t.based, RT_BLOCK, t.level_bytes, stream>>>(Pv);
+          else                rt_trace_kernel<true><<<t.primary, RT_BLOCK, t.level_bytes, stream>>>(Pv);
+        }
+        launches++;
+        // textures and the environment may still be in flight on the upload's copy stream: the primary trace reads
+        // nodes and triangles only, everything after the call's first one waits here (rt_scene.cu)
+        if (!shading_waited && p.shading_ready) cudaStreamWaitEvent(stream, p.shading_ready, 0);
+        shading_waited = true;
+        if (s0 == p.sample_begin && Pv.tiles) {
+          // every sample of the view's sky tiles in one launch, timed as a bounce-0 miss stage
+          StageParams S = Pv;
+          S.sample0 = p.sample_begin; S.n_samples = n_total;
+          S.per_sample_offset = 0;
+          S.hit_ids = p.hit_ids;
+          StageTimer st(RT_STAGE_MISS * RT_STAGE_BOUNCES, stream, t.dev);
+          if (p.fast) rt_fast_launch_sky(S, flat_grid(sm_count) * 4, stream);
+          else        rt_sky_kernel<<<flat_grid(sm_count) * 4, 256, 0, stream>>>(S);
+          launches++;
+        }
+      }
+      for (int b = 0; b < p.max_bounces; b++) {
+        P.bounce = b;
+        const int bslot = b < RT_STAGE_BOUNCES ? b : RT_STAGE_BOUNCES - 1;
+        if (b > 0) {
+          StageTimer st(RT_STAGE_TRACE * RT_STAGE_BOUNCES + bslot, stream, t.dev);
+          launch_bounce_trace(P, t, p.fast, stream);
+          launches++;
+        }
+        {
+          StageTimer st(RT_STAGE_MISS * RT_STAGE_BOUNCES + bslot, stream, t.dev);
+          if (p.fast) rt_fast_launch_miss(P, miss_grid(sm_count, b), stream);
+          else        rt_miss_kernel<<<miss_grid(sm_count, b), 256, 0, stream>>>(P);
+        }
+        {
+          StageTimer st(RT_STAGE_SHADE * RT_STAGE_BOUNCES + bslot, stream, t.dev);
+          if (p.fast) rt_fast_launch_shade(P, shade_grid(sm_count, b), stream);
+          else        rt_shade_kernel<<<shade_grid(sm_count, b), 256, 0, stream>>>(P);
+        }
+        launches += 2;
+      }
+      for (int v = v0; v < v1; v++) {
+        // view v's sums from its own paths: rad from base_v, its tile list, its accumulator
+        StageParams A = P;
+        A.tiles = tiles[(size_t)v];
+        A.accum = p.accum + (size_t)v * p.view_stride;
+        A.q.rad = P.q.rad + (size_t)(v - v0) * P.n_paths;
+        StageTimer st(RT_STAGE_ACCUMULATE * RT_STAGE_BOUNCES, stream, t.dev);
+        if (masked_sum) rt_accumulate_masked_kernel<<<flat_grid(sm_count) * 4, 256, 0, stream>>>(A);
+        else            rt_accumulate_kernel<<<flat_grid(sm_count) * 4, 256, 0, stream>>>(A);
         launches++;
       }
-      {
-        StageTimer st(RT_STAGE_MISS * RT_STAGE_BOUNCES + bslot, stream, t.dev);
-        if (p.fast) rt_fast_launch_miss(P, miss_grid(sm_count, b), stream);
-        else        rt_miss_kernel<<<miss_grid(sm_count, b), 256, 0, stream>>>(P);
-      }
-      {
-        StageTimer st(RT_STAGE_SHADE * RT_STAGE_BOUNCES + bslot, stream, t.dev);
-        if (p.fast) rt_fast_launch_shade(P, shade_grid(sm_count, b), stream);
-        else        rt_shade_kernel<<<shade_grid(sm_count, b), 256, 0, stream>>>(P);
-      }
-      launches += 2;
     }
-    {
-      StageTimer st(RT_STAGE_ACCUMULATE * RT_STAGE_BOUNCES, stream, t.dev);
-      if (masked_sum) rt_accumulate_masked_kernel<<<flat_grid(sm_count) * 4, 256, 0, stream>>>(P);
-      else            rt_accumulate_kernel<<<flat_grid(sm_count) * 4, 256, 0, stream>>>(P);
-    }
-    launches++;
   }
   if (n_launches) *n_launches += launches;
   return (int)cudaGetLastError();

@@ -80,6 +80,8 @@ struct __align__(16) StageParams {
   // tile ids ascending from [2] and the sky tile ids from [2 + n_tiles - 1] down.  The primary trace and the accumulate
   // cover the traced tiles only (path ids are built on the list), rt_sky_kernel the sky tiles.  NULL = every tile traced.
   const unsigned *tiles;
+  // many views in one call (rt_render.cu): the first path id of this view's primary trace; read by the BASED trace only
+  unsigned   path_base;
 };
 
 // raytracer.c:582-594, one lane of hash12x8.  Ray generation is spelled with round-to-nearest intrinsics, which are
@@ -156,7 +158,9 @@ __device__ __forceinline__ void path_pixel(const StageParams &P, unsigned path, 
 // bounce 1: more warps to cover the divergent loads), the short late queues lose 5-10 % to it (their time is the
 // slowest ray's latency, which spills lengthen) — the host picks per bounce (rt_render.cu, RT_TRACE_WIDE_BOUNCES).
 // MASKED (primary only): a path id whose pixel P.pixel_mask does not select takes no ray, as one outside the image.
-template <bool PRIMARY, int MIN_BLOCKS = (PRIMARY ? RT_TRACE_MIN_BLOCKS_PRIMARY : RT_TRACE_MIN_BLOCKS), bool MASKED = false>
+// BASED (primary only): the path handed on is P.path_base + q, so the views of one call own disjoint ranges of path ids.
+template <bool PRIMARY, int MIN_BLOCKS = (PRIMARY ? RT_TRACE_MIN_BLOCKS_PRIMARY : RT_TRACE_MIN_BLOCKS), bool MASKED = false,
+          bool BASED = false>
 __global__ void __launch_bounds__(RT_BLOCK, MIN_BLOCKS)
 RT_KN(rt_trace_kernel)(const __grid_constant__ StageParams P) {
   extern __shared__ float4 level_store[];          // [depth - 1][2][RT_BLOCK] entry distances of pending levels (2 .. depth)
@@ -187,7 +191,7 @@ RT_KN(rt_trace_kernel)(const __grid_constant__ StageParams P) {
       const bool is_hit = fin && w.hit_slot >= 0;
       const bool is_miss = fin && w.hit_slot < 0;
       if (__any_sync(RT_FULL, fin)) {
-        unsigned path = q;
+        unsigned path = BASED ? P.path_base + q : q;
         uint32_t rng = seed0;
         if (fin) {
           if (PRIMARY) {

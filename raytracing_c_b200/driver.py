@@ -347,6 +347,58 @@ def render_masked(loaded: LoadedScene, accum, sample_begin: int, sample_end: int
         counters.data_ptr() if counters is not None else None, st.cuda_stream))
 
 
+def _views_args(cameras, user_seeds):
+    """The host arrays of a many-view call: cameras (a sequence of Camera) and the optional per-view u32 seeds."""
+    cameras = list(cameras)
+    cams = (Camera * max(len(cameras), 1))(*cameras)
+    seeds = None
+    if user_seeds is not None:
+        seeds = np.ascontiguousarray(np.asarray(user_seeds, dtype=np.uint32).reshape(-1))
+        if len(seeds) != len(cameras):
+            raise ValueError(f"{len(seeds)} user_seeds for {len(cameras)} cameras")
+    return len(cameras), cams, seeds
+
+
+def render_views(loaded: LoadedScene, cameras, accum, sample_begin: int, sample_end: int, user_seeds=None,
+                 max_bounces: int = 8, accumulate: bool = False, counters=None, stream=None) -> None:
+    """Samples [sample_begin, sample_end) of one whole image per camera in one call (rt_gpu_render_views_device;
+    semantics in include/rt_gpu.h), enqueued on `stream` (default: torch's current stream).  `cameras` is a sequence of
+    Camera (as look_at returns); `accum` a contiguous (V, H, W, 3) float32 CUDA tensor whose slice v is, bit for bit, the
+    render of cameras[v] with the seed user_seeds[v] (default 0), continued with `accumulate`.  `counters` is an optional
+    8-element int64 CUDA tensor the work counters are added to.  The Scene's own camera is not used or changed.  Uploads
+    the scene if it is not resident."""
+    import torch
+    gpu = gpu_lib()
+    n, cams, seeds = _views_args(cameras, user_seeds)
+    if accum.dim() != 4:
+        raise ValueError("accum: a contiguous CUDA tensor of shape (V, H, W, 3) and dtype torch.float32 is required")
+    height, width = accum.shape[1], accum.shape[2]
+    _check_tensor(accum, (n, height, width, 3), (torch.float32,), "accum")
+    if counters is not None:
+        _check_tensor(counters, (8,), (torch.int64,), "counters")
+    _resident(loaded)
+    st = stream or torch.cuda.current_stream()
+    gpu_check(gpu.rt_gpu_render_views_device(
+        C.byref(loaded.scene), n, cams, seeds.ctypes.data if seeds is not None else None, width, height, sample_begin,
+        sample_end, max_bounces, int(accumulate), accum.data_ptr(), counters.data_ptr() if counters is not None else None,
+        st.cuda_stream))
+
+
+def render_views_images(loaded: LoadedScene, cameras, width: int, height: int, samples: int, max_bounces: int = 8,
+                        sample_begin: int = 0, user_seeds=None, want_accum: bool = False):
+    """The host-memory form (rt_gpu_render_views): the (V, H, W, 3) uint8 images of samples [sample_begin,
+    sample_begin + samples) of each camera, each the film of its view's sums; with want_accum, (images, sums) with the
+    (V, H, W, 3) float32 sums.  Uploads the scene if it is not resident."""
+    n, cams, seeds = _views_args(cameras, user_seeds)
+    _resident(loaded)
+    pixels = np.zeros((n, height, width, 3), dtype=np.uint8)
+    accum = np.zeros((n, height, width, 3), dtype=np.float32) if want_accum else None
+    gpu_check(gpu_lib().rt_gpu_render_views(C.byref(loaded.scene), n, cams, seeds.ctypes.data if seeds is not None else None,
+                                            width, height, sample_begin, sample_begin + samples, max_bounces,
+                                            accum.ctypes.data if accum is not None else None, pixels.ctypes.data))
+    return (pixels, accum) if want_accum else pixels
+
+
 def scene_positions(loaded: LoadedScene) -> np.ndarray:
     """A copy of the Scene's vertex positions in slot order, as the refit takes them: (3, 3, n_slots) float32, indexed
     [axis][vertex][slot] (the block order x0 x1 x2 y0 y1 y2 z0 z1 z2)."""
