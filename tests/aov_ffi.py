@@ -11,8 +11,8 @@ import os
 
 import numpy as np
 
-import cast_rays_ffi
 import oracle_ffi
+from helpers import CSRC, MODELS, ROOT, bits  # noqa: F401  (bits is re-exported)
 from raytracing_c_b200._ffi import Scene, isize
 
 FLOATS = 16
@@ -29,9 +29,9 @@ def aov_lib() -> C.CDLL:
     if _aov_lib is None:
         oracle_ffi.lib()                                   # builds liboracle.so if it is missing
         o = oracle_ffi.ORACLE_DIR
-        path = cast_rays_ffi._compile("libaov_oracle.so", [
-            "-O2", "-std=gnu11", "-mavx2", "-mfma", "-ffp-contract=off", "-I", os.path.join(cast_rays_ffi.ROOT, "include"),
-            "-I", o, os.path.join(cast_rays_ffi.CSRC, "aov_oracle.c"), "-lpthread", "-lm"])
+        path = oracle_ffi.build_lib("libaov_oracle.so", [
+            "-O2", "-std=gnu11", "-mavx2", "-mfma", "-ffp-contract=off", "-I", os.path.join(ROOT, "include"),
+            "-I", o, os.path.join(CSRC, "aov_oracle.c"), "-lpthread", "-lm"])
         lib = C.CDLL(path)
         lib.oracle_render_aov.argtypes = [C.POINTER(Scene), isize, isize, isize, isize, isize, C.c_void_p, C.c_void_p,
                                           C.c_int32]
@@ -73,14 +73,9 @@ def device_aov(loaded, width, height, sample_begin, sample_end, max_bounces=8, a
             "counters": dict(zip(oracle_ffi.COUNTER_NAMES, map(int, ctr.cpu().numpy())))}
 
 
-def bits(a):
-    return np.ascontiguousarray(a, dtype=np.float32).view(np.uint32)
-
-
 def load_default_camera(name):
     """A shipped model with the camera its loader sets (helpers.load overrides quad's and tower's, DESIGN.md §6
     deviation 6: the default camera sits inside those models, so camera rays meet back faces)."""
-    from helpers import MODELS
     from raytracing_c_b200 import driver
     return driver.load_scene(os.path.join(MODELS, name), shader_proc=oracle_ffi.shader_proc(),
                              background_proc=oracle_ffi.background_proc())

@@ -9,35 +9,19 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-import subprocess
-import tempfile
 
 import numpy as np
 
 import oracle_ffi
+from helpers import CSRC, ROOT, bits  # noqa: F401  (bits is re-exported)
 from raytracing_c_b200._ffi import Scene, isize
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CSRC = os.path.join(ROOT, "tests", "csrc")
-
-_build_dir = None
 _camera_lib = None
 _cast_lib = None
 
 
 def _ptr(a):
     return a.ctypes.data if a is not None else None
-
-
-def _compile(name, args):
-    global _build_dir
-    if _build_dir is None:
-        _build_dir = tempfile.mkdtemp(prefix="rt_cast_rays_")
-    out = os.path.join(_build_dir, name)
-    r = subprocess.run(["gcc", *args, "-shared", "-fPIC", "-o", out], capture_output=True, text=True)
-    if r.returncode:
-        raise RuntimeError(f"building {name} failed:\n{r.stdout}{r.stderr}")
-    return out
 
 
 def cast_lib() -> C.CDLL:
@@ -47,7 +31,7 @@ def cast_lib() -> C.CDLL:
     if _cast_lib is None:
         oracle_ffi.lib()                                   # builds liboracle.so if it is missing
         o = oracle_ffi.ORACLE_DIR
-        path = _compile("libcast_rays_oracle.so", [
+        path = oracle_ffi.build_lib("libcast_rays_oracle.so", [
             "-O2", "-std=gnu11", "-mavx2", "-mfma", "-ffp-contract=off", "-I", os.path.join(ROOT, "include"), "-I", o,
             os.path.join(CSRC, "cast_rays_oracle.c"), "-L", o, "-loracle", f"-Wl,-rpath,{o}", "-lpthread", "-lm"])
         lib = C.CDLL(path)
@@ -108,9 +92,9 @@ def ref_cast_ray_seeded(loaded, ray, key, sample, max_bounces, user_seed=0):
 def camera_lib() -> C.CDLL:
     global _camera_lib
     if _camera_lib is None:
-        lib = C.CDLL(_compile("libcamera_rays.so", ["-O2", "-std=gnu11", "-ffp-contract=off", "-I",
-                                                    os.path.join(ROOT, "include"), os.path.join(CSRC, "camera_rays.c"),
-                                                    "-lm"]))
+        lib = C.CDLL(oracle_ffi.build_lib("libcamera_rays.so", ["-O2", "-std=gnu11", "-ffp-contract=off", "-I",
+                                                              os.path.join(ROOT, "include"),
+                                                              os.path.join(CSRC, "camera_rays.c"), "-lm"]))
         lib.camera_rays.argtypes = [C.c_void_p, isize, isize, isize, C.c_void_p]
         lib.camera_rays.restype = None
         _camera_lib = lib
@@ -151,7 +135,3 @@ def device_cast_rays(loaded, rays, samples, max_bounces=8, sample_begin=0, user_
     if per is not None:
         out["per_sample"] = per[:n * samples].cpu().numpy().reshape(n, samples, 3)
     return out
-
-
-def bits(a):
-    return np.ascontiguousarray(a, dtype=np.float32).view(np.uint32)

@@ -10,10 +10,7 @@ import os
 import numpy as np
 
 import oracle_ffi
-
-
-def bits(a):
-    return np.ascontiguousarray(a, dtype=np.float32).view(np.uint32)
+from helpers import bits
 
 
 def sequential_sums(per_sample):

@@ -8,6 +8,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -41,6 +42,22 @@ def build_oracle() -> None:
     out = subprocess.run(["make", "-C", ORACLE_DIR, "all"], capture_output=True, text=True)
     if out.returncode:
         raise RuntimeError("oracle build failed:\n" + out.stdout + out.stderr)
+
+
+_build_dir = None
+
+
+def build_lib(name: str, args: list) -> str:
+    """Compiles a test-side C library, `gcc <args> -shared -fPIC -o <dir>/<name>`, into a private temporary directory (the
+    tree is never written) and returns its path.  `args` carry every flag: they decide the bits a reference computes."""
+    global _build_dir
+    if _build_dir is None:
+        _build_dir = tempfile.mkdtemp(prefix="rt_oracle_libs_")
+    out = os.path.join(_build_dir, name)
+    r = subprocess.run(["gcc", *args, "-shared", "-fPIC", "-o", out], capture_output=True, text=True)
+    if r.returncode:
+        raise RuntimeError(f"building {name} failed:\n{r.stdout}{r.stderr}")
+    return out
 
 
 _lib = None

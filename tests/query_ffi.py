@@ -9,44 +9,29 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-import subprocess
-import tempfile
 
 import numpy as np
 
 import oracle_ffi
+from helpers import CSRC, ROOT, bits  # noqa: F401  (bits is re-exported)
 from raytracing_c_b200._ffi import Scene, isize
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CSRC = os.path.join(ROOT, "tests", "csrc")
 EPS = np.float32(0.0001)                 # the reference's EPSILON
 SURFACE_FIELDS = {"point": slice(0, 3), "normal": slice(3, 6), "normal_geo": slice(6, 9), "tex_coords": slice(9, 11)}
 QUERY_COUNTERS = ["rays", "nodes", "leaves", "accepts"]
 HIT_DTYPE = np.dtype([("t", np.float32), ("u", np.float32), ("v", np.float32), ("slot", np.int32)])
 
-_build_dir = None
 _query_lib = None
 _ref_lib = None
-
-
-def _compile(name, args):
-    global _build_dir
-    if _build_dir is None:
-        _build_dir = tempfile.mkdtemp(prefix="rt_query_oracle_")
-    out = os.path.join(_build_dir, name)
-    r = subprocess.run(["gcc", *args, "-shared", "-fPIC", "-o", out], capture_output=True, text=True)
-    if r.returncode:
-        raise RuntimeError(f"building {name} failed:\n{r.stdout}{r.stderr}")
-    return out
 
 
 def query_lib() -> C.CDLL:
     """query_oracle_rays, built with the oracle's flags (no FMA contraction)."""
     global _query_lib
     if _query_lib is None:
-        path = _compile("libquery_oracle.so", ["-O2", "-std=gnu11", "-mavx2", "-mfma", "-ffp-contract=off",
-                                               "-I", os.path.join(ROOT, "include"), "-I", oracle_ffi.ORACLE_DIR,
-                                               os.path.join(CSRC, "query_oracle.c"), "-lpthread", "-lm"])
+        path = oracle_ffi.build_lib("libquery_oracle.so", [
+            "-O2", "-std=gnu11", "-mavx2", "-mfma", "-ffp-contract=off", "-I", os.path.join(ROOT, "include"),
+            "-I", oracle_ffi.ORACLE_DIR, os.path.join(CSRC, "query_oracle.c"), "-lpthread", "-lm"])
         lib = C.CDLL(path)
         lib.query_oracle_rays.argtypes = [C.POINTER(Scene), C.c_void_p, C.c_void_p, isize, C.c_int32, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]
@@ -64,7 +49,7 @@ def ref_query_lib() -> C.CDLL:
     global _ref_lib
     if _ref_lib is None:
         ref, o = os.environ["RT_REFERENCE_DIR"], oracle_ffi.ORACLE_DIR
-        path = _compile("libref_query.so", [
+        path = oracle_ffi.build_lib("libref_query.so", [
             "-O2", "-g", "-std=gnu11", "-mavx2", "-mfma", "-ffp-contract=off", "-w", "-Dmain=ref_driver_main",
             "-I", os.path.join(o, "codin_shim"), "-I", ref, "-I", os.path.join(ROOT, "include"), "-I", o,
             os.path.join(o, "ref_glue_common.c"), os.path.join(CSRC, "ref_query_glue.c"), os.path.join(o, "ref_glue_driver.c"),
@@ -215,7 +200,3 @@ def mixed_rays(loaded, seed, n_each=2048, grid=(64, 48)):
     surf = surface_rays(base, t0, rng)[:n_each]
     rays = np.concatenate([base, surf])
     return rays, oracle_query(loaded, rays)["t"]
-
-
-def bits(a):
-    return np.ascontiguousarray(a).view(np.uint32)

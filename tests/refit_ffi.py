@@ -12,7 +12,8 @@ import os
 
 import numpy as np
 
-import cast_rays_ffi
+import oracle_ffi
+from helpers import CSRC, ROOT
 from raytracing_c_b200._ffi import Scene
 
 _lib = None
@@ -21,9 +22,9 @@ _lib = None
 def refit_lib() -> C.CDLL:
     global _lib
     if _lib is None:
-        path = cast_rays_ffi._compile("librefit_oracle.so", [
-            "-O2", "-std=gnu11", "-mavx2", "-mfma", "-ffp-contract=off", "-I", os.path.join(cast_rays_ffi.ROOT, "include"),
-            os.path.join(cast_rays_ffi.CSRC, "refit_oracle.c"), "-lm"])
+        path = oracle_ffi.build_lib("librefit_oracle.so", [
+            "-O2", "-std=gnu11", "-mavx2", "-mfma", "-ffp-contract=off", "-I", os.path.join(ROOT, "include"),
+            os.path.join(CSRC, "refit_oracle.c"), "-lm"])
         lib = C.CDLL(path)
         lib.refit_oracle.argtypes = [C.POINTER(Scene), C.c_void_p, C.c_void_p]
         lib.refit_oracle.restype = None

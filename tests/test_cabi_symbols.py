@@ -6,9 +6,9 @@ import re
 
 import pytest
 
+from helpers import ROOT
 from raytracing_c_b200 import _ffi
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DECL = re.compile(r"^\s*(?:extern\s+)?(?:[A-Za-z_][\w\s\*]*?[\s\*])([a-z_][a-z0-9_]*)\s*\([^;{]*\)\s*;", re.M)
 
 

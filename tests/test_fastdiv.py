@@ -4,7 +4,7 @@ strided plus every multiple-of-d boundary for the large ones)."""
 import os
 import subprocess
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+from helpers import ROOT
 
 
 def test_fastdiv_equals_division(tmp_path):

@@ -2,40 +2,21 @@
 every field of every record and the eight work counters bit-exact on the six shipped models and inside tower.obj, for
 walk counts 0/1/2/8 and two sample offsets, and on one whole 1080p helmet frame; agreement with the renderer's own
 accumulator and counters; split ranges, chunked runs and the host form equal to one device call; ordering against
-uploads and renders; fast_math; refusals before launch; the compile-time budget of the two new kernels.
+uploads and renders; fast_math; refusals before launch.  The kernels' register budgets are in test_build_properties.py.
 """
-import contextlib
 import ctypes as C
 import os
-import re
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
 
 import aov_ffi as A
-from helpers import load
+from helpers import MODEL_NAMES, chunk_paths, load, upload
+from helpers import gpu_session  # noqa: F401
 from raytracing_c_b200 import driver, gpu_lib
 from raytracing_c_b200._ffi import gpu_check
 
 pytestmark = pytest.mark.gpu
-
-MODEL_NAMES = ["fov_test.obj", "quad.obj", "tower.obj", "spheres.glb", "sheen.glb", "helmet.glb"]
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "raytracing_c_b200", "csrc", "libraytracer_gpu.so")
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _gpu():
-    gpu_check(gpu_lib().rt_gpu_init(0))
-    yield
-    driver.set_options()
-
-
-def upload(loaded):
-    driver.register_callbacks(loaded)
-    gpu_check(gpu_lib().rt_gpu_scene_upload(C.byref(loaded.scene)))
 
 
 @pytest.fixture(scope="module", params=MODEL_NAMES + ["tower.obj:inside"])
@@ -50,20 +31,6 @@ def assert_equal(got, want):
     bad = A.bits(got["records"]) != A.bits(want["records"])
     assert not bad.any(), f"records differ on {int(bad.any(axis=-1).sum())} pixels, fields {np.nonzero(bad.any(axis=(0, 1)))[0]}"
     assert got["counters"] == want["counters"]
-
-
-@contextlib.contextmanager
-def chunk_paths(n):
-    """Path-queue chunks of at most n paths (RT_GPU_CHUNK_PATHS, read at every launch)."""
-    old = os.environ.get("RT_GPU_CHUNK_PATHS")
-    os.environ["RT_GPU_CHUNK_PATHS"] = str(n)
-    try:
-        yield
-    finally:
-        if old is None:
-            del os.environ["RT_GPU_CHUNK_PATHS"]
-        else:
-            os.environ["RT_GPU_CHUNK_PATHS"] = old
 
 
 # (max_bounces, sample_begin)
@@ -256,23 +223,3 @@ def test_refusals_and_empty_calls():
     finally:
         other.close()
         loaded.close()
-
-
-BUDGET = {   # mangled-name fragment -> (max registers per thread, max bytes of stack), from -Xptxas -v
-    "rt_aov_surface_kernel": (32, 0),
-    "rt_aov_accumulate_kernel": (64, 16),
-}
-
-
-@pytest.mark.skipif(shutil.which("cuobjdump") is None or not os.path.exists(LIB), reason="needs the built library and cuobjdump")
-def test_new_kernels_keep_their_register_budget():
-    out = subprocess.run(["cuobjdump", "-res-usage", LIB], capture_output=True, text=True).stdout
-    found = {}
-    for m in re.finditer(r"Function (\S+):\s*\n\s*REG:(\d+) STACK:(\d+)", out):
-        for key in BUDGET:
-            if key in m.group(1):
-                found[key] = (int(m.group(2)), int(m.group(3)))
-    assert set(found) == set(BUDGET), f"kernels missing from the library: {set(BUDGET) - set(found)}"
-    for key, (regs, stack) in found.items():
-        assert regs <= BUDGET[key][0], f"{key}: {regs} registers (budget {BUDGET[key][0]})"
-        assert stack <= BUDGET[key][1], f"{key}: {stack} bytes of stack (budget {BUDGET[key][1]})"

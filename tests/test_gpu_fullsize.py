@@ -16,17 +16,10 @@ import pytest
 
 import oracle_ffi
 from helpers import load
-from raytracing_c_b200 import driver, gpu_lib
-from raytracing_c_b200._ffi import gpu_check
+from helpers import gpu_session  # noqa: F401
+from raytracing_c_b200 import driver
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _gpu():
-    gpu_check(gpu_lib().rt_gpu_init(0))
-    yield
-    driver.set_options()
 
 
 def check_frame(name, w, h, spp, mask=None, threads=None):

@@ -7,17 +7,11 @@ import pytest
 
 import oracle_ffi
 from helpers import load
+from helpers import gpu_session  # noqa: F401
 from raytracing_c_b200 import driver, gpu_lib
-from raytracing_c_b200._ffi import Vec3, gpu_check
+from raytracing_c_b200._ffi import Vec3
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _gpu():
-    gpu_check(gpu_lib().rt_gpu_init(0))
-    yield
-    driver.set_options()
 
 
 @pytest.mark.parametrize("name,w,h,samples,seed", [("spheres.glb", 96, 80, 5, 0), ("tower.obj", 128, 64, 3, 9), ("sheen.glb", 64, 64, 4, 1)])

@@ -3,14 +3,10 @@ GPU.  Every accumulator, second moment and all eight work counters are compared 
 with its pixel_mask (six models and the inside-tower camera, six mask shapes, bounces 0/1/2/8, two sample offsets);
 composed passes against uniform renders at each pixel's own sample count; the buffer rules; the NULL mask against the
 renderer; chunked runs; fast_math; ordering against uploads and the other workspace users; refusals; one 1080p helmet
-pass; the film; the compile-time budget of the new kernels.
+pass; the film.  The kernels' register budgets are in test_build_properties.py.
 """
-import contextlib
 import ctypes as C
 import os
-import re
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
@@ -18,28 +14,14 @@ import pytest
 import aov_ffi as A
 import masked_ffi as M
 import oracle_ffi
-from helpers import load
+from helpers import MODEL_NAMES, chunk_paths, load, upload
+from helpers import gpu_session  # noqa: F401
 from raytracing_c_b200 import driver, gpu_lib
 from raytracing_c_b200._ffi import gpu_check
 
 pytestmark = pytest.mark.gpu
 
-MODEL_NAMES = ["fov_test.obj", "quad.obj", "tower.obj", "spheres.glb", "sheen.glb", "helmet.glb"]
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "raytracing_c_b200", "csrc", "libraytracer_gpu.so")
 ZERO_COUNTERS = dict.fromkeys(oracle_ffi.COUNTER_NAMES, 0)
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _gpu():
-    gpu_check(gpu_lib().rt_gpu_init(0))
-    yield
-    driver.set_options()
-
-
-def upload(loaded):
-    driver.register_callbacks(loaded)
-    gpu_check(gpu_lib().rt_gpu_scene_upload(C.byref(loaded.scene)))
 
 
 @pytest.fixture(scope="module", params=MODEL_NAMES + ["tower.obj:inside"])
@@ -48,20 +30,6 @@ def scene(request):
     upload(loaded)
     yield request.param, loaded
     loaded.close()
-
-
-@contextlib.contextmanager
-def chunk_paths(n):
-    """Path-queue chunks of at most n paths (RT_GPU_CHUNK_PATHS, read at every launch)."""
-    old = os.environ.get("RT_GPU_CHUNK_PATHS")
-    os.environ["RT_GPU_CHUNK_PATHS"] = str(n)
-    try:
-        yield
-    finally:
-        if old is None:
-            del os.environ["RT_GPU_CHUNK_PATHS"]
-        else:
-            os.environ["RT_GPU_CHUNK_PATHS"] = old
 
 
 def assert_same(got, want, where=None, counters=True):
@@ -381,24 +349,3 @@ def test_resolve_counts():
         assert (out[:, :w, 3] == 9).all() and (out[:, w:] == 9).all()
     finally:
         loaded.close()
-
-
-BUDGET = {   # mangled-name fragment -> (max registers per thread, max bytes of stack), from -Xptxas -v
-    "rt_trace_kernelILb1ELi4ELb1E": (64, 24),       # the unmasked primary trace's 64 registers and 24-byte frame
-    "rt_accumulate_masked_kernel": (40, 0),
-    "rt_resolve_counts_kernel": (32, 0),
-}
-
-
-@pytest.mark.skipif(shutil.which("cuobjdump") is None or not os.path.exists(LIB), reason="needs the built library and cuobjdump")
-def test_new_kernels_keep_their_register_budget():
-    out = subprocess.run(["cuobjdump", "-res-usage", LIB], capture_output=True, text=True).stdout
-    found = {}
-    for m in re.finditer(r"Function (\S+):\s*\n\s*REG:(\d+) STACK:(\d+)", out):
-        for key in BUDGET:
-            if key in m.group(1):
-                found[key] = (int(m.group(2)), int(m.group(3)))
-    assert set(found) == set(BUDGET), f"kernels missing from the library: {set(BUDGET) - set(found)}"
-    for key, (regs, stack) in found.items():
-        assert regs <= BUDGET[key][0], f"{key}: {regs} registers (budget {BUDGET[key][0]})"
-        assert stack <= BUDGET[key][1], f"{key}: {stack} bytes of stack (budget {BUDGET[key][1]})"

@@ -13,12 +13,11 @@ import numpy as np
 import pytest
 
 import oracle_ffi
-from helpers import MODELS, load
+from helpers import MODELS, ROOT, load
 from raytracing_c_b200 import driver, gpu_lib, sharding
 from raytracing_c_b200._ffi import SPLIT_CHUNKS, SPLIT_SAMPLES, REDUCE_NCCL, gpu_check
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 RT_DRIVER = os.path.join(ROOT, "raytracing_c_b200", "host", "rt_driver")
 
 

@@ -11,36 +11,12 @@ import numpy as np
 import pytest
 
 import oracle_ffi
+from helpers import MODELS, load
+from helpers import gpu_session  # noqa: F401
 from raytracing_c_b200 import driver, gpu_lib
 from raytracing_c_b200._ffi import gpu_check
 
 pytestmark = pytest.mark.gpu
-
-MODELS = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "assets", "models")
-
-# Camera overrides recorded in DESIGN.md (SURVEY §8d configs 2 and 5): the default camera sits
-# inside quad.obj's plane and inside tower.obj's footprint.
-CAMERAS = {
-    "quad.obj": dict(eye=(3.0, 0.0, 0.0), target=(0.0, 0.0, 0.0)),
-    "tower.obj": dict(eye=(0.0, 12.5, 40.0), target=(0.0, 12.5, 0.0)),
-}
-
-
-def load(name, **material_override):
-    cam = driver.look_at(**CAMERAS[name]) if name in CAMERAS else None
-    loaded = driver.load_scene(os.path.join(MODELS, name), shader_proc=oracle_ffi.shader_proc(),
-                               background_proc=oracle_ffi.background_proc(), camera=cam)
-    for i in range(loaded.model.n_materials):
-        for key, value in material_override.items():
-            setattr(loaded.model.materials[i], key, value)
-    return loaded
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _gpu():
-    gpu_check(gpu_lib().rt_gpu_init(0))
-    yield
-    driver.set_options()
 
 
 def gpu_render(loaded, w, h, spp, bounces=8, n_threads=1, **options):

@@ -9,20 +9,12 @@ import numpy as np
 import pytest
 
 import query_ffi as Q
-from helpers import MODELS, load
+from helpers import MODEL_NAMES, MODELS, load
+from helpers import gpu_session  # noqa: F401
 from raytracing_c_b200 import driver, gpu_lib
 from raytracing_c_b200._ffi import gpu_check
 
 pytestmark = pytest.mark.gpu
-
-MODEL_NAMES = ["fov_test.obj", "quad.obj", "tower.obj", "spheres.glb", "sheen.glb", "helmet.glb"]
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _gpu():
-    gpu_check(gpu_lib().rt_gpu_init(0))
-    yield
-    driver.set_options()
 
 
 @pytest.fixture(scope="module", params=MODEL_NAMES)

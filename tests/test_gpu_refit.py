@@ -13,24 +13,13 @@ import aov_ffi as A
 import oracle_ffi
 import query_ffi as Q
 import refit_ffi as R
-from helpers import load, scene_buffers
+from helpers import load, scene_buffers, upload
+from helpers import gpu_session  # noqa: F401
 from raytracing_c_b200 import driver, gpu_lib
 from raytracing_c_b200._ffi import gpu_check
 
 pytestmark = pytest.mark.gpu
 THREADS = os.cpu_count() or 8
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _gpu():
-    gpu_check(gpu_lib().rt_gpu_init(0))
-    yield
-    driver.set_options()
-
-
-def upload(loaded):
-    driver.register_callbacks(loaded)
-    gpu_check(gpu_lib().rt_gpu_scene_upload(C.byref(loaded.scene)))
 
 
 def host_nodes(loaded):

@@ -4,12 +4,8 @@ counters must stay bit for bit the oracle's, and counters_ex[1] (primary rays) t
 that see part, none or all of the model as sky, image sizes that are not whole tiles, sample offsets, chunked runs,
 masked passes across the sky boundary, pixel splits and fast mode.
 """
-import contextlib
 import ctypes as C
 import os
-import re
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
@@ -17,14 +13,13 @@ import pytest
 import aov_ffi as A
 import masked_ffi as M
 import oracle_ffi
-from helpers import load
+from helpers import chunk_paths, load
+from helpers import gpu_session  # noqa: F401
 from raytracing_c_b200 import driver, gpu_lib
 from raytracing_c_b200._ffi import gpu_check
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "raytracing_c_b200", "csrc", "libraytracer_gpu.so")
 
 # helmet.glb's bounds are about [-1, 1]^3 around the origin; its own camera sits at (1, -0.2, 1.73) facing it
 CAMERAS = {
@@ -33,26 +28,6 @@ CAMERAS = {
     "behind": dict(eye=(1.2, 0.0, 0.0), target=(1.2, 0.0, -5.0)),              # part of the model behind the camera plane
     "border": dict(eye=(0.0, 0.0, 3.0), target=(1.3, 0.0, 0.0)),               # the model cut by the image border
 }
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _gpu():
-    gpu_check(gpu_lib().rt_gpu_init(0))
-    yield
-    driver.set_options()
-
-
-@contextlib.contextmanager
-def chunk_paths(n):
-    old = os.environ.get("RT_GPU_CHUNK_PATHS")
-    os.environ["RT_GPU_CHUNK_PATHS"] = str(n)
-    try:
-        yield
-    finally:
-        if old is None:
-            del os.environ["RT_GPU_CHUNK_PATHS"]
-        else:
-            os.environ["RT_GPU_CHUNK_PATHS"] = old
 
 
 def counters_ex():
@@ -213,14 +188,3 @@ def test_fast_mode_close_to_exact(cam):
         assert fast["ex"][1] == exact["ex"][1] == w * h * spp
     finally:
         loaded.close()
-
-
-@pytest.mark.skipif(shutil.which("cuobjdump") is None or not os.path.exists(LIB), reason="needs cuobjdump")
-def test_sky_kernel_register_budget():
-    """64 registers (4 blocks of 256 threads per SM) and no spills, exact and fast."""
-    out = subprocess.run(["cuobjdump", "-res-usage", LIB], capture_output=True, text=True).stdout
-    found = {m.group(1): (int(m.group(2)), int(m.group(3)))
-             for m in re.finditer(r"Function (\S*rt_sky_kernel\S*):\s*\n\s*REG:(\d+) STACK:(\d+)", out)}
-    assert len(found) == 2, found
-    for name, (regs, stack) in found.items():
-        assert regs <= 64 and stack <= 16, (name, regs, stack)

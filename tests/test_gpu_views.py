@@ -5,14 +5,11 @@ inside-tower camera, camera sets with a duplicate, different fields of view, an 
 bounds, bounces 0/1/2/8, two sample offsets, NULL and distinct seeds.  Also: two views against the oracle renderer;
 chunked calls (sample chunks and view groups) and accumulation; fast_math; the one-view call against a render (bits,
 counters, launches); ordering against uploads, renders, AOV, cast_rays and a refit; refusals and empty calls; the host
-form and its film; the compile-time budget of the new primary trace.
+form and its film.  The primary trace's register budget is in test_build_properties.py.
 """
 import contextlib
 import ctypes as C
 import os
-import re
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
@@ -20,29 +17,15 @@ import pytest
 import aov_ffi as A
 import oracle_ffi
 import views_ffi as V
-from helpers import load
+from helpers import MODEL_NAMES, chunk_paths, load, upload
+from helpers import gpu_session  # noqa: F401
 from raytracing_c_b200 import driver, gpu_lib
 from raytracing_c_b200._ffi import Camera, gpu_check
 
 pytestmark = pytest.mark.gpu
 
-MODEL_NAMES = ["fov_test.obj", "quad.obj", "tower.obj", "spheres.glb", "sheen.glb", "helmet.glb"]
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "raytracing_c_b200", "csrc", "libraytracer_gpu.so")
 ZERO_COUNTERS = dict.fromkeys(oracle_ffi.COUNTER_NAMES, 0)
 W, H = 96, 64
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _gpu():
-    gpu_check(gpu_lib().rt_gpu_init(0))
-    yield
-    driver.set_options()
-
-
-def upload(loaded):
-    driver.register_callbacks(loaded)
-    gpu_check(gpu_lib().rt_gpu_scene_upload(C.byref(loaded.scene)))
 
 
 @pytest.fixture(scope="module", params=MODEL_NAMES + ["tower.obj:inside"])
@@ -51,20 +34,6 @@ def scene(request):
     upload(loaded)
     yield request.param, loaded
     loaded.close()
-
-
-@contextlib.contextmanager
-def chunk_paths(n):
-    """Path-queue chunks of at most n paths (RT_GPU_CHUNK_PATHS, read at every launch)."""
-    old = os.environ.get("RT_GPU_CHUNK_PATHS")
-    os.environ["RT_GPU_CHUNK_PATHS"] = str(n)
-    try:
-        yield
-    finally:
-        if old is None:
-            del os.environ["RT_GPU_CHUNK_PATHS"]
-        else:
-            os.environ["RT_GPU_CHUNK_PATHS"] = old
 
 
 def assert_views(got, want, counters=True):
@@ -377,22 +346,3 @@ def test_host_form_and_its_film():
             driver.render_views(loaded, cams, t[:2], 3, 12)
     finally:
         loaded.close()
-
-
-BUDGET = {   # mangled-name fragment -> (max registers per thread, max bytes of stack), from -Xptxas -v
-    "rt_trace_kernelILb1ELi4ELb0ELb1E": (64, 24),       # the unmasked primary trace's 64 registers and 24-byte frame
-}
-
-
-@pytest.mark.skipif(shutil.which("cuobjdump") is None or not os.path.exists(LIB), reason="needs the built library and cuobjdump")
-def test_new_primary_trace_keeps_its_register_budget():
-    out = subprocess.run(["cuobjdump", "-res-usage", LIB], capture_output=True, text=True).stdout
-    found = {}
-    for m in re.finditer(r"Function (\S+):\s*\n\s*REG:(\d+) STACK:(\d+)", out):
-        for key in BUDGET:
-            if key in m.group(1):
-                found[key] = (int(m.group(2)), int(m.group(3)))
-    assert set(found) == set(BUDGET), f"kernels missing from the library: {set(BUDGET) - set(found)}"
-    for key, (regs, stack) in found.items():
-        assert regs <= BUDGET[key][0], f"{key}: {regs} registers (budget {BUDGET[key][0]})"
-        assert stack <= BUDGET[key][1], f"{key}: {stack} bytes of stack (budget {BUDGET[key][1]})"

@@ -14,9 +14,7 @@ import aov_ffi as A
 import cast_rays_ffi as R
 import oracle_ffi
 import query_ffi as Q
-from helpers import load
-
-MODEL_NAMES = ["fov_test.obj", "quad.obj", "tower.obj", "spheres.glb", "sheen.glb", "helmet.glb"]
+from helpers import MODEL_NAMES, load
 
 
 @pytest.fixture(scope="module", params=MODEL_NAMES)

@@ -10,9 +10,7 @@ import pytest
 
 import masked_ffi as M
 import oracle_ffi
-from helpers import load
-
-MODEL_NAMES = ["fov_test.obj", "quad.obj", "tower.obj", "spheres.glb", "sheen.glb", "helmet.glb"]
+from helpers import MODEL_NAMES, load
 
 
 @pytest.fixture(scope="module", params=MODEL_NAMES)

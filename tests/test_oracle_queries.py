@@ -12,9 +12,7 @@ import numpy as np
 import pytest
 
 import query_ffi as Q
-from helpers import load
-
-MODEL_NAMES = ["fov_test.obj", "quad.obj", "tower.obj", "spheres.glb", "sheen.glb", "helmet.glb"]
+from helpers import MODEL_NAMES, load
 
 
 @pytest.fixture(scope="module", params=MODEL_NAMES)

@@ -5,11 +5,9 @@ import numpy as np
 import pytest
 
 import refit_ffi as R
-from helpers import load, scene_buffers, scene_digest
+from helpers import MODEL_NAMES, load, scene_buffers, scene_digest
 from raytracing_c_b200 import driver
 from raytracing_c_b200._ffi import Scene, host_lib
-
-MODEL_NAMES = ["fov_test.obj", "quad.obj", "tower.obj", "spheres.glb", "sheen.glb", "helmet.glb"]
 
 
 @pytest.fixture(scope="module", params=MODEL_NAMES)

@@ -9,13 +9,10 @@ import ctypes as C
 import numpy as np
 
 import oracle_ffi
+from helpers import bits  # noqa: F401  (bits is re-exported)
 from raytracing_c_b200._ffi import Camera
 
 CTR16_NAMES = oracle_ffi.COUNTER_NAMES + [f"ex{i}" for i in range(8)]
-
-
-def bits(a):
-    return np.ascontiguousarray(a, dtype=np.float32).view(np.uint32)
 
 
 def copy_camera(cam) -> Camera:
