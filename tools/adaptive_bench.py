@@ -21,17 +21,15 @@ The card name and power limit are read in the same run.
 """
 from __future__ import annotations
 
-import argparse
 import ctypes as C
 import json
-import os
-import subprocess
-import sys
 
 import numpy as np
+import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
+import benchkit  # first: it puts the repository root and tests/ on sys.path
+from raytracing_c_b200 import driver
+from raytracing_c_b200._ffi import gpu_check
 
 W, H, BOUNCES = 1920, 1080, 8
 PASS, CAP = 32, 1024
@@ -41,43 +39,18 @@ UNIFORM_SPPS = (32, 64, 128, 256, 512)
 LUMA = (0.2126, 0.7152, 0.0722)
 
 
-def card() -> dict:
-    out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                         capture_output=True, text=True).stdout.strip().splitlines()
-    name, power, clock = [s.strip() for s in out[0].split(",")]
-    return {"name": name, "power_limit": power, "max_sm_clock": clock}
-
-
 def main() -> None:
-    ap = argparse.ArgumentParser()
-    ap.add_argument("--reps", type=int, default=5)
-    ap.add_argument("--out", default=None, help="also write the result JSON here")
-    args = ap.parse_args()
-
-    import torch
-    from raytracing_c_b200 import driver, gpu_lib
-    from raytracing_c_b200._ffi import gpu_check
-
-    gpu = gpu_lib()
-    gpu_check(gpu.rt_gpu_init(0))
-    loaded = driver.load_scene(os.path.join(ROOT, "assets", "models", "helmet.glb"))
-    driver.register_callbacks(loaded)
-    gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+    args = benchkit.parser(reps=5).parse_args()
+    gpu = benchkit.init()
+    loaded = benchkit.resident("helmet.glb")
     scene = C.byref(loaded.scene)
     stream = torch.cuda.current_stream()
     st = stream.cuda_stream
     acc = torch.empty((H, W, 3), dtype=torch.float32, device="cuda")
     acc2 = torch.empty_like(acc)
     sq = torch.empty_like(acc)
-    result = {"card": card(), "model": "helmet.glb", "frame": f"{W}x{H}", "max_bounces": BOUNCES, "reps": args.reps}
-
-    def timed(fn):
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record(stream)
-        fn()
-        e1.record(stream)
-        torch.cuda.synchronize()
-        return e0.elapsed_time(e1)
+    result = {"card": benchkit.card(), "model": "helmet.glb", "frame": f"{W}x{H}", "max_bounces": BOUNCES,
+              "reps": args.reps}
 
     def render(begin, end, out, seed=0):
         gpu_check(gpu.rt_gpu_render_accum_device(scene, W, H, begin, end, BOUNCES, seed, 0, out.data_ptr(), None, None,
@@ -94,8 +67,8 @@ def main() -> None:
     torch.cuda.synchronize()
     t_render, t_null = [], []
     for _ in range(args.reps):
-        t_render.append(timed(lambda: render(0, spp, acc)))
-        t_null.append(timed(lambda: masked(None, 0, spp, acc2)))
+        t_render.append(benchkit.window_ms(lambda: render(0, spp, acc), stream))
+        t_null.append(benchkit.window_ms(lambda: masked(None, 0, spp, acc2), stream))
     identical = bool(torch.equal(acc.view(torch.int32), acc2.view(torch.int32)))
     r1 = {"spp": spp, "render_ms": [round(t, 3) for t in t_render], "null_mask_ms": [round(t, 3) for t in t_null],
           "render_median_ms": round(float(np.median(t_render)), 3), "null_mask_median_ms": round(float(np.median(t_null)), 3),
@@ -119,7 +92,7 @@ def main() -> None:
                 m.fill_(1)
             masked(m, 0, PASS, acc)
             torch.cuda.synchronize()
-            ts = [timed(lambda: masked(m, 0, PASS, acc)) for _ in range(args.reps)]
+            ts = [benchkit.window_ms(lambda: masked(m, 0, PASS, acc), stream) for _ in range(args.reps)]
             ms = float(np.median(ts))
             if full_ms is None:
                 full_ms = ms
@@ -161,40 +134,32 @@ def main() -> None:
                 counts.add_(m.to(torch.int32) * PASS)
                 passes.append(m)
                 n += PASS
-        ms = timed(loop)
+        ms = benchkit.window_ms(loop, stream)
         spent = int(counts.sum().item())
         px = driver.resolve_counts(acc, counts)
         eq_spp = max(1, round(spent / (W * H)))
         render(0, eq_spp, acc2)
         eq_px = driver.resolve_counts(acc2, torch.full((H, W), eq_spp, dtype=torch.int32, device="cuda"))
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record(stream); render(0, eq_spp, acc2); e1.record(stream)
-        torch.cuda.synchronize()
+        eq_ms = benchkit.window_ms(lambda: render(0, eq_spp, acc2), stream)
         hist = torch.bincount(counts.flatten().long() // PASS, minlength=CAP // PASS + 1).cpu().numpy()
         r = {"ms": round(ms, 3), "samples": spent, "mean_spp": round(spent / (W * H), 2),
              "passes": len(passes), "pixels_at_cap": int((counts == CAP).sum().item()),
              "spp_histogram": {str(k * PASS): int(v) for k, v in enumerate(hist) if v},
              "rmse_u8": round(rmse(px), 4),
-             "uniform_equal_samples": {"spp": eq_spp, "ms": round(e0.elapsed_time(e1), 3), "rmse_u8": round(rmse(eq_px), 4)}}
+             "uniform_equal_samples": {"spp": eq_spp, "ms": round(eq_ms, 3), "rmse_u8": round(rmse(eq_px), 4)}}
         r3["thresholds"][str(thr)] = r
         print(json.dumps({f"adaptive_{thr}": r}), flush=True)
     # the uniform curve the loop is compared with: RMSE and time of a uniform render per sample count
     r3["uniform"] = {}
     for spp in UNIFORM_SPPS:
-        ms = timed(lambda: render(0, spp, acc2))
+        ms = benchkit.window_ms(lambda: render(0, spp, acc2), stream)
         px = driver.resolve_counts(acc2, torch.full((H, W), spp, dtype=torch.int32, device="cuda"))
         r3["uniform"][str(spp)] = {"ms": round(ms, 3), "rmse_u8": round(rmse(px), 4)}
     print(json.dumps({"uniform": r3["uniform"]}), flush=True)
     result["adaptive_loop"] = r3
 
     result["parity_ok"] = identical
-    print(json.dumps({"card": result["card"], "parity_ok": result["parity_ok"]}), flush=True)
-    if args.out:
-        with open(args.out, "w") as f:
-            json.dump(result, f, indent=1)
-    loaded.close()
-    if not identical:
-        sys.exit(1)
+    benchkit.finish(args, result, ("parity_ok",), loaded)
 
 
 if __name__ == "__main__":

@@ -16,79 +16,50 @@ limit are read in the same run.
 """
 from __future__ import annotations
 
-import argparse
 import ctypes as C
 import json
 import os
-import subprocess
-import sys
 
 import numpy as np
+import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tests"))
+import benchkit  # first: it puts the repository root and tests/ on sys.path
+import cast_rays_ffi as R
+import helpers
+import query_ffi as Q
+from raytracing_c_b200._ffi import gpu_check
 
 W, H = 1920, 1080
 FRAME_SPP, PROBES, PROBE_SPP, BOUNCES = 64, 1 << 20, 256, 8
 PARITY_RAYS = 1024
 
 
-def card() -> dict:
-    out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                         capture_output=True, text=True).stdout.strip().splitlines()
-    name, power, clock = [s.strip() for s in out[0].split(",")]
-    return {"name": name, "power_limit": power, "max_sm_clock": clock}
-
-
 def main() -> None:
-    ap = argparse.ArgumentParser()
-    ap.add_argument("--reps", type=int, default=20)
-    ap.add_argument("--out", default=None, help="also write the result JSON here")
-    args = ap.parse_args()
-
-    import torch
-    import cast_rays_ffi as R
-    import query_ffi as Q
-    from raytracing_c_b200 import driver, gpu_lib
-    from raytracing_c_b200._ffi import gpu_check
-
-    gpu = gpu_lib()
-    gpu_check(gpu.rt_gpu_init(0))
-    loaded = driver.load_scene(os.path.join(ROOT, "assets", "models", "helmet.glb"))
-    oracle_scene = driver.load_scene(os.path.join(ROOT, "assets", "models", "helmet.glb"),
-                                     shader_proc=R.oracle_ffi.shader_proc(), background_proc=R.oracle_ffi.background_proc())
-    driver.register_callbacks(loaded)
-    gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+    args = benchkit.parser(reps=20).parse_args()
+    gpu = benchkit.init()
+    loaded = benchkit.resident("helmet.glb")
+    oracle_scene = helpers.load("helmet.glb")
     scene = C.byref(loaded.scene)
     stream = torch.cuda.current_stream()
     dev = "cuda"
-    result = {"card": card(), "model": "helmet.glb", "max_bounces": BOUNCES, "reps": args.reps, "workloads": {}}
+    result = {"card": benchkit.card(), "model": "helmet.glb", "max_bounces": BOUNCES, "reps": args.reps,
+              "workloads": {}}
 
     def cast(rays, keys, samples, radiance, counters=None):
-        return gpu.rt_gpu_cast_rays_device(scene, rays.data_ptr(), keys.data_ptr() if keys is not None else None,
-                                           rays.shape[0], 0, samples, BOUNCES, 0, 0, radiance.data_ptr(), None,
-                                           counters.data_ptr() if counters is not None else None, stream.cuda_stream)
-
-    def timed(fn):
-        gpu_check(fn())                                           # warm-up: workspace, kernel modules
-        torch.cuda.synchronize()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record(stream)
-        for _ in range(args.reps):
-            gpu_check(fn())
-        e1.record(stream)
-        torch.cuda.synchronize()
-        return e0.elapsed_time(e1) / args.reps
+        gpu_check(gpu.rt_gpu_cast_rays_device(scene, rays.data_ptr(), keys.data_ptr() if keys is not None else None,
+                                              rays.shape[0], 0, samples, BOUNCES, 0, 0, radiance.data_ptr(), None,
+                                              counters.data_ptr() if counters is not None else None, stream.cuda_stream))
 
     def measure(name, rays, keys, samples):
         n = rays.shape[0]
         rad = torch.empty((n, 3), dtype=torch.float32, device=dev)
         ctr = torch.zeros(8, dtype=torch.int64, device=dev)
-        gpu_check(cast(rays, keys, samples, rad, ctr))
+        cast(rays, keys, samples, rad, ctr)
         torch.cuda.synchronize()
         c = dict(zip(R.oracle_ffi.COUNTER_NAMES, map(int, ctr.cpu().numpy())))
-        ms = timed(lambda: cast(rays, keys, samples, rad))
+        cast(rays, keys, samples, rad)                            # warm-up: workspace, kernel modules
+        torch.cuda.synchronize()
+        ms = benchkit.per_call_ms(lambda: cast(rays, keys, samples, rad), stream, args.reps)
         w = {"rays": n, "samples_per_ray": samples, "paths": n * samples, "ms": round(ms, 2),
              "Msamples_per_s": round(n * samples / (ms * 1e-3) / 1e6, 1), "rays_traced_per_path": round(c["rays"] / (n * samples), 3),
              "counters_samples_ok": c["samples"] == n * samples}
@@ -112,8 +83,14 @@ def main() -> None:
     del cam, pixels
     torch.cuda.empty_cache()
     accum = torch.empty(W * H * 3, dtype=torch.float32, device=dev)
-    ms = timed(lambda: gpu.rt_gpu_render_accum_device(scene, W, H, 0, FRAME_SPP, BOUNCES, 0, 0, accum.data_ptr(), None, None,
-                                                      None, stream.cuda_stream))
+
+    def render():
+        gpu_check(gpu.rt_gpu_render_accum_device(scene, W, H, 0, FRAME_SPP, BOUNCES, 0, 0, accum.data_ptr(), None, None,
+                                                 None, stream.cuda_stream))
+
+    render()                                                      # warm-up: workspace, kernel modules
+    torch.cuda.synchronize()
+    ms = benchkit.per_call_ms(render, stream, args.reps)
     result["renderer_frame"] = {"frame": f"helmet.glb {W}x{H}, {FRAME_SPP} spp, {BOUNCES} bounces (rt_gpu_render_accum_device)",
                                 "ms": round(ms, 2), "Msamples_per_s": round(W * H * FRAME_SPP / (ms * 1e-3) / 1e6, 1)}
     print(json.dumps({"renderer_frame": result["renderer_frame"]}), flush=True)
@@ -132,15 +109,7 @@ def main() -> None:
                                          result["renderer_frame"]["Msamples_per_s"], 3)
     result["parity_ok"] = all(all(v for k, v in w["parity"].items() if k != "rays") and w["counters_samples_ok"]
                               for w in result["workloads"].values())
-    print(json.dumps({"card": result["card"], "camera_vs_renderer": result["camera_vs_renderer"],
-                      "parity_ok": result["parity_ok"]}), flush=True)
-    if args.out:
-        with open(args.out, "w") as f:
-            json.dump(result, f, indent=1)
-    oracle_scene.close()
-    loaded.close()
-    if not result["parity_ok"]:
-        sys.exit(1)
+    benchkit.finish(args, result, ("camera_vs_renderer", "parity_ok"), oracle_scene, loaded)
 
 
 if __name__ == "__main__":

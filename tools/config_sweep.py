@@ -10,15 +10,13 @@ import argparse
 import ctypes as C
 import json
 import os
-import sys
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
+import torch
 
-import torch  # noqa: E402
-
-from raytracing_c_b200 import driver, gpu_lib  # noqa: E402
-from raytracing_c_b200._ffi import gpu_check  # noqa: E402
+import benchkit  # first: it puts the repository root and tests/ on sys.path
+from helpers import upload
+from raytracing_c_b200 import driver
+from raytracing_c_b200._ffi import gpu_check
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--quick", action="store_true", help="cap spp at 64")
@@ -30,19 +28,17 @@ RUNS = [("spheres.glb", 1024, 1024, [16], False), ("quad.obj", 1024, 1024, [1], 
         ("fov_test.obj", 1024, 1024, [1], False), ("helmet.glb", 1920, 1080, [1024], False),
         ("sheen.glb", 1024, 1024, [16], True), ("tower.obj", 3840, 2160, [1, 4, 16, 64, 256, 1024], False)]
 
-gpu = gpu_lib()
-gpu_check(gpu.rt_gpu_init(0))
+gpu = benchkit.init()
 torch.cuda.set_device(0)
 stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
 for model, W, H, spps, denoise in RUNS:
     cam = driver.look_at(**CAMERAS[model]) if model in CAMERAS else None
-    loaded = driver.load_scene(os.path.join(ROOT, "assets", "models", model), camera=cam)
+    loaded = driver.load_scene(os.path.join(benchkit.ROOT, "assets", "models", model), camera=cam)
     if model == "sheen.glb":                       # the asset declares no sheen: inject it (SURVEY fact 7)
         for i in range(loaded.model.n_materials):
             loaded.model.materials[i].sheen, loaded.model.materials[i].sheen_tint = 1.0, 0.5
-    driver.register_callbacks(loaded)
+    upload(loaded)
     scene = C.byref(loaded.scene)
-    gpu_check(gpu.rt_gpu_scene_upload(scene))
     accum = torch.zeros(W * H * 3, dtype=torch.float32, device="cuda")
     pixels = torch.zeros(W * H * 3, dtype=torch.uint8, device="cuda")
     pixels2 = torch.zeros(W * H * 3, dtype=torch.uint8, device="cuda")

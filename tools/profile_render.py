@@ -4,16 +4,12 @@
 Prints the CUDA-event time per launch (never quote a number taken under a profiler)."""
 import argparse
 import ctypes as C
-import os
-import sys
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
+import torch
 
-import torch  # noqa: E402
-
-from raytracing_c_b200 import driver, gpu_lib  # noqa: E402
-from raytracing_c_b200._ffi import gpu_check  # noqa: E402
+import benchkit  # first: it puts the repository root and tests/ on sys.path
+from raytracing_c_b200 import driver
+from raytracing_c_b200._ffi import gpu_check
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--model", default="helmet.glb")
@@ -27,14 +23,11 @@ ap.add_argument("--eye", type=float, nargs=3, default=None, help="camera positio
 ap.add_argument("--target", type=float, nargs=3, default=(0.0, 0.0, 0.0))
 args = ap.parse_args()
 
-gpu = gpu_lib()
-gpu_check(gpu.rt_gpu_init(0))
+gpu = benchkit.init()
 torch.cuda.set_device(0)
 camera = driver.look_at(args.eye, args.target) if args.eye else None
-loaded = driver.load_scene(os.path.join(ROOT, "assets", "models", args.model), camera=camera)
-driver.register_callbacks(loaded)
+loaded = benchkit.resident(args.model, camera=camera)
 scene = C.byref(loaded.scene)
-gpu_check(gpu.rt_gpu_scene_upload(scene))
 W, H = args.width, args.height
 accum = torch.zeros(W * H * 3, dtype=torch.float32, device="cuda")
 pixels = torch.zeros(W * H * 3, dtype=torch.uint8, device="cuda")

@@ -16,18 +16,17 @@ four counters bit-exact).  The card name and power limit are read in the same ru
 """
 from __future__ import annotations
 
-import argparse
 import ctypes as C
 import json
 import os
-import subprocess
-import sys
 
 import numpy as np
+import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tests"))
+import benchkit  # first: it puts the repository root and tests/ on sys.path
+import query_ffi as Q
+from raytracing_c_b200 import driver
+from raytracing_c_b200._ffi import gpu_check
 
 W, H, SPP_RAYS = 1920, 1080, 16
 AO_PER_HIT = 4
@@ -35,34 +34,15 @@ EPS = 0.0001
 PARITY_RAYS = 65536
 
 
-def card() -> dict:
-    out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                         capture_output=True, text=True).stdout.strip().splitlines()
-    name, power, clock = [s.strip() for s in out[0].split(",")]
-    return {"name": name, "power_limit": power, "max_sm_clock": clock}
-
-
 def main() -> None:
-    ap = argparse.ArgumentParser()
-    ap.add_argument("--reps", type=int, default=20)
-    ap.add_argument("--out", default=None, help="also write the result JSON here")
-    args = ap.parse_args()
-
-    import torch
-    import query_ffi as Q
-    from raytracing_c_b200 import driver, gpu_lib
-    from raytracing_c_b200._ffi import gpu_check
-
-    gpu = gpu_lib()
-    gpu_check(gpu.rt_gpu_init(0))
-    loaded = driver.load_scene(os.path.join(ROOT, "assets", "models", "helmet.glb"))
-    driver.register_callbacks(loaded)
-    gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+    args = benchkit.parser(reps=20).parse_args()
+    gpu = benchkit.init()
+    loaded = benchkit.resident("helmet.glb")
     scene = C.byref(loaded.scene)
     stream = torch.cuda.current_stream()
     dev = "cuda"
     g = torch.Generator(device=dev).manual_seed(2026)
-    result = {"card": card(), "model": "helmet.glb", "reps": args.reps, "families": {}}
+    result = {"card": benchkit.card(), "model": "helmet.glb", "reps": args.reps, "families": {}}
 
     def query(rays, t_max, kind, hits=None, surf=None, occ=None, ctr=None):
         n = rays.shape[0]
@@ -83,13 +63,7 @@ def main() -> None:
             ctr = torch.zeros(4, dtype=torch.int64, device=dev)
             gpu_check(query(rays, t_max, kind, hits, surf, occ, ctr))          # warm-up, and the counters of one pass
             torch.cuda.synchronize()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record(stream)
-            for _ in range(args.reps):
-                gpu_check(query(rays, t_max, kind, hits, surf, occ))
-            e1.record(stream)
-            torch.cuda.synchronize()
-            ms = e0.elapsed_time(e1) / args.reps
+            ms = benchkit.per_call_ms(lambda: gpu_check(query(rays, t_max, kind, hits, surf, occ)), stream, args.reps)
             c = ctr.cpu().numpy()
             fam[kind] = {"ms": round(ms, 3), "Mrays_per_s": round(n / (ms * 1e-3) / 1e6, 1),
                          "nodes_per_ray": round(float(c[1]) / n, 3), "leaves_per_ray": round(float(c[2]) / n, 3),
@@ -194,14 +168,7 @@ def main() -> None:
     result["parity_ok"] = all(all(v for k, v in f["parity"].items() if k != "rays") for f in result["families"].values())
     result["occluded_not_slower_at_inf"] = all(f["occluded_vs_closest_time"] <= 1.0 for k, f in result["families"].items()
                                                if k in ("camera", "ao_inf", "interior"))
-    print(json.dumps({"card": result["card"], "parity_ok": result["parity_ok"],
-                      "occluded_not_slower_at_inf": result["occluded_not_slower_at_inf"]}), flush=True)
-    if args.out:
-        with open(args.out, "w") as f:
-            json.dump(result, f, indent=1)
-    loaded.close()
-    if not result["parity_ok"]:
-        sys.exit(1)
+    benchkit.finish(args, result, ("parity_ok", "occluded_not_slower_at_inf"), loaded)
 
 
 if __name__ == "__main__":

@@ -19,48 +19,27 @@ The card name and power limit are read in the same run.
 """
 from __future__ import annotations
 
-import argparse
 import ctypes as C
 import json
-import os
-import subprocess
-import sys
 import time
 
 import numpy as np
+import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
+import benchkit  # first: it puts the repository root and tests/ on sys.path
+from raytracing_c_b200 import driver, host_lib
+from raytracing_c_b200._ffi import Scene, gpu_check
+from refit_ffi import deform
 
 MODELS = {"helmet.glb": None, "tower.obj": dict(eye=(0.0, 12.5, 40.0), target=(0.0, 12.5, 0.0))}
 W, H, SPP, BOUNCES = 480, 270, 4, 8
 
 
-def card() -> dict:
-    out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                         capture_output=True, text=True).stdout.strip().splitlines()
-    name, power, clock = [s.strip() for s in out[0].split(",")]
-    return {"name": name, "power_limit": power, "max_sm_clock": clock}
-
-
-def deform(p, amount, freq):
-    a, f = np.float32(amount), np.float32(freq)
-    return np.stack([p[0] + a * np.sin(f * p[1]), p[1] + a * np.sin(f * p[2]), p[2] + a * np.sin(f * p[0])]).astype(np.float32)
-
-
 def main() -> None:
-    ap = argparse.ArgumentParser()
-    ap.add_argument("--reps", type=int, default=20)
-    ap.add_argument("--out", default=None, help="also write the result JSON here")
-    args = ap.parse_args()
-
-    import torch
-    from raytracing_c_b200 import driver, gpu_lib, host_lib
-    from raytracing_c_b200._ffi import Scene, gpu_check
-
-    gpu, host = gpu_lib(), host_lib()
-    gpu_check(gpu.rt_gpu_init(0))
-    result = {"card": card(), "reps": args.reps, "frame": f"{W}x{H}", "spp": SPP, "max_bounces": BOUNCES, "models": {}}
+    args = benchkit.parser(reps=20).parse_args()
+    gpu, host = benchkit.init(), host_lib()
+    result = {"card": benchkit.card(), "reps": args.reps, "frame": f"{W}x{H}", "spp": SPP, "max_bounces": BOUNCES,
+              "models": {}}
     stream = torch.cuda.current_stream()
 
     def trace_work(loaded):
@@ -69,10 +48,7 @@ def main() -> None:
         return {"nodes_per_ray": round(c["nodes"] / c["rays"], 3), "leaves_per_ray": round(c["leaves"] / c["rays"], 3)}
 
     for name, cam in MODELS.items():
-        loaded = driver.load_scene(os.path.join(ROOT, "assets", "models", name),
-                                   camera=driver.look_at(**cam) if cam else None)
-        driver.register_callbacks(loaded)
-        gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+        loaded = benchkit.resident(name, camera=driver.look_at(**cam) if cam else None)
         n_tri, slots = loaded.n_triangles, loaded.scene.triangles.len
         p0 = driver.scene_positions(loaded)
         src = np.ctypeslib.as_array((C.c_float * (n_tri * 28)).from_address(C.addressof(loaded.model.triangles.data.contents)))
@@ -154,10 +130,7 @@ def main() -> None:
         print(json.dumps({name: r}), flush=True)
         loaded.close()
 
-    print(json.dumps({"card": result["card"]}), flush=True)
-    if args.out:
-        with open(args.out, "w") as f:
-            json.dump(result, f, indent=1)
+    benchkit.finish(args, result, ())
 
 
 if __name__ == "__main__":

@@ -13,28 +13,20 @@ limit are read in the same run.
 """
 from __future__ import annotations
 
-import argparse
 import ctypes as C
 import json
-import os
-import subprocess
-import sys
 
 import numpy as np
+import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
+import benchkit  # first: it puts the repository root and tests/ on sys.path
+from raytracing_c_b200 import driver
+from raytracing_c_b200._ffi import Camera, gpu_check
+from views_ffi import copy_camera
 
 BOUNCES = 8
 WORKLOADS = {"a": dict(views=64, width=256, height=256, spp=16), "b": dict(views=4, width=1920, height=1080, spp=64)}
 QUICK = {"a": dict(views=8, width=64, height=64, spp=4), "b": dict(views=2, width=192, height=108, spp=4)}
-
-
-def card() -> dict:
-    out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                         capture_output=True, text=True).stdout.strip().splitlines()
-    name, power, clock = [s.strip() for s in out[0].split(",")]
-    return {"name": name, "power_limit": power, "max_sm_clock": clock}
 
 
 def orbit_cameras(driver, loaded, n):
@@ -52,39 +44,20 @@ def orbit_cameras(driver, loaded, n):
 
 
 def main() -> None:
-    ap = argparse.ArgumentParser()
-    ap.add_argument("--reps", type=int, default=7)
-    ap.add_argument("--out", default=None, help="also write the result JSON here")
+    ap = benchkit.parser(reps=7)
     ap.add_argument("--quick", action="store_true", help="small workloads (a dry run of the script)")
     args = ap.parse_args()
-
-    import torch
-    from raytracing_c_b200 import driver, gpu_lib
-    from raytracing_c_b200._ffi import Camera, gpu_check
-
-    gpu = gpu_lib()
-    gpu_check(gpu.rt_gpu_init(0))
-    loaded = driver.load_scene(os.path.join(ROOT, "assets", "models", "helmet.glb"))
-    driver.register_callbacks(loaded)
-    gpu_check(gpu.rt_gpu_scene_upload(C.byref(loaded.scene)))
+    gpu = benchkit.init()
+    loaded = benchkit.resident("helmet.glb")
     scene = C.byref(loaded.scene)
     stream = torch.cuda.current_stream()
     st = stream.cuda_stream
-    own_camera = Camera()
-    C.memmove(C.addressof(own_camera), C.addressof(loaded.scene.camera), C.sizeof(Camera))
-    result = {"card": card(), "model": "helmet.glb", "max_bounces": BOUNCES, "reps": args.reps,
+    own_camera = copy_camera(loaded.scene.camera)
+    result = {"card": benchkit.card(), "model": "helmet.glb", "max_bounces": BOUNCES, "reps": args.reps,
               "cameras": "orbit at 1.6 bounding radii, 15 degrees up, 60-degree field of view",
               "timing": "CUDA events around the batched call / the whole loop, host enqueue included; median of reps",
               "workloads": {}}
     all_identical = True
-
-    def timed(fn):
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record(stream)
-        fn()
-        e1.record(stream)
-        torch.cuda.synchronize()
-        return e0.elapsed_time(e1)
 
     for key, wl in (QUICK if args.quick else WORKLOADS).items():
         n, w, h, spp = wl["views"], wl["width"], wl["height"], wl["spp"]
@@ -108,8 +81,8 @@ def main() -> None:
         torch.cuda.synchronize()
         t_views, t_loop, identical = [], [], True
         for _ in range(args.reps):
-            t_views.append(timed(views))
-            t_loop.append(timed(loop))
+            t_views.append(benchkit.window_ms(views, stream))
+            t_loop.append(benchkit.window_ms(loop, stream))
             identical &= bool(torch.equal(batched.view(torch.int32), looped.view(torch.int32)))
         samples = n * w * h * spp
         mv, ml = float(np.median(t_views)), float(np.median(t_loop))
@@ -124,13 +97,7 @@ def main() -> None:
         print(json.dumps({key: r}), flush=True)
 
     result["parity_ok"] = all_identical
-    print(json.dumps({"card": result["card"], "parity_ok": all_identical}), flush=True)
-    if args.out:
-        with open(args.out, "w") as f:
-            json.dump(result, f, indent=1)
-    loaded.close()
-    if not all_identical:
-        sys.exit(1)
+    benchkit.finish(args, result, ("parity_ok",), loaded)
 
 
 if __name__ == "__main__":
